@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference ...                     # the reference algorithm on host cores
+    python bench.py ... --dump-outputs DIR                   # also write what the last timed step computed
 
 One step = one pass of the hot path over one synthetic batch: gated GCN stack
 forward + loss (CE + 0.01 xy + 0.01 kl, train.py:115-118) + backward + Adam step.
@@ -20,6 +21,7 @@ import subprocess
 import sys
 import threading
 import time
+import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -183,6 +185,30 @@ class KernelTimer:
         return agg
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every tensor as ``out_dir/<name>.npy`` in float32, at most DUMP_BYTES in all, so two builds can be compared
+    output for output.  The smallest arrays are written whole; an array larger than its share of what is left keeps
+    the first rows of a permutation seeded by its name, in ascending order, and their indices go to
+    ``<name>.rows.npy`` (float64).  A smaller share keeps a subset of the rows a larger one keeps, so two dumps whose
+    budgets split differently (one array more or less) still line up on the rows they share."""
+    os.makedirs(out_dir, exist_ok=True)
+    items = sorted(((k, v.detach().float().cpu().numpy()) for k, v in arrays.items()), key=lambda kv: kv[1].nbytes)
+    left = DUMP_BYTES - 2 * 256 * len(items)      # room for the .npy headers of each array and its row indices
+    for i, (name, a) in enumerate(items):
+        share = left // (len(items) - i)
+        if a.nbytes > share:
+            perm = np.random.default_rng(zlib.crc32(name.encode())).permutation(a.shape[0])
+            rows = np.sort(perm[:max(1, share // (a.nbytes // a.shape[0] + 8))]).astype(np.float64)
+            np.save(os.path.join(out_dir, name + ".rows.npy"), rows)
+            a = a[rows.astype(np.int64)]
+            left -= rows.nbytes
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        left -= a.nbytes
+
+
 # ---------------------------------------------------------------------------------------------
 def build_model(c, device, torch_head=False):
     import ed_gated_gcn_b200 as E
@@ -268,6 +294,11 @@ def run_b200(args):
     dist_dev = E.tree_distance(graph, anchor)
     tgt = tgt_host.to(dev)
 
+    # what the latest step computed; under a CUDA graph these are the buffers every replay rewrites.  The gradients are
+    # taken here, not from p.grad later: the steps that follow the capture (zero_grad, the e2e graphs) rebind p.grad
+    last = {}
+    named = [("stack." + n, p) for n, p in stack.named_parameters()] + [("dense." + n, p) for n, p in dense.named_parameters()]
+
     def step_resident():
         opt.zero_grad(set_to_none=True)
         x_dev.grad = None
@@ -276,6 +307,11 @@ def run_b200(args):
         loss.backward()
         reducer()
         opt.step()
+        last.clear()
+        last.update(loss=loss.detach(), logits=out.logits.detach(), xy=out.xy.detach(), kl=out.kl.detach(),
+                    scores=out.scores.detach(), pooled=out.pooled.detach())
+        last["x.grad"] = x_dev.grad[:, :c["D"]]
+        last.update({"grad." + n: p.grad for n, p in named if p.grad is not None})
         return loss
 
     # ---- host-resident inputs through the public API (the `e2e` number)
@@ -383,6 +419,8 @@ def run_b200(args):
     if rank == 0:
         sampler.start()
     ms_total = timed(run_resident, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {**last, **{"param." + n: p for n, p in named}})    # params: after this step's Adam
     launches = kernels_per_step * args.steps
     loss_val = float(run_resident().item())
     ms_e2e = timed(run_e2e, args.steps, max(3, args.warmup // 2))
@@ -597,7 +635,15 @@ def main():
     ap.add_argument("--torch-adam", action="store_true", help="torch.optim.Adam(fused, capturable) instead of edg_adam_multi")
     ap.add_argument("--no-graph", action="store_true", help="enqueue kernels from Python instead of replaying a CUDA graph")
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (loss, logits, xy, kl, scores, "
+                         "pooled, the input and parameter gradients, the updated parameters) as DIR/<name>.npy, float32, "
+                         "<= 64 MB in all (larger arrays: a seeded sample of their rows, indices in DIR/<name>.rows.npy)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -15,7 +15,7 @@ reference's own source files are then imported unmodified:
   autograd backward run; the tensors entering and leaving the gated block are
   captured with hooks.
 
-Run:  python oracle/make_golden.py        (writes tests/golden/*.npz)
+Run:  python oracle/make_golden.py        (writes tests/golden/*.npz, see oracle/fixtures.py)
 This script is test infrastructure; it cannot run on the GPU box (no reference
 there) -- which is why its outputs are committed.
 """
@@ -67,8 +67,8 @@ def _install_stubs() -> None:
 
 def golden_gcn_layer(GraphConvolution) -> None:
     from ed_gated_gcn_b200 import synth
-    from oracle import ref_oracle as O
-    out = {}
+    from oracle import fixtures, ref_oracle as O
+    out, drawn = {}, {}
     cases = [(3, 9, 16, 16, True, 0), (2, 50, 300, 300, True, 1), (4, 12, 24, 40, False, 2)]
     for ci, (B, T, Din, Dout, bias, seed) in enumerate(cases):
         g = torch.Generator().manual_seed(100 + seed)
@@ -86,15 +86,17 @@ def golden_gcn_layer(GraphConvolution) -> None:
         out[pre + "T"] = np.int64(T)
         out[pre + "text"] = text.detach().numpy()
         out[pre + "weight"] = layer.weight.detach().numpy()
+        drawn[pre + "weight"] = (100 + seed, 0)                     # the first draws of g, bias next (reference_init_)
         if bias:
             out[pre + "bias"] = layer.bias.detach().numpy()
             out[pre + "dbias"] = layer.bias.grad.numpy()
+            drawn[pre + "bias"] = (100 + seed, Din * Dout)
         out[pre + "probe"] = probe.numpy()
         out[pre + "y"] = y.detach().numpy()
         out[pre + "dtext"] = text.grad.numpy()
         out[pre + "dweight"] = layer.weight.grad.numpy()
     out["n_cases"] = np.int64(len(cases))
-    np.savez_compressed(os.path.join(GOLD, "gcn_layer.npz"), **out)
+    fixtures.save(os.path.join(GOLD, "gcn_layer.npz"), out, drawn=drawn)
     print("gcn_layer.npz", len(out))
 
 
@@ -155,7 +157,7 @@ def golden_block55(BertAmir55, fname: str = "block55.npz", seed: int = 55) -> No
     front of the Linear, bert_amir5.py:464-465) and in the ``dense`` head (two Linears over cat[aspect, out,
     pooled_output], :443-446, :536)."""
     from ed_gated_gcn_b200 import synth
-    from oracle import ref_oracle as O
+    from oracle import fixtures, ref_oracle as O
     torch.manual_seed(seed)
     B, ORI_ML, BERT_ML, C = 6, 20, 24, 5
     batch = synth.make_batch(B, 4, 14, seed=55)
@@ -237,16 +239,19 @@ def golden_block55(BertAmir55, fname: str = "block55.npz", seed: int = 55) -> No
         "scores": scores.detach().numpy(), "loss": loss.detach().numpy(),
     }
     keep = ("gc1.", "gc2.", "gate1.", "gate2.", "fc.", "dense.")
+    drawn, offset = {}, 0
     for n, p in model.named_parameters():
         if n.startswith(keep):
             out["p_" + n] = p.detach().numpy()
+            drawn["p_" + n] = (555, offset)                            # its place in the stream of g above
             if p.numel() < 500_000:                                    # BertAmir54's dense.0.weight is 768 x 1280: keep the
                 out["g_" + n] = p.grad.numpy()                         # fixture small, its bias gradient pins that layer
+        offset += p.numel()
     if fname != "block55.npz":
         out.pop("anchor_rep")
     else:
         out.pop("dense_in")                                            # block55.npz keeps its committed layout
-    np.savez_compressed(os.path.join(GOLD, fname), **out)
+    fixtures.save(os.path.join(GOLD, fname), out, drawn=drawn, sampled=[k for k in out if k.startswith("g_")])
     print(fname, {k: v.shape for k, v in out.items() if k[:2] not in ("p_", "g_")})
 
 

@@ -9,7 +9,7 @@ import torch
 
 from conftest import GOLDEN
 from gpu_util import DEV, rel, tol_for, dense_inputs, pack_rows
-from oracle import ref_oracle as O
+from oracle import fixtures, ref_oracle as O
 
 pytestmark = pytest.mark.gpu
 DTYPES = [torch.float32, torch.bfloat16]
@@ -20,7 +20,7 @@ DTYPES = [torch.float32, torch.bfloat16]
 def test_graph_convolution_matches_reference_outputs(dtype):
     """models/gcn.py run by the reference itself (golden) vs the drop-in module, dense interface."""
     import ed_gated_gcn_b200 as E
-    z = np.load(os.path.join(GOLDEN, "gcn_layer.npz"))
+    z = fixtures.load(os.path.join(GOLDEN, "gcn_layer.npz"))
     tol = tol_for(dtype)
     for ci in range(int(z["n_cases"])):
         p = f"c{ci}_"
@@ -120,7 +120,7 @@ def _load_stack_from_golden(z, dtype):
     C, D2 = z["p_fc.0.weight"].shape
     D = D2 // 2
     stack = E.GatedGCNStack(D, n_layers=2, n_classes=C, gate_arch="sig-2", compute_dtype=dtype).to(DEV)
-    sd = {k[2:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("p_") and not k.startswith("p_dense.")}
+    sd = {k[2:]: torch.from_numpy(z[k]) for k in z if k.startswith("p_") and not k.startswith("p_dense.")}
     stack.load_state_dict(sd)                                        # same keys as BertAmir55 (bert_amir5.py:559-572)
     dense = torch.nn.Linear(z["p_dense.weight"].shape[1], C).to(DEV)
     with torch.no_grad():
@@ -222,7 +222,7 @@ def test_stack_matches_full_reference_forward_backward(dtype):
     """BertAmir55.forward + backward as run by the reference (golden block55), dense-compat layout:
     every sentence has T rows, pad rows are live self-loop singletons (SURVEY fact 6)."""
     import ed_gated_gcn_b200 as E
-    z = np.load(os.path.join(GOLDEN, "block55.npz"))
+    z = fixtures.load(os.path.join(GOLDEN, "block55.npz"))
     tol = tol_for(dtype)
     stack, dense = _load_stack_from_golden(z, dtype)
     x = torch.from_numpy(z["x"]).to(DEV).requires_grad_(True)          # LSTM output [B,T,D]
@@ -248,12 +248,12 @@ def test_stack_matches_full_reference_forward_backward(dtype):
         # backward against the reference's own numbers
         assert rel(x.grad, z["dx"]) < tol
         got = dict(stack.named_parameters())
-        for k in z.files:
+        for k in z:
             if k.startswith("g_") and k != "g_fc.0.bias":
                 name = k[2:]
                 g = dense.weight.grad if name == "dense.weight" else dense.bias.grad if name == "dense.bias" \
                     else got[name].grad
-                assert rel(g, z[k]) < tol, name
+                assert rel(fixtures.pick(z, k, g), z[k]) < tol, name
         return
     # bf16: gradients against the oracle (pinned to the same fixture) with the CUDA path's routing
     sents = [(torch.from_numpy(z["x"][b]), torch.from_numpy(z["adj"][b]), int(z["anchor"][b]),
@@ -318,15 +318,15 @@ def test_bert_amir54_variant_matches_full_reference_forward_backward(dtype):
     """BertAmir54.forward + backward as run by the reference (golden block54): fc = Sequential(Sigmoid, Linear)
     (bert_amir5.py:464-465), dense = two Linears over cat[aspect, out, pooled_output] (:443-446, :536)."""
     import ed_gated_gcn_b200 as E
-    z = np.load(os.path.join(GOLDEN, "block54.npz"))
+    z = fixtures.load(os.path.join(GOLDEN, "block54.npz"))
     tol = tol_for(dtype)
     C, D2 = z["p_fc.1.weight"].shape
     D = D2 // 2
     stack = E.GatedGCNStack(D, n_layers=2, n_classes=C, gate_arch="sig-2", compute_dtype=dtype, fc_sigmoid=True).to(DEV)
-    sd = {k[2:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("p_") and not k.startswith("p_dense.")}
+    sd = {k[2:]: torch.from_numpy(z[k]) for k in z if k.startswith("p_") and not k.startswith("p_dense.")}
     stack.load_state_dict(sd)                                         # keys of BertAmir54 incl. fc.1.*
     dense = torch.nn.Sequential(torch.nn.Linear(2 * D + 768, 768), torch.nn.Linear(768, C)).to(DEV)
-    dense.load_state_dict({k[len("p_dense."):]: torch.from_numpy(z[k]) for k in z.files if k.startswith("p_dense.")})
+    dense.load_state_dict({k[len("p_dense."):]: torch.from_numpy(z[k]) for k in z if k.startswith("p_dense.")})
     x = torch.from_numpy(z["x"]).to(DEV).requires_grad_(True)
     adj = torch.from_numpy(z["adj"]).to(DEV)
     anchor = torch.from_numpy(z["anchor"]).to(DEV)
@@ -345,9 +345,9 @@ def test_bert_amir54_variant_matches_full_reference_forward_backward(dtype):
         assert rel(x.grad, z["dx"]) < tol
         got = dict(stack.named_parameters())
         got.update({"dense." + n: p for n, p in dense.named_parameters()})
-        for k in z.files:
+        for k in z:
             if k.startswith("g_") and k not in ("g_fc.1.bias", "g_fc.1.weight"):
-                assert rel(got[k[2:]].grad, z[k]) < tol, k
+                assert rel(fixtures.pick(z, k, got[k[2:]].grad), z[k]) < tol, k
         # fc.1.weight: d kl / d fc.weight = sum_b sum_t ds_bt logits_b (x) sigmoid(cat[x_out_t, a_b]) with sum_t ds_bt = 0
         # (a softmax derivative): a 2.9e-6 remainder of summands that add up to 4.9e-4 in absolute value.  The
         # reference's OWN fp32 value is 1.6e-5 away from an fp64 evaluation of the same lines, i.e. outside the 1e-5
@@ -405,7 +405,7 @@ def test_bert_amir_variant_matches_full_reference_forward_backward(dtype):
 def _fp64_fc_weight_grad_block54(z):
     """fp64 evaluation of the reference block on the block54 fixture (oracle restatement of bert_amir5.py:515-540 with
     fc = Sequential(Sigmoid, Linear)): d loss / d fc.1.weight and max_cj sum_bt |ds_bt logits_bc sigmoid(cat)_j|."""
-    P = {k[2:]: torch.from_numpy(z[k]).double().requires_grad_(True) for k in z.files if k.startswith("p_")}
+    P = {k[2:]: torch.from_numpy(z[k]).double().requires_grad_(True) for k in z if k.startswith("p_")}
     D = z["x"].shape[2]
     x, adj = torch.from_numpy(z["x"]).double(), torch.from_numpy(z["adj"]).double()
     po = torch.from_numpy(z["dense_in"][:, 2 * D:]).double()
