@@ -120,8 +120,11 @@ def graph_from_dense(adj: torch.Tensor, check: bool = True) -> DepGraph:
     with torch.cuda.device(dev):
         L.call("edg_csr_from_dense_count", L.ptr(adj), is64, B, T, adj.stride(0), adj.stride(1), adj.stride(2),
                L.ptr(row_ptr), L.ptr(flags), L.stream())
-        host = torch.cat([row_ptr[rows:rows + 1], flags]).cpu()     # one small device->host read
-        nnz, odd, asym = (int(v) for v in host)
+        # the largest CSR entry count of one sentence: any symmetric pattern is accepted, so the tree bound 3T - 2 that
+        # DepGraph.tile_plan assumes otherwise does not hold (a dense sentence can overflow the fused kernels' tiles)
+        sent_nnz = (row_ptr[T::T] - row_ptr[:rows:T]).max().view(1)
+        host = torch.cat([row_ptr[rows:rows + 1], flags, sent_nnz]).cpu()     # one small device->host read
+        nnz, odd, asym, max_sent_nnz = (int(v) for v in host)
         if check and (odd or asym):
             raise L.EdgError(
                 f"dense adjacency is not a 0/1 symmetric pattern ({odd} non-binary, {asym} asymmetric entries); "
@@ -131,7 +134,7 @@ def graph_from_dense(adj: torch.Tensor, check: bool = True) -> DepGraph:
                L.ptr(row_ptr), L.ptr(col), L.stream())
     sent_ptr = torch.arange(0, rows + 1, T, dtype=torch.int32, device=dev)
     row_sent = torch.arange(B, dtype=torch.int32, device=dev).repeat_interleave(T)
-    return DepGraph(sent_ptr, row_ptr, col, row_sent, B, rows, T, padded_T=T)
+    return DepGraph(sent_ptr, row_ptr, col, row_sent, B, rows, T, padded_T=T, max_sent_nnz=max_sent_nnz)
 
 
 def tree_distance(graph: DepGraph, anchor_index: torch.Tensor, pad: Optional[str] = None,

@@ -149,7 +149,7 @@ int edg_fused_tile_rows(int32_t K, int32_t Nout);
  * arguments of the mode-1 call that produces d h_1.  g_xy: device scalar (NULL = 0). */
 int edg_views_bwd_hmax(const float* hmax, const float* gates, const float* g_xy, int32_t V, int32_t B, int32_t D,
                        float* patch_val, int64_t ldp, float* dgates, int acc_view, edg_stream stream);
-/* Greedy packing of whole sentences into tiles of <= max_rows rows (<= 8 sentences, <= 512 CSR entries):
+/* Greedy packing of whole sentences into tiles of <= max_rows rows (<= 6 sentences, <= 512 CSR entries):
  * tile_info int32 [B+1][8] = {s0, s1, r0, r1, e0, e1, 0, 0} (sentence, row and CSR-entry ranges), n_tiles = device
  * scalar.  One small kernel, no host synchronisation. */
 int edg_tile_plan(const int32_t* sent_ptr, const int32_t* row_ptr, int32_t B, int32_t max_rows,

@@ -37,25 +37,33 @@ def _dense_ops(batch):
     return out
 
 
-def test_tile_plan_covers_every_sentence_once():
+def check_tile_plan(sp, g, rows, plan):
+    """The tiles of edg_tile_plan cover every sentence once, in order, greedily, within the row, sentence and CSR-entry
+    caps of the fused kernels; returns the plan's tile_info rows on the host."""
     from ed_gated_gcn_b200 import ops
-    batch, g, _, _, _, rows, plan = _setup(700, 1, 50, 3, 64, 64)
     info, n_tiles = plan
     nt = int(n_tiles.item())
     info = info[:nt].cpu().numpy()
-    sp = batch.sent_ptr
     rp = g.row_ptr.cpu().numpy()
-    assert info[0, 0] == 0 and info[-1, 1] == batch.n_graphs
+    assert info[0, 0] == 0 and info[-1, 1] == len(sp) - 1
     assert np.array_equal(info[1:, 0], info[:-1, 1])
     assert np.array_equal(info[:, 2], sp[info[:, 0]]) and np.array_equal(info[:, 3], sp[info[:, 1]])
     assert np.array_equal(info[:, 4], rp[info[:, 2]]) and np.array_equal(info[:, 5], rp[info[:, 3]])
     assert ((info[:, 3] - info[:, 2]) <= rows).all() and ((info[:, 1] - info[:, 0]) <= ops.FUSED_MAX_SENTENCES).all()
+    assert ((info[:, 5] - info[:, 4]) <= 512).all()
     assert ((info[:, 1] - info[:, 0]) >= 1).all()
-    # greedy: the next sentence would not have fitted (rows) unless the sentence cap stopped the tile
+    # greedy: the next sentence would not have fitted (rows or CSR entries) unless the sentence cap stopped the tile
     for t in range(nt - 1):
         s1 = info[t, 1]
-        full = (sp[s1 + 1] - info[t, 2] > rows) or (info[t, 1] - info[t, 0] == ops.FUSED_MAX_SENTENCES)
-        assert full
+        full = (sp[s1 + 1] - info[t, 2] > rows) or (rp[sp[s1 + 1]] - info[t, 4] > 512) \
+            or (info[t, 1] - info[t, 0] == ops.FUSED_MAX_SENTENCES)
+        assert full, t
+    return info
+
+
+def test_tile_plan_covers_every_sentence_once():
+    batch, g, _, _, _, rows, plan = _setup(700, 1, 50, 3, 64, 64)
+    check_tile_plan(batch.sent_ptr, g, rows, plan)
 
 
 @pytest.mark.parametrize("shape", [(300, 300), (64, 64), (256, 256), (300, 160), (128, 320), (48, 16)])
