@@ -29,6 +29,8 @@ SIGNATURES = {
     "edg_strerror": (c_char_p, [c_int]),
     "edg_last_cuda_error": (c_char_p, []),
     "edg_csr_from_heads": (c_int, [_P, _P, _I, _I, _I, _P, _P, _P, _P, _P]),
+    "edg_csr_from_heads_edges_workspace": (_Z, [_I, _I, _I]),
+    "edg_csr_from_heads_edges": (c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _P, _Z, _P]),
     "edg_csr_from_dense_count": (c_int, [_P, c_int, _I, _I, _L, _L, _L, _P, _P, _P]),
     "edg_csr_from_dense_fill": (c_int, [_P, c_int, _I, _I, _L, _L, _L, _P, _P, _P]),
     "edg_tree_dist": (c_int, [_P, _P, _P, _P, _I, _I, _P, _P]),
@@ -141,6 +143,8 @@ def _kernels_of(name: str, args) -> int:
         return 2 + (2 if args[11] else 0)
     if name == "edg_csr_from_heads":
         return 3
+    if name == "edg_csr_from_heads_edges":
+        return 0 if args[4] == 0 else (3 if (args[5] == 0 or args[6] == 0) else 7)
     if name == "edg_wgrad_split":
         return 4
     if name == "edg_dense_head_bwd":

@@ -16,19 +16,116 @@ __device__ __forceinline__ int clean_head(const int32_t* __restrict__ hs, int i,
   return (hs[h] == i && i > h) ? -1 : h;
 }
 
+// ---- extra undirected edges (heads + edges -> CSR) ---------------------------
+// Pair e of the edge list belongs to the sentence b with edge_ptr[b] <= e < edge_ptr[b+1] (empty sentences allowed).
+__device__ __forceinline__ int pair_sentence(const int32_t* __restrict__ edge_ptr, int B, int e) {
+  int lo = 0, hi = B - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (edge_ptr[mid] <= e) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
+// Pair e as sentence-local (i, j) of the sentence starting at global row `base`.  False for a pair that adds nothing to
+// the forest's pattern: an endpoint outside [0, n), i == j, or the edge of a (cleaned) head in either direction.  The
+// pair count and scatter passes both decide with this one function, so they agree; duplicates are removed per row by
+// extra_sort_kernel.
+__device__ __forceinline__ bool extra_pair(const int32_t* __restrict__ heads, const int32_t* __restrict__ sent_ptr,
+                                           const int32_t* __restrict__ edges, const int32_t* __restrict__ edge_ptr,
+                                           int B, int e, int& base, int& i, int& j) {
+  const int b = pair_sentence(edge_ptr, B, e);
+  base = sent_ptr[b];
+  const int n = sent_ptr[b + 1] - base;
+  i = edges[2 * (int64_t)e];
+  j = edges[2 * (int64_t)e + 1];
+  if (i < 0 || i >= n || j < 0 || j >= n || i == j) return false;
+  return clean_head(heads + base, i, n) != j && clean_head(heads + base, j, n) != i;
+}
+
+// per-row count of extra entries (both directions of every kept pair); cnt[N] zeroed by the caller
+__global__ void pairs_count_kernel(const int32_t* __restrict__ heads, const int32_t* __restrict__ sent_ptr,
+                                   const int32_t* __restrict__ edges, const int32_t* __restrict__ edge_ptr, int B, int E,
+                                   int32_t* __restrict__ cnt) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  int base, i, j;
+  if (e >= E || !extra_pair(heads, sent_ptr, edges, edge_ptr, B, e, base, i, j)) return;
+  atomicAdd(&cnt[base + i], 1);
+  atomicAdd(&cnt[base + j], 1);
+}
+
+// row r's extra neighbours (sentence-local, unordered, maybe repeated) into xl[xoff[r] ..); cur[N] zeroed by the caller
+__global__ void pairs_scatter_kernel(const int32_t* __restrict__ heads, const int32_t* __restrict__ sent_ptr,
+                                     const int32_t* __restrict__ edges, const int32_t* __restrict__ edge_ptr, int B,
+                                     int E, const int32_t* __restrict__ xoff, int32_t* __restrict__ cur,
+                                     int32_t* __restrict__ xl) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  int base, i, j;
+  if (e >= E || !extra_pair(heads, sent_ptr, edges, edge_ptr, B, e, base, i, j)) return;
+  xl[xoff[base + i] + atomicAdd(&cur[base + i], 1)] = j;
+  xl[xoff[base + j] + atomicAdd(&cur[base + j], 1)] = i;
+}
+
+// One warp per row: sort and de-duplicate the row's extra list in place through a bitmap of the sentence's tokens
+// (`words` 32-bit words per warp in shared memory), so the result is a set in ascending order whatever the order of the
+// pairs or of the scatter's atomics.  xu[r]: on entry the list length, on return the number of distinct entries.
+__global__ void extra_sort_kernel(const int32_t* __restrict__ xoff, int32_t* __restrict__ xl, int32_t* __restrict__ xu,
+                                  int N, int words) {
+  extern __shared__ uint32_t bm_all[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int r = blockIdx.x * (blockDim.x >> 5) + warp;
+  if (r >= N) return;                      // warp-uniform
+  const int beg = xoff[r], k = xoff[r + 1] - beg;
+  if (k <= 1) return;                      // xu[r] = k already
+  uint32_t* bm = bm_all + warp * words;
+  for (int q = lane; q < words; q += 32) bm[q] = 0u;
+  __syncwarp();
+  for (int e = lane; e < k; e += 32) {
+    const int c = xl[beg + e];
+    if (c >= 32 * words) __trap();         // a sentence longer than the caller's max_len (see heads_fill_kernel)
+    atomicOr(&bm[c >> 5], 1u << (c & 31));
+  }
+  __syncwarp();
+  int w = beg;
+  for (int q0 = 0; q0 < words; q0 += 32) {
+    const int q = q0 + lane;
+    uint32_t m = q < words ? bm[q] : 0u;
+    const int c = __popc(m);
+    int incl = c;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int t = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= o) incl += t;
+    }
+    for (int p = w + incl - c; m; m &= m - 1u) xl[p++] = 32 * q + __ffs(m) - 1;
+    w += __shfl_sync(0xffffffffu, incl, 31);
+  }
+  if (lane == 0) xu[r] = w - beg;
+}
+
 // ---- heads -> CSR ----------------------------------------------------------
-// pass 1: non-zeros of each sentence = n + 2 * (tokens that have a head)
+// pass 1: non-zeros of each sentence = n + 2 * (tokens that have a head) [+ the rows' distinct extra entries xu].
+// With extras, a sentence over a positive caller bound *nnz_cap fails loudly, and mx[0] collects the largest count.
+template <bool kExtra>
 __global__ void heads_count_kernel(const int32_t* __restrict__ heads, const int32_t* __restrict__ sent_ptr,
-                                   int B, int32_t* __restrict__ sent_nnz) {
+                                   int B, int32_t* __restrict__ sent_nnz, const int32_t* __restrict__ xu = nullptr,
+                                   const int32_t* __restrict__ nnz_cap = nullptr, int32_t* __restrict__ mx = nullptr) {
   int b = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (b >= B) return;
   int lane = threadIdx.x & 31;
   int base = sent_ptr[b], n = sent_ptr[b + 1] - base;
   int cnt = 0;
-  for (int i = lane; i < n; i += 32) cnt += 1 + 2 * (clean_head(heads + base, i, n) >= 0);
+  for (int i = lane; i < n; i += 32) cnt += 1 + 2 * (clean_head(heads + base, i, n) >= 0) + (kExtra ? xu[base + i] : 0);
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
-  if (lane == 0) sent_nnz[b] = cnt;
+  if (lane == 0) {
+    sent_nnz[b] = cnt;
+    if (kExtra) {
+      const int cap = *nnz_cap;
+      if (cap > 0 && cnt > cap) __trap();   // the caller's max_sent_nnz is smaller than this sentence: fail loudly
+      atomicMax(mx, cnt);
+    }
+  }
 }
 
 // single-block exclusive scan: out[0..n] (n+1 entries), out[n] = total
@@ -71,13 +168,20 @@ __global__ void scan_exclusive_kernel(const int32_t* in, int32_t* out, int n) { 
 
 // pass 2: one block per sentence; thread i builds row i by scanning the sentence
 // in ascending token order, which yields the ascending column order directly.
+// With extras, row r's distinct extra neighbours xl[xoff[r] .. + xu[r]) are ascending and disjoint from self, parent
+// and children (extra_pair, extra_sort_kernel), so the same scan merges them in; block 0 publishes mx[0].
+template <bool kExtra>
 __global__ void heads_fill_kernel(const int32_t* __restrict__ heads, const int32_t* __restrict__ sent_ptr,
                                   const int32_t* __restrict__ sent_off, int32_t* __restrict__ row_ptr,
-                                  int32_t* __restrict__ col, int32_t* __restrict__ row_sent, int B, int N, int cap) {
+                                  int32_t* __restrict__ col, int32_t* __restrict__ row_sent, int B, int N, int cap,
+                                  const int32_t* __restrict__ xoff = nullptr, const int32_t* __restrict__ xl = nullptr,
+                                  const int32_t* __restrict__ xu = nullptr, const int32_t* __restrict__ mx = nullptr,
+                                  int32_t* __restrict__ sent_max_nnz = nullptr) {
   extern __shared__ int32_t sm[];
   const int b = blockIdx.x;
   const int base = sent_ptr[b], n = sent_ptr[b + 1] - base;
   if (n > cap) __trap();      // the caller's max_len (it sizes the shared arrays) is smaller than this sentence: fail loudly
+  if (kExtra && b == 0 && threadIdx.x == 0) *sent_max_nnz = *mx;
   int32_t* h = sm;            // cleaned heads [n]
   int32_t* deg = sm + n;      // row lengths -> exclusive offsets [n+1]
   for (int i = threadIdx.x; i < n; i += blockDim.x) {
@@ -86,7 +190,7 @@ __global__ void heads_fill_kernel(const int32_t* __restrict__ heads, const int32
   }
   __syncthreads();
   for (int i = threadIdx.x; i < n; i += blockDim.x) {
-    atomicAdd(&deg[i], 1 + (h[i] >= 0));
+    atomicAdd(&deg[i], 1 + (h[i] >= 0) + (kExtra ? xu[base + i] : 0));
     if (h[i] >= 0) atomicAdd(&deg[h[i]], 1);
   }
   __syncthreads();
@@ -112,8 +216,18 @@ __global__ void heads_fill_kernel(const int32_t* __restrict__ heads, const int32
     row_ptr[base + i] = w;
     row_sent[base + i] = b;
     const int hi = h[i];
-    for (int k = 0; k < n; ++k)
-      if (k == i || k == hi || h[k] == i) col[w++] = base + k;
+    if (kExtra) {
+      int xp = xoff[base + i];
+      const int xe = xp + xu[base + i];
+      for (int k = 0; k < n; ++k) {
+        bool nz = k == i || k == hi || h[k] == i;
+        if (!nz && xp < xe && xl[xp] == k) { nz = true; ++xp; }
+        if (nz) col[w++] = base + k;
+      }
+    } else {
+      for (int k = 0; k < n; ++k)
+        if (k == i || k == hi || h[k] == i) col[w++] = base + k;
+    }
   }
   if (b == B - 1 && threadIdx.x == 0) row_ptr[N] = off0 + deg[n];
 }
@@ -230,11 +344,58 @@ extern "C" int edg_csr_from_heads(const int32_t* heads, const int32_t* sent_ptr,
   cudaStream_t s = (cudaStream_t)stream;
   if (B == 0) { cudaMemsetAsync(row_ptr, 0, sizeof(int32_t), s); return check_launch(); }
   int32_t* sent_nnz = ws;   // B ints, scanned in place into B+1 offsets
-  heads_count_kernel<<<(B + 7) / 8, 256, 0, s>>>(heads, sent_ptr, B, sent_nnz);
+  heads_count_kernel<false><<<(B + 7) / 8, 256, 0, s>>>(heads, sent_ptr, B, sent_nnz);
   scan_exclusive_kernel<<<1, 1024, 0, s>>>(sent_nnz, sent_nnz, B);
   int threads = max_len <= 64 ? 64 : (max_len <= 128 ? 128 : 256);
   size_t smem = (2 * (size_t)max_len + 1) * sizeof(int32_t);
-  heads_fill_kernel<<<B, threads, smem, s>>>(heads, sent_ptr, sent_nnz, row_ptr, col, row_sent, B, N, max_len);
+  heads_fill_kernel<false><<<B, threads, smem, s>>>(heads, sent_ptr, sent_nnz, row_ptr, col, row_sent, B, N, max_len);
+  return check_launch();
+}
+
+// workspace of edg_csr_from_heads_edges, in int32: sentence counts -> offsets [B+1] | extra entries per row -> offsets
+// [N+1] | distinct extra entries per row [N] | largest sentence count [1] | extra lists [2E]
+static size_t heads_edges_ws_ints(int64_t B, int64_t N, int64_t E) { return (B + 1) + (N + 1) + N + 1 + 2 * E; }
+
+extern "C" size_t edg_csr_from_heads_edges_workspace(int32_t B, int32_t N, int32_t E) {
+  if (B < 0 || N < 0 || E < 0) return 0;
+  return heads_edges_ws_ints(B, N, E) * sizeof(int32_t);
+}
+
+extern "C" int edg_csr_from_heads_edges(const int32_t* heads, const int32_t* sent_ptr, const int32_t* edges,
+                                        const int32_t* edge_ptr, int32_t B, int32_t N, int32_t E, int32_t max_len,
+                                        int32_t* row_ptr, int32_t* col, int32_t* row_sent, int32_t* sent_max_nnz,
+                                        void* ws, size_t ws_bytes, edg_stream stream) {
+  if (B < 0 || N < 0 || E < 0 || max_len < 0) return EDG_ERR_ARG;
+  if (!sent_ptr || !row_ptr || !sent_max_nnz || !ws) return EDG_ERR_ARG;
+  if (N > 0 && (!heads || !col || !row_sent)) return EDG_ERR_ARG;
+  if (E > 0 && (!edges || !edge_ptr)) return EDG_ERR_ARG;
+  if (max_len > kMaxSentence) return EDG_ERR_UNSUPPORTED;
+  if (ws_bytes < edg_csr_from_heads_edges_workspace(B, N, E)) return EDG_ERR_WORKSPACE;
+  cudaStream_t s = (cudaStream_t)stream;
+  if (B == 0) {
+    cudaMemsetAsync(row_ptr, 0, sizeof(int32_t), s);
+    cudaMemsetAsync(sent_max_nnz, 0, sizeof(int32_t), s);
+    return check_launch();
+  }
+  int32_t* sent_nnz = (int32_t*)ws;
+  int32_t* xoff = sent_nnz + (B + 1);
+  int32_t* xu = xoff + (N + 1);
+  int32_t* mx = xu + N;
+  int32_t* xl = mx + 1;
+  cudaMemsetAsync(xoff, 0, (2 * (size_t)N + 2) * sizeof(int32_t), s);     // xoff, xu, mx
+  if (E > 0 && N > 0) {
+    const int words = max(1, (max_len + 31) / 32);
+    pairs_count_kernel<<<(E + 255) / 256, 256, 0, s>>>(heads, sent_ptr, edges, edge_ptr, B, E, xoff);
+    scan_exclusive_kernel<<<1, 1024, 0, s>>>(xoff, xoff, N);
+    pairs_scatter_kernel<<<(E + 255) / 256, 256, 0, s>>>(heads, sent_ptr, edges, edge_ptr, B, E, xoff, xu, xl);
+    extra_sort_kernel<<<(N + 7) / 8, 256, 8 * words * sizeof(uint32_t), s>>>(xoff, xl, xu, N, words);
+  }
+  heads_count_kernel<true><<<(B + 7) / 8, 256, 0, s>>>(heads, sent_ptr, B, sent_nnz, xu, sent_max_nnz, mx);
+  scan_exclusive_kernel<<<1, 1024, 0, s>>>(sent_nnz, sent_nnz, B);
+  int threads = max_len <= 64 ? 64 : (max_len <= 128 ? 128 : 256);
+  size_t smem = (2 * (size_t)max_len + 1) * sizeof(int32_t);
+  heads_fill_kernel<true><<<B, threads, smem, s>>>(heads, sent_ptr, sent_nnz, row_ptr, col, row_sent, B, N, max_len,
+                                                   xoff, xl, xu, mx, sent_max_nnz);
   return check_launch();
 }
 

@@ -73,14 +73,29 @@ def _i32(t: torch.Tensor, device) -> torch.Tensor:
 
 
 def build_graph(heads: torch.Tensor, sent_ptr: torch.Tensor, max_len: Optional[int] = None,
-                device: Optional[torch.device] = None) -> DepGraph:
+                device: Optional[torch.device] = None, extra_edges: Optional[torch.Tensor] = None,
+                edge_ptr: Optional[torch.Tensor] = None, max_sent_nnz: Optional[int] = None) -> DepGraph:
     """heads int [N] (sentence-local head index, -1 = root), sent_ptr int [B+1].
 
     The packed counterpart of ``gen_graph`` (graph.py:62-75).  ``max_len`` (longest
-    sentence) may be passed to avoid one device->host read."""
+    sentence) may be passed to avoid one device->host read.
+
+    Graphs that are not forests (enhanced dependencies, graph.py:63-64) come as the forest of ``heads`` plus
+    ``extra_edges`` int [E, 2] of sentence-local undirected pairs, sentence b owning pairs ``edge_ptr[b]`` ..
+    ``edge_ptr[b+1] - 1`` (``wire.split_adjacency`` / ``collate_packed`` produce both).  Pairs follow set semantics:
+    duplicates, reversed pairs, pairs that repeat a head edge and self pairs change nothing; pairs with an endpoint
+    outside the sentence are dropped.  The graph then carries ``max_sent_nnz``, the largest CSR entry count of one
+    sentence (it decides whether the fused layer kernels can take the batch).  ``max_sent_nnz`` may be passed as an
+    upper bound the caller guarantees, like ``max_len`` (``PackedBatch.max_sent_nnz`` is exact); the kernels trap on a
+    sentence above it.  With both ``max_len`` and ``max_sent_nnz`` given the build makes no device->host read and can
+    be captured in a CUDA graph.  Otherwise a missing ``max_sent_nnz`` is read back after the build (one 4-byte copy),
+    and a missing ``max_len`` is computed from ``sent_ptr`` before it (a read only when ``sent_ptr`` is on the GPU).
+    Without ``extra_edges``, ``edge_ptr`` and ``max_sent_nnz`` are ignored."""
     device = torch.device(device) if device is not None else heads.device
     if device.type != "cuda":
         raise L.EdgError("build_graph needs a CUDA device (there is no CPU path)")
+    if extra_edges is not None:
+        return _build_graph_edges(heads, sent_ptr, max_len, device, extra_edges, edge_ptr, max_sent_nnz)
     heads = _i32(heads, device)
     sent_ptr = _i32(sent_ptr, device)
     B = sent_ptr.numel() - 1
@@ -95,6 +110,39 @@ def build_graph(heads: torch.Tensor, sent_ptr: torch.Tensor, max_len: Optional[i
         L.call("edg_csr_from_heads", L.ptr(heads), L.ptr(sent_ptr), B, N, max_len, L.ptr(row_ptr), L.ptr(col),
                L.ptr(row_sent), L.ptr(ws), L.stream())
     return DepGraph(sent_ptr, row_ptr, col, row_sent[:N], B, N, max_len)
+
+
+def _build_graph_edges(heads, sent_ptr, max_len, device, extra_edges, edge_ptr, max_sent_nnz) -> DepGraph:
+    if edge_ptr is None:
+        raise L.EdgError("extra_edges needs edge_ptr (int [B+1]: the pairs of sentence b are edge_ptr[b] .. [b+1] - 1)")
+    if extra_edges.dim() != 2 or extra_edges.shape[1] != 2:
+        raise L.EdgError(f"extra_edges must be [E, 2], got {tuple(extra_edges.shape)}")
+    if edge_ptr.numel() != sent_ptr.numel():
+        raise L.EdgError(f"edge_ptr has {edge_ptr.numel()} entries, sent_ptr {sent_ptr.numel()}")
+    if max_len is None and not sent_ptr.is_cuda:
+        sp = sent_ptr.to(torch.int64)
+        max_len = int((sp[1:] - sp[:-1]).max()) if sp.numel() > 1 else 0
+    heads = _i32(heads, device)
+    sent_ptr = _i32(sent_ptr, device)
+    edges = _i32(extra_edges, device)
+    edge_ptr = _i32(edge_ptr, device)
+    B, N, E = sent_ptr.numel() - 1, heads.numel(), edges.shape[0]
+    if max_len is None:
+        max_len = int((sent_ptr[1:] - sent_ptr[:-1]).max().item()) if B > 0 else 0
+    row_ptr = torch.empty(N + 1, dtype=torch.int32, device=device)
+    col = torch.empty(max(3 * N + 2 * E, 1), dtype=torch.int32, device=device)
+    row_sent = torch.empty(max(N, 1), dtype=torch.int32, device=device)
+    # in: the caller's bound (0 = none), out: the largest sentence
+    smn = torch.full((1,), int(max_sent_nnz or 0), dtype=torch.int32, device=device)
+    with torch.cuda.device(device):
+        nbytes = L.load().edg_csr_from_heads_edges_workspace(B, N, E)
+        ws = torch.empty(max(nbytes, 4), dtype=torch.uint8, device=device)
+        L.call("edg_csr_from_heads_edges", L.ptr(heads), L.ptr(sent_ptr), L.ptr(edges) if E else None, L.ptr(edge_ptr),
+               B, N, E, max_len, L.ptr(row_ptr), L.ptr(col), L.ptr(row_sent), L.ptr(smn), L.ptr(ws), ws.numel(),
+               L.stream())
+        if max_sent_nnz is None:
+            max_sent_nnz = int(smn.item())          # one small device->host read
+    return DepGraph(sent_ptr, row_ptr, col, row_sent[:N], B, N, max_len, max_sent_nnz=int(max_sent_nnz))
 
 
 def graph_from_dense(adj: torch.Tensor, check: bool = True) -> DepGraph:
@@ -143,7 +191,12 @@ def tree_distance(graph: DepGraph, anchor_index: torch.Tensor, pad: Optional[str
 
     ``pad=None`` -> packed int32 ``[N]``.  ``pad='max+1'`` (data_utils.py:486-488) or
     ``'zero'`` (:593-594) -> int64 ``[B,T]`` laid out like the collated
-    ``dist_to_target`` column (data_utils.py:378)."""
+    ``dist_to_target`` column (data_utils.py:378).
+
+    The kernel counts breadth-first hops.  On a graph with extra edges (``build_graph(..., extra_edges=...)``) it
+    returns those hop counts; the reference's depth-first walk depends on the order it visits neighbours on a cycle and
+    can over-estimate there (``tests/golden/tree_dist_cycle.npz``).  Where parity with the reference's distances
+    matters, use the items' own ``dist_to_target`` (``PackedBatch.dist``)."""
     dev = graph.device
     anchor = _i32(anchor_index, dev)
     dist = torch.empty(max(graph.n_rows, 1), dtype=torch.int32, device=dev)

@@ -27,7 +27,7 @@ def shard_graphs(lengths: Sequence[int], world_size: int, rank: int) -> np.ndarr
 
 
 def shard_tree_batch(batch, world_size: int, rank: int):
-    """Sub-batch (a ``synth.TreeBatch``) holding only this rank's graphs."""
+    """Sub-batch (a ``synth.TreeBatch``) holding only this rank's graphs, with their extra edges if it has any."""
     from .synth import TreeBatch
     idx = shard_graphs(batch.lengths, world_size, rank)
     lengths = batch.lengths[idx]
@@ -35,7 +35,14 @@ def shard_tree_batch(batch, world_size: int, rank: int):
     np.cumsum(lengths, out=sent_ptr[1:])
     heads = np.concatenate([batch.heads[batch.sent_ptr[b]:batch.sent_ptr[b + 1]] for b in idx]) if len(idx) else \
         np.zeros(0, dtype=np.int32)
-    return TreeBatch(heads=heads.astype(np.int32), sent_ptr=sent_ptr, anchor=batch.anchor[idx], lengths=lengths), idx
+    extra_edges = edge_ptr = None
+    if getattr(batch, "extra_edges", None) is not None:
+        ep = batch.edge_ptr
+        extra_edges = np.concatenate([np.zeros((0, 2), dtype=np.int32)] + [batch.extra_edges[ep[b]:ep[b + 1]] for b in idx])
+        edge_ptr = np.zeros(len(idx) + 1, dtype=np.int32)
+        np.cumsum(ep[idx + 1] - ep[idx], out=edge_ptr[1:])
+    return TreeBatch(heads=heads.astype(np.int32), sent_ptr=sent_ptr, anchor=batch.anchor[idx], lengths=lengths,
+                     extra_edges=extra_edges, edge_ptr=edge_ptr), idx
 
 
 class GradientAllReducer:

@@ -49,6 +49,8 @@ class TreeBatch:
     sent_ptr: np.ndarray     # int32 [B+1] row offsets of the sentences
     anchor: np.ndarray       # int32 [B]   sentence-local trigger index
     lengths: np.ndarray      # int32 [B]
+    extra_edges: Optional[np.ndarray] = None   # int32 [E,2] sentence-local (i, j), i < j: edges beyond the tree
+    edge_ptr: Optional[np.ndarray] = None      # int32 [B+1] pairs of sentence b: edge_ptr[b] .. edge_ptr[b+1] - 1
 
     @property
     def n_graphs(self) -> int:
@@ -60,6 +62,12 @@ class TreeBatch:
 
     def heads_list(self) -> List[np.ndarray]:
         return [self.heads[self.sent_ptr[b]:self.sent_ptr[b + 1]] for b in range(self.n_graphs)]
+
+    def extras_list(self) -> List[np.ndarray]:
+        """Extra edges of every sentence (int32 [E_b, 2]; empty without extras)."""
+        if self.extra_edges is None:
+            return [np.zeros((0, 2), dtype=np.int32) for _ in range(self.n_graphs)]
+        return [self.extra_edges[self.edge_ptr[b]:self.edge_ptr[b + 1]] for b in range(self.n_graphs)]
 
 
 def make_batch(n_graphs: int, n_min: int, n_max: int, seed: int = REFERENCE_SEED,
@@ -76,6 +84,40 @@ def make_batch(n_graphs: int, n_min: int, n_max: int, seed: int = REFERENCE_SEED
         heads[sent_ptr[b]:sent_ptr[b + 1]] = random_tree(int(lengths[b]), rng, skewed)
     anchor = (rng.random(n_graphs) * lengths).astype(np.int32)
     return TreeBatch(heads=heads, sent_ptr=sent_ptr, anchor=anchor, lengths=lengths)
+
+
+DEFAULT_EXTRA_RATE = 0.1
+
+
+def with_extra_edges(batch: TreeBatch, rate: float = DEFAULT_EXTRA_RATE, seed: int = REFERENCE_SEED) -> TreeBatch:
+    """``batch`` plus edges like those CoreNLP's enhanced dependencies add to a tree (propagated conjunct subjects,
+    controlled subjects): each token that has a head gets, with probability ``rate``, one extra edge to its
+    grandparent or to a sibling, closing a triangle.  Edges are drawn from a generator of their own (``seed``), so the
+    tree arrays -- which the result shares with ``batch`` -- and every seeded stream of ``make_batch`` stay as they
+    are.  Per sentence the edges are distinct, never repeat a tree edge, and come as (i, j), i < j, in ascending order.
+
+    The default rate is a synthetic choice: no statistic of real CoreNLP output was available to calibrate it."""
+    rng = np.random.default_rng(seed)
+    pairs = set()
+    for b, h in enumerate(batch.heads_list()):
+        cand = np.nonzero((h >= 0) & (rng.random(len(h)) < rate))[0]
+        to_grandparent = rng.random(len(cand)) < 0.5
+        for i, up in zip(cand.tolist(), to_grandparent.tolist()):
+            p = int(h[i])
+            sibs = np.nonzero(h == p)[0]
+            sibs = sibs[sibs != i]
+            if up and h[p] >= 0:
+                j = int(h[p])
+            elif len(sibs):
+                j = int(sibs[rng.integers(len(sibs))])
+            else:
+                continue
+            pairs.add((b, min(i, j), max(i, j)))
+    rows = np.array(sorted(pairs), dtype=np.int32).reshape(-1, 3)
+    edge_ptr = np.zeros(batch.n_graphs + 1, dtype=np.int32)
+    np.cumsum(np.bincount(rows[:, 0], minlength=batch.n_graphs), out=edge_ptr[1:])
+    return TreeBatch(heads=batch.heads, sent_ptr=batch.sent_ptr, anchor=batch.anchor, lengths=batch.lengths,
+                     extra_edges=np.ascontiguousarray(rows[:, 1:]), edge_ptr=edge_ptr)
 
 
 # BASELINE.json configs (SURVEY.md 8d "Per-config shapes")

@@ -8,6 +8,10 @@ per batch (train.py:108).  The hot path only needs ~16 bytes per token:
     heads int32[N] (-1 = root), sent_ptr int32[B+1], anchor int32[B], dist int32[N] (optional: the GPU
     recomputes it), seg_start/seg_len int32[N] + piece_ptr int32[B+1] (word pieces of every word)
 
+Dependency graphs that are not forests (CoreNLP enhanced dependencies add edges that close cycles) travel as their
+breadth-first forest in ``heads`` plus the remaining edges, ``extra_edges`` int32[E,2] + ``edge_ptr`` int32[B+1]
+(8 bytes per extra edge; both absent when every sentence is a forest).
+
 ``collate_packed`` builds that from the reference's own per-sentence item dicts (host, numpy);
 ``PackedBatch.pin`` / ``.to`` move it with one small copy per field.  Host-side only: no kernels here.
 """
@@ -20,16 +24,9 @@ import numpy as np
 import torch
 
 
-def heads_from_adjacency(adj, n: int) -> np.ndarray:
-    """Orient the symmetric 0/1 matrix of graph.py:66-75 (first ``n`` rows/cols) as head indices: every
-    connected component is rooted at its smallest token (-1), every other token points at the neighbour that
-    discovered it in a breadth-first sweep.  The CSR built from these heads (self + parent + children) is the
-    non-zero pattern of the matrix.  Raises ValueError when the matrix is not a forest (an edge would be lost)."""
-    a = np.asarray(adj)[:n, :n] != 0
-    if not np.array_equal(a, a.T):
-        raise ValueError("adjacency is not symmetric")
+def _bfs_heads(a: np.ndarray, n: int):
+    """Heads of the breadth-first orientation of the boolean pattern ``a`` and the number of edges it holds."""
     heads = np.full(n, -2, dtype=np.int32)
-    n_edges = (int(a.sum()) - int(np.trace(a))) // 2
     used = 0
     for root in range(n):
         if heads[root] != -2:
@@ -45,9 +42,45 @@ def heads_from_adjacency(adj, n: int) -> np.ndarray:
                         used += 1
                         nxt.append(int(v))
             frontier = nxt
+    return heads, used
+
+
+def _pattern(adj, n: int) -> np.ndarray:
+    a = np.asarray(adj)[:n, :n] != 0
+    if not np.array_equal(a, a.T):
+        raise ValueError("adjacency is not symmetric")
+    return a
+
+
+def heads_from_adjacency(adj, n: int) -> np.ndarray:
+    """Orient the symmetric 0/1 matrix of graph.py:66-75 (first ``n`` rows/cols) as head indices: every
+    connected component is rooted at its smallest token (-1), every other token points at the neighbour that
+    discovered it in a breadth-first sweep.  The CSR built from these heads (self + parent + children) is the
+    non-zero pattern of the matrix.  Raises ValueError when the matrix is not a forest (an edge would be lost;
+    ``split_adjacency`` keeps such edges)."""
+    a = _pattern(adj, n)
+    heads, used = _bfs_heads(a, n)
+    n_edges = (int(a.sum()) - int(np.trace(a))) // 2
     if used != n_edges:
-        raise ValueError(f"adjacency is not a forest ({n_edges} edges, {used} fit a head array): use graph_from_dense")
+        raise ValueError(f"adjacency is not a forest ({n_edges} edges, {used} fit a head array): "
+                         "use split_adjacency or graph_from_dense")
     return heads
+
+
+def split_adjacency(adj, n: int):
+    """Any symmetric 0/1 matrix of graph.py:66-75 (first ``n`` rows/cols), e.g. one built from CoreNLP enhanced
+    dependencies whose extra edges close cycles -> ``(heads, extra)``.  ``heads`` is the breadth-first forest
+    ``heads_from_adjacency`` returns for every input; ``extra`` int32 ``[E_b, 2]`` holds the remaining edges as
+    ``(i, j)`` with ``i < j``, in ascending order (empty for a forest).  The forest's CSR plus these edges
+    (``graph.build_graph(..., extra_edges=...)``) is the non-zero pattern of the matrix.  Raises ValueError on an
+    asymmetric matrix."""
+    a = _pattern(adj, n)
+    heads, _ = _bfs_heads(a, n)
+    rest = np.triu(a, 1)
+    kids = np.nonzero(heads >= 0)[0]
+    par = heads[kids]
+    rest[np.minimum(kids, par), np.maximum(kids, par)] = False
+    return heads, np.argwhere(rest).astype(np.int32).reshape(-1, 2)
 
 
 def segments_from_transform_rows(transform, n_words: int):
@@ -70,6 +103,9 @@ class PackedBatch:
     seg_len: Optional[torch.Tensor] = None     # int32 [N]
     piece_ptr: Optional[torch.Tensor] = None   # int32 [B+1] word-piece rows of sentence b ([CLS] .. [SEP])
     max_len: int = 0
+    extra_edges: Optional[torch.Tensor] = None  # int32 [E,2] sentence-local (i, j), i < j: edges a head array cannot hold
+    edge_ptr: Optional[torch.Tensor] = None     # int32 [B+1] pairs of sentence b; both None when no sentence has one
+    max_sent_nnz: int = 0               # largest CSR entry count of one sentence: n_b + 2 (forest edges) + 2 E_b
 
     @property
     def n_graphs(self) -> int:
@@ -103,11 +139,16 @@ def collate_packed(items: Sequence[dict], with_dist: bool = True, with_transform
     (keys ``dependency_graph``, ``anchor_index``, ``sentence_length``, ``dist_to_target``, ``transform``,
     ``cls_text_sep_length``, ``polarity``; data_utils.py:362-379)."""
     heads: List[np.ndarray] = []
+    extras: List[np.ndarray] = []
     lens, anchors, dists, pols = [], [], [], []
     seg_s, seg_n, piece_ptr = [], [], [0]
+    max_sent_nnz = 0
     for it in items:
         n = int(it["sentence_length"])
-        heads.append(heads_from_adjacency(it["dependency_graph"], n))
+        h, x = split_adjacency(it["dependency_graph"], n)
+        heads.append(h)
+        extras.append(x)
+        max_sent_nnz = max(max_sent_nnz, n + 2 * int((h >= 0).sum()) + 2 * len(x))
         lens.append(n)
         anchors.append(int(it["anchor_index"]))
         if with_dist and "dist_to_target" in it:
@@ -124,6 +165,11 @@ def collate_packed(items: Sequence[dict], with_dist: bool = True, with_transform
     np.cumsum(np.asarray(lens, dtype=np.int32), out=sent_ptr[1:])
     t = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dtype=dt))
     cat = lambda xs, dt: t(np.concatenate(xs) if xs else np.zeros(0, dtype=dt), dt)
+    n_extra = np.asarray([len(x) for x in extras], dtype=np.int32)
+    edge_ptr = None
+    if n_extra.sum() > 0:
+        edge_ptr = np.zeros(len(items) + 1, dtype=np.int32)
+        np.cumsum(n_extra, out=edge_ptr[1:])
     return PackedBatch(
         heads=cat(heads, np.int32), sent_ptr=t(sent_ptr, np.int32), anchor=t(np.asarray(anchors), np.int32),
         dist=cat(dists, np.int32) if len(dists) == len(items) and items else None,
@@ -131,4 +177,7 @@ def collate_packed(items: Sequence[dict], with_dist: bool = True, with_transform
         seg_start=cat(seg_s, np.int32) if len(seg_s) == len(items) and items else None,
         seg_len=cat(seg_n, np.int32) if len(seg_n) == len(items) and items else None,
         piece_ptr=t(np.asarray(piece_ptr), np.int32) if len(seg_s) == len(items) and items else None,
-        max_len=int(max(lens)) if lens else 0)
+        max_len=int(max(lens)) if lens else 0,
+        extra_edges=t(np.concatenate(extras), np.int32) if edge_ptr is not None else None,
+        edge_ptr=t(edge_ptr, np.int32) if edge_ptr is not None else None,
+        max_sent_nnz=max_sent_nnz)

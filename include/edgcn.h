@@ -73,6 +73,26 @@ int edg_csr_from_heads(const int32_t* heads, const int32_t* sent_ptr, int32_t B,
                        int32_t max_len, int32_t* row_ptr, int32_t* col, int32_t* row_sent,
                        int32_t* ws, edg_stream stream);
 
+/* graph.py:66-75 for graphs that are not forests (CoreNLP enhanced dependencies,
+ * graph.py:63-64): the forest of heads[] (as in edg_csr_from_heads) plus E extra
+ * undirected edges.  edges[E][2] holds sentence-local (i, j) pairs; sentence b owns
+ * pairs edge_ptr[b] .. edge_ptr[b+1]-1 (edge_ptr[B+1], edge_ptr[0] = 0, edge_ptr[B] = E).
+ * Set semantics: duplicate pairs, both orientations of one pair, pairs that repeat a
+ * forest edge and i == j change nothing; a pair with an endpoint outside [0, n_b) is
+ * dropped.  Each row lists self, parent, children and extra neighbours once, as
+ * global ids in ascending order, so the output does not depend on the order of the
+ * pairs.  Writes row_ptr[N+1], col (capacity >= 3N + 2E), row_sent[N] and
+ * sent_max_nnz[0] = the largest CSR entry count of one sentence.  On entry,
+ * sent_max_nnz[0] > 0 is an upper bound the caller guarantees for that count (a
+ * sentence above it traps, as one longer than max_len does); 0 = no bound.
+ * ws: edg_csr_from_heads_edges_workspace(B, N, E) bytes.  max_len <= 4096; any
+ * number of pairs per sentence.  Enqueues 3 kernels when E = 0 or N = 0, 7 otherwise. */
+size_t edg_csr_from_heads_edges_workspace(int32_t B, int32_t N, int32_t E);
+int edg_csr_from_heads_edges(const int32_t* heads, const int32_t* sent_ptr, const int32_t* edges,
+                             const int32_t* edge_ptr, int32_t B, int32_t N, int32_t E, int32_t max_len,
+                             int32_t* row_ptr, int32_t* col, int32_t* row_sent, int32_t* sent_max_nnz,
+                             void* ws, size_t ws_bytes, edg_stream stream);
+
 /* Compat path for the unchanged forward(text, adj) signature (models/gcn.py:30):
  * dense [B,T,T] adjacency (fp32 or int64, any strides) -> packed CSR over B*T rows
  * (padding rows are self-loop singletons, graph.py:66).  Two calls because the
