@@ -29,12 +29,11 @@ pool_staged_kernel(const T* __restrict__ h, int64_t ldh, const int32_t* __restri
   __shared__ __align__(8) uint64_t bar;
   __shared__ int sh[4];
   const RowWindow w = stage_window<T>(h, ldh, N, B, tile_rows, sent_ptr, row_sent, win, &bar, sh);
-  if (w.r1 <= w.r0) return;
   const int pitch = (int)(ldh * (int64_t)sizeof(T));
   const int c = threadIdx.x * E;
   const int64_t BD = (int64_t)B * D;
   const uint32_t xs = stg_smem_u32(win) + threadIdx.x * 16;
-  bool waited = false;
+  bool waited = !w.has_rows();           // a window without rows still writes its (empty) sentences
   for (int s = w.s0 + threadIdx.y; s < w.s1; s += blockDim.y) {
     const int beg = __ldg(sent_ptr + s), end = __ldg(sent_ptr + s + 1);
     // the gate vectors do not depend on the window: issue their loads BEFORE blocking on the bulk copy
@@ -99,7 +98,6 @@ scores_staged_kernel(const T* __restrict__ h, int64_t ldh, const int32_t* __rest
   __shared__ __align__(8) uint64_t bar;
   __shared__ int sh[4];
   const RowWindow w = stage_window<T>(h, ldh, N, B, tile_rows, sent_ptr, row_sent, win, &bar, sh);
-  if (w.r1 <= w.r0) return;
   const int pitch = (int)(ldh * (int64_t)sizeof(T));
   const int lane = threadIdx.x, warp = threadIdx.y;
   const int width = chunks * E;
@@ -107,7 +105,7 @@ scores_staged_kernel(const T* __restrict__ h, int64_t ldh, const int32_t* __rest
   const uint32_t w_a = stg_smem_u32(w_s);
   const uint32_t xs = stg_smem_u32(win);
   const float invB = 1.0f / (float)B;
-  bool waited = false;
+  bool waited = !w.has_rows();           // a window without rows still writes its (empty) sentences
   for (int s = w.s0 + warp; s < w.s1; s += kScoresWarps) {
     const int beg = __ldg(sent_ptr + s) - w.r0, end = __ldg(sent_ptr + s + 1) - w.r0;
     const int n = end - beg;
@@ -268,7 +266,6 @@ head_bwd_staged_kernel(const T* __restrict__ h, int64_t ldh, const int32_t* __re
   __shared__ __align__(8) uint64_t bar;
   __shared__ int sh[4];
   const RowWindow w = stage_window<T>(h, ldh, N, B, tile_rows, sent_ptr, row_sent, win, &bar, sh);
-  if (w.r1 <= w.r0) return;
   const int pitch = (int)(ldh * (int64_t)sizeof(T));
   float* ds_s = reinterpret_cast<float*>(win + (size_t)cap_rows * pitch);      // [cap_rows] d loss / d scores
   const int nthreads = blockDim.x * blockDim.y;
@@ -330,7 +327,7 @@ head_bwd_staged_kernel(const T* __restrict__ h, int64_t ldh, const int32_t* __re
   int s = w.s0 + threadIdx.y;
   if (s < w.s1) load_sentence(s);          // in flight while the block waits below
   __syncthreads();                         // publishes ds_s (phase 1)
-  wait_window(&bar);
+  if (w.has_rows()) wait_window(&bar);     // a window without rows still writes its (empty) sentences
   for (bool first = true; s < w.s1; s += blockDim.y, first = false) {
     if (!first) load_sentence(s);
     float gv[E], ggp[E], sf[E], xg[E];
@@ -362,7 +359,7 @@ head_bwd_staged_kernel(const T* __restrict__ h, int64_t ldh, const int32_t* __re
       if (c + k < D) {
         const int64_t o = (int64_t)s * D + c + k;
         float dg = fmaf(vv[k], sf[k], xg[k]);
-        if (where[k] >= 0) {
+        if (where[k] >= beg && where[k] < end) {      // as the per-sentence kernel: only a row of the sentence
           const T* hp = reinterpret_cast<const T*>(win + (size_t)(where[k] - w.r0) * pitch) + c + k;
           dg = fmaf(gp[k], to_f32(*hp), dg);
         }
@@ -382,13 +379,14 @@ static inline dim3 chunk_block(int chunks) {
   return dim3(chunks, y);
 }
 
-// returns 1 when the staged path does not apply (caller falls back to the per-sentence kernels)
+// returns 1 when the staged path does not apply (caller falls back to the per-sentence kernels); N == 0 (every
+// sentence empty) is one such case: it would be a grid of 0 blocks
 template <typename T>
 int pool_fwd_staged(const void* h, int64_t ldh, const int32_t* sent_ptr, const int32_t* row_sent, int N, int B, int D,
                     int max_len, const float* gates, int V, float* pooled, int32_t* arg, float* hmax, cudaStream_t s) {
   constexpr int E = Vec16<T>::kElems;
   const int chunks = (D + E - 1) / E;
-  if (!row_sent || max_len <= 0 || chunks > 256) return 1;
+  if (!row_sent || max_len <= 0 || N <= 0 || chunks > 256) return 1;
   const dim3 blk = chunk_block(chunks);
   const WindowPlan p = plan_window((size_t)ldh * sizeof(T), max_len);
   if (p.tile_rows < 8) return 1;
@@ -437,7 +435,7 @@ int scores_kl_staged(const void* h, int64_t ldh, const int32_t* sent_ptr, const 
                      float* scores, float* kl_b, float* dv_unit, float* dc_unit, float* u_unit, float* sf_unit, cudaStream_t s) {
   constexpr int E = Vec16<T>::kElems;
   const int chunks = (D + E - 1) / E;
-  if (!row_sent || max_len <= 0 || chunks > 32 * kSMaxQ || max_len > 32 * kSMaxPass) return 1;
+  if (!row_sent || max_len <= 0 || N <= 0 || chunks > 32 * kSMaxQ || max_len > 32 * kSMaxPass) return 1;
   const size_t wbuf = (size_t)kScoresWarps * chunks * E * sizeof(float);          // per-warp gate*v of the current sentence
   const WindowPlan p = plan_window((size_t)ldh * sizeof(T), max_len, 0, wbuf);
   if (p.tile_rows < 8) return 1;
@@ -465,7 +463,7 @@ int head_bwd_staged(const void* h, int64_t ldh, const int32_t* sent_ptr, const i
                     cudaStream_t s) {
   constexpr int E = Vec16<T>::kElems;
   const int chunks = (D + E - 1) / E;
-  if (!row_sent || max_len <= 0 || chunks > 256) return 1;
+  if (!row_sent || max_len <= 0 || N <= 0 || chunks > 256) return 1;
   const dim3 blk = chunk_block(chunks);
   const WindowPlan p = plan_window((size_t)ldh * sizeof(T), max_len, 4);
   if (p.tile_rows < 8) return 1;

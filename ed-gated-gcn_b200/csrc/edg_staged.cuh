@@ -5,12 +5,20 @@
 // completion) brings them into shared memory; all per-row work then runs on 128-bit shared-memory
 // loads.  DRAM latency is paid once per window and hidden by the other resident blocks, instead of
 // once per row of a sequential per-sentence loop.
+//
+// Every sentence has exactly one owner, empty ones (0 rows) included: window 0 also owns the empty sentences
+// before the first row, and a window that lies inside one long sentence owns the empty sentences that start at its
+// end.  Such a window has no rows to stage (r1 <= r0) and issues no copy, but it still writes the outputs of its
+// sentences (all of them empty); it must then not wait on the barrier (has_rows() is false).
 #pragma once
 #include "edg_common.cuh"
 
 namespace edg {
 
-struct RowWindow { int r0, r1, s0, s1; };
+struct RowWindow {
+  int r0, r1, s0, s1;
+  __device__ __forceinline__ bool has_rows() const { return r1 > r0; }   // false: no copy was issued, do not wait
+};
 
 __device__ __forceinline__ uint32_t stg_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -28,7 +36,7 @@ __device__ __forceinline__ RowWindow stage_window(const T* __restrict__ x, int64
     const int p0 = __ldg(sent_ptr + a0), q0 = a0 < B ? __ldg(sent_ptr + a0 + 1) : p0;
     const int p1 = __ldg(sent_ptr + a1), q1 = a1 < B ? __ldg(sent_ptr + a1 + 1) : p1;
     const bool up0 = w0 < N && p0 < w0, up1 = w1 < N && p1 < w1;
-    const int s0 = a0 + up0, s1 = a1 + up1;
+    const int s0 = w0 == 0 ? 0 : a0 + up0, s1 = a1 + up1;     // row_sent names no leading empty sentence
     const int r0 = up0 ? q0 : p0, r1 = up1 ? q1 : p1;
     sh[0] = r0; sh[1] = r1; sh[2] = s0; sh[3] = s1;
     const uint32_t b32 = stg_smem_u32(bar);

@@ -266,6 +266,7 @@ int edg_trigger_scatter_add(const float* da, const float* extra, int32_t n_extra
 
 /* bert_amir5.py:627-636,640: pooled[v,b,:] = max_t h[t,:]*gates[v,b,:] over the
  * sentence's rows, arg = global row of the maximum (first row wins ties).
+ * An empty sentence (0 rows) gets pooled 0, arg -1 and hmax 0.
  * row_sent[N] + max_len (may be NULL/0) enable the shared-memory staged kernel: the rows of the sentences
  * starting in a window are brought in by one bulk async copy instead of one dependent load per row;
  * the same holds for edg_scores_kl_fwd and edg_head_bwd.
@@ -298,7 +299,8 @@ int edg_views_bwd(const float* pooled, const int32_t* arg, const float* gates, c
  * Optional (NULL to skip): dv_unit[B,D], dc_unit[B] = d kl / d v, d kl / d c per unit upstream
  * gradient, so that the backward pass needs no extra sweep over h when only kl carries gradient; with them (optional)
  * u_unit[N] = d kl / d scores[i] = P_i (Q_i - kl_b) / B and sf_unit[B,D] = sum_t u_t h[t,:] (dv_unit without the gate),
- * the per-row scalars and per-sentence vectors edg_head_du builds the top layer's gradient from. */
+ * the per-row scalars and per-sentence vectors edg_head_du builds the top layer's gradient from.
+ * An empty sentence (0 rows) gets kl_b 0, and dv_unit, dc_unit, sf_unit 0. */
 int edg_scores_kl_fwd(const void* h, int dtype, int64_t ldh, const int32_t* sent_ptr, int32_t B,
                       int32_t D, const float* gate, const float* v, const float* c,
                       const void* dist, int dist_i64, float* scores, float* kl_b,
@@ -353,7 +355,8 @@ int edg_fc_head_bwd(const float* logits, int64_t ldl, const float* fc_w, int64_t
  * g_kl: device scalar or NULL; g_scores, g_pooled, g_xout may be NULL.
  * dh/dgate may be NULL (first pass: only dv/dc, which the host needs before it can
  * back-propagate through the classifier head to obtain g_pooled).
- * max_len = longest sentence (sizes the shared-memory ds buffer; <= 8192). */
+ * max_len = longest sentence (sizes the shared-memory ds buffer; <= 8192).
+ * An empty sentence (0 rows) gets dgate, dv and dc 0. */
 int edg_head_bwd(const void* h, int dtype, int64_t ldh, const int32_t* sent_ptr, int32_t B,
                  int32_t D, const float* gate, const float* v, const void* dist, int dist_i64,
                  const float* scores, const float* kl_b, const float* g_kl, const float* g_scores,
