@@ -94,6 +94,13 @@ SIGNATURES = {
     "edg_sum_scaled": (c_int, [_P, _L, _F, _P, _P]),
     "edg_colsum_workspace": (_Z, [_I, _I]),
     "edg_colsum": (c_int, [_P, c_int, _L, _I, _I, _P, c_int, _P, _Z, _P]),
+    "edg_tree_dist_pairs": (c_int, [_P, _P, _P, _P, _P, _P, _I, _I, _P, _P]),
+    "edg_scores_kl_pairs_fwd": (c_int, [_P, c_int, _L, _P, _P, _P, _I, _I, _P, _P, _P, _P, c_int, _P, _P, _P, _P, _P, _P,
+                                        _P]),
+    "edg_head_bwd_pairs": (c_int, [_P, c_int, _L, _P, _I, _P, _I, _P, _P, _P, _I, _I, _P, _P, _P, c_int, _P, _P, _P, _P, _P, _P,
+                                   _P, _L, _P, _P, _P, _P, _P]),
+    "edg_views_bwd_hmax_pairs": (c_int, [_P, _P, _P, _I, _I, _P, _I, _I, _P, _L, _P, c_int, _P]),
+    "edg_trigger_scatter_add_pairs": (c_int, [_P, _P, _I, _I, _P, _I, _I, _P, _P, _P, c_int, _L, _P]),
 }
 
 
@@ -157,6 +164,8 @@ def _kernels_of(name: str, args) -> int:
         return 2 if args[23] else 1
     if name == "edg_adam_multi":
         return 2 if args[0] else 0
+    if name == "edg_head_bwd_pairs":
+        return 2 if args[22] else 1
     if name == "edg_pool_fwd":
         return (args[7] + 3) // 4
     return 1

@@ -284,16 +284,11 @@ __global__ void dense_fill_kernel(const T* __restrict__ adj, int rows, int Tn, i
 // ---- distance to the trigger -------------------------------------------------
 // one block per sentence, level-synchronous BFS over the CSR (true hop counts;
 // equals data_utils.py:302-323 on trees and forests, SURVEY fact 8).
-__global__ void tree_dist_kernel(const int32_t* __restrict__ row_ptr, const int32_t* __restrict__ col,
-                                 const int32_t* __restrict__ sent_ptr, const int32_t* __restrict__ anchor,
-                                 int32_t* __restrict__ dist, int cap) {
-  extern __shared__ int32_t d[];
-  const int b = blockIdx.x;
-  const int base = sent_ptr[b], n = sent_ptr[b + 1] - base;
-  if (n > cap) __trap();      // max_len smaller than this sentence (see heads_fill_kernel)
+// level-synchronous BFS of one sentence (rows base .. base + n - 1) from sentence-local row `a`, written to out[0..n)
+__device__ __forceinline__ void bfs_sentence(const int32_t* __restrict__ row_ptr, const int32_t* __restrict__ col, int base,
+                                             int n, int a, int32_t* __restrict__ out, int32_t* d) {
   for (int i = threadIdx.x; i < n; i += blockDim.x) d[i] = -1;
   __syncthreads();
-  int a = anchor[b];
   if (threadIdx.x == 0 && a >= 0 && a < n) d[a] = 0;
   __syncthreads();
   for (int level = 0; level < n; ++level) {
@@ -309,7 +304,33 @@ __global__ void tree_dist_kernel(const int32_t* __restrict__ row_ptr, const int3
     if (!__syncthreads_or(grew)) break;
   }
   for (int i = threadIdx.x; i < n; i += blockDim.x)
-    dist[base + i] = d[i] >= 0 ? d[i] + 1 : kUnreachablePlusOne;
+    out[i] = d[i] >= 0 ? d[i] + 1 : kUnreachablePlusOne;
+}
+
+// one block per sentence, level-synchronous BFS over the CSR (true hop counts;
+// equals data_utils.py:302-323 on trees and forests, SURVEY fact 8).
+__global__ void tree_dist_kernel(const int32_t* __restrict__ row_ptr, const int32_t* __restrict__ col,
+                                 const int32_t* __restrict__ sent_ptr, const int32_t* __restrict__ anchor,
+                                 int32_t* __restrict__ dist, int cap) {
+  extern __shared__ int32_t d[];
+  const int b = blockIdx.x;
+  const int base = sent_ptr[b], n = sent_ptr[b + 1] - base;
+  if (n > cap) __trap();      // max_len smaller than this sentence (see heads_fill_kernel)
+  bfs_sentence(row_ptr, col, base, n, anchor[b], dist + base, d);
+}
+
+// the same per (sentence, trigger) pair: block p walks sentence pair_sent[p] from anchor[p] and writes that pair's copy
+// of the sentence's distances at pair_row_ptr[p]
+__global__ void tree_dist_pairs_kernel(const int32_t* __restrict__ row_ptr, const int32_t* __restrict__ col,
+                                       const int32_t* __restrict__ sent_ptr, const int32_t* __restrict__ pair_sent,
+                                       const int32_t* __restrict__ pair_row_ptr, const int32_t* __restrict__ anchor,
+                                       int32_t* __restrict__ dist, int cap) {
+  extern __shared__ int32_t d[];
+  const int p = blockIdx.x;
+  const int s = pair_sent[p];
+  const int base = sent_ptr[s], n = sent_ptr[s + 1] - base;
+  if (n > cap) __trap();      // max_len smaller than this sentence
+  bfs_sentence(row_ptr, col, base, n, anchor[p], dist + pair_row_ptr[p], d);
 }
 
 __global__ void dist_pad_kernel(const int32_t* __restrict__ dist, const int32_t* __restrict__ sent_ptr,
@@ -439,6 +460,19 @@ extern "C" int edg_tree_dist(const int32_t* row_ptr, const int32_t* col, const i
   if (max_len > 8192) return EDG_ERR_UNSUPPORTED;
   int threads = max_len <= 64 ? 64 : (max_len <= 128 ? 128 : 256);
   tree_dist_kernel<<<B, threads, (size_t)max_len * sizeof(int32_t), (cudaStream_t)stream>>>(row_ptr, col, sent_ptr, anchor, dist, max_len);
+  return check_launch();
+}
+
+extern "C" int edg_tree_dist_pairs(const int32_t* row_ptr, const int32_t* col, const int32_t* sent_ptr,
+                                   const int32_t* pair_sent, const int32_t* pair_row_ptr, const int32_t* anchor, int32_t P,
+                                   int32_t max_len, int32_t* dist, edg_stream stream) {
+  if (P < 0 || max_len < 0) return EDG_ERR_ARG;
+  if (P == 0) return EDG_OK;
+  if (!row_ptr || !col || !sent_ptr || !pair_sent || !pair_row_ptr || !anchor || !dist) return EDG_ERR_ARG;
+  if (max_len > 8192) return EDG_ERR_UNSUPPORTED;
+  int threads = max_len <= 64 ? 64 : (max_len <= 128 ? 128 : 256);
+  tree_dist_pairs_kernel<<<P, threads, (size_t)(max_len > 0 ? max_len : 1) * sizeof(int32_t), (cudaStream_t)stream>>>(
+      row_ptr, col, sent_ptr, pair_sent, pair_row_ptr, anchor, dist, max_len);
   return check_launch();
 }
 

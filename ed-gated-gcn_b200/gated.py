@@ -28,7 +28,7 @@ import torch.nn as nn
 from . import _lib as L
 from . import ops
 from .gcn import GraphConvolution, _compute_dtype
-from .graph import DepGraph
+from .graph import DepGraph, TriggerPairs
 
 # name -> (leading Sigmoid?, number of (Linear, Sigmoid) pairs); SURVEY 8a variant matrix
 GATE_ARCHS = {
@@ -721,6 +721,362 @@ class _GatedStackFn(torch.autograd.Function):
         return (None, dx, d_aspect) + tuple(grads_out) + tuple(head_grads)
 
 
+class _GatedPairsFn(torch.autograd.Function):
+    """The block for (sentence, trigger) pairs (``GatedGCNStack.forward(..., pairs=)``): the GCN chain runs once on the
+    sentence rows, everything that depends on the trigger runs per pair.  Positive gates give
+    ``max_t (h_t * g) = g * max_t h_t`` with a gate-independent arg-max row, so every per-pair pooled view is
+    ``g_p * hmax[sentence(p)]``; only the scores / kl pass over the sentence's rows once per pair.  Same inputs as
+    :class:`_GatedStackFn` (without ``aspect``)."""
+
+    @staticmethod
+    def forward(ctx, cfg, x, *params):
+        graph: DepGraph = cfg["graph"]
+        pairs = cfg["pairs"]
+        cd: torch.dtype = cfg["cdtype"]
+        Lyr, npr, lead = cfg["L"], cfg["gate_pairs"], cfg["lead"]
+        anchor, dist, logits_fn = cfg["anchor"], cfg["dist"], cfg["logits_fn"]
+        D = cfg["D"]
+        S, P = graph.n_graphs, pairs.n_pairs
+        gcn_p = [(params[2 * l], params[2 * l + 1]) for l in range(Lyr)]
+        o = 2 * Lyr
+        gate_p = [[(params[o + 2 * (g * npr + i)], params[o + 2 * (g * npr + i) + 1]) for i in range(npr)]
+                  for g in range(Lyr)]
+        o += 2 * Lyr * npr
+        fc_w, fc_b = params[o], params[o + 1]
+        n_head = cfg["n_head"]
+        params = params[:len(params) - n_head] if n_head else params
+        ctx.x_padded = x.shape[1] != D
+        xr = ops.as_rows(x[:, :D] if ctx.x_padded else x, cd)
+        flat_w = [w for (w, _) in gcn_p] + [w for gp in gate_p for (w, _) in gp]
+        casted = ops.cast_weights_batch([(w, True) for w in flat_w] + [(w, False) for w in flat_w], cd)
+        nW = len(flat_w)
+        w_t = {id(w): casted[i] for i, w in enumerate(flat_w)}
+        w_n = {id(w): casted[nW + i] for i, w in enumerate(flat_w)}
+        ctx.w_t = [casted[i] for i in range(nW)]
+        ctx.w_n = [casted[nW + i] for i in range(nW)]
+        gated = cfg["gated"]
+        # ---- per pair: the trigger row of its sentence and the gate MLPs on P rows
+        a_raw, s0 = ops.trigger_gather(xr, ops.PairRows(pairs), anchor, lead)
+        gate_saved = []
+        if gated:
+            gates = torch.empty((Lyr, P, D), dtype=torch.float32, device=x.device)
+        else:
+            gates = torch.ones((Lyr, P, D), dtype=torch.float32, device=x.device)
+        use_chain = gated and _chain_ok(cd, D, Lyr, npr)
+        ctx.use_chain = use_chain
+        if use_chain:
+            stages = []
+            for g in range(Lyr):
+                acts, st = [s0], []
+                for i, (w, b) in enumerate(gate_p[g]):
+                    last = i == npr - 1
+                    out = gates[g] if last else ops.alloc_rows(P, D, cd, x.device)
+                    st.append(dict(w=w_n[id(w)], bias=b.detach().float().contiguous(), out=out))
+                    if not last:
+                        acts.append(out)
+                stages.append(st)
+                gate_saved.append(acts)
+            if P > 0:
+                ops.mlp_chain(0, [s0] * Lyr, stages, P, D)
+        for g in range(Lyr if (gated and not use_chain and P > 0) else 0):
+            s = s0
+            acts = [s0]
+            for i, (w, b) in enumerate(gate_p[g]):
+                last = i == npr - 1
+                s = ops.linear(s, w_n[id(w)], b.detach().float().contiguous(), act=L.ACT_SIGMOID,
+                               out_dtype=torch.float32 if last else cd, out=gates[g] if last else None)
+                if not last:
+                    acts.append(s)
+            gate_saved.append(acts)
+        # ---- the GCN chain once per sentence, with the column maxima of h_1 (views) and h_L (final pool)
+        h = xr
+        ms, hs, ms_split = [], [], []
+        hmax1 = harg1 = hmaxL = hargL = None
+        fused = _fused_plan(cfg, cd, D, graph, 0.0)
+        ctx.fused = fused
+        ones = None
+        for l, (w, b) in enumerate(gcn_p):
+            want_pool = (l == 0 and gated) or l == Lyr - 1
+            b32 = b.detach().float().contiguous() if b is not None else None
+            if fused is not None:
+                rows, plan = fused
+                h, hm, ha, _ = ops.gcn_layer(h, w_t[id(w)], b32, graph, 0, plan, rows, want_pool=want_pool)
+                ms.append(None)
+                ms_split.append(None)
+            else:
+                m = ops.aggregate(h, graph, mode=0)
+                wt = w_t[id(w)]
+                act = L.ACT_RELU if cfg["relu"] else L.ACT_NONE
+                if (cd == torch.float32 and ops.f32_tc(m.shape[0], m.shape[1], wt.shape[0])
+                        and ops.f32_tc(m.shape[0], wt.shape[0], m.shape[1])):
+                    m2 = ops.split_rows(m)
+                    h = ops.linear_split(m2, ops.split_rows(wt), b32, act)
+                    ms_split.append((m2.amax, m2.rows, m2.cols))
+                    m = m2.data
+                else:
+                    h = ops.linear(m, wt, b32, act=act)
+                    ms_split.append(None)
+                ms.append(m)
+                if want_pool:
+                    if ones is None:
+                        ones = torch.ones((1, S, D), dtype=torch.float32, device=x.device)
+                    _, ha, hm = ops.pool_fwd(h, graph, ones, want_hmax=True)
+                    ha = ha[0]
+            hs.append(h)
+            if l == 0 and gated:
+                hmax1, harg1 = hm, ha
+            if l == Lyr - 1:
+                hmaxL, hargL = hm, ha
+        ps = pairs.pair_sent.long()
+        xy = torch.zeros((), dtype=torch.float32, device=x.device)
+        v_arg = None
+        if gated:
+            v_arg = harg1[ps].unsqueeze(0).expand(Lyr, P, D).contiguous()
+            if Lyr > 1 and P > 0:
+                xy = ops.diversity_fwd(gates * hmax1[ps].unsqueeze(0))     # views g_{v,p} * max_t h_1
+        gL = gates[Lyr - 1]
+        hL = hs[-1]
+        pooled = gL * hmaxL[ps]
+        p_arg = hargL[ps]
+        # ---- classifier head on [P,D], then the per-pair scores / kl over the sentence rows
+        dense_head = cfg.get("dense_head")
+        a_leaf = p_leaf = None
+        if dense_head is not None:
+            hp = cfg["head_params"]
+            logits = ops.dense_head_fwd(a_raw, pooled, hp[0], hp[1] if len(hp) > 1 else None)
+        else:
+            with torch.enable_grad():
+                a_leaf = a_raw.detach().requires_grad_(True)
+                p_leaf = pooled.detach().requires_grad_(True)
+                logits = logits_fn(a_leaf, p_leaf)
+            if logits.requires_grad and cfg["grad_enabled"]:
+                _check_head_leaves(logits, (a_leaf, p_leaf), cfg["head_params"])
+        lg = logits.detach().float().contiguous()
+        fcw32, fcb32 = fc_w.detach().float().contiguous(), fc_b.detach().float().contiguous()
+        v, c = ops.fc_head_fwd(lg, fcw32, fcb32, a_raw)
+        scores, kl_b, kl, dvu, dcu = ops.scores_kl_pairs_fwd(hL, graph, pairs, gL, v, c, dist)
+        ctx.kl_units = (dvu, dcu)
+        ctx.set_materialize_grads(False)
+        ctx.cfg = cfg
+        ctx.head = (a_leaf, p_leaf, logits, lg, a_raw, v)
+        ctx.pooled_head = pooled.detach() if dense_head is not None else None
+        ctx.gate_saved = gate_saved
+        ctx.n_params = len(params)
+        ctx.n_head = n_head
+        ctx.x_dtype = x.dtype
+        ctx.x_cols = x.shape[1]
+        ctx.ms_split = ms_split
+        ctx.pool_rows = (hmax1, harg1, hargL)
+        ctx.save_for_backward(xr, gates, scores, kl_b, *[m for m in ms if m is not None], *hs, *params)
+        ctx.n_ms = sum(m is not None for m in ms)
+        if v_arg is None:
+            v_arg = torch.empty((0,), dtype=torch.int32, device=x.device)
+        ctx.mark_non_differentiable(p_arg, v_arg)
+        return logits.detach(), xy, kl, scores, pooled, p_arg, v_arg
+
+    @staticmethod
+    def backward(ctx, g_logits, g_xy, g_kl, g_scores, g_pooled, _g_parg=None, _g_varg=None):
+        cfg = ctx.cfg
+        graph: DepGraph = cfg["graph"]
+        pairs = cfg["pairs"]
+        cd: torch.dtype = cfg["cdtype"]
+        Lyr, npr, lead = cfg["L"], cfg["gate_pairs"], cfg["lead"]
+        anchor, dist = cfg["anchor"], cfg["dist"]
+        saved = ctx.saved_tensors
+        xr, gates, scores, kl_b = saved[:4]
+        o = 4
+        ms = list(saved[o:o + ctx.n_ms]) if ctx.n_ms else [None] * Lyr
+        o += ctx.n_ms
+        hs = saved[o:o + Lyr]
+        params = saved[o + Lyr:]
+        P, N, D = pairs.n_pairs, graph.n_rows, xr.shape[1]
+        dev = xr.device
+        a_leaf, p_leaf, logits, lg, a_raw, v = ctx.head
+        hmax1, harg1, hargL = ctx.pool_rows
+        gL = gates[Lyr - 1]
+        hL = hs[-1]
+
+        def f32(t):
+            return None if t is None else t.detach().float().contiguous()
+
+        g_xy, g_kl, g_scores, g_pooled = f32(g_xy), f32(g_kl), f32(g_scores), f32(g_pooled)
+        need_scores = g_kl is not None or g_scores is not None
+        grad_hook = cfg.get("grad_hook") or (lambda ts: None)
+        gated = cfg["gated"]
+        views_active = g_xy is not None and Lyr > 1 and gated
+        dgates = torch.empty((Lyr, P, D), dtype=torch.float32, device=dev)
+        # ---- d v, d c (per pair) and the fc head
+        fc_w, fc_b = params[-2], params[-1]
+        d_fcw = d_fcb = da_fc = g_lg2 = None
+        g_lg = g_logits.float() if g_logits is not None else None
+        if need_scores:
+            if g_scores is None:
+                dv_in, dc_in, scale = ctx.kl_units[0], ctx.kl_units[1], g_kl
+            else:
+                _, _, dv_in, dc_in = ops.head_bwd_pairs(hL, graph, pairs, gL, v, dist, scores, kl_b, g_kl, g_scores,
+                                                        None, None, want_dh=False)
+                scale = None
+            fcw32, fcb32 = fc_w.detach().float().contiguous(), fc_b.detach().float().contiguous()
+            d_lg, da_fc, d_fcw, d_fcb = ops.fc_head_bwd(lg, fcw32, fcb32, a_raw, dv_in, dc_in, scale, parts=3)
+            d_fcw, d_fcb = d_fcw.to(fc_w.dtype), d_fcb.to(fc_b.dtype)
+            if cfg.get("dense_head") is not None and g_lg is not None:
+                g_lg2 = d_lg
+            else:
+                g_lg = d_lg if g_lg is None else g_lg + d_lg
+        # ---- classifier head backward: d a, d pooled (per pair) and the head's parameters
+        ga_head = gp_head = None
+        head_grads: List[Optional[torch.Tensor]] = [None] * ctx.n_head
+        if g_lg is not None and cfg.get("dense_head") is not None:
+            hp = cfg["head_params"]
+            ga_head, gp_head, d_hw, d_hb = ops.dense_head_bwd(g_lg, a_raw, ctx.pooled_head, hp[0], parts=3, g2=g_lg2,
+                                                              da_add=da_fc, dp_add=g_pooled)
+            da_fc = g_pooled = None
+            if hp[0].requires_grad:
+                head_grads[0] = d_hw.to(hp[0].dtype)
+            if len(hp) > 1 and hp[1].requires_grad:
+                head_grads[1] = d_hb.to(hp[1].dtype)
+        elif g_lg is not None and logits.requires_grad:
+            cap = [(i, p) for i, p in enumerate(cfg["head_params"]) if p.requires_grad]
+            res = torch.autograd.grad([logits], [a_leaf, p_leaf] + [p for _, p in cap], [g_lg.to(logits.dtype)],
+                                      allow_unused=True, retain_graph=True)
+            ga_head, gp_head = res[0], res[1]
+            for (i, _), g in zip(cap, res[2:]):
+                head_grads[i] = g
+        grad_hook([g for g in head_grads if g is not None and g.dtype == torch.float32])
+        if da_fc is not None:
+            ga_head = da_fc if ga_head is None else ga_head.float() + da_fc
+        gp_total = g_pooled
+        if gp_head is not None:
+            gp_total = gp_head.float() if gp_total is None else gp_total + gp_head.float()
+        # ---- d h_L over the sentence rows (every pair of a sentence summed in pair order), d gate_L per pair
+        if not views_active and Lyr > 1:
+            dgates[:Lyr - 1].zero_()
+        dh, _, _, _ = ops.head_bwd_pairs(hL, graph, pairs, gL, v if need_scores else None, dist,
+                                         scores if need_scores else None, kl_b, g_kl, g_scores,
+                                         gp_total.contiguous() if gp_total is not None else None, hargL, want_dh=True,
+                                         dgate_out=dgates[Lyr - 1])
+        patch_val = None
+        if views_active:
+            patch_val = ops.views_bwd_hmax_pairs(hmax1, gates, g_xy, dgates, pairs, acc_view=Lyr - 1)
+        grads_out: List[Optional[torch.Tensor]] = [None] * ctx.n_params
+        o = 2 * Lyr
+        # ---- gate MLPs (dgates complete)
+        da_gate = None
+        da_extra = None
+        if gated and P > 0:
+            dz_all = ops.sigmoid_bwd(gates.view(Lyr * P, D), dgates.view(Lyr * P, D), cd)
+            if ctx.use_chain:
+                da_extra = torch.empty((Lyr, P, D), dtype=torch.float32, device=dev)
+                dz_in = [[None] * npr for _ in range(Lyr)]
+                stages = []
+                for g in range(Lyr):
+                    acts = ctx.gate_saved[g]
+                    dz_in[g][npr - 1] = dz_all[g * P:(g + 1) * P]
+                    st = []
+                    for i in range(npr - 1, -1, -1):
+                        wt = ctx.w_t[Lyr + g * npr + i]
+                        if i > 0:
+                            out = ops.alloc_rows(P, D, cd, dev)
+                            dz_in[g][i - 1] = out
+                            st.append(dict(w=wt, y=acts[i], out=out))
+                        else:
+                            st.append(dict(w=wt, y=acts[0] if lead else None, out=da_extra[g]))
+                    stages.append(st)
+                ops.mlp_chain(1, [dz_in[g][npr - 1] for g in range(Lyr)], stages, P, D)
+                idx = [(g, i) for g in range(Lyr) for i in range(npr)]
+                for c0 in range(0, len(idx), 8):
+                    part = idx[c0:c0 + 8]
+                    dWs, dbs = ops.wgrad_batch([dz_in[g][i] for g, i in part], [ctx.gate_saved[g][i] for g, i in part],
+                                               bias_of=1)
+                    for (g, i), dW, db in zip(part, dWs, dbs):
+                        w, b = params[o + 2 * (g * npr + i)], params[o + 2 * (g * npr + i) + 1]
+                        grads_out[o + 2 * (g * npr + i)] = dW.to(w.dtype)
+                        grads_out[o + 2 * (g * npr + i) + 1] = db.to(b.dtype)
+            else:
+                for g in range(Lyr):
+                    acts = ctx.gate_saved[g]
+                    dz = dz_all[g * P:(g + 1) * P]
+                    for i in range(npr - 1, -1, -1):
+                        w, b = params[o + 2 * (g * npr + i)], params[o + 2 * (g * npr + i) + 1]
+                        dW, db = ops.wgrad(dz, acts[i], bias_of=1)
+                        grads_out[o + 2 * (g * npr + i)] = dW.to(w.dtype)
+                        grads_out[o + 2 * (g * npr + i) + 1] = db.to(b.dtype)
+                        wt = ctx.w_t[Lyr + g * npr + i]
+                        if i > 0:
+                            dz = ops.sigmoid_bwd(acts[i], ops.linear(dz, wt, None), cd)
+                        elif lead:
+                            ds = ops.linear(dz, wt, None)
+                            if da_gate is None:
+                                da_gate = ops.sigmoid_bwd(acts[0], ds, torch.float32,
+                                                          out=torch.empty((P, D), dtype=torch.float32, device=dev))
+                            else:
+                                ops.sigmoid_bwd(acts[0], ds, torch.float32, out=da_gate, accumulate=True)
+                        else:
+                            dlast = ops.linear(dz, wt, None, out_dtype=torch.float32)
+                            da_gate = dlast if da_gate is None else da_gate + dlast
+            grad_hook(grads_out[o:o + 2 * Lyr * npr])
+        elif gated:                                # no pairs: the gate parameters get zero gradients
+            for k in range(o, o + 2 * Lyr * npr):
+                grads_out[k] = torch.zeros_like(params[k])
+        # ---- the GCN chain backward on the sentence rows, exactly as for unpaired batches
+        fused = ctx.fused
+        if fused is not None:
+            rows, plan = fused
+            db_next = ops.colsum(dh)
+            du = ops.aggregate(dh, graph, mode=1)
+            for l in range(Lyr - 1, -1, -1):
+                w, b = params[2 * l], params[2 * l + 1]
+                dW, _ = ops.wgrad(hs[l - 1] if l > 0 else xr, du, bias_of=0)
+                grads_out[2 * l], grads_out[2 * l + 1] = dW.to(w.dtype), db_next.to(b.dtype)
+                grad_hook(grads_out[2 * l:2 * l + 2])
+                wk = ctx.w_n[l]
+                if l > 0:
+                    patch = (patch_val, harg1) if (l == 1 and patch_val is not None) else None
+                    du, _, _, db_next = ops.gcn_layer(du, wk, None, graph, 1, plan, rows, patch=patch, want_colsum=True)
+                else:
+                    dh = ops.linear(du, wk, None)
+        else:
+            for l in range(Lyr - 1, -1, -1):
+                if l == 0 and patch_val is not None:
+                    # the views' share of d h_1 at the sentences' arg-max rows ((row, column) targets are distinct):
+                    # edg_views_bwd_parts with one unit view adds g_pooled = patch_val at arg
+                    zero = torch.zeros((1, graph.n_graphs, D), dtype=torch.float32, device=dev)
+                    ops.views_bwd(zero, harg1.unsqueeze(0), zero + 1.0, hs[0], None, patch_val.unsqueeze(0), dh, None,
+                                  parts=1)
+                w, b = params[2 * l], params[2 * l + 1]
+                if cfg["relu"]:
+                    dh = ops.as_rows(dh * (hs[l] > 0), cd)
+                msp = ctx.ms_split[l]
+                dh2 = ops.split_rows(dh) if msp is not None else None
+                if msp is not None:
+                    dW, db = ops.wgrad_split(ops.SplitRows(ms[l], *msp), dh2, bias_of=2)
+                else:
+                    dW, db = ops.wgrad(ms[l], dh, bias_of=2)
+                grads_out[2 * l], grads_out[2 * l + 1] = dW.to(w.dtype), db.to(b.dtype)
+                grad_hook(grads_out[2 * l:2 * l + 2])
+                wk = ctx.w_n[l]
+                dm = ops.linear_split(dh2, ops.split_rows(wk), None) if msp is not None else ops.linear(dh, wk, None)
+                dh = ops.aggregate(dm, graph, mode=1)
+        dx = dh
+        # ---- d x at the trigger rows: the head's and the gate MLPs' d a of every pair, in pair order
+        da = ga_head.float() if ga_head is not None else None
+        if da_gate is not None:
+            da = da_gate if da is None else da + da_gate
+        if (da is not None or da_extra is not None) and P > 0:
+            ops.trigger_scatter_add_pairs(da, pairs, anchor, dx, extra=da_extra)
+        grads_out[-2], grads_out[-1] = d_fcw, d_fcb
+        grad_hook([g for g in (d_fcw, d_fcb) if g is not None])
+        if ctx.x_padded:
+            dx = dx.as_strided((N, dx.stride(0)), (dx.stride(0), 1))
+            if dx.shape[1] != ctx.x_cols:
+                full = torch.zeros((N, ctx.x_cols), dtype=dx.dtype, device=dev)
+                full[:, :D] = dx[:, :D]
+                dx = full
+        if dx.dtype != ctx.x_dtype:
+            dx = dx.to(ctx.x_dtype)
+        return (None, dx) + tuple(grads_out) + tuple(head_grads)
+
+
 class GatedGCNStack(nn.Module):
     """Owns gc1..gcL, gate1..gateL and fc with the reference's parameter names
     (state-dict keys ``gc1.weight``, ``gate1.1.weight``, ``fc.0.weight`` ...,
@@ -770,7 +1126,8 @@ class GatedGCNStack(nn.Module):
     def forward(self, x: torch.Tensor, graph: DepGraph, anchor_index: torch.Tensor, dist_to_target: torch.Tensor,
                 logits_fn: Callable[[torch.Tensor, torch.Tensor], torch.Tensor],
                 head_params: Sequence[torch.Tensor] = (), return_x_out: bool = False,
-                aspect: Optional[torch.Tensor] = None, view_len: Optional[torch.Tensor] = None) -> StackOutput:
+                aspect: Optional[torch.Tensor] = None, view_len: Optional[torch.Tensor] = None,
+                pairs: Optional[TriggerPairs] = None) -> StackOutput:
         """x [N,D] packed rows (or [B,T,D] with a dense-compat graph), graph, sentence-local
         trigger index [B], distances (packed [N] or [B,T] for a dense-compat graph; int32/int64),
         ``logits_fn(a [B,D], pooled [B,D]) -> [B,C]`` = the model's ``dense`` head (:643), and the
@@ -780,9 +1137,22 @@ class GatedGCNStack(nn.Module):
         LSTM output over the trigger's word pieces, bert_amir.py:118, :259) instead of taking the trigger row of ``x``;
         its gradient is returned through autograd.  ``view_len int [B]`` (optional): the two diversity pools only see the
         first ``view_len[b]`` rows of sentence b -- ``masked_fill(mask, -1e12)`` of bert_amir.py:141-142 with the
-        reference's zeros-then-ones mask (``view_len = (mask == 0).sum(1)``); the final pool stays unmasked (:146)."""
+        reference's zeros-then-ones mask (``view_len = (mask == 0).sum(1)``); the final pool stays unmasked (:146).
+
+        ``pairs`` (:class:`graph.TriggerPairs`, ``graph.pairs_from_ptr``): score every candidate trigger of a sentence
+        from ONE pass of the GCN chain.  ``x [N,D]`` and ``graph`` then hold every sentence once; ``anchor_index [P]``
+        and ``dist_to_target`` (per-pair packed, ``[pairs.n_pair_rows]``) are per (sentence, trigger) pair.  Every
+        output is per pair -- ``logits [P,C]``, ``pooled [P,D]``, ``scores [n_pair_rows]``, ``pooled_arg [P,D]`` and
+        ``view_arg [V,P,D]`` (global sentence rows) -- and ``xy`` / ``kl`` are means over the P pairs; ``logits_fn``
+        receives ``[P,D]`` inputs.  The result equals the block run on the batch with each sentence repeated once per
+        pair, ``dx`` being the sum over a sentence's pairs.  Valid only when ``x`` does not depend on the trigger
+        (no trigger marker or position features upstream).  Not covered (``EdgError``): train-mode gate dropout,
+        ``fc_sigmoid``, ``view_len``, ``aspect``, ``return_x_out`` and 3-D dense-compat ``x``."""
         if not x.is_cuda:
             raise L.EdgError("GatedGCNStack runs on CUDA tensors only (there is no CPU path)")
+        if pairs is not None:
+            return self._forward_pairs(x, graph, anchor_index, dist_to_target, logits_fn, head_params, return_x_out,
+                                       aspect, view_len, pairs)
         drop_p, seed = 0.0, None
         if self.training and self.dropout_p > 0 and self.gated:
             # nn.Dropout on the broadcast gates (bert_amir5.py:624-625).  The seed is a DEVICE scalar drawn from
@@ -817,3 +1187,50 @@ class GatedGCNStack(nn.Module):
             if x_out is not None:
                 x_out = x_out.reshape(shape3)
         return StackOutput(logits, xy, kl, scores, pooled, x_out, p_arg, v_arg)
+
+    def _forward_pairs(self, x, graph, anchor_index, dist_to_target, logits_fn, head_params, return_x_out, aspect,
+                       view_len, pairs: TriggerPairs) -> StackOutput:
+        declined = []
+        if self.training and self.dropout_p > 0 and self.gated:
+            declined.append("train-mode gate dropout (p > 0)")
+        if self.fc_sigmoid:
+            declined.append("fc_sigmoid")
+        if view_len is not None:
+            declined.append("view_len")
+        if aspect is not None:
+            declined.append("aspect")
+        if return_x_out:
+            declined.append("return_x_out")
+        if x.dim() != 2:
+            declined.append("3-D dense-compat x")
+        if self.grad_bucket_hook is not None:
+            declined.append("grad_bucket_hook (sharded grouped batches)")
+        if declined:
+            raise L.EdgError("pairs= does not cover: " + ", ".join(declined))
+        if pairs.n_sentences != graph.n_graphs:
+            raise L.EdgError(f"pairs were built for {pairs.n_sentences} sentences, the graph has {graph.n_graphs}")
+        if x.shape[0] != graph.n_rows:
+            raise L.EdgError(f"x has {x.shape[0]} rows, the graph {graph.n_rows} (pass each sentence once)")
+        if anchor_index.numel() != pairs.n_pairs:
+            raise L.EdgError(f"expected {pairs.n_pairs} anchors (one per pair), got {anchor_index.numel()}")
+        dist = dist_to_target.reshape(-1)
+        if dist.numel() != pairs.n_pair_rows:
+            raise L.EdgError(f"dist_to_target must be per-pair packed ({pairs.n_pair_rows} entries), got {dist.numel()}")
+        if dist.dtype not in (torch.int32, torch.int64):
+            dist = dist.long()
+        dist = dist.contiguous()
+        lead, npr = GATE_ARCHS[self.gate_arch]
+        if x.shape[-1] != self.hidden and x.shape[-1] != ops.row_pitch(self.hidden, x.dtype):
+            raise L.EdgError(f"expected {self.hidden} feature columns (or the padded pitch), got {x.shape[-1]}")
+        from .head import DenseHead
+        dense_head = logits_fn if isinstance(logits_fn, DenseHead) and logits_fn.fusable(self.hidden) else None
+        if isinstance(logits_fn, DenseHead):
+            head_params = [p for p in (logits_fn.weight, logits_fn.bias) if p is not None]
+        cfg = dict(graph=graph, pairs=pairs, cdtype=self.compute_dtype, D=self.hidden, dense_head=dense_head,
+                   L=self.n_layers, gate_pairs=npr, lead=lead, anchor=anchor_index.to(torch.int32).contiguous(), dist=dist,
+                   logits_fn=logits_fn, head_params=list(head_params), n_head=len(list(head_params)),
+                   grad_enabled=torch.is_grad_enabled(), grad_hook=self.grad_ready_hook, relu=self.relu,
+                   gated=self.gated, fc_sigmoid=False)
+        logits, xy, kl, scores, pooled, p_arg, v_arg = _GatedPairsFn.apply(cfg, x, *self._flat_params(),
+                                                                           *cfg["head_params"])
+        return StackOutput(logits, xy, kl, scores, pooled, None, p_arg, v_arg)

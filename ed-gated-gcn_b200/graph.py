@@ -68,6 +68,75 @@ class DepGraph:
         return plan
 
 
+@dataclass
+class TriggerPairs:
+    """(sentence, candidate trigger) pairs over the sentences of a ``DepGraph``, grouped by sentence: the pairs of
+    sentence ``s`` are ``pair_ptr[s] .. pair_ptr[s+1] - 1`` (a sentence may have none; pairs may share an anchor).
+    Per-pair row data (distances, scores) uses the per-pair packed layout: pair ``p``'s copy of its sentence's rows
+    starts at ``pair_row_ptr[p]``.  All tensors live on the graph's device.  Built by :func:`pairs_from_ptr`."""
+    pair_ptr: torch.Tensor        # int32 [S+1]
+    pair_sent: torch.Tensor       # int32 [P]   sentence of every pair
+    pair_start: torch.Tensor      # int32 [P]   = sent_ptr[pair_sent]: first packed row of the pair's sentence
+    anchor: torch.Tensor          # int32 [P]   sentence-local trigger index
+    pair_row_ptr: torch.Tensor    # int32 [P+1] offsets of the pairs' copies of their sentences
+    n_pairs: int
+    n_sentences: int
+    n_pair_rows: int
+
+    @property
+    def device(self):
+        return self.pair_ptr.device
+
+
+def pairs_from_ptr(graph: DepGraph, pair_ptr: torch.Tensor, anchor: torch.Tensor,
+                   n_pair_rows: Optional[int] = None) -> TriggerPairs:
+    """``pair_ptr`` int ``[S+1]`` (S = ``graph.n_graphs``; monotone, ``pair_ptr[0] = 0``, ``pair_ptr[S] = P``) and the
+    sentence-local ``anchor`` int ``[P]`` of every pair -> :class:`TriggerPairs`, built with torch ops on the graph's
+    device.
+
+    ``n_pair_rows`` (the sum of the pairs' sentence lengths, ``PackedBatch.n_pair_rows``) may be passed as the caller
+    knows it: the build then makes no device->host read and can be captured in a CUDA graph, like
+    ``build_graph(max_len=, max_sent_nnz=)``; device-side values of ``pair_ptr`` / ``anchor`` are then not checked
+    (host tensors still are).  Without it one small read returns ``n_pair_rows`` together with the checks: ``pair_ptr``
+    monotone from 0 to P, and every anchor inside its sentence."""
+    dev = graph.device
+    S = graph.n_graphs
+    if pair_ptr.dim() != 1 or pair_ptr.numel() != S + 1:
+        raise L.EdgError(f"pair_ptr must be int [S+1] = [{S + 1}], got {tuple(pair_ptr.shape)}")
+    if anchor.dim() != 1:
+        raise L.EdgError(f"anchor must be int [P], got {tuple(anchor.shape)}")
+    P = anchor.numel()
+    if not pair_ptr.is_cuda:                 # host-side checks cost no device read
+        pp = pair_ptr.to(torch.int64)
+        if int(pp[0]) != 0 or int(pp[-1]) != P or bool((pp[1:] < pp[:-1]).any()):
+            raise L.EdgError(f"pair_ptr must rise monotonically from 0 to P = {P}")
+    pair_ptr = _i32(pair_ptr, dev)
+    anchor = _i32(anchor, dev)
+    sp = graph.sent_ptr
+    lens = sp[1:] - sp[:-1]
+    # sentence of pair p = number of sentences whose pairs end at or before p (empty ranges included); no host read
+    idx = torch.arange(P, dtype=torch.int32, device=dev)
+    pair_sent = torch.searchsorted(pair_ptr[1:], idx, right=True, out_int32=True).clamp_(max=max(S - 1, 0))
+    if S == 0:
+        pair_sent = pair_sent[:0]
+    pair_start = sp[:-1][pair_sent.long()] if P else pair_sent.clone()
+    plen = lens[pair_sent.long()] if P else pair_sent.clone()
+    pair_row_ptr = torch.zeros(P + 1, dtype=torch.int32, device=dev)
+    if P:
+        pair_row_ptr[1:] = torch.cumsum(plen, 0, dtype=torch.int32)
+    if n_pair_rows is None:
+        bad_ptr = (pair_ptr[0] != 0) | (pair_ptr[-1] != P) | (pair_ptr[1:] < pair_ptr[:-1]).any()
+        bad_anchor = ((anchor < 0) | (anchor >= plen)).any() if P else torch.zeros((), dtype=torch.bool, device=dev)
+        host = torch.stack([pair_row_ptr[-1].long(), bad_ptr.long(), bad_anchor.long()]).cpu()   # one small read
+        n_pair_rows, bp, ba = (int(v) for v in host)
+        if bp:
+            raise L.EdgError(f"pair_ptr must rise monotonically from 0 to P = {P}")
+        if ba:
+            raise L.EdgError("a pair's anchor lies outside its sentence")
+    return TriggerPairs(pair_ptr, pair_sent.contiguous(), pair_start.contiguous(), anchor, pair_row_ptr, P, S,
+                        int(n_pair_rows))
+
+
 def _i32(t: torch.Tensor, device) -> torch.Tensor:
     return t.to(device=device, dtype=torch.int32).contiguous()
 
@@ -186,7 +255,7 @@ def graph_from_dense(adj: torch.Tensor, check: bool = True) -> DepGraph:
 
 
 def tree_distance(graph: DepGraph, anchor_index: torch.Tensor, pad: Optional[str] = None,
-                  T: Optional[int] = None) -> torch.Tensor:
+                  T: Optional[int] = None, pairs: Optional[TriggerPairs] = None) -> torch.Tensor:
     """``get_dist_to_target`` (data_utils.py:319-323) for every sentence of the batch.
 
     ``pad=None`` -> packed int32 ``[N]``.  ``pad='max+1'`` (data_utils.py:486-488) or
@@ -196,9 +265,23 @@ def tree_distance(graph: DepGraph, anchor_index: torch.Tensor, pad: Optional[str
     The kernel counts breadth-first hops.  On a graph with extra edges (``build_graph(..., extra_edges=...)``) it
     returns those hop counts; the reference's depth-first walk depends on the order it visits neighbours on a cycle and
     can over-estimate there (``tests/golden/tree_dist_cycle.npz``).  Where parity with the reference's distances
-    matters, use the items' own ``dist_to_target`` (``PackedBatch.dist``)."""
+    matters, use the items' own ``dist_to_target`` (``PackedBatch.dist``).
+
+    ``pairs`` (:class:`TriggerPairs`): ``anchor_index`` holds one anchor per pair, and the result is the per-pair packed
+    ``int32 [pairs.n_pair_rows]`` (pair p's distances start at ``pairs.pair_row_ptr[p]``); ``pad`` must be None."""
     dev = graph.device
     anchor = _i32(anchor_index, dev)
+    if pairs is not None:
+        if pad is not None:
+            raise L.EdgError("tree_distance(pairs=) returns the per-pair packed layout only (pad must be None)")
+        if anchor.numel() != pairs.n_pairs:
+            raise L.EdgError(f"expected {pairs.n_pairs} anchors (one per pair), got {anchor.numel()}")
+        dist = torch.empty(max(pairs.n_pair_rows, 1), dtype=torch.int32, device=dev)
+        with torch.cuda.device(dev):
+            L.call("edg_tree_dist_pairs", L.ptr(graph.row_ptr), L.ptr(graph.col), L.ptr(graph.sent_ptr),
+                   L.ptr(pairs.pair_sent), L.ptr(pairs.pair_row_ptr), L.ptr(anchor), pairs.n_pairs, graph.max_len,
+                   L.ptr(dist), L.stream())
+        return dist[:pairs.n_pair_rows]
     dist = torch.empty(max(graph.n_rows, 1), dtype=torch.int32, device=dev)
     with torch.cuda.device(dev):
         L.call("edg_tree_dist", L.ptr(graph.row_ptr), L.ptr(graph.col), L.ptr(graph.sent_ptr), L.ptr(anchor),

@@ -578,3 +578,81 @@ def dropout_rows(x: torch.Tensor, seed: torch.Tensor, stream_id: int, p: float, 
     L.call("edg_dropout_rows", L.ptr(x), L.dt(x), ld(x), L.ptr(out), ld(out), N, D, L.ptr(seed), int(stream_id), float(p),
            int(accumulate), L.stream())
     return out
+
+
+# ---------------------------------------------------------------------------
+# (sentence, trigger) pairs over sentence rows (graph.TriggerPairs; include/edgcn.h "Trigger pairs")
+class PairRows:
+    """The pairs seen as B = P 'sentences' starting at ``pair_start``: what ``edg_trigger_gather`` reads (``sent_ptr[b]``
+    only), so the per-pair trigger rows of the sentence rows come from the existing gather."""
+    __slots__ = ("sent_ptr", "n_graphs")
+
+    def __init__(self, pairs):
+        self.sent_ptr, self.n_graphs = pairs.pair_start, pairs.n_pairs
+
+
+def scores_kl_pairs_fwd(h, graph, pairs, gate, v, c, dist, want_units: bool = True):
+    """``edg_scores_kl_pairs_fwd`` -> ``(scores [n_pair_rows], kl_b [P], kl, dv_unit [P,D], dc_unit [P])`` (units None
+    without ``want_units``); ``kl`` is the mean over the P pairs."""
+    P, D = gate.shape
+    dev = h.device
+    R = pairs.n_pair_rows
+    scores = torch.empty((max(R, 1),), dtype=torch.float32, device=dev)[:R]
+    kl_b = torch.empty((P,), dtype=torch.float32, device=dev)
+    dvu = torch.empty((P, D), dtype=torch.float32, device=dev) if want_units else None
+    dcu = torch.empty((P,), dtype=torch.float32, device=dev) if want_units else None
+    L.call("edg_scores_kl_pairs_fwd", L.ptr(h), L.dt(h), ld(h), L.ptr(graph.sent_ptr), L.ptr(pairs.pair_sent),
+           L.ptr(pairs.pair_row_ptr), P, D, L.ptr(gate), L.ptr(v), L.ptr(c), L.ptr(dist), _dist_flag(dist), L.ptr(scores),
+           L.ptr(kl_b), L.ptr(dvu), L.ptr(dcu), None, None, L.stream())
+    kl = torch.empty((), dtype=torch.float32, device=dev)
+    L.call("edg_sum_scaled", L.ptr(kl_b), P, 1.0 / max(P, 1), L.ptr(kl), L.stream())
+    return scores, kl_b, kl, dvu, dcu
+
+
+def head_bwd_pairs(h, graph, pairs, gate, v, dist, scores, kl_b, g_kl, g_scores, g_pooled, arg, want_dh: bool,
+                   dgate_out: Optional[torch.Tensor] = None):
+    """``edg_head_bwd_pairs``.  ``want_dh``: the full pass -> ``(dh [N,D] compute dtype, dgate [P,D], None, None)``;
+    otherwise the first pass -> ``(None, None, dv [P,D], dc [P])``.  ``arg`` int32 [S,D] = the sentences' arg-max rows."""
+    P, D = gate.shape
+    N = h.shape[0]
+    dev = h.device
+    dh = alloc_rows(N, D, h.dtype, dev) if want_dh else None
+    dgate = (dgate_out if dgate_out is not None else torch.empty((P, D), dtype=torch.float32, device=dev)) \
+        if want_dh else None
+    dv = None if want_dh else torch.empty((P, D), dtype=torch.float32, device=dev)
+    dc = None if want_dh else torch.empty((P,), dtype=torch.float32, device=dev)
+    ds_ws = torch.empty((max(pairs.n_pair_rows, 1),), dtype=torch.float32, device=dev)
+    if want_dh and graph.row_sent is None:
+        raise L.EdgError("the pairs head backward needs graph.row_sent (build_graph / graph_from_dense set it)")
+    L.call("edg_head_bwd_pairs", L.ptr(h), L.dt(h), ld(h), L.ptr(graph.sent_ptr), graph.n_graphs,
+           L.ptr(graph.row_sent) if N > 0 else None, N, L.ptr(pairs.pair_ptr),
+           L.ptr(pairs.pair_sent), L.ptr(pairs.pair_row_ptr), P, D, L.ptr(gate), L.ptr(v), L.ptr(dist),
+           _dist_flag(dist) if dist is not None else 0, L.ptr(scores), L.ptr(kl_b), L.ptr(g_kl), L.ptr(g_scores),
+           L.ptr(g_pooled), L.ptr(arg), L.ptr(dh), ld(dh) if dh is not None else 0, L.ptr(dgate), L.ptr(dv), L.ptr(dc),
+           L.ptr(ds_ws), L.stream())
+    return dh, dgate, dv, dc
+
+
+def views_bwd_hmax_pairs(hmax: torch.Tensor, gates: torch.Tensor, g_xy, dgates: torch.Tensor, pairs,
+                         acc_view: int = -1) -> torch.Tensor:
+    """``edg_views_bwd_hmax_pairs``: writes ``dgates [V,P,D]`` and returns ``patch_val fp32 [S,D]`` (what the arg-max
+    rows of the sentences' d h_1 receive)."""
+    V, P, D = gates.shape
+    S = hmax.shape[0]
+    patch_val = torch.empty((S, D), dtype=torch.float32, device=hmax.device)
+    L.call("edg_views_bwd_hmax_pairs", L.ptr(hmax), L.ptr(gates), L.ptr(g_xy), V, S, L.ptr(pairs.pair_ptr), P, D,
+           L.ptr(patch_val), D, L.ptr(dgates), int(acc_view), L.stream())
+    return patch_val
+
+
+def trigger_scatter_add_pairs(da: Optional[torch.Tensor], pairs, anchor: torch.Tensor, dx: torch.Tensor,
+                              extra: Optional[torch.Tensor] = None) -> None:
+    """``dx[pair_start[p] + anchor[p]] += da[p] + extra.sum(0)[p]`` in pair order per sentence (anchors may repeat)."""
+    if extra is not None:
+        extra = _f32c(extra)
+    if da is not None:
+        da = _f32c(da)
+    P, D = (da.shape if da is not None else extra.shape[1:])
+    L.call("edg_trigger_scatter_add_pairs", L.ptr(da), L.ptr(extra), extra.shape[0] if extra is not None else 0,
+           pairs.n_sentences, L.ptr(pairs.pair_ptr), P, D, L.ptr(pairs.pair_start), L.ptr(anchor), L.ptr(dx), L.dt(dx),
+           ld(dx), L.stream())

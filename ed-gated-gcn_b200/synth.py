@@ -120,6 +120,29 @@ def with_extra_edges(batch: TreeBatch, rate: float = DEFAULT_EXTRA_RATE, seed: i
                      extra_edges=np.ascontiguousarray(rows[:, 1:]), edge_ptr=edge_ptr)
 
 
+def candidate_pairs(batch: TreeBatch, per_sentence: Optional[int] = None, none_rate: float = 0.0,
+                    seed: int = REFERENCE_SEED):
+    """(sentence, candidate trigger) pairs over ``batch``, grouped by sentence, as ``(pair_ptr int32 [B+1], anchor int32
+    [P])`` for ``graph.pairs_from_ptr``.  ``per_sentence=None``: every token of every sentence is a candidate, in token
+    order (what the LitBank reader makes, data_utils.py:456-508).  Otherwise ``per_sentence`` anchors drawn uniformly
+    with replacement (so anchors may repeat).  Each sentence gets no pairs with probability ``none_rate``; empty
+    sentences never have any.  Draws come from a generator of their own (``seed``): every seeded stream of
+    ``make_batch`` stays as it is."""
+    rng = np.random.default_rng(seed)
+    counts, anchors = [], []
+    for n in batch.lengths.tolist():
+        if n == 0 or (none_rate > 0 and rng.random() < none_rate):
+            counts.append(0)
+            continue
+        a = np.arange(n, dtype=np.int32) if per_sentence is None else rng.integers(0, n, size=per_sentence).astype(np.int32)
+        counts.append(len(a))
+        anchors.append(a)
+    pair_ptr = np.zeros(batch.n_graphs + 1, dtype=np.int32)
+    np.cumsum(np.asarray(counts, dtype=np.int32), out=pair_ptr[1:])
+    anchor = np.concatenate(anchors).astype(np.int32) if anchors else np.zeros(0, dtype=np.int32)
+    return pair_ptr, anchor
+
+
 # BASELINE.json configs (SURVEY.md 8d "Per-config shapes")
 CONFIGS = {
     "C1": dict(n_graphs=32, n_min=5, n_max=50, D=300, L=2, C=34, dtype="f32", skewed=False),

@@ -12,6 +12,10 @@ Dependency graphs that are not forests (CoreNLP enhanced dependencies add edges 
 breadth-first forest in ``heads`` plus the remaining edges, ``extra_edges`` int32[E,2] + ``edge_ptr`` int32[B+1]
 (8 bytes per extra edge; both absent when every sentence is a forest).
 
+The LitBank reader makes one item per (sentence, candidate trigger) pair, so a sentence arrives once per candidate.
+``collate_packed(..., group_sentences=True)`` sends such a sentence once, with ``pair_ptr`` int32[S+1] grouping the
+pairs by sentence; ``anchor``, ``polarity`` and ``dist`` are then per pair (``dist`` in the per-pair packed layout).
+
 ``collate_packed`` builds that from the reference's own per-sentence item dicts (host, numpy);
 ``PackedBatch.pin`` / ``.to`` move it with one small copy per field.  Host-side only: no kernels here.
 """
@@ -106,9 +110,16 @@ class PackedBatch:
     extra_edges: Optional[torch.Tensor] = None  # int32 [E,2] sentence-local (i, j), i < j: edges a head array cannot hold
     edge_ptr: Optional[torch.Tensor] = None     # int32 [B+1] pairs of sentence b; both None when no sentence has one
     max_sent_nnz: int = 0               # largest CSR entry count of one sentence: n_b + 2 (forest edges) + 2 E_b
+    pair_ptr: Optional[torch.Tensor] = None    # int32 [S+1] pairs of sentence s (grouped batches; None otherwise)
+    n_pair_rows: int = 0                # grouped batches: sum over the pairs of their sentence's length (= dist rows)
 
     @property
     def n_graphs(self) -> int:
+        """Sentences of the batch (= items unless grouped)."""
+        return self.anchor.numel() if self.pair_ptr is None else self.sent_ptr.numel() - 1
+
+    @property
+    def n_pairs(self) -> int:
         return self.anchor.numel()
 
     @property
@@ -134,17 +145,55 @@ class PackedBatch:
         return self._map(lambda t: t.to(device, non_blocking=non_blocking))
 
 
-def collate_packed(items: Sequence[dict], with_dist: bool = True, with_transform: bool = True) -> PackedBatch:
+def _sentence_key(it: dict):
+    """What makes two items the same sentence: length, word-piece ids and the adjacency pattern.  None for an item
+    without ``cls_text_sep_indices`` (never grouped)."""
+    if "cls_text_sep_indices" not in it:
+        return None
+    n = int(it["sentence_length"])
+    m = int(it.get("cls_text_sep_length", len(it["cls_text_sep_indices"])))
+    ids = np.asarray(it["cls_text_sep_indices"])[:m]
+    return n, m, ids, np.asarray(it["dependency_graph"])[:n, :n] != 0
+
+
+def _same_sentence(a, b) -> bool:
+    return (a is not None and b is not None and a[0] == b[0] and a[1] == b[1] and np.array_equal(a[2], b[2])
+            and np.array_equal(a[3], b[3]))
+
+
+def collate_packed(items: Sequence[dict], with_dist: bool = True, with_transform: bool = True,
+                   group_sentences: bool = False) -> PackedBatch:
     """The packed counterpart of ``collate_fn`` (data_utils.py:381-402) over the same item dicts
     (keys ``dependency_graph``, ``anchor_index``, ``sentence_length``, ``dist_to_target``, ``transform``,
-    ``cls_text_sep_length``, ``polarity``; data_utils.py:362-379)."""
+    ``cls_text_sep_length``, ``polarity``; data_utils.py:362-379).
+
+    ``group_sentences=True``: CONSECUTIVE items holding the same sentence (equal ``sentence_length``,
+    ``cls_text_sep_length``, ``cls_text_sep_indices[:length]`` and non-zero pattern of ``dependency_graph[:n, :n]``)
+    become one sentence with several (sentence, trigger) pairs; items without ``cls_text_sep_indices`` are never
+    merged.  Pairs keep the item order, so per-pair outputs line up with the items.  Sentence-level fields (heads,
+    sent_ptr, extra edges, word-piece segments, max_len) then hold each sentence once; ``anchor`` and ``polarity`` are
+    per pair, ``dist`` is per-pair packed, and ``pair_ptr`` groups the pairs (see ``graph.pairs_from_ptr``)."""
     heads: List[np.ndarray] = []
     extras: List[np.ndarray] = []
     lens, anchors, dists, pols = [], [], [], []
     seg_s, seg_n, piece_ptr = [], [], [0]
     max_sent_nnz = 0
+    pair_counts: List[int] = []
+    prev_key = None
     for it in items:
         n = int(it["sentence_length"])
+        if group_sentences:
+            key = _sentence_key(it)
+            if pair_counts and _same_sentence(prev_key, key):
+                pair_counts[-1] += 1
+                anchors.append(int(it["anchor_index"]))
+                if with_dist and "dist_to_target" in it:
+                    dists.append(np.asarray(it["dist_to_target"][:n], dtype=np.int32))
+                if "polarity" in it:
+                    pols.append(int(it["polarity"]))
+                continue
+            prev_key = key
+            pair_counts.append(1)
         h, x = split_adjacency(it["dependency_graph"], n)
         heads.append(h)
         extras.append(x)
@@ -161,23 +210,31 @@ def collate_packed(items: Sequence[dict], with_dist: bool = True, with_transform
             seg_n.append(l)
             n_pieces = int(it["cls_text_sep_length"]) if "cls_text_sep_length" in it else int((s + l).max(initial=0)) + 1
             piece_ptr.append(piece_ptr[-1] + n_pieces)
-    sent_ptr = np.zeros(len(items) + 1, dtype=np.int32)
+    S = len(lens)
+    sent_ptr = np.zeros(S + 1, dtype=np.int32)
     np.cumsum(np.asarray(lens, dtype=np.int32), out=sent_ptr[1:])
     t = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dtype=dt))
     cat = lambda xs, dt: t(np.concatenate(xs) if xs else np.zeros(0, dtype=dt), dt)
     n_extra = np.asarray([len(x) for x in extras], dtype=np.int32)
     edge_ptr = None
     if n_extra.sum() > 0:
-        edge_ptr = np.zeros(len(items) + 1, dtype=np.int32)
+        edge_ptr = np.zeros(S + 1, dtype=np.int32)
         np.cumsum(n_extra, out=edge_ptr[1:])
+    pair_ptr = None
+    n_pair_rows = 0
+    if group_sentences:
+        pair_ptr = np.zeros(S + 1, dtype=np.int32)
+        np.cumsum(np.asarray(pair_counts, dtype=np.int32), out=pair_ptr[1:])
+        n_pair_rows = int(np.dot(np.asarray(lens, dtype=np.int64), np.asarray(pair_counts, dtype=np.int64))) if S else 0
     return PackedBatch(
         heads=cat(heads, np.int32), sent_ptr=t(sent_ptr, np.int32), anchor=t(np.asarray(anchors), np.int32),
         dist=cat(dists, np.int32) if len(dists) == len(items) and items else None,
         polarity=t(np.asarray(pols), np.int64) if len(pols) == len(items) and items else None,
-        seg_start=cat(seg_s, np.int32) if len(seg_s) == len(items) and items else None,
-        seg_len=cat(seg_n, np.int32) if len(seg_n) == len(items) and items else None,
-        piece_ptr=t(np.asarray(piece_ptr), np.int32) if len(seg_s) == len(items) and items else None,
+        seg_start=cat(seg_s, np.int32) if len(seg_s) == S and items else None,
+        seg_len=cat(seg_n, np.int32) if len(seg_n) == S and items else None,
+        piece_ptr=t(np.asarray(piece_ptr), np.int32) if len(seg_s) == S and items else None,
         max_len=int(max(lens)) if lens else 0,
         extra_edges=t(np.concatenate(extras), np.int32) if edge_ptr is not None else None,
         edge_ptr=t(edge_ptr, np.int32) if edge_ptr is not None else None,
-        max_sent_nnz=max_sent_nnz)
+        max_sent_nnz=max_sent_nnz,
+        pair_ptr=t(pair_ptr, np.int32) if pair_ptr is not None else None, n_pair_rows=n_pair_rows)

@@ -538,6 +538,54 @@ int edg_loss_combine(const float* t0, const float* t1, const float* t2, float w0
                      edg_stream stream);
 int edg_loss_combine_bwd(const float* g, float w0, float w1, float w2, float* out3, edg_stream stream);
 
+/* ---- Trigger pairs: every candidate trigger of a sentence from one pass of the GCN chain ----------------------------
+ * The LitBank reader makes one example per (sentence, candidate trigger) pair; the GCN chain h_1 .. h_L depends on the
+ * sentence only (its input x carries no trigger marker), so the sentence's rows are run once and only what depends on
+ * the trigger runs per pair.  S sentences own rows [sent_ptr[s], sent_ptr[s+1]); the P pairs are grouped by sentence,
+ * pairs of sentence s = [pair_ptr[s], pair_ptr[s+1]) (a sentence may have none); pair_sent[P] names each pair's
+ * sentence, pair_start[P] = sent_ptr[pair_sent], anchor[P] is sentence-local.  Per-pair row data (distances, scores)
+ * lives in the per-pair packed layout: pair p's copy of its sentence's n rows starts at pair_row_ptr[p] (P+1 entries).
+ * Every sum over the pairs of a sentence runs in ascending pair order in one thread: results are deterministic.
+ * The forward trigger gather is edg_trigger_gather with sent_ptr = pair_start and B = P. */
+
+/* edg_tree_dist per pair: pair p walks sentence pair_sent[p] from anchor[p]; dist[pair_row_ptr[P]] is per-pair packed. */
+int edg_tree_dist_pairs(const int32_t* row_ptr, const int32_t* col, const int32_t* sent_ptr, const int32_t* pair_sent,
+                        const int32_t* pair_row_ptr, const int32_t* anchor, int32_t P, int32_t max_len, int32_t* dist,
+                        edg_stream stream);
+/* edg_scores_kl_fwd per pair over the sentence rows h [N, ldh]: gate, v fp32 [P,D], c fp32 [P] (NULL = 0), dist per-pair
+ * packed; scores [pair_row_ptr[P]], kl_b [P]; optional dv_unit [P,D], dc_unit [P], u_unit [pair_row_ptr[P]],
+ * sf_unit [P,D] as in edg_scores_kl_fwd with the mean taken over the P pairs (u_t = P_t (Q_t - kl_b) / P).
+ * A pair whose sentence is empty gets kl_b 0 and zero unit outputs. */
+int edg_scores_kl_pairs_fwd(const void* h, int dtype, int64_t ldh, const int32_t* sent_ptr, const int32_t* pair_sent,
+                            const int32_t* pair_row_ptr, int32_t P, int32_t D, const float* gate, const float* v,
+                            const float* c, const void* dist, int dist_i64, float* scores, float* kl_b, float* dv_unit,
+                            float* dc_unit, float* u_unit, float* sf_unit, edg_stream stream);
+/* Backward of the per-pair scores / kl and the final pool (pooled_p = gate_p * max_t h_t), same two-pass contract as
+ * edg_head_bwd.  With ds_{p,t} = g_kl / P * P_{p,t} (Q_{p,t} - kl_b[p]) + g_scores[pair_row_ptr[p] + t]:
+ *   first pass (dh = dgate = NULL): dv_p = gate_p * sum_t ds_{p,t} h_t, dc_p = sum_t ds_{p,t};
+ *   full pass: dh [N, lddh] (compute dtype, every row written)
+ *     dh_t = sum_{p of s} ds_{p,t} (gate_p * v_p) + [t = arg[s]] sum_{p of s} gate_p * g_pooled_p,
+ *   dgate_p = v_p * sum_t ds_{p,t} h_t + g_pooled_p * h[arg[s]], and dv / dc when given.
+ * arg int32 [S,D] = the sentence's global arg-max rows (-1 for an empty sentence), g_pooled fp32 [P,D] (NULL = 0).
+ * ds_ws: fp32 workspace of pair_row_ptr[P] entries.  row_sent[N] (sentence of every row) is needed for dh. */
+int edg_head_bwd_pairs(const void* h, int dtype, int64_t ldh, const int32_t* sent_ptr, int32_t S, const int32_t* row_sent,
+                       int32_t N, const int32_t* pair_ptr,
+                       const int32_t* pair_sent, const int32_t* pair_row_ptr, int32_t P, int32_t D, const float* gate,
+                       const float* v, const void* dist, int dist_i64, const float* scores, const float* kl_b,
+                       const float* g_kl, const float* g_scores, const float* g_pooled, const int32_t* arg, void* dh,
+                       int64_t lddh, float* dgate, float* dv, float* dc, float* ds_ws, edg_stream stream);
+/* edg_views_bwd_hmax per pair: gates / dgates [V,P,D], hmax [S,D] of the sentences;
+ *   patch_val[s,d] = sum_{p of s} sum_v gates[v,p,d] dP_{v,p},  dgates[v,p,d] (+)= dP_{v,p} * hmax[s,d]
+ * with dP_{v,p} = g_xy / P * sum_{v' != v} gates[v',p,d] * hmax[s,d].  A sentence without pairs gets patch_val 0. */
+int edg_views_bwd_hmax_pairs(const float* hmax, const float* gates, const float* g_xy, int32_t V, int32_t S,
+                             const int32_t* pair_ptr, int32_t P, int32_t D, float* patch_val, int64_t ldp, float* dgates,
+                             int acc_view, edg_stream stream);
+/* edg_trigger_scatter_add per pair: dx[pair_start[p] + anchor[p]] += da[p] + sum_k extra[k][p], the pairs of a
+ * sentence in ascending order (pairs may share a row). */
+int edg_trigger_scatter_add_pairs(const float* da, const float* extra, int32_t n_extra, int32_t S, const int32_t* pair_ptr,
+                                  int32_t P, int32_t D, const int32_t* pair_start, const int32_t* anchor, void* dx,
+                                  int dtype, int64_t lddx, edg_stream stream);
+
 #ifdef __cplusplus
 }
 #endif
