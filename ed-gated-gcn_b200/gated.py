@@ -18,6 +18,7 @@ reference block.  CUDA only; no fallback.
 """
 from __future__ import annotations
 
+import contextlib
 import os
 from collections import namedtuple
 from typing import Callable, List, Optional, Sequence
@@ -26,11 +27,11 @@ import torch
 import torch.nn as nn
 
 from . import _lib as L
-from . import ops
+from . import gcn, ops
 from .gcn import GraphConvolution, _compute_dtype
 from .graph import DepGraph, TriggerPairs
 
-# name -> (leading Sigmoid?, number of (Linear, Sigmoid) pairs); SURVEY 8a variant matrix
+# name -> (leading Sigmoid?, Linears per gate, each followed by a Sigmoid); SURVEY 8a variant matrix
 GATE_ARCHS = {
     "sig-2": (True, 2),     # BertAmir52/53/54/55   bert_amir5.py:562-571
     "2": (False, 2),        # BertAmir5/51          bert_amir5.py:27-30
@@ -40,11 +41,11 @@ GATE_ARCHS = {
 
 
 
-def _chain_ok(cd: torch.dtype, D: int, n_gates: int, pairs: int) -> bool:
+def _chain_ok(cd: torch.dtype, D: int, n_gates: int, gate_linears: int) -> bool:
     """The fused gate-MLP kernel (``edg_mlp_chain``) covers bf16, D <= 320, <= 4 gates, <= 3 Linears per gate;
     everything else runs one ``edg_linear`` per layer.  EDG_MLP_CHAIN=0 forces the per-layer kernels (bring-up)."""
     return (cd == torch.bfloat16 and 16 <= D <= ops.MLP_CHAIN_MAX_D and n_gates <= ops.MLP_CHAIN_MAX_GROUPS
-            and pairs <= ops.MLP_CHAIN_MAX_STAGES and os.environ.get("EDG_MLP_CHAIN", "1") != "0")
+            and gate_linears <= ops.MLP_CHAIN_MAX_STAGES and os.environ.get("EDG_MLP_CHAIN", "1") != "0")
 
 
 # Opt-in (EDG_VIEWS_PATCH=1): the views' backward folded into the adjoint aggregation (edg_views_patch +
@@ -131,7 +132,6 @@ class _Side:
         self.dirty = False
 
     def region(self):
-        import contextlib
         if not self.enabled:
             return contextlib.nullcontext()
         self.side.wait_stream(self.main)
@@ -165,46 +165,314 @@ StackOutput = namedtuple("StackOutput", ["logits", "xy", "kl", "scores", "pooled
 
 
 def make_gate(D: int, arch: str) -> nn.Sequential:
-    lead, pairs = GATE_ARCHS[arch]
+    lead, gate_linears = GATE_ARCHS[arch]
     mods: List[nn.Module] = [nn.Sigmoid()] if lead else []
-    for _ in range(pairs):
+    for _ in range(gate_linears):
         mods += [nn.Linear(D, D), nn.Sigmoid()]
     return nn.Sequential(*mods)
 
 
+def _f32(t):
+    return None if t is None else t.detach().float().contiguous()
+
+
+def _x_rows(ctx, x: torch.Tensor, D: int, cd: torch.dtype) -> torch.Tensor:
+    """x is [N, D], or the whole padded allocation [N, pitch >= D] (then dx comes back in the same dense layout and
+    autograd can keep it without a copy): the compute-dtype rows, with what :func:`_dx_like_x` needs kept on ``ctx``."""
+    ctx.x_padded, ctx.x_cols, ctx.x_dtype = x.shape[1] != D, x.shape[1], x.dtype
+    return ops.as_rows(x[:, :D] if ctx.x_padded else x, cd)
+
+
+def _dx_like_x(ctx, dx: torch.Tensor) -> torch.Tensor:
+    """dx in the caller's layout: with a padded x, the whole [N, pitch] allocation (padding columns are finite)."""
+    if ctx.x_padded:
+        N, D = dx.shape
+        dx = dx.as_strided((N, dx.stride(0)), (dx.stride(0), 1))
+        if dx.shape[1] != ctx.x_cols:
+            full = torch.zeros((N, ctx.x_cols), dtype=dx.dtype, device=dx.device)
+            full[:, :D] = dx[:, :D]
+            dx = full
+    return dx if dx.dtype == ctx.x_dtype else dx.to(ctx.x_dtype)
+
+
+def _param_groups(params, n_layers: int, gate_linears: int):
+    """The block's parameter inputs -> (per layer (weight, bias), per gate per Linear (weight, bias) gate by gate,
+    fc.weight, fc.bias)."""
+    o = 2 * n_layers
+    gate_p = [(params[k], params[k + 1]) for k in range(o, o + 2 * n_layers * gate_linears, 2)]
+    return [(params[2 * l], params[2 * l + 1]) for l in range(n_layers)], gate_p, params[-2], params[-1]
+
+
+def _unpack(params, cfg):
+    """The Function's parameter inputs (the block's, then the classifier head's, whose gradients backward returns) ->
+    (the block's parameters, GCN (weight, bias) per layer, gate (weight, bias) per Linear, fc.weight, fc.bias, w_t,
+    w_n).  w_t / w_n are every compute-dtype weight copy of the step, transposed and in the same orientation (forward
+    and backward operands), cast in one launch: the GCN layers' first, then the gates' in ``gate_p`` order."""
+    n_head = cfg["n_head"]
+    params = params[:len(params) - n_head] if n_head else params
+    gcn_p, gate_p, fc_w, fc_b = _param_groups(params, cfg["L"], cfg["gate_linears"])
+    flat_w = [w for (w, _) in gcn_p] + [w for (w, _) in gate_p]
+    casted = ops.cast_weights_batch([(w, True) for w in flat_w] + [(w, False) for w in flat_w], cfg["cdtype"])
+    nW = len(flat_w)
+    return params, gcn_p, gate_p, fc_w, fc_b, casted[:nW], casted[nW:]
+
+
+def _gates_fwd(s0, gate_p, w_n, gates: torch.Tensor, cd: torch.dtype, use_chain: bool):
+    """The gate MLPs (bert_amir5.py:562-571) on ``s0 [M,D]``, the trigger rows after the leading Sigmoid of the
+    architectures that have one: gate g's last Sigmoid writes ``gates[g]`` (fp32 ``[L,M,D]``).  ``gate_p`` / ``w_n``:
+    the gates' parameters and same-orientation weights, gate by gate.  Returns per gate the inputs of its Linears."""
+    Lyr, M, D = gates.shape
+    n = len(gate_p) // Lyr
+    saved = []
+    if use_chain:
+        # every Linear+Sigmoid of every gate in ONE launch (activation tile resident in shared memory)
+        stages = []
+        for g in range(Lyr):
+            acts, st = [s0], []
+            for i in range(n):
+                last = i == n - 1
+                out = gates[g] if last else ops.alloc_rows(M, D, cd, s0.device)
+                st.append(dict(w=w_n[g * n + i], bias=_f32(gate_p[g * n + i][1]), out=out))
+                if not last:
+                    acts.append(out)
+            stages.append(st)
+            saved.append(acts)
+        ops.mlp_chain(0, [s0] * Lyr, stages, M, D)
+        return saved
+    for g in range(Lyr):
+        s, acts = s0, [s0]
+        for i in range(n):
+            last = i == n - 1                                           # nn.Linear [out,in] is K-major
+            s = ops.linear(s, w_n[g * n + i], _f32(gate_p[g * n + i][1]), act=L.ACT_SIGMOID,
+                           out_dtype=torch.float32 if last else cd, out=gates[g] if last else None)
+            if not last:
+                acts.append(s)
+        saved.append(acts)
+    return saved
+
+
+def _gates_bwd(gates, dgates, saved, gate_p, w_t, lead: bool, cd: torch.dtype, use_chain: bool, grad_hook):
+    """Backward of :func:`_gates_fwd` from the complete ``dgates``.  Returns ``(da_gate [M,D] or None, da_extra [L,M,D]
+    or None, the gate parameters' gradients in parameter order)``: the gates' input gradients come back summed
+    (``da_gate``, per-layer kernels) or as one slab per gate (``da_extra``, summed where it is consumed)."""
+    Lyr, M, D = gates.shape
+    n = len(gate_p) // Lyr
+    dev = gates.device
+    grads: List[Optional[torch.Tensor]] = [None] * (2 * len(gate_p))
+
+    def put(g, i, dW, db):
+        w, b = gate_p[g * n + i]
+        grads[2 * (g * n + i)], grads[2 * (g * n + i) + 1] = dW.to(w.dtype), db.to(b.dtype)
+
+    # the last Sigmoid of every gate in one launch (gates / dgates are [V*M, D] row blocks)
+    dz_all = ops.sigmoid_bwd(gates.view(Lyr * M, D), dgates.view(Lyr * M, D), cd)
+    da_gate = da_extra = None
+    if use_chain:
+        # d z chain of every gate in ONE launch, then every weight gradient in batched launches
+        da_extra = torch.empty((Lyr, M, D), dtype=torch.float32, device=dev)
+        dz_in = [[None] * n for _ in range(Lyr)]          # gradient at the pre-activation output of Linear i
+        stages = []
+        for g in range(Lyr):
+            acts = saved[g]
+            dz_in[g][n - 1] = dz_all[g * M:(g + 1) * M]
+            st = []
+            for i in range(n - 1, -1, -1):
+                wt = w_t[g * n + i]                                     # [in,out]: row n = input column n
+                if i > 0:
+                    out = ops.alloc_rows(M, D, cd, dev)
+                    dz_in[g][i - 1] = out
+                    st.append(dict(w=wt, y=acts[i], out=out))
+                else:
+                    st.append(dict(w=wt, y=acts[0] if lead else None, out=da_extra[g]))
+            stages.append(st)
+        ops.mlp_chain(1, [dz_in[g][n - 1] for g in range(Lyr)], stages, M, D)
+        idx = [(g, i) for g in range(Lyr) for i in range(n)]
+        for c0 in range(0, len(idx), 8):
+            part = idx[c0:c0 + 8]
+            dWs, dbs = ops.wgrad_batch([dz_in[g][i] for g, i in part], [saved[g][i] for g, i in part], bias_of=1)
+            for (g, i), dW, db in zip(part, dWs, dbs):
+                put(g, i, dW, db)
+    else:
+        for g in range(Lyr):
+            acts = saved[g]
+            dz = dz_all[g * M:(g + 1) * M]
+            for i in range(n - 1, -1, -1):
+                put(g, i, *ops.wgrad(dz, acts[i], bias_of=1))            # [out,in], [out]
+                wt = w_t[g * n + i]                                      # [in,out]
+                if i > 0:
+                    dz = ops.sigmoid_bwd(acts[i], ops.linear(dz, wt, None), cd)
+                elif lead:
+                    ds = ops.linear(dz, wt, None)
+                    if da_gate is None:
+                        da_gate = ops.sigmoid_bwd(acts[0], ds, torch.float32,
+                                                  out=torch.empty((M, D), dtype=torch.float32, device=dev))
+                    else:
+                        ops.sigmoid_bwd(acts[0], ds, torch.float32, out=da_gate, accumulate=True)
+                else:
+                    dlast = ops.linear(dz, wt, None, out_dtype=torch.float32)
+                    da_gate = dlast if da_gate is None else da_gate + dlast
+    grad_hook(grads)
+    return da_gate, da_extra, grads
+
+
+def _head_fwd(ctx, a_raw, pooled, a_fc, fc_w, fc_b):
+    """Classifier head: ``logits_fn`` is the model's own dense head (host torch, :643); a head.DenseHead (= the
+    reference's nn.Linear on cat[a, pooled]) is run by the block's own kernels: no inner autograd graph, its weight and
+    bias are head_params[0:2].  Then the per-row operands of the collapsed scores, [v_b | va_b] = logits_b @ fc.weight
+    and c_b = a_b . va_b + logits_b . fc.bias  (= logits_b . (Wfc[:, D:] a_b + bfc), SURVEY A9), in one kernel.
+    Returns (logits, v, c); what :func:`_head_bwd` reads stays on ``ctx``."""
+    cfg = ctx.cfg
+    dense_head = cfg.get("dense_head")
+    a_leaf = p_leaf = None
+    if dense_head is not None:
+        hp = cfg["head_params"]
+        logits = ops.dense_head_fwd(a_raw, pooled, hp[0], hp[1] if len(hp) > 1 else None)
+    else:
+        with torch.enable_grad():
+            a_leaf = a_raw.detach().requires_grad_(True)
+            p_leaf = pooled.detach().requires_grad_(True)
+            logits = cfg["logits_fn"](a_leaf, p_leaf)
+        if logits.requires_grad and cfg["grad_enabled"]:
+            _check_head_leaves(logits, (a_leaf, p_leaf), cfg["head_params"])
+    lg = logits.detach().float().contiguous()
+    v, c = ops.fc_head_fwd(lg, _f32(fc_w), _f32(fc_b), a_fc)
+    ctx.head = (a_leaf, p_leaf, logits, lg, a_raw, v)
+    # (detached alias: `pooled` itself is an output of this node, and an output stored on its own node is a reference
+    # cycle that keeps the whole graph -- and its AccumulateGrad nodes with their stream -- alive until the cyclic GC)
+    ctx.pooled_head = pooled.detach() if dense_head is not None else None
+    return logits, v, c
+
+
+def _head_bwd(ctx, g_logits, g_pooled, dvc, fc_w, fc_b, side: Optional[_Side], grad_hook):
+    """Backward of :func:`_head_fwd`.  ``dvc = (d v, d c, scale)`` when the scores carry gradient (else None): the fc
+    head's backward adds its d logits to ``g_logits``, then the classifier head's backward gives d a, d pooled and the
+    head parameters' gradients.  With ``side``, each launch runs as parts=1 here and parts=2 (the parameter gradients,
+    which nothing downstream waits for) in ``side``'s region, where ``grad_hook`` receives them; with ``side=None`` each
+    runs once as parts=3 and the caller hands the gradients on.
+    Returns (d a or None, d pooled or None, d fc.weight, d fc.bias, head parameter gradients)."""
+    cfg = ctx.cfg
+    a_leaf, p_leaf, logits, lg, a_raw, v = ctx.head
+    dense = cfg.get("dense_head") is not None
+    region = side.region if side is not None else contextlib.nullcontext
+    d_fcw = d_fcb = da_fc = g_lg2 = None
+    g_lg = g_logits.float() if g_logits is not None else None
+    if dvc is not None:
+        # backward of [v | va] = logits @ fc.weight, c = a . va + logits . fc.bias  (one kernel + a reduction)
+        a_fc = ctx.fc_sig[2] if ctx.fc_sig else a_raw
+        fcw32, fcb32 = _f32(fc_w), _f32(fc_b)
+        d_lg, da_fc, d_fcw, d_fcb = ops.fc_head_bwd(lg, fcw32, fcb32, a_fc, *dvc, parts=3 if side is None else 1)
+        with region():
+            if side is not None:
+                _, _, d_fcw, d_fcb = ops.fc_head_bwd(lg, fcw32, fcb32, a_fc, *dvc, parts=2)
+            d_fcw, d_fcb = d_fcw.to(fc_w.dtype), d_fcb.to(fc_b.dtype)
+            if side is not None:
+                grad_hook([d_fcw, d_fcb])
+        if ctx.fc_sig:
+            da_fc = da_fc * a_fc * (1.0 - a_fc)                   # through sigmoid(a)
+        if dense and g_lg is not None:
+            g_lg2 = d_lg                      # the fused head adds the two d logits terms while it loads them
+        else:
+            g_lg = d_lg if g_lg is None else g_lg + d_lg
+    # ---- classifier head backward: d a, d pooled, and .grad of the parameters it closes over
+    ga_head = gp_head = None
+    head_grads: List[Optional[torch.Tensor]] = [None] * ctx.n_head
+    if g_lg is not None and dense:
+        hp = cfg["head_params"]
+        # d a and d pooled leave with everything else that flows into a / pooled already added (da_fc, g_pooled)
+        ga_head, gp_head, d_hw, d_hb = ops.dense_head_bwd(g_lg, a_raw, ctx.pooled_head, hp[0],
+                                                          parts=3 if side is None else 1, g2=g_lg2,
+                                                          da_add=da_fc, dp_add=g_pooled)
+        da_fc = g_pooled = None
+        with region():
+            if side is not None:
+                _, _, d_hw, d_hb = ops.dense_head_bwd(g_lg, a_raw, ctx.pooled_head, hp[0], parts=2, g2=g_lg2)
+            if hp[0].requires_grad:
+                head_grads[0] = d_hw.to(hp[0].dtype)
+            if len(hp) > 1 and hp[1].requires_grad:
+                head_grads[1] = d_hb.to(hp[1].dtype)
+            if side is not None:
+                grad_hook([g for g in head_grads if g is not None and g.dtype == torch.float32])
+    elif g_lg is not None and logits.requires_grad:
+        cap = [(i, p) for i, p in enumerate(cfg["head_params"]) if p.requires_grad]
+        res = torch.autograd.grad([logits], [a_leaf, p_leaf] + [p for _, p in cap], [g_lg.to(logits.dtype)],
+                                  allow_unused=True, retain_graph=True)
+        ga_head, gp_head = res[0], res[1]
+        for (i, _), g in zip(cap, res[2:]):
+            head_grads[i] = g
+        if side is not None:
+            grad_hook([g for g in head_grads if g is not None and g.dtype == torch.float32])
+    if da_fc is not None:
+        ga_head = da_fc if ga_head is None else ga_head.float() + da_fc
+    gp_total = g_pooled
+    if gp_head is not None:
+        gp_total = gp_head.float() if gp_total is None else gp_total + gp_head.float()
+    return ga_head, gp_total, d_fcw, d_fcb, head_grads
+
+
+def _layer_fwd(h, wt, b, graph: DepGraph, cd: torch.dtype, relu: bool, fused, want_pool: bool):
+    """One layer of the GCN chain -> (h_l, saved rows, split metadata, column maxima, their rows).  ``fused``: one
+    ``edg_gcn_layer`` launch, h_l = A^ (h_{l-1} W_l) + b_l with the column maxima of every sentence (and their first
+    rows) from the epilogue when ``want_pool`` -- the aggregated rows and the pooling passes never touch HBM.
+    Otherwise aggregate -> projection (:func:`gcn.layer_fwd`), with no maxima."""
+    if fused is not None:
+        rows, plan = fused
+        h, hm, ha, _ = ops.gcn_layer(h, wt, _f32(b), graph, 0, plan, rows, want_pool=want_pool)
+        return h, None, None, hm, ha
+    m = ops.aggregate(h, graph, mode=0)
+    h, m, split = gcn.layer_fwd(m, wt, _f32(b), cd, L.ACT_RELU if relu else L.ACT_NONE)
+    return h, m, split, None, None
+
+
+def _unfused_layer_bwd(ctx, l: int, dh, hs, ms, params, grads_out, grad_hook, side_w: _Side):
+    """Layer l of the unfused chain backward from d h_l: the ReLU mask, the weight gradient (in ``side_w``'s region,
+    handed to ``grad_hook``) and d h_l W_l^T, which the caller aggregates with A^T."""
+    w, b = params[2 * l], params[2 * l + 1]
+    if ctx.cfg["relu"]:
+        dh = ops.as_rows(dh * (hs[l] > 0), ctx.cfg["cdtype"])
+    split = ctx.ms_split[l]
+    dh2 = gcn.layer_dy_split(dh, split)                                 # shared by dW and the input gradient
+    with side_w.region():
+        dW, db = gcn.layer_wgrad(ms[l], split, dh, dh2, bias_of=2)
+        grads_out[2 * l], grads_out[2 * l + 1] = dW.to(w.dtype), db.to(b.dtype)
+        grad_hook(grads_out[2 * l:2 * l + 2])
+    return gcn.layer_dgrad(dh, dh2, ctx.w_n[l])                          # w_n[l] [in,out] = B operand of dh W^T
+
+
+def _fused_chain_bwd(ctx, du, db_next, xr, hs, params, grads_out, grad_hook, patch=None, patch_ready=None):
+    """The fused chain backward from du_L = A^T dh_L and db_L.  With u_l = h_{l-1} W_l and h_l = A^ u_l + b_l:
+    db_l = colsum(dh_l), du_l = A^T dh_l, dW_l = h_{l-1}^T du_l, dh_{l-1} = du_l W_l^T.  One fused launch per layer
+    produces du_{l-1} = A^T (du_l W_l^T + views patch) and the column sums of its argument (= db_{l-1}); neither
+    dh_{l-1} nor the aggregated rows exist in HBM.  ``patch`` (the views' share of d h_1) enters the layer-1 launch,
+    after ``patch_ready`` when given.  Returns du_1 once the weight gradient of layer 1 is handed to ``grad_hook``:
+    dx = du_1 W_1^T is the caller's."""
+    rows, plan = ctx.fused
+    graph = ctx.cfg["graph"]
+    for l in range(len(hs) - 1, -1, -1):
+        w, b = params[2 * l], params[2 * l + 1]
+        dW, _ = ops.wgrad(hs[l - 1] if l > 0 else xr, du, bias_of=0)
+        grads_out[2 * l], grads_out[2 * l + 1] = dW.to(w.dtype), db_next.to(b.dtype)
+        grad_hook(grads_out[2 * l:2 * l + 2])
+        if l > 0:
+            if l == 1 and patch_ready is not None:
+                torch.cuda.current_stream(xr.device).wait_event(patch_ready)
+            du, _, _, db_next = ops.gcn_layer(du, ctx.w_n[l], None, graph, 1, plan, rows,
+                                              patch=patch if l == 1 else None, want_colsum=True)
+    return du
+
+
 class _GatedStackFn(torch.autograd.Function):
-    """inputs: x, then per layer (weight, bias), then per gate per pair (weight, bias),
+    """inputs: x, then per layer (weight, bias), then per gate per Linear (weight, bias),
     then fc.weight, fc.bias.  ``cfg`` carries the non-tensor arguments."""
 
     @staticmethod
     def forward(ctx, cfg, x, aspect, *params):
         graph: DepGraph = cfg["graph"]
         cd: torch.dtype = cfg["cdtype"]
-        Lyr, pairs, lead = cfg["L"], cfg["pairs"], cfg["lead"]
-        anchor, dist, logits_fn = cfg["anchor"], cfg["dist"], cfg["logits_fn"]
-        D = cfg["D"]
-        B, N = graph.n_graphs, graph.n_rows
-        gcn_p = [(params[2 * l], params[2 * l + 1]) for l in range(Lyr)]
-        o = 2 * Lyr
-        gate_p = [[(params[o + 2 * (g * pairs + i)], params[o + 2 * (g * pairs + i) + 1]) for i in range(pairs)]
-                  for g in range(Lyr)]
-        o += 2 * Lyr * pairs
-        fc_w, fc_b = params[o], params[o + 1]
-        n_head = cfg["n_head"]                 # the caller's classifier-head parameters ride along as inputs (their gradients
-        params = params[:len(params) - n_head] if n_head else params     # are returned by backward: autograd accumulates them)
-
-        # x is [N, D], or the whole padded allocation [N, pitch >= D] (then dx comes back in the same dense
-        # layout and autograd can keep it without a copy)
-        ctx.x_padded = x.shape[1] != D
-        xr = ops.as_rows(x[:, :D] if ctx.x_padded else x, cd)
-        # every compute-dtype weight copy of the step (both orientations: forward and backward operands) in one launch
-        flat_w = [w for (w, _) in gcn_p] + [w for gp in gate_p for (w, _) in gp]
-        casted = ops.cast_weights_batch([(w, True) for w in flat_w] + [(w, False) for w in flat_w], cd)
-        nW = len(flat_w)
-        w_t = {id(w): casted[i] for i, w in enumerate(flat_w)}            # transposed copies
-        w_n = {id(w): casted[nW + i] for i, w in enumerate(flat_w)}       # same-orientation copies
-        ctx.w_t = [casted[i] for i in range(nW)]
-        ctx.w_n = [casted[nW + i] for i in range(nW)]
+        Lyr, lead, D = cfg["L"], cfg["lead"], cfg["D"]
+        B = graph.n_graphs
+        xr = _x_rows(ctx, x, D, cd)
+        params, gcn_p, gate_p, fc_w, fc_b, w_t, w_n = _unpack(params, cfg)
+        ctx.w_t, ctx.w_n = w_t, w_n
         # ---- trigger vector and the gate MLPs (bert_amir5.py:615-622)
         gated = cfg["gated"]
         drop_p, seed = (cfg["drop_p"], cfg["seed"]) if gated else (0.0, None)
@@ -215,180 +483,100 @@ class _GatedStackFn(torch.autograd.Function):
             # trigger's word pieces, bert_amir.py:118) instead of the trigger row of x (bert_amir5.py:615-618)
             a_raw = aspect.detach().float().contiguous()
             s0 = ops.as_rows(torch.sigmoid(a_raw) if lead else a_raw, cd)
-        side = _Side(_OVERLAP and cfg["gated"], x.device)
+        side = _Side(_OVERLAP and gated, x.device)
         if aspect is None:
             with side.region():                   # the gather feeds the gate MLPs only: it runs on their (side) stream
-                a_raw, s0 = ops.trigger_gather(xr, graph, anchor, lead)
-        gate_saved = []
-        if gated:
-            gates = torch.empty((Lyr, B, D), dtype=torch.float32, device=x.device)
-        else:
-            # ungated ablation (BertAmir55NoGate, bert_amir5.py:731-749): x = gc2(gc1(x)), out = max_t x, xy = 0.0;
-            # the same kernels run with a unit gate
-            gates = torch.ones((Lyr, B, D), dtype=torch.float32, device=x.device)
-        use_chain = gated and _chain_ok(cd, D, Lyr, pairs)
-        ctx.use_chain = use_chain
+                a_raw, s0 = ops.trigger_gather(xr, graph, cfg["anchor"], lead)
+        # ungated ablation (BertAmir55NoGate, bert_amir5.py:731-749): x = gc2(gc1(x)), out = max_t x, xy = 0.0; the same
+        # kernels run with a unit gate
+        gates = (torch.empty if gated else torch.ones)((Lyr, B, D), dtype=torch.float32, device=x.device)
+        ctx.use_chain = gated and _chain_ok(cd, D, Lyr, cfg["gate_linears"])
         with side.region():                       # overlaps the first aggregate -> projection below
-            if use_chain:
-                # every Linear+Sigmoid of every gate in ONE launch (activation tile resident in shared memory)
-                stages = []
-                for g in range(Lyr):
-                    acts, st = [s0], []
-                    for i, (w, b) in enumerate(gate_p[g]):
-                        last = i == pairs - 1
-                        out = gates[g] if last else ops.alloc_rows(B, D, cd, x.device)
-                        st.append(dict(w=w_n[id(w)], bias=b.detach().float().contiguous(), out=out))
-                        if not last:
-                            acts.append(out)
-                    stages.append(st)
-                    gate_saved.append(acts)
-                ops.mlp_chain(0, [s0] * Lyr, stages, B, D)
-            for g in range(Lyr if (gated and not use_chain) else 0):
-                s = s0
-                acts = [s0]
-                for i, (w, b) in enumerate(gate_p[g]):
-                    wk = w_n[id(w)]                                                 # nn.Linear [out,in] is K-major
-                    last = i == pairs - 1
-                    s = ops.linear(s, wk, b.detach().float().contiguous(), act=L.ACT_SIGMOID,
-                                   out_dtype=torch.float32 if last else cd, out=gates[g] if last else None)
-                    if not last:
-                        acts.append(s)
-                gate_saved.append(acts)
+            gate_saved = _gates_fwd(s0, gate_p, w_n[Lyr:], gates, cd, ctx.use_chain) if gated else []
         # ---- ungated GCN chain (bert_amir5.py:626, :639; gcn.py:33-45); after layer 1 the gated views of h_1 and
         # the diversity term (:627-638) go to the side stream (behind the gate MLPs) while layers 2.. run here
         h = xr
         ms, hs, ms_split = [], [], []
         v_pooled = v_arg = v_hmax = None
-        hmaxL = None
         xy = torch.zeros((), dtype=torch.float32, device=x.device)
         fused = _fused_plan(cfg, cd, D, graph, drop_p)
         ctx.fused = fused
-        if fused is not None:
-            # one launch per layer: h_l = A^ (h_{l-1} W_l) + b_l with the column maxima of every sentence (and their
-            # first rows) from the epilogue -- the aggregated rows and the pooling passes never touch HBM
-            rows, plan = fused
-            for l, (w, b) in enumerate(gcn_p):
-                views_here = l == 0 and gated
-                want_pool = views_here or l == Lyr - 1
-                h, hm, ha, _ = ops.gcn_layer(h, w_t[id(w)], b.detach().float().contiguous() if b is not None else None,
-                                             graph, 0, plan, rows, want_pool=want_pool)
-                hs.append(h)
-                if views_here:
-                    v_hmax = hm
-                    v_arg = ha.unsqueeze(0).expand(Lyr, B, D)     # positive gates: the views share their arg-max row
-                    if Lyr > 1:
-                        with side.region():
-                            v_pooled = gates * hm.unsqueeze(0)    # max_t (h_t g) = g max_t h_t for g > 0
-                            xy = ops.diversity_fwd(v_pooled)
-                if l == Lyr - 1:
-                    hmaxL, p_arg = hm, ha
-        else:
-            for l, (w, b) in enumerate(gcn_p):
-                m = ops.aggregate(h, graph, mode=0)
-                wt = w_t[id(w)]                                                     # [out,in]: K-major B operand
-                b32 = b.detach().float().contiguous() if b is not None else None
-                act = L.ACT_RELU if cfg["relu"] else L.ACT_NONE
-                if (cd == torch.float32 and ops.f32_tc(m.shape[0], m.shape[1], wt.shape[0])
-                        and ops.f32_tc(m.shape[0], wt.shape[0], m.shape[1])):
-                    # fp32 mode: the projection reads split operands (ops.SplitRows); the split form of A^ h is also what
-                    # the weight gradient reads, so it is kept INSTEAD of the fp32 rows (same bytes, one split per layer)
-                    m2 = ops.split_rows(m)
-                    h = ops.linear_split(m2, ops.split_rows(wt), b32, act)
-                    ms_split.append((m2.amax, m2.rows, m2.cols))
-                    m = m2.data
-                else:
-                    h = ops.linear(m, wt, b32, act=act)
-                    ms_split.append(None)
-                ms.append(m)
-                hs.append(h)
-                if l == 0 and gated:
+        for l, (_, b) in enumerate(gcn_p):
+            views_here = l == 0 and gated
+            h, m, split, hm, ha = _layer_fwd(h, w_t[l], b, graph, cd, cfg["relu"], fused, views_here or l == Lyr - 1)
+            ms.append(m)
+            ms_split.append(split)
+            hs.append(h)
+            if views_here and fused is not None:
+                v_hmax = hm
+                v_arg = ha.unsqueeze(0).expand(Lyr, B, D)     # positive gates: the views share their arg-max row
+                if Lyr > 1:
                     with side.region():
-                        if drop_p > 0:
-                            # gate dropout (:624-625): view v sees h_1 under the per-token mask of gate v
-                            h1m = [ops.dropout_rows(hs[0], seed, v, drop_p) for v in range(Lyr)]
-                            v_pooled = torch.empty((Lyr, B, D), dtype=torch.float32, device=x.device)
-                            v_arg = torch.empty((Lyr, B, D), dtype=torch.int32, device=x.device)
-                            for v in range(Lyr):
-                                pv, av = ops.pool_fwd(h1m[v], graph, gates[v:v + 1])
-                                v_pooled[v], v_arg[v] = pv[0], av[0]
-                        elif cfg.get("view_len") is not None:
-                            v_pooled, v_arg = _masked_view_pool(hs[0], graph, gates, cfg["view_len"])
-                        elif _PATCH_VIEWS:
-                            v_pooled, v_arg, v_hmax = ops.pool_fwd(hs[0], graph, gates, want_hmax=True)
-                        else:
-                            v_pooled, v_arg = ops.pool_fwd(hs[0], graph, gates)
-                        if Lyr > 1:
-                            xy = ops.diversity_fwd(v_pooled)
+                        v_pooled = gates * hm.unsqueeze(0)    # max_t (h_t g) = g max_t h_t for g > 0
+                        xy = ops.diversity_fwd(v_pooled)
+            elif views_here:
+                with side.region():
+                    if drop_p > 0:
+                        # gate dropout (:624-625): view v sees h_1 under the per-token mask of gate v
+                        h1m = [ops.dropout_rows(hs[0], seed, v, drop_p) for v in range(Lyr)]
+                        v_pooled = torch.empty((Lyr, B, D), dtype=torch.float32, device=x.device)
+                        v_arg = torch.empty((Lyr, B, D), dtype=torch.int32, device=x.device)
+                        for v in range(Lyr):
+                            pv, av = ops.pool_fwd(h1m[v], graph, gates[v:v + 1])
+                            v_pooled[v], v_arg[v] = pv[0], av[0]
+                    elif cfg.get("view_len") is not None:
+                        v_pooled, v_arg = _masked_view_pool(hs[0], graph, gates, cfg["view_len"])
+                    elif _PATCH_VIEWS:
+                        v_pooled, v_arg, v_hmax = ops.pool_fwd(hs[0], graph, gates, want_hmax=True)
+                    else:
+                        v_pooled, v_arg = ops.pool_fwd(hs[0], graph, gates)
+                    if Lyr > 1:
+                        xy = ops.diversity_fwd(v_pooled)
         side.join()                                # gates (and the views) are complete from here on
         # ---- output pooling (:639-640); under gate dropout x_out = gate_L * (h_L * mask_L / (1-p))
         gL = gates[Lyr - 1]
         if fused is not None:
-            hL = hs[-1]
-            pooled = gL * hmaxL                        # the arg-max rows came with the maxima (p_arg)
+            hL, hmaxL, p_arg = hs[-1], hm, ha
+            pooled = gL * hmaxL                        # the arg-max rows came with the maxima
         else:
             hL = ops.dropout_rows(hs[-1], seed, Lyr - 1, drop_p) if drop_p > 0 else hs[-1]
+            hmaxL = None
             pooled, p_arg = ops.pool_fwd(hL, graph, gL.unsqueeze(0))
             pooled, p_arg = pooled[0], p_arg[0]
-        # ---- classifier head: logits_fn is the model's own dense head (host torch, :643); the per-sentence
-        # operands of the collapsed scores, [v_b | va_b] = logits_b @ fc.weight and
-        # c_b = a_b . va_b + logits_b . fc.bias  (= logits_b . (Wfc[:, D:] a_b + bfc), SURVEY A9), are one kernel
-        # A head.DenseHead (= the reference's nn.Linear on cat[a, pooled]) is run by the block's own kernels: no inner
-        # autograd graph, its weight and bias are head_params[0:2].
-        dense_head = cfg.get("dense_head")
-        a_leaf = p_leaf = None
-        if dense_head is not None:
-            hp = cfg["head_params"]
-            logits = ops.dense_head_fwd(a_raw, pooled, hp[0], hp[1] if len(hp) > 1 else None)
-        else:
-            with torch.enable_grad():
-                a_leaf = a_raw.detach().requires_grad_(True)
-                p_leaf = pooled.detach().requires_grad_(True)
-                logits = logits_fn(a_leaf, p_leaf)
-            if logits.requires_grad and cfg["grad_enabled"]:
-                _check_head_leaves(logits, (a_leaf, p_leaf), cfg["head_params"])
-        lg = logits.detach().float().contiguous()
-        fcw32, fcb32 = fc_w.detach().float().contiguous(), fc_b.detach().float().contiguous()
+        # ---- classifier head (:643) and the scores' per-sentence operands
+        ctx.set_materialize_grads(False)          # unused outputs arrive as None, not zero tensors
+        ctx.cfg = cfg
         fc_sig = cfg["fc_sigmoid"]
         # BertAmir54: fc = Sequential(Sigmoid, Linear) (:464-465): the scores read z = sigmoid(x_out) (materialised
         # rows, unit gate) and sigmoid(a); everything downstream is the same kernels
         a_fc = torch.sigmoid(a_raw) if fc_sig else a_raw
-        v, c = ops.fc_head_fwd(lg, fcw32, fcb32, a_fc)
+        logits, v, c = _head_fwd(ctx, a_raw, pooled, a_fc, fc_w, fc_b)
         # ---- importance scores and the softmax product (:645-648)
         # (also d kl/d v, d kl/d c per unit gradient: saves the backward pass one sweep over h_L)
         if fc_sig:
             z = ops.gate_rows(hL, graph, gL, cd, act=L.ACT_SIGMOID)
             ones = torch.ones((B, D), dtype=torch.float32, device=x.device)
-            scores, kl_b, kl, dvu, dcu = ops.scores_kl_fwd(z, graph, ones, v, c, dist, want_units=True)
+            scores, kl_b, kl, dvu, dcu = ops.scores_kl_fwd(z, graph, ones, v, c, cfg["dist"], want_units=True)
             ctx.fc_sig = (z, ones, a_fc)
         else:
             if fused is not None:
-                scores, kl_b, kl, dvu, dcu, uu, sfu = ops.scores_kl_fwd(hL, graph, gL, v, c, dist, want_units=True, want_rows=True)
+                scores, kl_b, kl, dvu, dcu, uu, sfu = ops.scores_kl_fwd(hL, graph, gL, v, c, cfg["dist"],
+                                                                        want_units=True, want_rows=True)
                 ctx.kl_rows = (uu, sfu)
             else:
-                scores, kl_b, kl, dvu, dcu = ops.scores_kl_fwd(hL, graph, gL, v, c, dist, want_units=True)
+                scores, kl_b, kl, dvu, dcu = ops.scores_kl_fwd(hL, graph, gL, v, c, cfg["dist"], want_units=True)
             ctx.fc_sig = None
         ctx.kl_units = (dvu, dcu)
         x_out = ops.gate_rows(hL, graph, gL, cd) if cfg["return_x_out"] else None
         ctx.drop = (drop_p, seed, h1m, hL) if drop_p > 0 else None
-
-        ctx.set_materialize_grads(False)          # unused outputs arrive as None, not zero tensors
-        ctx.cfg = cfg
-        ctx.head = (a_leaf, p_leaf, logits, lg, a_raw, v)
-        # (detached alias: `pooled` itself is an output of this node, and an output stored on its own node is a reference
-        # cycle that keeps the whole graph -- and its AccumulateGrad nodes with their stream -- alive until the cyclic GC)
-        ctx.pooled_head = pooled.detach() if dense_head is not None else None
         ctx.gate_saved = gate_saved
         ctx.n_params = len(params)
-        ctx.n_head = n_head
-        ctx.x_dtype = x.dtype
-        ctx.x_cols = x.shape[1]
+        ctx.n_head = cfg["n_head"]
         ctx.v_hmax = v_hmax
         ctx.hmaxL = hmaxL
-        if fused is not None:
-            ms = [None] * Lyr                     # never materialised
-            ms_split = [None] * Lyr
-            v_arg = v_arg.contiguous() if v_arg is not None else None
         ctx.ms_split = ms_split
+        if fused is not None and v_arg is not None:
+            v_arg = v_arg.contiguous()
         ctx.save_for_backward(xr, gates, v_pooled, v_arg, p_arg, scores, kl_b, *ms, *hs, *params)
         # arg-max rows (global row ids), like the indices torch.max returns at :635-636/:640
         if v_arg is None:
@@ -401,24 +589,20 @@ class _GatedStackFn(torch.autograd.Function):
         cfg = ctx.cfg
         graph: DepGraph = cfg["graph"]
         cd: torch.dtype = cfg["cdtype"]
-        Lyr, pairs, lead = cfg["L"], cfg["pairs"], cfg["lead"]
-        anchor, dist = cfg["anchor"], cfg["dist"]
+        Lyr, dist = cfg["L"], cfg["dist"]
         saved = ctx.saved_tensors
         xr, gates, v_pooled, v_arg, p_arg, scores, kl_b = saved[:7]
         ms = saved[7:7 + Lyr]
         hs = saved[7 + Lyr:7 + 2 * Lyr]
         params = saved[7 + 2 * Lyr:]
+        _, gate_p, fc_w, fc_b = _param_groups(params, Lyr, cfg["gate_linears"])
         B, N, D = graph.n_graphs, graph.n_rows, xr.shape[1]
         dev = xr.device
-        a_leaf, p_leaf, logits, lg, a_raw, v = ctx.head
+        v = ctx.head[5]
         gL = gates[Lyr - 1]
         drop = ctx.drop
         hL = drop[3] if drop else hs[-1]          # under gate dropout the block ran on the masked rows of h_L
-
-        def f32(t):
-            return None if t is None else t.detach().float().contiguous()
-
-        g_xy, g_kl, g_scores, g_pooled = f32(g_xy), f32(g_kl), f32(g_scores), f32(g_pooled)
+        g_xy, g_kl, g_scores, g_pooled = _f32(g_xy), _f32(g_kl), _f32(g_scores), _f32(g_pooled)
         if g_xout is not None:
             g_xout = ops.as_rows(g_xout, cd)
         need_scores = g_kl is not None or g_scores is not None
@@ -435,85 +619,39 @@ class _GatedStackFn(torch.autograd.Function):
         early_views = views_active and not drop and _PATCH_VIEWS and fused is None
         if early_views:
             # the dgates half of the views' backward needs only forward tensors and d xy: it runs on the side stream
-            # from the very start, so the gate MLPs' backward can follow right after edg_head_bwd.  (With
-            # EDG_VIEWS_PATCH=1 what goes to d h_1 comes back as patch arrays for the adjoint aggregation of layer 2.)
+            # from the very start, so the gate MLPs' backward can follow right after edg_head_bwd; what goes to d h_1
+            # comes back as patch arrays for the adjoint aggregation of layer 2
             with side.region():
-                if _PATCH_VIEWS:
-                    patch = ops.views_patch(v_pooled, v_arg, gates, ctx.v_hmax, graph, g_xy, None, dgates, acc_view=-1)
-                    if side.enabled:
-                        patch_ev = torch.cuda.Event()
-                        patch_ev.record(side.side)
-                else:
-                    ops.views_bwd(v_pooled, v_arg, gates, hs[0], g_xy, None, None, dgates, acc_view=-1, parts=2)
+                patch = ops.views_patch(v_pooled, v_arg, gates, ctx.v_hmax, graph, g_xy, None, dgates, acc_view=-1)
+                if side.enabled:
+                    patch_ev = torch.cuda.Event()
+                    patch_ev.record(side.side)
         # ---- d v, d c: the per-unit gradients of the forward sweep times d kl, or (when scores itself carries
-        # gradient) pass A over h_L
-        fc_w, fc_b = params[-2], params[-1]
-        d_fcw = d_fcb = da_fc = g_lg2 = None
-        g_lg = g_logits.float() if g_logits is not None else None
+        # gradient) pass A over h_L; then the fc and classifier heads
+        dvc = None
         if need_scores:
             if g_scores is None:
-                dv_in, dc_in, scale = ctx.kl_units[0], ctx.kl_units[1], g_kl
+                dvc = (ctx.kl_units[0], ctx.kl_units[1], g_kl)
             else:
                 rows_s, gate_s = (ctx.fc_sig[0], ctx.fc_sig[1]) if ctx.fc_sig else (hL, gL)
                 _, _, dv_in, dc_in = ops.head_bwd(rows_s, graph, gate_s, v, dist, scores, kl_b, g_kl, g_scores,
                                                   None, None, None, want_dh=False, want_dv=True)
-                scale = None
-            # backward of [v | va] = logits @ fc.weight, c = a . va + logits . fc.bias  (one kernel + a reduction)
-            a_fc = ctx.fc_sig[2] if ctx.fc_sig else a_raw
-            fcw32, fcb32 = fc_w.detach().float().contiguous(), fc_b.detach().float().contiguous()
-            d_lg, da_fc, _, _ = ops.fc_head_bwd(lg, fcw32, fcb32, a_fc, dv_in, dc_in, scale, parts=1)
-            with side.region():       # nothing downstream waits for the fc parameter gradients: side stream
-                _, _, d_fcw, d_fcb = ops.fc_head_bwd(lg, fcw32, fcb32, a_fc, dv_in, dc_in, scale, parts=2)
-                d_fcw, d_fcb = d_fcw.to(fc_w.dtype), d_fcb.to(fc_b.dtype)
-                grad_hook([d_fcw, d_fcb])
-            if ctx.fc_sig:
-                da_fc = da_fc * a_fc * (1.0 - a_fc)                   # through sigmoid(a)
-            if cfg.get("dense_head") is not None and g_lg is not None:
-                g_lg2 = d_lg                      # the fused head adds the two d logits terms while it loads them
-            else:
-                g_lg = d_lg if g_lg is None else g_lg + d_lg
-        # ---- host head backward through logits_fn: d a, d pooled, and .grad of the parameters it closes over
-        ga_head = gp_head = None
-        head_grads: List[Optional[torch.Tensor]] = [None] * ctx.n_head
-        if g_lg is not None and cfg.get("dense_head") is not None:
-            hp = cfg["head_params"]
-            # d a and d pooled leave with everything else that flows into a / pooled already added (da_fc, g_pooled)
-            ga_head, gp_head, _, _ = ops.dense_head_bwd(g_lg, a_raw, ctx.pooled_head, hp[0], parts=1, g2=g_lg2,
-                                                        da_add=da_fc, dp_add=g_pooled)
-            da_fc = g_pooled = None
-            with side.region():       # nothing downstream waits for the head's parameter gradients: side stream
-                _, _, d_hw, d_hb = ops.dense_head_bwd(g_lg, a_raw, ctx.pooled_head, hp[0], parts=2, g2=g_lg2)
-                if hp[0].requires_grad:
-                    head_grads[0] = d_hw.to(hp[0].dtype)
-                if len(hp) > 1 and hp[1].requires_grad:
-                    head_grads[1] = d_hb.to(hp[1].dtype)
-                grad_hook([g for g in head_grads if g is not None and g.dtype == torch.float32])
-        elif g_lg is not None and logits.requires_grad:
-            cap = [(i, p) for i, p in enumerate(cfg["head_params"]) if p.requires_grad]
-            res = torch.autograd.grad([logits], [a_leaf, p_leaf] + [p for _, p in cap], [g_lg.to(logits.dtype)],
-                                      allow_unused=True, retain_graph=True)
-            ga_head, gp_head = res[0], res[1]
-            for (i, _), g in zip(cap, res[2:]):
-                head_grads[i] = g
-            grad_hook([g for g in head_grads if g is not None and g.dtype == torch.float32])
-        if da_fc is not None:
-            ga_head = da_fc if ga_head is None else ga_head.float() + da_fc
-        gp_total = g_pooled
-        if gp_head is not None:
-            gp_total = gp_head.float() if gp_total is None else gp_total + gp_head.float()
+                dvc = (dv_in, dc_in, None)
+        ga_head, gp_total, d_fcw, d_fcb, head_grads = _head_bwd(ctx, g_logits, g_pooled, dvc, fc_w, fc_b, side,
+                                                                grad_hook)
+        gp_total = gp_total.contiguous() if gp_total is not None else None
         # ---- pass B over h_L: dh_L, dgate_L
         if not views_active and Lyr > 1:
             dgates[:Lyr - 1].zero_()                                  # no diversity gradient: the other gates get none
-        early_gate = early_views              # dgates[L-1] already holds the views' share: head_bwd writes elsewhere
-        dgL = torch.empty((B, D), dtype=torch.float32, device=dev) if early_gate else dgates[Lyr - 1]
+        # (early views: dgates[L-1] already holds the views' share, head_bwd writes elsewhere)
+        dgL = torch.empty((B, D), dtype=torch.float32, device=dev) if early_views else dgates[Lyr - 1]
         du_top = db_top = None
         if fused is not None and g_xout is None:
             # top of the chain straight in aggregated form: du_L = A^T dh_L, db_L, d gate_L from [N]- and [B,D]-sized
             # inputs only (h_L is not read again, dh_L never exists)
             uu, sfu = ctx.kl_rows
-            du_top, db_top, _ = ops.head_du(uu, g_kl if need_scores else None, g_scores, gL, v,
-                                            gp_total.contiguous() if gp_total is not None else None, p_arg, sfu, ctx.hmaxL,
-                                            graph, fused[1], want_dgate=True, dgate_out=dgL)
+            du_top, db_top, _ = ops.head_du(uu, g_kl if need_scores else None, g_scores, gL, v, gp_total, p_arg, sfu,
+                                            ctx.hmaxL, graph, fused[1], want_dgate=True, dgate_out=dgL)
             if g_scores is not None:
                 # scores itself carries gradient: d gate_L also needs sum_t g_scores_t h_t -- one sweep over h_L
                 _, _, dv_s, _ = ops.head_bwd(hL, graph, gL, v, dist, scores, kl_b, None, g_scores, None, None, None,
@@ -528,92 +666,33 @@ class _GatedStackFn(torch.autograd.Function):
             dxo = ops.sigmoid_bwd(z, dz, cd)
             if g_xout is not None:
                 dxo = ops.as_rows(dxo + g_xout, cd)
-            dh, _, _, _ = ops.head_bwd(hL, graph, gL, None, dist, None, kl_b, None, None,
-                                       gp_total.contiguous() if gp_total is not None else None, p_arg, dxo,
+            dh, _, _, _ = ops.head_bwd(hL, graph, gL, None, dist, None, kl_b, None, None, gp_total, p_arg, dxo,
                                        want_dh=True, want_dv=False, dgate_out=dgL)
         else:
             dh, _, _, _ = ops.head_bwd(hL, graph, gL, v if need_scores else None, dist,
-                                       scores if need_scores else None, kl_b, g_kl, g_scores,
-                                       gp_total.contiguous() if gp_total is not None else None, p_arg, g_xout,
+                                       scores if need_scores else None, kl_b, g_kl, g_scores, gp_total, p_arg, g_xout,
                                        want_dh=True, want_dv=False, dgate_out=dgL)
         if drop:
             dh = ops.dropout_rows(dh, drop[1], Lyr - 1, drop[0])      # d h_L = d (h_L * mask / (1-p)) * mask / (1-p)
         grads_out: List[Optional[torch.Tensor]] = [None] * ctx.n_params
         o = 2 * Lyr
 
-        # ---- gate MLP backward (bert_amir5.py:562-571): needs the complete dgates, nothing else of the GCN chain
+        # ---- gate MLP backward (bert_amir5.py:562-571): needs the complete dgates, nothing else of the GCN chain;
+        # it runs on the side stream next to the GCN chain backward
         def gate_backward():
-            # the last Sigmoid of every gate in one launch (gates / dgates are [V*B, D] row blocks)
-            dz_all = ops.sigmoid_bwd(gates.view(Lyr * B, D), dgates.view(Lyr * B, D), cd)
-            da_g = None
-            if ctx.use_chain:
-                # d z chain of every gate in ONE launch, then every weight gradient in one batched launch
-                da_parts = torch.empty((Lyr, B, D), dtype=torch.float32, device=dev)
-                dz_in = [[None] * pairs for _ in range(Lyr)]      # gradient at the pre-activation output of Linear i
-                stages = []
-                for g in range(Lyr):
-                    acts = ctx.gate_saved[g]
-                    dz_in[g][pairs - 1] = dz_all[g * B:(g + 1) * B]
-                    st = []
-                    for i in range(pairs - 1, -1, -1):
-                        wt = ctx.w_t[Lyr + g * pairs + i]                       # [in,out]: row n = input column n
-                        if i > 0:
-                            out = ops.alloc_rows(B, D, cd, dev)
-                            dz_in[g][i - 1] = out
-                            st.append(dict(w=wt, y=acts[i], out=out))
-                        else:
-                            st.append(dict(w=wt, y=acts[0] if lead else None, out=da_parts[g]))
-                    stages.append(st)
-                ops.mlp_chain(1, [dz_in[g][pairs - 1] for g in range(Lyr)], stages, B, D)
-                idx = [(g, i) for g in range(Lyr) for i in range(pairs)]
-                for c0 in range(0, len(idx), 8):
-                    part = idx[c0:c0 + 8]
-                    dWs, dbs = ops.wgrad_batch([dz_in[g][i] for g, i in part], [ctx.gate_saved[g][i] for g, i in part],
-                                               bias_of=1)
-                    for (g, i), dW, db in zip(part, dWs, dbs):
-                        w, b = params[o + 2 * (g * pairs + i)], params[o + 2 * (g * pairs + i) + 1]
-                        grads_out[o + 2 * (g * pairs + i)] = dW.to(w.dtype)
-                        grads_out[o + 2 * (g * pairs + i) + 1] = db.to(b.dtype)
-                grad_hook(grads_out[o:o + 2 * Lyr * pairs])
-                return ("parts", da_parts)         # [L,B,D], summed where it is consumed (edg_trigger_scatter_add)
-            for g in range(Lyr):
-                acts = ctx.gate_saved[g]
-                dz = dz_all[g * B:(g + 1) * B]
-                for i in range(pairs - 1, -1, -1):
-                    w, b = params[o + 2 * (g * pairs + i)], params[o + 2 * (g * pairs + i) + 1]
-                    dW, db = ops.wgrad(dz, acts[i], bias_of=1)                  # [out,in], [out]
-                    grads_out[o + 2 * (g * pairs + i)] = dW.to(w.dtype)
-                    grads_out[o + 2 * (g * pairs + i) + 1] = db.to(b.dtype)
-                    wt = ctx.w_t[Lyr + g * pairs + i]                           # [in,out]
-                    if i > 0:
-                        ds = ops.linear(dz, wt, None)
-                        dz = ops.sigmoid_bwd(acts[i], ds, cd)
-                    elif lead:
-                        ds = ops.linear(dz, wt, None)
-                        if da_g is None:
-                            da_g = ops.sigmoid_bwd(acts[0], ds, torch.float32,
-                                                   out=torch.empty((B, D), dtype=torch.float32, device=dev))
-                        else:
-                            ops.sigmoid_bwd(acts[0], ds, torch.float32, out=da_g, accumulate=True)
-                    else:
-                        dlast = ops.linear(dz, wt, None, out_dtype=torch.float32)
-                        da_g = dlast if da_g is None else da_g + dlast
-            grad_hook(grads_out[o:o + 2 * Lyr * pairs])
-            return da_g
+            da_g, da_x, gg = _gates_bwd(gates, dgates, ctx.gate_saved, gate_p, ctx.w_t[Lyr:], cfg["lead"], cd,
+                                        ctx.use_chain, grad_hook)
+            grads_out[o:o + len(gg)] = gg
+            return da_g, da_x
 
-        # ---- GCN chain backward (gcn.py:33-45); the gate MLPs' backward runs on the side stream next to it
         # (opt-in) the weight gradient of a layer next to its input gradient: both start from dh
         side_w = _Side(_OVERLAP_WGRAD, dev, which=1)
-        da_gate = None
-        if early_gate:
+        da_gate = da_extra = None
+        if early_views:
             with side.region():                   # after head_bwd: dgates are complete
                 dgates[Lyr - 1].add_(dgL)
-                da_gate = gate_backward()
+                da_gate, da_extra = gate_backward()
         if fused is not None:
-            # with u_l = h_{l-1} W_l and h_l = A^ u_l + b_l:  db_l = colsum(dh_l), du_l = A^T dh_l, dW_l = h_{l-1}^T du_l,
-            # dh_{l-1} = du_l W_l^T.  One fused launch per layer produces du_{l-1} = A^T (du_l W_l^T + views patch) and the
-            # column sums of its argument (= db_{l-1}); neither dh_{l-1} nor the aggregated rows exist in HBM.
-            rows, plan = fused
             if du_top is not None:
                 du, db_next = du_top, db_top
             else:                                 # a direct gradient on x_out came in: dh_L exists, aggregate it
@@ -624,41 +703,31 @@ class _GatedStackFn(torch.autograd.Function):
             if gated:
                 # side stream, behind edg_head_du (which wrote d gate_L): the views' share of d gates / the patch for d h_1,
                 # then the gate MLPs' backward; this stream goes straight on to the weight gradient of layer L and only
-                # waits for the patch where it is consumed (the layer-1 launch below)
+                # waits for the patch where it is consumed (the layer-1 launch)
                 with side.region():
                     if views_active:
                         patch = (ops.views_bwd_hmax(ctx.v_hmax, gates, g_xy, dgates, acc_view=Lyr - 1), v_arg[0])
                         if side.enabled:
                             patch_ready = torch.cuda.Event()
                             patch_ready.record(side.side)
-                    da_gate = gate_backward()     # dgates are complete from here on
-            for l in range(Lyr - 1, -1, -1):
-                w, b = params[2 * l], params[2 * l + 1]
-                dW, _ = ops.wgrad(hs[l - 1] if l > 0 else xr, du, bias_of=0)
-                grads_out[2 * l], grads_out[2 * l + 1] = dW.to(w.dtype), db_next.to(b.dtype)
-                grad_hook(grads_out[2 * l:2 * l + 2])
-                wk = ctx.w_n[l]                                                 # [in,out] = B operand of du W^T
-                if l == 0 and bucket_hook is not None:
-                    # every parameter gradient of the block exists now (the gate MLPs' come from the side stream): hand
-                    # them to the all-reduce and let it run NEXT to the input-gradient projection, which leaves it SMs
-                    side.join()
-                    side_w.join()
-                    grads_out[-2], grads_out[-1] = d_fcw, d_fcb
-                    n_out = len(grads_out)
-                    reduced = bucket_hook(list(grads_out) + list(head_grads))
-                    grads_out[:] = reduced[:n_out]
-                    head_grads = list(reduced[n_out:])
-                    d_fcw, d_fcb = grads_out[-2], grads_out[-1]
-                    with ops.sm_budget(_BUCKET_LINEAR_SMS):
-                        dh = ops.linear(du, wk, None)
-                    continue
-                if l > 0:
-                    if l == 1 and patch_ready is not None:
-                        torch.cuda.current_stream(dev).wait_event(patch_ready)
-                    du, _, _, db_next = ops.gcn_layer(du, wk, None, graph, 1, plan, rows,
-                                                      patch=patch if l == 1 else None, want_colsum=True)
-                else:
+                    da_gate, da_extra = gate_backward()     # dgates are complete from here on
+            du = _fused_chain_bwd(ctx, du, db_next, xr, hs, params, grads_out, grad_hook, patch, patch_ready)
+            wk = ctx.w_n[0]                                                 # [in,out] = B operand of du W^T
+            if bucket_hook is not None:
+                # every parameter gradient of the block exists now (the gate MLPs' come from the side stream): hand
+                # them to the all-reduce and let it run NEXT to the input-gradient projection, which leaves it SMs
+                side.join()
+                side_w.join()
+                grads_out[-2], grads_out[-1] = d_fcw, d_fcb
+                n_out = len(grads_out)
+                reduced = bucket_hook(list(grads_out) + list(head_grads))
+                grads_out[:] = reduced[:n_out]
+                head_grads = list(reduced[n_out:])
+                d_fcw, d_fcb = grads_out[-2], grads_out[-1]
+                with ops.sm_budget(_BUCKET_LINEAR_SMS):
                     dh = ops.linear(du, wk, None)
+            else:
+                dh = ops.linear(du, wk, None)
         else:
             for l in range(Lyr - 1, -1, -1):
                 if l == 0 and views_active and drop:
@@ -672,23 +741,10 @@ class _GatedStackFn(torch.autograd.Function):
                 elif l == 0 and views_active and not _PATCH_VIEWS:
                     # gated views of h_1 feed xy (:627-638): add their gradient to d h_1 before leaving layer 1
                     ops.views_bwd(v_pooled, v_arg, gates, hs[0], g_xy, None, dh, dgates, acc_view=Lyr - 1)
-                if l == 0 and gated and not early_gate:
+                if l == 0 and gated and not early_views:
                     with side.region():               # dgates are complete from here on
-                        da_gate = gate_backward()
-                w, b = params[2 * l], params[2 * l + 1]
-                if cfg["relu"]:
-                    dh = ops.as_rows(dh * (hs[l] > 0), cd)
-                msp = ctx.ms_split[l]
-                dh2 = ops.split_rows(dh) if msp is not None else None              # shared by dW and the input gradient
-                with side_w.region():
-                    if msp is not None:
-                        dW, db = ops.wgrad_split(ops.SplitRows(ms[l], *msp), dh2, bias_of=2)
-                    else:
-                        dW, db = ops.wgrad(ms[l], dh, bias_of=2)
-                    grads_out[2 * l], grads_out[2 * l + 1] = dW.to(w.dtype), db.to(b.dtype)
-                    grad_hook(grads_out[2 * l:2 * l + 2])
-                wk = ctx.w_n[l]                                                     # [in,out] = B operand of dh W^T
-                dm = ops.linear_split(dh2, ops.split_rows(wk), None) if msp is not None else ops.linear(dh, wk, None)
+                        da_gate, da_extra = gate_backward()
+                dm = _unfused_layer_bwd(ctx, l, dh, hs, ms, params, grads_out, grad_hook, side_w)
                 if l == 1 and patch is not None and patch_ev is not None:
                     torch.cuda.current_stream(dev).wait_event(patch_ev)       # the patch arrays come from the side stream
                 dh = ops.aggregate(dm, graph, mode=1, patch=patch if l == 1 else None)
@@ -696,11 +752,8 @@ class _GatedStackFn(torch.autograd.Function):
         side.join()
         side_w.join()
         da = ga_head.float() if ga_head is not None else None
-        da_extra = None
-        if isinstance(da_gate, tuple):            # the gate MLPs' input gradients, one [B,D] slab per gate
-            da_extra, da_gate = da_gate[1], None
-            if ctx.ext_aspect:                    # the caller gets d aspect as a tensor: sum them here
-                da_gate, da_extra = (da_extra.sum(0) if da_extra.shape[0] > 1 else da_extra[0]), None
+        if da_extra is not None and ctx.ext_aspect:   # the caller gets d aspect as a tensor: sum the gates' slabs here
+            da_gate, da_extra = (da_extra.sum(0) if da_extra.shape[0] > 1 else da_extra[0]), None
         if da_gate is not None:
             da = da_gate if da is None else da + da_gate
         d_aspect = None
@@ -708,17 +761,9 @@ class _GatedStackFn(torch.autograd.Function):
             if ctx.ext_aspect:
                 d_aspect = da
             else:
-                ops.trigger_scatter_add(da, graph, anchor, dx, extra=da_extra)
+                ops.trigger_scatter_add(da, graph, cfg["anchor"], dx, extra=da_extra)
         grads_out[-2], grads_out[-1] = d_fcw, d_fcb
-        if ctx.x_padded:        # hand back the whole [N, pitch] allocation (padding columns are finite)
-            dx = dx.as_strided((N, dx.stride(0)), (dx.stride(0), 1))
-            if dx.shape[1] != ctx.x_cols:
-                full = torch.zeros((N, ctx.x_cols), dtype=dx.dtype, device=dev)
-                full[:, :D] = dx[:, :D]
-                dx = full
-        if dx.dtype != ctx.x_dtype:
-            dx = dx.to(ctx.x_dtype)
-        return (None, dx, d_aspect) + tuple(grads_out) + tuple(head_grads)
+        return (None, _dx_like_x(ctx, dx), d_aspect) + tuple(grads_out) + tuple(head_grads)
 
 
 class _GatedPairsFn(torch.autograd.Function):
@@ -731,102 +776,39 @@ class _GatedPairsFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, cfg, x, *params):
         graph: DepGraph = cfg["graph"]
-        pairs = cfg["pairs"]
+        pairs: TriggerPairs = cfg["pairs"]
         cd: torch.dtype = cfg["cdtype"]
-        Lyr, npr, lead = cfg["L"], cfg["gate_pairs"], cfg["lead"]
-        anchor, dist, logits_fn = cfg["anchor"], cfg["dist"], cfg["logits_fn"]
-        D = cfg["D"]
+        Lyr, D, gated = cfg["L"], cfg["D"], cfg["gated"]
         S, P = graph.n_graphs, pairs.n_pairs
-        gcn_p = [(params[2 * l], params[2 * l + 1]) for l in range(Lyr)]
-        o = 2 * Lyr
-        gate_p = [[(params[o + 2 * (g * npr + i)], params[o + 2 * (g * npr + i) + 1]) for i in range(npr)]
-                  for g in range(Lyr)]
-        o += 2 * Lyr * npr
-        fc_w, fc_b = params[o], params[o + 1]
-        n_head = cfg["n_head"]
-        params = params[:len(params) - n_head] if n_head else params
-        ctx.x_padded = x.shape[1] != D
-        xr = ops.as_rows(x[:, :D] if ctx.x_padded else x, cd)
-        flat_w = [w for (w, _) in gcn_p] + [w for gp in gate_p for (w, _) in gp]
-        casted = ops.cast_weights_batch([(w, True) for w in flat_w] + [(w, False) for w in flat_w], cd)
-        nW = len(flat_w)
-        w_t = {id(w): casted[i] for i, w in enumerate(flat_w)}
-        w_n = {id(w): casted[nW + i] for i, w in enumerate(flat_w)}
-        ctx.w_t = [casted[i] for i in range(nW)]
-        ctx.w_n = [casted[nW + i] for i in range(nW)]
-        gated = cfg["gated"]
+        xr = _x_rows(ctx, x, D, cd)
+        params, gcn_p, gate_p, fc_w, fc_b, w_t, w_n = _unpack(params, cfg)
+        ctx.w_t, ctx.w_n = w_t, w_n
         # ---- per pair: the trigger row of its sentence and the gate MLPs on P rows
-        a_raw, s0 = ops.trigger_gather(xr, ops.PairRows(pairs), anchor, lead)
-        gate_saved = []
-        if gated:
-            gates = torch.empty((Lyr, P, D), dtype=torch.float32, device=x.device)
-        else:
-            gates = torch.ones((Lyr, P, D), dtype=torch.float32, device=x.device)
-        use_chain = gated and _chain_ok(cd, D, Lyr, npr)
-        ctx.use_chain = use_chain
-        if use_chain:
-            stages = []
-            for g in range(Lyr):
-                acts, st = [s0], []
-                for i, (w, b) in enumerate(gate_p[g]):
-                    last = i == npr - 1
-                    out = gates[g] if last else ops.alloc_rows(P, D, cd, x.device)
-                    st.append(dict(w=w_n[id(w)], bias=b.detach().float().contiguous(), out=out))
-                    if not last:
-                        acts.append(out)
-                stages.append(st)
-                gate_saved.append(acts)
-            if P > 0:
-                ops.mlp_chain(0, [s0] * Lyr, stages, P, D)
-        for g in range(Lyr if (gated and not use_chain and P > 0) else 0):
-            s = s0
-            acts = [s0]
-            for i, (w, b) in enumerate(gate_p[g]):
-                last = i == npr - 1
-                s = ops.linear(s, w_n[id(w)], b.detach().float().contiguous(), act=L.ACT_SIGMOID,
-                               out_dtype=torch.float32 if last else cd, out=gates[g] if last else None)
-                if not last:
-                    acts.append(s)
-            gate_saved.append(acts)
+        a_raw, s0 = ops.trigger_gather(xr, ops.PairRows(pairs), cfg["anchor"], cfg["lead"])
+        gates = (torch.empty if gated else torch.ones)((Lyr, P, D), dtype=torch.float32, device=x.device)
+        ctx.use_chain = gated and _chain_ok(cd, D, Lyr, cfg["gate_linears"])
+        gate_saved = _gates_fwd(s0, gate_p, w_n[Lyr:], gates, cd, ctx.use_chain) if gated and P > 0 else []
         # ---- the GCN chain once per sentence, with the column maxima of h_1 (views) and h_L (final pool)
         h = xr
         ms, hs, ms_split = [], [], []
-        hmax1 = harg1 = hmaxL = hargL = None
+        hmax1 = harg1 = None
         fused = _fused_plan(cfg, cd, D, graph, 0.0)
         ctx.fused = fused
         ones = None
-        for l, (w, b) in enumerate(gcn_p):
+        for l, (_, b) in enumerate(gcn_p):
             want_pool = (l == 0 and gated) or l == Lyr - 1
-            b32 = b.detach().float().contiguous() if b is not None else None
-            if fused is not None:
-                rows, plan = fused
-                h, hm, ha, _ = ops.gcn_layer(h, w_t[id(w)], b32, graph, 0, plan, rows, want_pool=want_pool)
-                ms.append(None)
-                ms_split.append(None)
-            else:
-                m = ops.aggregate(h, graph, mode=0)
-                wt = w_t[id(w)]
-                act = L.ACT_RELU if cfg["relu"] else L.ACT_NONE
-                if (cd == torch.float32 and ops.f32_tc(m.shape[0], m.shape[1], wt.shape[0])
-                        and ops.f32_tc(m.shape[0], wt.shape[0], m.shape[1])):
-                    m2 = ops.split_rows(m)
-                    h = ops.linear_split(m2, ops.split_rows(wt), b32, act)
-                    ms_split.append((m2.amax, m2.rows, m2.cols))
-                    m = m2.data
-                else:
-                    h = ops.linear(m, wt, b32, act=act)
-                    ms_split.append(None)
-                ms.append(m)
-                if want_pool:
-                    if ones is None:
-                        ones = torch.ones((1, S, D), dtype=torch.float32, device=x.device)
-                    _, ha, hm = ops.pool_fwd(h, graph, ones, want_hmax=True)
-                    ha = ha[0]
+            h, m, split, hm, ha = _layer_fwd(h, w_t[l], b, graph, cd, cfg["relu"], fused, want_pool)
+            if fused is None and want_pool:
+                if ones is None:
+                    ones = torch.ones((1, S, D), dtype=torch.float32, device=x.device)
+                _, ha, hm = ops.pool_fwd(h, graph, ones, want_hmax=True)
+                ha = ha[0]
+            ms.append(m)
+            ms_split.append(split)
             hs.append(h)
             if l == 0 and gated:
                 hmax1, harg1 = hm, ha
-            if l == Lyr - 1:
-                hmaxL, hargL = hm, ha
+        hmaxL, hargL = hm, ha
         ps = pairs.pair_sent.long()
         xy = torch.zeros((), dtype=torch.float32, device=x.device)
         v_arg = None
@@ -839,36 +821,18 @@ class _GatedPairsFn(torch.autograd.Function):
         pooled = gL * hmaxL[ps]
         p_arg = hargL[ps]
         # ---- classifier head on [P,D], then the per-pair scores / kl over the sentence rows
-        dense_head = cfg.get("dense_head")
-        a_leaf = p_leaf = None
-        if dense_head is not None:
-            hp = cfg["head_params"]
-            logits = ops.dense_head_fwd(a_raw, pooled, hp[0], hp[1] if len(hp) > 1 else None)
-        else:
-            with torch.enable_grad():
-                a_leaf = a_raw.detach().requires_grad_(True)
-                p_leaf = pooled.detach().requires_grad_(True)
-                logits = logits_fn(a_leaf, p_leaf)
-            if logits.requires_grad and cfg["grad_enabled"]:
-                _check_head_leaves(logits, (a_leaf, p_leaf), cfg["head_params"])
-        lg = logits.detach().float().contiguous()
-        fcw32, fcb32 = fc_w.detach().float().contiguous(), fc_b.detach().float().contiguous()
-        v, c = ops.fc_head_fwd(lg, fcw32, fcb32, a_raw)
-        scores, kl_b, kl, dvu, dcu = ops.scores_kl_pairs_fwd(hL, graph, pairs, gL, v, c, dist)
-        ctx.kl_units = (dvu, dcu)
         ctx.set_materialize_grads(False)
         ctx.cfg = cfg
-        ctx.head = (a_leaf, p_leaf, logits, lg, a_raw, v)
-        ctx.pooled_head = pooled.detach() if dense_head is not None else None
+        ctx.fc_sig = None
+        logits, v, c = _head_fwd(ctx, a_raw, pooled, a_raw, fc_w, fc_b)
+        scores, kl_b, kl, dvu, dcu = ops.scores_kl_pairs_fwd(hL, graph, pairs, gL, v, c, cfg["dist"])
+        ctx.kl_units = (dvu, dcu)
         ctx.gate_saved = gate_saved
         ctx.n_params = len(params)
-        ctx.n_head = n_head
-        ctx.x_dtype = x.dtype
-        ctx.x_cols = x.shape[1]
+        ctx.n_head = cfg["n_head"]
         ctx.ms_split = ms_split
         ctx.pool_rows = (hmax1, harg1, hargL)
-        ctx.save_for_backward(xr, gates, scores, kl_b, *[m for m in ms if m is not None], *hs, *params)
-        ctx.n_ms = sum(m is not None for m in ms)
+        ctx.save_for_backward(xr, gates, scores, kl_b, *ms, *hs, *params)
         if v_arg is None:
             v_arg = torch.empty((0,), dtype=torch.int32, device=x.device)
         ctx.mark_non_differentiable(p_arg, v_arg)
@@ -878,76 +842,37 @@ class _GatedPairsFn(torch.autograd.Function):
     def backward(ctx, g_logits, g_xy, g_kl, g_scores, g_pooled, _g_parg=None, _g_varg=None):
         cfg = ctx.cfg
         graph: DepGraph = cfg["graph"]
-        pairs = cfg["pairs"]
-        cd: torch.dtype = cfg["cdtype"]
-        Lyr, npr, lead = cfg["L"], cfg["gate_pairs"], cfg["lead"]
-        anchor, dist = cfg["anchor"], cfg["dist"]
+        pairs: TriggerPairs = cfg["pairs"]
+        Lyr, dist = cfg["L"], cfg["dist"]
         saved = ctx.saved_tensors
         xr, gates, scores, kl_b = saved[:4]
-        o = 4
-        ms = list(saved[o:o + ctx.n_ms]) if ctx.n_ms else [None] * Lyr
-        o += ctx.n_ms
-        hs = saved[o:o + Lyr]
-        params = saved[o + Lyr:]
-        P, N, D = pairs.n_pairs, graph.n_rows, xr.shape[1]
+        ms = saved[4:4 + Lyr]
+        hs = saved[4 + Lyr:4 + 2 * Lyr]
+        params = saved[4 + 2 * Lyr:]
+        _, gate_p, fc_w, fc_b = _param_groups(params, Lyr, cfg["gate_linears"])
+        P, D = pairs.n_pairs, xr.shape[1]
         dev = xr.device
-        a_leaf, p_leaf, logits, lg, a_raw, v = ctx.head
+        v = ctx.head[5]
         hmax1, harg1, hargL = ctx.pool_rows
         gL = gates[Lyr - 1]
         hL = hs[-1]
-
-        def f32(t):
-            return None if t is None else t.detach().float().contiguous()
-
-        g_xy, g_kl, g_scores, g_pooled = f32(g_xy), f32(g_kl), f32(g_scores), f32(g_pooled)
+        g_xy, g_kl, g_scores, g_pooled = _f32(g_xy), _f32(g_kl), _f32(g_scores), _f32(g_pooled)
         need_scores = g_kl is not None or g_scores is not None
         grad_hook = cfg.get("grad_hook") or (lambda ts: None)
         gated = cfg["gated"]
         views_active = g_xy is not None and Lyr > 1 and gated
         dgates = torch.empty((Lyr, P, D), dtype=torch.float32, device=dev)
-        # ---- d v, d c (per pair) and the fc head
-        fc_w, fc_b = params[-2], params[-1]
-        d_fcw = d_fcb = da_fc = g_lg2 = None
-        g_lg = g_logits.float() if g_logits is not None else None
+        # ---- d v, d c (per pair), the fc head and the classifier head
+        dvc = None
         if need_scores:
             if g_scores is None:
-                dv_in, dc_in, scale = ctx.kl_units[0], ctx.kl_units[1], g_kl
+                dvc = (ctx.kl_units[0], ctx.kl_units[1], g_kl)
             else:
                 _, _, dv_in, dc_in = ops.head_bwd_pairs(hL, graph, pairs, gL, v, dist, scores, kl_b, g_kl, g_scores,
                                                         None, None, want_dh=False)
-                scale = None
-            fcw32, fcb32 = fc_w.detach().float().contiguous(), fc_b.detach().float().contiguous()
-            d_lg, da_fc, d_fcw, d_fcb = ops.fc_head_bwd(lg, fcw32, fcb32, a_raw, dv_in, dc_in, scale, parts=3)
-            d_fcw, d_fcb = d_fcw.to(fc_w.dtype), d_fcb.to(fc_b.dtype)
-            if cfg.get("dense_head") is not None and g_lg is not None:
-                g_lg2 = d_lg
-            else:
-                g_lg = d_lg if g_lg is None else g_lg + d_lg
-        # ---- classifier head backward: d a, d pooled (per pair) and the head's parameters
-        ga_head = gp_head = None
-        head_grads: List[Optional[torch.Tensor]] = [None] * ctx.n_head
-        if g_lg is not None and cfg.get("dense_head") is not None:
-            hp = cfg["head_params"]
-            ga_head, gp_head, d_hw, d_hb = ops.dense_head_bwd(g_lg, a_raw, ctx.pooled_head, hp[0], parts=3, g2=g_lg2,
-                                                              da_add=da_fc, dp_add=g_pooled)
-            da_fc = g_pooled = None
-            if hp[0].requires_grad:
-                head_grads[0] = d_hw.to(hp[0].dtype)
-            if len(hp) > 1 and hp[1].requires_grad:
-                head_grads[1] = d_hb.to(hp[1].dtype)
-        elif g_lg is not None and logits.requires_grad:
-            cap = [(i, p) for i, p in enumerate(cfg["head_params"]) if p.requires_grad]
-            res = torch.autograd.grad([logits], [a_leaf, p_leaf] + [p for _, p in cap], [g_lg.to(logits.dtype)],
-                                      allow_unused=True, retain_graph=True)
-            ga_head, gp_head = res[0], res[1]
-            for (i, _), g in zip(cap, res[2:]):
-                head_grads[i] = g
+                dvc = (dv_in, dc_in, None)
+        ga_head, gp_total, d_fcw, d_fcb, head_grads = _head_bwd(ctx, g_logits, g_pooled, dvc, fc_w, fc_b, None, None)
         grad_hook([g for g in head_grads if g is not None and g.dtype == torch.float32])
-        if da_fc is not None:
-            ga_head = da_fc if ga_head is None else ga_head.float() + da_fc
-        gp_total = g_pooled
-        if gp_head is not None:
-            gp_total = gp_head.float() if gp_total is None else gp_total + gp_head.float()
         # ---- d h_L over the sentence rows (every pair of a sentence summed in pair order), d gate_L per pair
         if not views_active and Lyr > 1:
             dgates[:Lyr - 1].zero_()
@@ -961,81 +886,23 @@ class _GatedPairsFn(torch.autograd.Function):
         grads_out: List[Optional[torch.Tensor]] = [None] * ctx.n_params
         o = 2 * Lyr
         # ---- gate MLPs (dgates complete)
-        da_gate = None
-        da_extra = None
+        da_gate = da_extra = None
         if gated and P > 0:
-            dz_all = ops.sigmoid_bwd(gates.view(Lyr * P, D), dgates.view(Lyr * P, D), cd)
-            if ctx.use_chain:
-                da_extra = torch.empty((Lyr, P, D), dtype=torch.float32, device=dev)
-                dz_in = [[None] * npr for _ in range(Lyr)]
-                stages = []
-                for g in range(Lyr):
-                    acts = ctx.gate_saved[g]
-                    dz_in[g][npr - 1] = dz_all[g * P:(g + 1) * P]
-                    st = []
-                    for i in range(npr - 1, -1, -1):
-                        wt = ctx.w_t[Lyr + g * npr + i]
-                        if i > 0:
-                            out = ops.alloc_rows(P, D, cd, dev)
-                            dz_in[g][i - 1] = out
-                            st.append(dict(w=wt, y=acts[i], out=out))
-                        else:
-                            st.append(dict(w=wt, y=acts[0] if lead else None, out=da_extra[g]))
-                    stages.append(st)
-                ops.mlp_chain(1, [dz_in[g][npr - 1] for g in range(Lyr)], stages, P, D)
-                idx = [(g, i) for g in range(Lyr) for i in range(npr)]
-                for c0 in range(0, len(idx), 8):
-                    part = idx[c0:c0 + 8]
-                    dWs, dbs = ops.wgrad_batch([dz_in[g][i] for g, i in part], [ctx.gate_saved[g][i] for g, i in part],
-                                               bias_of=1)
-                    for (g, i), dW, db in zip(part, dWs, dbs):
-                        w, b = params[o + 2 * (g * npr + i)], params[o + 2 * (g * npr + i) + 1]
-                        grads_out[o + 2 * (g * npr + i)] = dW.to(w.dtype)
-                        grads_out[o + 2 * (g * npr + i) + 1] = db.to(b.dtype)
-            else:
-                for g in range(Lyr):
-                    acts = ctx.gate_saved[g]
-                    dz = dz_all[g * P:(g + 1) * P]
-                    for i in range(npr - 1, -1, -1):
-                        w, b = params[o + 2 * (g * npr + i)], params[o + 2 * (g * npr + i) + 1]
-                        dW, db = ops.wgrad(dz, acts[i], bias_of=1)
-                        grads_out[o + 2 * (g * npr + i)] = dW.to(w.dtype)
-                        grads_out[o + 2 * (g * npr + i) + 1] = db.to(b.dtype)
-                        wt = ctx.w_t[Lyr + g * npr + i]
-                        if i > 0:
-                            dz = ops.sigmoid_bwd(acts[i], ops.linear(dz, wt, None), cd)
-                        elif lead:
-                            ds = ops.linear(dz, wt, None)
-                            if da_gate is None:
-                                da_gate = ops.sigmoid_bwd(acts[0], ds, torch.float32,
-                                                          out=torch.empty((P, D), dtype=torch.float32, device=dev))
-                            else:
-                                ops.sigmoid_bwd(acts[0], ds, torch.float32, out=da_gate, accumulate=True)
-                        else:
-                            dlast = ops.linear(dz, wt, None, out_dtype=torch.float32)
-                            da_gate = dlast if da_gate is None else da_gate + dlast
-            grad_hook(grads_out[o:o + 2 * Lyr * npr])
+            da_gate, da_extra, gg = _gates_bwd(gates, dgates, ctx.gate_saved, gate_p, ctx.w_t[Lyr:], cfg["lead"],
+                                               cfg["cdtype"], ctx.use_chain, grad_hook)
+            grads_out[o:o + len(gg)] = gg
         elif gated:                                # no pairs: the gate parameters get zero gradients
-            for k in range(o, o + 2 * Lyr * npr):
+            for k in range(o, o + 2 * len(gate_p)):
                 grads_out[k] = torch.zeros_like(params[k])
         # ---- the GCN chain backward on the sentence rows, exactly as for unpaired batches
-        fused = ctx.fused
-        if fused is not None:
-            rows, plan = fused
+        if ctx.fused is not None:
+            patch = (patch_val, harg1) if patch_val is not None else None
             db_next = ops.colsum(dh)
-            du = ops.aggregate(dh, graph, mode=1)
-            for l in range(Lyr - 1, -1, -1):
-                w, b = params[2 * l], params[2 * l + 1]
-                dW, _ = ops.wgrad(hs[l - 1] if l > 0 else xr, du, bias_of=0)
-                grads_out[2 * l], grads_out[2 * l + 1] = dW.to(w.dtype), db_next.to(b.dtype)
-                grad_hook(grads_out[2 * l:2 * l + 2])
-                wk = ctx.w_n[l]
-                if l > 0:
-                    patch = (patch_val, harg1) if (l == 1 and patch_val is not None) else None
-                    du, _, _, db_next = ops.gcn_layer(du, wk, None, graph, 1, plan, rows, patch=patch, want_colsum=True)
-                else:
-                    dh = ops.linear(du, wk, None)
+            du = _fused_chain_bwd(ctx, ops.aggregate(dh, graph, mode=1), db_next, xr, hs, params, grads_out, grad_hook,
+                                  patch)
+            dh = ops.linear(du, ctx.w_n[0], None)
         else:
+            no_side = _Side(False, dev)
             for l in range(Lyr - 1, -1, -1):
                 if l == 0 and patch_val is not None:
                     # the views' share of d h_1 at the sentences' arg-max rows ((row, column) targets are distinct):
@@ -1043,38 +910,18 @@ class _GatedPairsFn(torch.autograd.Function):
                     zero = torch.zeros((1, graph.n_graphs, D), dtype=torch.float32, device=dev)
                     ops.views_bwd(zero, harg1.unsqueeze(0), zero + 1.0, hs[0], None, patch_val.unsqueeze(0), dh, None,
                                   parts=1)
-                w, b = params[2 * l], params[2 * l + 1]
-                if cfg["relu"]:
-                    dh = ops.as_rows(dh * (hs[l] > 0), cd)
-                msp = ctx.ms_split[l]
-                dh2 = ops.split_rows(dh) if msp is not None else None
-                if msp is not None:
-                    dW, db = ops.wgrad_split(ops.SplitRows(ms[l], *msp), dh2, bias_of=2)
-                else:
-                    dW, db = ops.wgrad(ms[l], dh, bias_of=2)
-                grads_out[2 * l], grads_out[2 * l + 1] = dW.to(w.dtype), db.to(b.dtype)
-                grad_hook(grads_out[2 * l:2 * l + 2])
-                wk = ctx.w_n[l]
-                dm = ops.linear_split(dh2, ops.split_rows(wk), None) if msp is not None else ops.linear(dh, wk, None)
-                dh = ops.aggregate(dm, graph, mode=1)
+                dh = ops.aggregate(_unfused_layer_bwd(ctx, l, dh, hs, ms, params, grads_out, grad_hook, no_side),
+                                   graph, mode=1)
         dx = dh
         # ---- d x at the trigger rows: the head's and the gate MLPs' d a of every pair, in pair order
         da = ga_head.float() if ga_head is not None else None
         if da_gate is not None:
             da = da_gate if da is None else da + da_gate
         if (da is not None or da_extra is not None) and P > 0:
-            ops.trigger_scatter_add_pairs(da, pairs, anchor, dx, extra=da_extra)
+            ops.trigger_scatter_add_pairs(da, pairs, cfg["anchor"], dx, extra=da_extra)
         grads_out[-2], grads_out[-1] = d_fcw, d_fcb
         grad_hook([g for g in (d_fcw, d_fcb) if g is not None])
-        if ctx.x_padded:
-            dx = dx.as_strided((N, dx.stride(0)), (dx.stride(0), 1))
-            if dx.shape[1] != ctx.x_cols:
-                full = torch.zeros((N, ctx.x_cols), dtype=dx.dtype, device=dev)
-                full[:, :D] = dx[:, :D]
-                dx = full
-        if dx.dtype != ctx.x_dtype:
-            dx = dx.to(ctx.x_dtype)
-        return (None, dx) + tuple(grads_out) + tuple(head_grads)
+        return (None, _dx_like_x(ctx, dx)) + tuple(grads_out) + tuple(head_grads)
 
 
 class GatedGCNStack(nn.Module):
@@ -1164,22 +1011,9 @@ class GatedGCNStack(nn.Module):
         if x.dim() == 3:
             shape3 = x.shape
             x = x.reshape(-1, x.shape[-1])
-        dist = dist_to_target.reshape(-1)
-        if dist.dtype not in (torch.int32, torch.int64):
-            dist = dist.long()
-        dist = dist.contiguous()
-        lead, pairs = GATE_ARCHS[self.gate_arch]
-        if x.shape[-1] != self.hidden and x.shape[-1] != ops.row_pitch(self.hidden, x.dtype):
-            raise L.EdgError(f"expected {self.hidden} feature columns (or the padded pitch), got {x.shape[-1]}")
-        from .head import DenseHead
-        dense_head = logits_fn if isinstance(logits_fn, DenseHead) and logits_fn.fusable(self.hidden) else None
-        if isinstance(logits_fn, DenseHead):        # its parameters are the head parameters: nothing to declare
-            head_params = [p for p in (logits_fn.weight, logits_fn.bias) if p is not None]
-        cfg = dict(graph=graph, cdtype=self.compute_dtype, D=self.hidden, dense_head=dense_head, L=self.n_layers, pairs=pairs, lead=lead,
-                   anchor=anchor_index.to(torch.int32).contiguous(), dist=dist, logits_fn=logits_fn,
-                   head_params=list(head_params), n_head=len(list(head_params)), grad_enabled=torch.is_grad_enabled(), grad_hook=self.grad_ready_hook, bucket_hook=self.grad_bucket_hook,
-                   relu=self.relu, return_x_out=return_x_out, gated=self.gated,
-                   drop_p=drop_p, seed=seed, fc_sigmoid=self.fc_sigmoid, view_len=view_len)
+        cfg = self._cfg(x, graph, anchor_index, dist_to_target.reshape(-1), logits_fn, head_params)
+        cfg.update(bucket_hook=self.grad_bucket_hook, return_x_out=return_x_out, drop_p=drop_p, seed=seed,
+                   view_len=view_len)
         logits, xy, kl, scores, pooled, x_out, p_arg, v_arg = _GatedStackFn.apply(cfg, x, aspect, *self._flat_params(),
                                                                                  *cfg["head_params"])
         if shape3 is not None:
@@ -1187,6 +1021,24 @@ class GatedGCNStack(nn.Module):
             if x_out is not None:
                 x_out = x_out.reshape(shape3)
         return StackOutput(logits, xy, kl, scores, pooled, x_out, p_arg, v_arg)
+
+    def _cfg(self, x, graph, anchor_index, dist, logits_fn, head_params) -> dict:
+        """The non-tensor arguments both block Functions read (``dist`` flat)."""
+        if dist.dtype not in (torch.int32, torch.int64):
+            dist = dist.long()
+        if x.shape[-1] != self.hidden and x.shape[-1] != ops.row_pitch(self.hidden, x.dtype):
+            raise L.EdgError(f"expected {self.hidden} feature columns (or the padded pitch), got {x.shape[-1]}")
+        lead, gate_linears = GATE_ARCHS[self.gate_arch]
+        from .head import DenseHead
+        dense_head = logits_fn if isinstance(logits_fn, DenseHead) and logits_fn.fusable(self.hidden) else None
+        if isinstance(logits_fn, DenseHead):        # its parameters are the head parameters: nothing to declare
+            head_params = [p for p in (logits_fn.weight, logits_fn.bias) if p is not None]
+        head_params = list(head_params)
+        return dict(graph=graph, cdtype=self.compute_dtype, D=self.hidden, dense_head=dense_head, L=self.n_layers,
+                    gate_linears=gate_linears, lead=lead, anchor=anchor_index.to(torch.int32).contiguous(),
+                    dist=dist.contiguous(), logits_fn=logits_fn, head_params=head_params, n_head=len(head_params),
+                    grad_enabled=torch.is_grad_enabled(), grad_hook=self.grad_ready_hook, relu=self.relu,
+                    gated=self.gated, fc_sigmoid=self.fc_sigmoid)
 
     def _forward_pairs(self, x, graph, anchor_index, dist_to_target, logits_fn, head_params, return_x_out, aspect,
                        view_len, pairs: TriggerPairs) -> StackOutput:
@@ -1216,21 +1068,8 @@ class GatedGCNStack(nn.Module):
         dist = dist_to_target.reshape(-1)
         if dist.numel() != pairs.n_pair_rows:
             raise L.EdgError(f"dist_to_target must be per-pair packed ({pairs.n_pair_rows} entries), got {dist.numel()}")
-        if dist.dtype not in (torch.int32, torch.int64):
-            dist = dist.long()
-        dist = dist.contiguous()
-        lead, npr = GATE_ARCHS[self.gate_arch]
-        if x.shape[-1] != self.hidden and x.shape[-1] != ops.row_pitch(self.hidden, x.dtype):
-            raise L.EdgError(f"expected {self.hidden} feature columns (or the padded pitch), got {x.shape[-1]}")
-        from .head import DenseHead
-        dense_head = logits_fn if isinstance(logits_fn, DenseHead) and logits_fn.fusable(self.hidden) else None
-        if isinstance(logits_fn, DenseHead):
-            head_params = [p for p in (logits_fn.weight, logits_fn.bias) if p is not None]
-        cfg = dict(graph=graph, pairs=pairs, cdtype=self.compute_dtype, D=self.hidden, dense_head=dense_head,
-                   L=self.n_layers, gate_pairs=npr, lead=lead, anchor=anchor_index.to(torch.int32).contiguous(), dist=dist,
-                   logits_fn=logits_fn, head_params=list(head_params), n_head=len(list(head_params)),
-                   grad_enabled=torch.is_grad_enabled(), grad_hook=self.grad_ready_hook, relu=self.relu,
-                   gated=self.gated, fc_sigmoid=False)
+        cfg = self._cfg(x, graph, anchor_index, dist, logits_fn, head_params)
+        cfg["pairs"] = pairs
         logits, xy, kl, scores, pooled, p_arg, v_arg = _GatedPairsFn.apply(cfg, x, *self._flat_params(),
                                                                            *cfg["head_params"])
         return StackOutput(logits, xy, kl, scores, pooled, None, p_arg, v_arg)

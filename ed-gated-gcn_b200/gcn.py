@@ -47,6 +47,36 @@ def cached_graph_from_dense(adj: torch.Tensor) -> DepGraph:
     return g
 
 
+def layer_fwd(m: torch.Tensor, wt: torch.Tensor, bias32: Optional[torch.Tensor], cdtype: torch.dtype, act: int):
+    """Projection of an unfused layer: ``act(m W + b)`` from the aggregated rows ``m = A_hat x`` and the K-major weight
+    ``wt [Dout,Din]``.  Returns ``(y, saved, split)``: ``saved`` is what :func:`layer_wgrad` reads, and ``split`` is None
+    or the metadata of its fp32 split form.  In fp32 the projection runs on the tensor cores from split operands
+    (ops.SplitRows); the split form of ``m`` is what the weight gradient reads, so it is saved instead of the fp32 rows
+    (same bytes, one split per layer)."""
+    if (cdtype == torch.float32 and ops.f32_tc(m.shape[0], m.shape[1], wt.shape[0])
+            and ops.f32_tc(m.shape[0], wt.shape[0], m.shape[1])):
+        m2 = ops.split_rows(m)
+        return ops.linear_split(m2, ops.split_rows(wt), bias32, act), m2.data, (m2.amax, m2.rows, m2.cols)
+    return ops.linear(m, wt, bias32, act=act), m, None
+
+
+def layer_dy_split(dy: torch.Tensor, split):
+    """The split form of ``dy`` when the layer ran split (shared by :func:`layer_wgrad` and :func:`layer_dgrad`)."""
+    return ops.split_rows(dy) if split is not None else None
+
+
+def layer_wgrad(saved: torch.Tensor, split, dy: torch.Tensor, dy2, bias_of: int):
+    """``dW = (A_hat x)^T dy [Din,Dout]`` and ``db = colsum(dy)`` from :func:`layer_fwd`'s saved rows."""
+    if split is not None:
+        return ops.wgrad_split(ops.SplitRows(saved, *split), dy2, bias_of=bias_of)
+    return ops.wgrad(saved, dy, bias_of=bias_of)
+
+
+def layer_dgrad(dy: torch.Tensor, dy2, w: torch.Tensor) -> torch.Tensor:
+    """``dy W^T`` with ``w [Din,Dout]`` (the input gradient before the adjoint aggregation)."""
+    return ops.linear_split(dy2, ops.split_rows(w), None) if dy2 is not None else ops.linear(dy, w, None)
+
+
 class _GCNLayerFn(torch.autograd.Function):
     """One graph convolution on packed rows: y = act((A_hat x) W + b).
 
@@ -59,20 +89,9 @@ class _GCNLayerFn(torch.autograd.Function):
         m = ops.aggregate(xr, graph, mode=0)                               # A_hat x          [N,Din]
         wt = ops.cast_weight(weight, cdtype, transpose=True)               # [Dout,Din], K-major
         b32 = bias.detach().float().contiguous() if bias is not None else None
-        act = L.ACT_RELU if relu else L.ACT_NONE
-        # fp32 mode: the projection runs on the tensor cores from split operands (ops.SplitRows); the split form
-        # of A_hat x is what the weight gradient reads, so it is saved instead of the fp32 rows
-        split = cdtype == torch.float32 and ops.f32_tc(m.shape[0], m.shape[1], wt.shape[0]) \
-            and ops.f32_tc(m.shape[0], wt.shape[0], m.shape[1])
-        if split:
-            m2 = ops.split_rows(m)
-            y = ops.linear_split(m2, ops.split_rows(wt), b32, act)
-            ctx.m_amax, ctx.m_shape = m2.amax, m2.shape
-            m = m2.data
-        else:
-            y = ops.linear(m, wt, b32, act=act)                            # [N,Dout]
+        y, m, ctx.split = layer_fwd(m, wt, b32, cdtype, L.ACT_RELU if relu else L.ACT_NONE)
         ctx.set_materialize_grads(False)
-        ctx.graph, ctx.cdtype, ctx.relu, ctx.has_bias, ctx.split = graph, cdtype, relu, bias is not None, split
+        ctx.graph, ctx.cdtype, ctx.relu, ctx.has_bias = graph, cdtype, relu, bias is not None
         ctx.x_dtype = x.dtype
         ctx.save_for_backward(m, weight, y if relu else None)
         return y
@@ -87,18 +106,13 @@ class _GCNLayerFn(torch.autograd.Function):
             dy = dy * (y > 0)
         dyr = ops.as_rows(dy, cdtype)
         dW = db = dx = None
-        want_w = ctx.needs_input_grad[1] or ctx.has_bias
-        dy2 = ops.split_rows(dyr) if ctx.split else None                   # shared by dW and dx
-        if want_w:
-            if ctx.split:
-                m2 = ops.SplitRows(m, ctx.m_amax, *ctx.m_shape)
-                dW, db = ops.wgrad_split(m2, dy2, bias_of=2 if ctx.has_bias else 0)
-            else:
-                dW, db = ops.wgrad(m, dyr, bias_of=2 if ctx.has_bias else 0)   # [Din,Dout], [Dout]
+        dy2 = layer_dy_split(dyr, ctx.split)
+        if ctx.needs_input_grad[1] or ctx.has_bias:
+            dW, db = layer_wgrad(m, ctx.split, dyr, dy2, bias_of=2 if ctx.has_bias else 0)   # [Din,Dout], [Dout]
         if ctx.needs_input_grad[0]:
             w = ops.cast_weight(weight, cdtype, transpose=False)           # [Din,Dout] = B operand of dy W^T
-            dm = ops.linear_split(dy2, ops.split_rows(w), None) if ctx.split else ops.linear(dyr, w, None)   # [N,Din]
-            dx = ops.aggregate(dm, graph, mode=1, out_dtype=ctx.x_dtype if ctx.x_dtype in L.DTYPES else cdtype)
+            dx = ops.aggregate(layer_dgrad(dyr, dy2, w), graph, mode=1,
+                               out_dtype=ctx.x_dtype if ctx.x_dtype in L.DTYPES else cdtype)
             if dx.dtype != ctx.x_dtype:
                 dx = dx.to(ctx.x_dtype)
         return dx, dW, db, None, None, None
