@@ -109,4 +109,28 @@ __device__ __forceinline__ void store_from_f32(void* p, int dtype, int64_t idx, 
 
 __device__ __forceinline__ float sigmoidf_(float x) { return 1.0f / (1.0f + expf(-x)); }
 
+// ---- gate dropout mask (include/edgcn.h, edg_dropout_rows) ----------------------------------------------------
+// keep(seed, stream, row, column) is a counter-based hash, so every kernel that applies or differentiates the mask
+// regenerates it where it needs it and nothing is stored.  The format is restated bit for bit by the tests (numpy).
+__host__ __device__ __forceinline__ uint32_t mix32(uint32_t x) {
+  x ^= x >> 16; x *= 0x7feb352dU; x ^= x >> 15; x *= 0x846ca68bU; x ^= x >> 16;
+  return x;
+}
+struct DropKey { uint32_t lo, hi; };
+// the per-stream key from the DEVICE seed (a captured graph reads a new seed on every replay)
+__device__ __forceinline__ DropKey dropout_key(const int64_t* seed, uint32_t stream_id) {
+  const uint64_t sd = (uint64_t)__ldg(seed);
+  return DropKey{(uint32_t)sd ^ (stream_id * 0xC2B2AE3DU), (uint32_t)(sd >> 32)};
+}
+__device__ __forceinline__ bool dropout_keep(DropKey k, uint32_t row, uint32_t col, uint32_t thr) {
+  const uint32_t u = mix32(mix32(row * 0x9E3779B1U + k.lo) ^ (col * 0x85EBCA77U + k.hi));
+  return u >= thr;
+}
+// an element is kept when its hash is >= floor(p * 2^32); p in [0, 1)
+inline uint32_t dropout_threshold(float p) {
+  const double t = (double)p * 4294967296.0;
+  return t >= 4294967295.0 ? 4294967295U : (uint32_t)t;
+}
+inline bool dropout_p_ok(float p) { return p >= 0.f && p < 1.f; }
+
 }  // namespace edg

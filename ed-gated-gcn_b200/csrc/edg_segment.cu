@@ -236,17 +236,8 @@ extern "C" int edg_lr_pool_bwd(const float* g, const int32_t* arg, int32_t B, in
 //     y[t,d] (+)= x[t,d] * keep(t,d) / (1 - p),
 // and every kernel of the gated block then runs unchanged on the masked rows; the backward pass multiplies the row
 // gradient by the same mask, regenerated from the seed (nothing is stored).
-// keep(t,d) is a counter-based hash of (seed, stream, row, column) -- restated in tests with numpy, bit for bit.
+// keep(t,d) is a counter-based hash of (seed, stream, row, column) (edg_common.cuh, dropout_keep).
 namespace edg {
-
-__host__ __device__ __forceinline__ uint32_t mix32(uint32_t x) {
-  x ^= x >> 16; x *= 0x7feb352dU; x ^= x >> 15; x *= 0x846ca68bU; x ^= x >> 16;
-  return x;
-}
-__device__ __forceinline__ bool dropout_keep(uint32_t key_lo, uint32_t key_hi, uint32_t row, uint32_t col, uint32_t thr) {
-  const uint32_t u = mix32(mix32(row * 0x9E3779B1U + key_lo) ^ (col * 0x85EBCA77U + key_hi));
-  return u >= thr;
-}
 
 template <typename T>
 __global__ void __launch_bounds__(256)
@@ -257,14 +248,13 @@ dropout_rows_kernel(const T* __restrict__ x, int64_t ldx, T* __restrict__ y, int
   const int row = (int)(idx / chunks);
   if (row >= N) return;
   const int c = (int)(idx - (int64_t)row * chunks) * E;
-  const uint64_t sd = (uint64_t)__ldg(seed);
-  const uint32_t key_lo = (uint32_t)sd ^ (stream_id * 0xC2B2AE3DU), key_hi = (uint32_t)(sd >> 32);
+  const DropKey key = dropout_key(seed, stream_id);
   float f[E], o[E];
   Vec16<T>::load(x + (int64_t)row * ldx + c, f);
   if (accumulate) Vec16<T>::load(y + (int64_t)row * ldy + c, o);
 #pragma unroll
   for (int k = 0; k < E; ++k) {
-    const float v = (c + k < D && dropout_keep(key_lo, key_hi, (uint32_t)row, (uint32_t)(c + k), thr)) ? f[k] * scale : 0.f;
+    const float v = (c + k < D && dropout_keep(key, (uint32_t)row, (uint32_t)(c + k), thr)) ? f[k] * scale : 0.f;
     o[k] = accumulate ? o[k] + v : v;
   }
   Vec16<T>::store(y + (int64_t)row * ldy + c, o);
@@ -274,15 +264,14 @@ dropout_rows_kernel(const T* __restrict__ x, int64_t ldx, T* __restrict__ y, int
 
 extern "C" int edg_dropout_rows(const void* x, int dtype, int64_t ldx, void* y, int64_t ldy, int32_t N, int32_t D,
                                 const int64_t* seed, int32_t stream_id, float p, int accumulate, edg_stream stream) {
-  if (N < 0 || D <= 0 || !(p >= 0.f) || !(p < 1.f)) return EDG_ERR_ARG;
+  if (N < 0 || D <= 0 || !edg::dropout_p_ok(p)) return EDG_ERR_ARG;
   if (N == 0) return EDG_OK;
   if (!x || !y || !seed || ldx < D || ldy < D) return EDG_ERR_ARG;
   if (!edg::aligned16(x) || !edg::aligned16(y) || !edg::row_pitch_ok(dtype, ldx) || !edg::row_pitch_ok(dtype, ldy)) return EDG_ERR_ALIGN;
   const int E = dtype == EDG_BF16 ? 8 : 4;
   const int chunks = (D + E - 1) / E;
   if ((int64_t)chunks * E > ldx || (int64_t)chunks * E > ldy) return EDG_ERR_ALIGN;
-  double t = (double)p * 4294967296.0;
-  const uint32_t thr = t >= 4294967295.0 ? 4294967295U : (uint32_t)t;
+  const uint32_t thr = edg::dropout_threshold(p);
   const float scale = 1.0f / (1.0f - p);
   const int64_t total = (int64_t)N * chunks;
   const unsigned grid = (unsigned)((total + 255) / 256);

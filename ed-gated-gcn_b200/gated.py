@@ -76,6 +76,12 @@ _BUCKET_LINEAR_SMS = 148 - int(os.environ.get("EDG_ALLREDUCE_SMS", "32"))
 _FUSED = os.environ.get("EDG_FUSED", "1") != "0"
 
 
+def _dropout_seed(device) -> torch.Tensor:
+    """The gate-dropout seed of one forward pass: a DEVICE int64 scalar drawn from torch's CUDA generator, so a captured
+    CUDA graph draws fresh masks on every replay and ``torch.manual_seed`` makes them reproducible."""
+    return torch.randint(0, 2 ** 62, (1,), dtype=torch.int64, device=device)
+
+
 def _fused_plan(cfg, cd, D, graph, drop_p):
     """(tile_rows, plan) when the whole GCN chain can run on ``edg_gcn_layer``: bf16, no ReLU, no gate dropout, no
     BertAmir54 head, every sentence fits a tile.  Otherwise None (the unfused kernels cover everything)."""
@@ -788,15 +794,18 @@ class _GatedPairsFn(torch.autograd.Function):
         gates = (torch.empty if gated else torch.ones)((Lyr, P, D), dtype=torch.float32, device=x.device)
         ctx.use_chain = gated and _chain_ok(cd, D, Lyr, cfg["gate_linears"])
         gate_saved = _gates_fwd(s0, gate_p, w_n[Lyr:], gates, cd, ctx.use_chain) if gated and P > 0 else []
+        # gate dropout (pair_dropout=True): every pair pools and scores its own masked copy of the sentence rows, so the
+        # per-sentence column maxima below are not used
+        drop_p, seed = (cfg["drop_p"], cfg["seed"]) if gated else (0.0, None)
         # ---- the GCN chain once per sentence, with the column maxima of h_1 (views) and h_L (final pool)
         h = xr
         ms, hs, ms_split = [], [], []
-        hmax1 = harg1 = None
-        fused = _fused_plan(cfg, cd, D, graph, 0.0)
+        hmax1 = harg1 = hm = ha = None
+        fused = _fused_plan(cfg, cd, D, graph, drop_p)
         ctx.fused = fused
         ones = None
         for l, (_, b) in enumerate(gcn_p):
-            want_pool = (l == 0 and gated) or l == Lyr - 1
+            want_pool = ((l == 0 and gated) or l == Lyr - 1) and drop_p == 0
             h, m, split, hm, ha = _layer_fwd(h, w_t[l], b, graph, cd, cfg["relu"], fused, want_pool)
             if fused is None and want_pool:
                 if ones is None:
@@ -812,20 +821,34 @@ class _GatedPairsFn(torch.autograd.Function):
         ps = pairs.pair_sent.long()
         xy = torch.zeros((), dtype=torch.float32, device=x.device)
         v_arg = None
-        if gated:
-            v_arg = harg1[ps].unsqueeze(0).expand(Lyr, P, D).contiguous()
-            if Lyr > 1 and P > 0:
-                xy = ops.diversity_fwd(gates * hmax1[ps].unsqueeze(0))     # views g_{v,p} * max_t h_1
         gL = gates[Lyr - 1]
         hL = hs[-1]
-        pooled = gL * hmaxL[ps]
-        p_arg = hargL[ps]
+        ctx.drop = None
+        if drop_p > 0:
+            # views: h_1 under the masks of streams 0..L-1; final pool and scores: h_L under stream L-1
+            v_pooled, v_arg, v_mmax = ops.pool_drop_pairs(hs[0], graph, pairs, gates, seed, 0, drop_p)
+            if Lyr > 1 and P > 0:
+                xy = ops.diversity_fwd(v_pooled)
+            pooled, p_arg, mmaxL = (t[0] for t in ops.pool_drop_pairs(hL, graph, pairs, gL.unsqueeze(0), seed, Lyr - 1,
+                                                                      drop_p))
+            ctx.drop = (drop_p, seed, v_pooled, v_mmax, v_arg.detach(), p_arg.detach(), mmaxL)
+        else:
+            if gated:
+                v_arg = harg1[ps].unsqueeze(0).expand(Lyr, P, D).contiguous()
+                if Lyr > 1 and P > 0:
+                    xy = ops.diversity_fwd(gates * hmax1[ps].unsqueeze(0))     # views g_{v,p} * max_t h_1
+            pooled = gL * hmaxL[ps]
+            p_arg = hargL[ps]
         # ---- classifier head on [P,D], then the per-pair scores / kl over the sentence rows
         ctx.set_materialize_grads(False)
         ctx.cfg = cfg
         ctx.fc_sig = None
         logits, v, c = _head_fwd(ctx, a_raw, pooled, a_raw, fc_w, fc_b)
-        scores, kl_b, kl, dvu, dcu = ops.scores_kl_pairs_fwd(hL, graph, pairs, gL, v, c, cfg["dist"])
+        if drop_p > 0:
+            scores, kl_b, kl, dvu, dcu = ops.scores_kl_drop_pairs_fwd(hL, graph, pairs, gL, v, c, cfg["dist"], seed,
+                                                                      Lyr - 1, drop_p)
+        else:
+            scores, kl_b, kl, dvu, dcu = ops.scores_kl_pairs_fwd(hL, graph, pairs, gL, v, c, cfg["dist"])
         ctx.kl_units = (dvu, dcu)
         ctx.gate_saved = gate_saved
         ctx.n_params = len(params)
@@ -862,26 +885,38 @@ class _GatedPairsFn(torch.autograd.Function):
         gated = cfg["gated"]
         views_active = g_xy is not None and Lyr > 1 and gated
         dgates = torch.empty((Lyr, P, D), dtype=torch.float32, device=dev)
+        drop = ctx.drop
+        if drop:
+            # the head backward on every pair's masked rows of h_L (stream L-1), with the pair's own final-pool rows
+            drop_p, seed, v_pooled, v_mmax, v_arg, p_arg, mmaxL = drop
+
+            def head_bwd(*a, **kw):
+                return ops.head_bwd_drop_pairs(*a, p_arg, mmaxL, seed, Lyr - 1, drop_p, **kw)
+        else:
+            def head_bwd(*a, **kw):
+                return ops.head_bwd_pairs(*a, hargL, **kw)
         # ---- d v, d c (per pair), the fc head and the classifier head
         dvc = None
         if need_scores:
             if g_scores is None:
                 dvc = (ctx.kl_units[0], ctx.kl_units[1], g_kl)
             else:
-                _, _, dv_in, dc_in = ops.head_bwd_pairs(hL, graph, pairs, gL, v, dist, scores, kl_b, g_kl, g_scores,
-                                                        None, None, want_dh=False)
+                _, _, dv_in, dc_in = head_bwd(hL, graph, pairs, gL, v, dist, scores, kl_b, g_kl, g_scores, None,
+                                              want_dh=False)
                 dvc = (dv_in, dc_in, None)
         ga_head, gp_total, d_fcw, d_fcb, head_grads = _head_bwd(ctx, g_logits, g_pooled, dvc, fc_w, fc_b, None, None)
         grad_hook([g for g in head_grads if g is not None and g.dtype == torch.float32])
         # ---- d h_L over the sentence rows (every pair of a sentence summed in pair order), d gate_L per pair
         if not views_active and Lyr > 1:
             dgates[:Lyr - 1].zero_()
-        dh, _, _, _ = ops.head_bwd_pairs(hL, graph, pairs, gL, v if need_scores else None, dist,
-                                         scores if need_scores else None, kl_b, g_kl, g_scores,
-                                         gp_total.contiguous() if gp_total is not None else None, hargL, want_dh=True,
-                                         dgate_out=dgates[Lyr - 1])
+        dh, _, _, _ = head_bwd(hL, graph, pairs, gL, v if need_scores else None, dist, scores if need_scores else None,
+                               kl_b, g_kl, g_scores, gp_total.contiguous() if gp_total is not None else None,
+                               want_dh=True, dgate_out=dgates[Lyr - 1])
         patch_val = None
-        if views_active:
+        if views_active and drop:
+            ops.views_bwd_drop_pairs(v_pooled, v_mmax, v_arg, gates, g_xy, graph, pairs, seed, drop_p, dgates=dgates,
+                                     acc_view=Lyr - 1)
+        elif views_active:
             patch_val = ops.views_bwd_hmax_pairs(hmax1, gates, g_xy, dgates, pairs, acc_view=Lyr - 1)
         grads_out: List[Optional[torch.Tensor]] = [None] * ctx.n_params
         o = 2 * Lyr
@@ -904,6 +939,9 @@ class _GatedPairsFn(torch.autograd.Function):
         else:
             no_side = _Side(False, dev)
             for l in range(Lyr - 1, -1, -1):
+                if l == 0 and views_active and drop:
+                    # the views' share of d h_1: every pair's view arg-max rows under that view's mask
+                    ops.views_bwd_drop_pairs(v_pooled, v_mmax, v_arg, gates, g_xy, graph, pairs, seed, drop_p, dh=dh)
                 if l == 0 and patch_val is not None:
                     # the views' share of d h_1 at the sentences' arg-max rows ((row, column) targets are distinct):
                     # edg_views_bwd_parts with one unit view adds g_pooled = patch_val at arg
@@ -931,7 +969,7 @@ class GatedGCNStack(nn.Module):
 
     def __init__(self, hidden: int, n_layers: int = 2, n_classes: int = 2, gate_arch: str = "sig-2",
                  relu: bool = False, dropout: float = 0.0, compute_dtype="f32", gated: bool = True,
-                 fc_sigmoid: bool = False):
+                 fc_sigmoid: bool = False, pair_dropout: bool = False):
         super().__init__()
         if hidden % 4:
             raise ValueError("hidden size must be a multiple of 4 (16-byte fp32 rows)")
@@ -940,6 +978,9 @@ class GatedGCNStack(nn.Module):
         self.gated = gated            # False = BertAmir55NoGate (gates constructed, as there, but unused: :672-681, :731-748)
         self.relu = relu
         self.dropout_p = dropout
+        # train-mode gate dropout on the pairs= path (per-pair passes over the sentence rows instead of [P,D] products:
+        # the caller asks for that cost explicitly); no effect without pairs, in eval mode, at p = 0 or ungated
+        self.pair_dropout = pair_dropout
         self.compute_dtype = _compute_dtype(compute_dtype)
         for l in range(1, n_layers + 1):
             setattr(self, f"gc{l}", GraphConvolution(hidden, hidden, None, compute_dtype=self.compute_dtype))
@@ -993,8 +1034,13 @@ class GatedGCNStack(nn.Module):
         ``view_arg [V,P,D]`` (global sentence rows) -- and ``xy`` / ``kl`` are means over the P pairs; ``logits_fn``
         receives ``[P,D]`` inputs.  The result equals the block run on the batch with each sentence repeated once per
         pair, ``dx`` being the sum over a sentence's pairs.  Valid only when ``x`` does not depend on the trigger
-        (no trigger marker or position features upstream).  Not covered (``EdgError``): train-mode gate dropout,
-        ``fc_sigmoid``, ``view_len``, ``aspect``, ``return_x_out`` and 3-D dense-compat ``x``."""
+        (no trigger marker or position features upstream).  Train-mode gate dropout (``dropout > 0``) needs
+        ``pair_dropout=True``: each pair then applies the masks the expanded batch would apply to its copy of the
+        sentence (keyed on the per-pair packed row ``pairs.pair_row_ptr[p] + t``), so for the same
+        ``last_dropout_seed`` the result equals the expanded run's, every pair with its own masks; the views and the
+        final pool become per-pair passes over the sentence rows.  Not covered (``EdgError``): train-mode gate dropout
+        without ``pair_dropout``, ``fc_sigmoid``, ``view_len``, ``aspect``, ``return_x_out`` and 3-D dense-compat
+        ``x``."""
         if not x.is_cuda:
             raise L.EdgError("GatedGCNStack runs on CUDA tensors only (there is no CPU path)")
         if pairs is not None:
@@ -1005,7 +1051,7 @@ class GatedGCNStack(nn.Module):
             # nn.Dropout on the broadcast gates (bert_amir5.py:624-625).  The seed is a DEVICE scalar drawn from
             # torch's CUDA generator, so a captured CUDA graph draws a fresh mask on every replay.
             drop_p = float(self.dropout_p)
-            seed = torch.randint(0, 2 ** 62, (1,), dtype=torch.int64, device=x.device)
+            seed = _dropout_seed(x.device)
             self.last_dropout_seed = seed
         shape3 = None
         if x.dim() == 3:
@@ -1043,8 +1089,9 @@ class GatedGCNStack(nn.Module):
     def _forward_pairs(self, x, graph, anchor_index, dist_to_target, logits_fn, head_params, return_x_out, aspect,
                        view_len, pairs: TriggerPairs) -> StackOutput:
         declined = []
-        if self.training and self.dropout_p > 0 and self.gated:
-            declined.append("train-mode gate dropout (p > 0)")
+        drop = self.training and self.dropout_p > 0 and self.gated
+        if drop and not self.pair_dropout:
+            declined.append("train-mode gate dropout (p > 0) unless GatedGCNStack(pair_dropout=True)")
         if self.fc_sigmoid:
             declined.append("fc_sigmoid")
         if view_len is not None:
@@ -1059,6 +1106,11 @@ class GatedGCNStack(nn.Module):
             declined.append("grad_bucket_hook (sharded grouped batches)")
         if declined:
             raise L.EdgError("pairs= does not cover: " + ", ".join(declined))
+        drop_p, seed = 0.0, None
+        if drop:
+            drop_p = float(self.dropout_p)
+            seed = _dropout_seed(x.device)
+            self.last_dropout_seed = seed
         if pairs.n_sentences != graph.n_graphs:
             raise L.EdgError(f"pairs were built for {pairs.n_sentences} sentences, the graph has {graph.n_graphs}")
         if x.shape[0] != graph.n_rows:
@@ -1069,7 +1121,7 @@ class GatedGCNStack(nn.Module):
         if dist.numel() != pairs.n_pair_rows:
             raise L.EdgError(f"dist_to_target must be per-pair packed ({pairs.n_pair_rows} entries), got {dist.numel()}")
         cfg = self._cfg(x, graph, anchor_index, dist, logits_fn, head_params)
-        cfg["pairs"] = pairs
+        cfg.update(pairs=pairs, drop_p=drop_p, seed=seed)
         logits, xy, kl, scores, pooled, p_arg, v_arg = _GatedPairsFn.apply(cfg, x, *self._flat_params(),
                                                                            *cfg["head_params"])
         return StackOutput(logits, xy, kl, scores, pooled, None, p_arg, v_arg)

@@ -645,6 +645,77 @@ def views_bwd_hmax_pairs(hmax: torch.Tensor, gates: torch.Tensor, g_xy, dgates: 
     return patch_val
 
 
+def pool_drop_pairs(h, graph, pairs, gates: torch.Tensor, seed: torch.Tensor, stream0: int, p: float):
+    """``edg_pool_drop_pairs``: the gated max-pool of every pair's masked rows, view v under dropout stream
+    ``stream0 + v`` -> ``(pooled fp32 [V,P,D], arg int32 [V,P,D] (global sentence rows), mmax fp32 [V,P,D])``."""
+    V, P, D = gates.shape
+    dev = h.device
+    pooled = torch.empty((V, P, D), dtype=torch.float32, device=dev)
+    arg = torch.empty((V, P, D), dtype=torch.int32, device=dev)
+    mmax = torch.empty((V, P, D), dtype=torch.float32, device=dev)
+    L.call("edg_pool_drop_pairs", L.ptr(h), L.dt(h), ld(h), L.ptr(graph.sent_ptr), L.ptr(pairs.pair_sent),
+           L.ptr(pairs.pair_row_ptr), P, D, L.ptr(gates.contiguous()), V, L.ptr(seed), int(stream0), float(p),
+           L.ptr(pooled), L.ptr(arg), L.ptr(mmax), L.stream())
+    return pooled, arg, mmax
+
+
+def scores_kl_drop_pairs_fwd(h, graph, pairs, gate, v, c, dist, seed: torch.Tensor, stream_id: int, p: float):
+    """:func:`scores_kl_pairs_fwd` on the pairs' masked rows of dropout stream ``stream_id``."""
+    P, D = gate.shape
+    dev = h.device
+    R = pairs.n_pair_rows
+    scores = torch.empty((max(R, 1),), dtype=torch.float32, device=dev)[:R]
+    kl_b = torch.empty((P,), dtype=torch.float32, device=dev)
+    dvu = torch.empty((P, D), dtype=torch.float32, device=dev)
+    dcu = torch.empty((P,), dtype=torch.float32, device=dev)
+    L.call("edg_scores_kl_drop_pairs_fwd", L.ptr(h), L.dt(h), ld(h), L.ptr(graph.sent_ptr), L.ptr(pairs.pair_sent),
+           L.ptr(pairs.pair_row_ptr), P, D, L.ptr(gate), L.ptr(v), L.ptr(c), L.ptr(dist), _dist_flag(dist), L.ptr(scores),
+           L.ptr(kl_b), L.ptr(dvu), L.ptr(dcu), None, None, L.ptr(seed), int(stream_id), float(p), L.stream())
+    kl = torch.empty((), dtype=torch.float32, device=dev)
+    L.call("edg_sum_scaled", L.ptr(kl_b), P, 1.0 / max(P, 1), L.ptr(kl), L.stream())
+    return scores, kl_b, kl, dvu, dcu
+
+
+def head_bwd_drop_pairs(h, graph, pairs, gate, v, dist, scores, kl_b, g_kl, g_scores, g_pooled, arg, mmax,
+                        seed: torch.Tensor, stream_id: int, p: float, want_dh: bool,
+                        dgate_out: Optional[torch.Tensor] = None):
+    """:func:`head_bwd_pairs` on the pairs' masked rows of dropout stream ``stream_id``; ``arg`` int32 / ``mmax`` fp32
+    ``[P,D]`` are the final pool's per-pair arg-max rows and masked maxima (:func:`pool_drop_pairs`)."""
+    P, D = gate.shape
+    N = h.shape[0]
+    dev = h.device
+    dh = alloc_rows(N, D, h.dtype, dev) if want_dh else None
+    dgate = (dgate_out if dgate_out is not None else torch.empty((P, D), dtype=torch.float32, device=dev)) \
+        if want_dh else None
+    dv = None if want_dh else torch.empty((P, D), dtype=torch.float32, device=dev)
+    dc = None if want_dh else torch.empty((P,), dtype=torch.float32, device=dev)
+    ds_ws = torch.empty((max(pairs.n_pair_rows, 1),), dtype=torch.float32, device=dev)
+    if want_dh and graph.row_sent is None:
+        raise L.EdgError("the pairs head backward needs graph.row_sent (build_graph / graph_from_dense set it)")
+    L.call("edg_head_bwd_drop_pairs", L.ptr(h), L.dt(h), ld(h), L.ptr(graph.sent_ptr), graph.n_graphs,
+           L.ptr(graph.row_sent) if N > 0 else None, N, L.ptr(pairs.pair_ptr),
+           L.ptr(pairs.pair_sent), L.ptr(pairs.pair_row_ptr), P, D, L.ptr(gate), L.ptr(v), L.ptr(dist),
+           _dist_flag(dist) if dist is not None else 0, L.ptr(scores), L.ptr(kl_b), L.ptr(g_kl), L.ptr(g_scores),
+           L.ptr(g_pooled), L.ptr(arg), L.ptr(mmax), L.ptr(dh), ld(dh) if dh is not None else 0, L.ptr(dgate), L.ptr(dv),
+           L.ptr(dc), L.ptr(ds_ws), L.ptr(seed), int(stream_id), float(p), L.stream())
+    return dh, dgate, dv, dc
+
+
+def views_bwd_drop_pairs(pooled, mmax, arg, gates, g_xy, graph, pairs, seed: torch.Tensor, p: float,
+                         dh: Optional[torch.Tensor] = None, dgates: Optional[torch.Tensor] = None,
+                         acc_view: int = -1) -> None:
+    """``edg_views_bwd_drop_pairs`` for the views of :func:`pool_drop_pairs` (streams 0..V-1): writes ``dgates
+    [V,P,D]`` (``acc_view`` accumulates) and / or adds the views' share of d h_1 into ``dh``."""
+    V, P, D = pooled.shape
+    N = graph.n_rows
+    if dh is not None and graph.row_sent is None:
+        raise L.EdgError("the pairs views backward needs graph.row_sent (build_graph / graph_from_dense set it)")
+    L.call("edg_views_bwd_drop_pairs", L.ptr(pooled), L.ptr(mmax), L.ptr(arg), L.ptr(gates), L.ptr(g_xy), V,
+           L.ptr(graph.sent_ptr), L.ptr(graph.row_sent) if (dh is not None and N > 0) else None, N, L.ptr(pairs.pair_ptr),
+           L.ptr(pairs.pair_row_ptr), P, D, L.ptr(seed), float(p), L.ptr(dh), L.dt(dh) if dh is not None else 0,
+           ld(dh) if dh is not None else 0, L.ptr(dgates), int(acc_view), L.stream())
+
+
 def trigger_scatter_add_pairs(da: Optional[torch.Tensor], pairs, anchor: torch.Tensor, dx: torch.Tensor,
                               extra: Optional[torch.Tensor] = None) -> None:
     """``dx[pair_start[p] + anchor[p]] += da[p] + extra.sum(0)[p]`` in pair order per sentence (anchors may repeat)."""

@@ -567,7 +567,8 @@ int edg_scores_kl_pairs_fwd(const void* h, int dtype, int64_t ldh, const int32_t
  *     dh_t = sum_{p of s} ds_{p,t} (gate_p * v_p) + [t = arg[s]] sum_{p of s} gate_p * g_pooled_p,
  *   dgate_p = v_p * sum_t ds_{p,t} h_t + g_pooled_p * h[arg[s]], and dv / dc when given.
  * arg int32 [S,D] = the sentence's global arg-max rows (-1 for an empty sentence), g_pooled fp32 [P,D] (NULL = 0).
- * ds_ws: fp32 workspace of pair_row_ptr[P] entries.  row_sent[N] (sentence of every row) is needed for dh. */
+ * ds_ws: fp32 workspace of pair_row_ptr[P] entries.  row_sent[N] (sentence of every row) is needed for dh.
+ * With P = 0 the per-pair arrays may be NULL: dh (when given) is written as 0, nothing else is written. */
 int edg_head_bwd_pairs(const void* h, int dtype, int64_t ldh, const int32_t* sent_ptr, int32_t S, const int32_t* row_sent,
                        int32_t N, const int32_t* pair_ptr,
                        const int32_t* pair_sent, const int32_t* pair_row_ptr, int32_t P, int32_t D, const float* gate,
@@ -580,6 +581,49 @@ int edg_head_bwd_pairs(const void* h, int dtype, int64_t ldh, const int32_t* sen
 int edg_views_bwd_hmax_pairs(const float* hmax, const float* gates, const float* g_xy, int32_t V, int32_t S,
                              const int32_t* pair_ptr, int32_t P, int32_t D, float* patch_val, int64_t ldp, float* dgates,
                              int acc_view, edg_stream stream);
+/* Gate dropout of the pairs (bert_amir5.py:624-625 on the expanded batch): pair p reads row t of its sentence under the
+ * edg_dropout_rows mask of that row's copy, keep(seed, stream, pair_row_ptr[p] + t, column), so for one seed the pairs
+ * apply exactly the masks the expanded batch applies; a kept element reads as T(h * 1/(1-p)) (rounded to the row dtype),
+ * a dropped one as 0.  Streams: v for view v of h_1, L-1 for the final pool / scores of h_L.  seed: device int64 scalar,
+ * p in [0, 1).  Masks are regenerated from the seed in both directions (nothing is stored per (pair, row)).
+ *
+ * Gated max-pool of the masked rows per pair, views v = 0..V-1 under streams stream0 + v (gates [V,P,D]): mmax [V,P,D]
+ * = column maximum of the pair's masked rows, pooled = mmax * gates, arg = its first row (global sentence row; the
+ * sentence's first row where the gate is 0).  A pair of an empty sentence gets pooled 0, arg -1, mmax 0; P = 0 does
+ * nothing. */
+int edg_pool_drop_pairs(const void* h, int dtype, int64_t ldh, const int32_t* sent_ptr, const int32_t* pair_sent,
+                        const int32_t* pair_row_ptr, int32_t P, int32_t D, const float* gates, int32_t V,
+                        const int64_t* seed, int32_t stream0, float p, float* pooled, int32_t* arg, float* mmax,
+                        edg_stream stream);
+/* edg_scores_kl_pairs_fwd on the masked rows of stream stream_id (same outputs, same empty-sentence and P = 0 rules). */
+int edg_scores_kl_drop_pairs_fwd(const void* h, int dtype, int64_t ldh, const int32_t* sent_ptr, const int32_t* pair_sent,
+                                 const int32_t* pair_row_ptr, int32_t P, int32_t D, const float* gate, const float* v,
+                                 const float* c, const void* dist, int dist_i64, float* scores, float* kl_b,
+                                 float* dv_unit, float* dc_unit, float* u_unit, float* sf_unit, const int64_t* seed,
+                                 int32_t stream_id, float p, edg_stream stream);
+/* edg_head_bwd_pairs on the masked rows of stream stream_id, with the final pool per pair: arg int32 [P,D] and mmax fp32
+ * [P,D] from edg_pool_drop_pairs (dgate_p = v_p * sum_t ds_{p,t} m_{p,t} + g_pooled_p * mmax_p) and
+ *   dh_t = sum_{p of s} keep_{p,t} / (1-p) * (ds_{p,t} gate_p v_p + [t = arg_p] gate_p g_pooled_p)
+ * (every row written; 0 where the sentence has no pairs, so P = 0 gives dh = 0).  A pair of an empty sentence gets
+ * dgate, dv and dc 0. */
+int edg_head_bwd_drop_pairs(const void* h, int dtype, int64_t ldh, const int32_t* sent_ptr, int32_t S,
+                            const int32_t* row_sent, int32_t N, const int32_t* pair_ptr, const int32_t* pair_sent,
+                            const int32_t* pair_row_ptr, int32_t P, int32_t D, const float* gate, const float* v,
+                            const void* dist, int dist_i64, const float* scores, const float* kl_b, const float* g_kl,
+                            const float* g_scores, const float* g_pooled, const int32_t* arg, const float* mmax, void* dh,
+                            int64_t lddh, float* dgate, float* dv, float* dc, float* ds_ws, const int64_t* seed,
+                            int32_t stream_id, float p, edg_stream stream);
+/* Backward of the masked views (streams 0..V-1) and the diversity term from edg_pool_drop_pairs' pooled / mmax / arg
+ * [V,P,D], with dP_{v,p} = g_xy / P * (sum_{v'} pooled_{v',p} - pooled_{v,p}):
+ *   dgates (optional) [V,P,D]:  dgates[v,p] (+)= dP_{v,p} * mmax_{v,p}   (+= for v = acc_view)
+ *   dh (optional, [N, lddh] compute dtype):  dh_t += sum_{p of s} sum_v [t = arg_{v,p}] keep_{v,p,t} / (1-p) gates_{v,p}
+ *       dP_{v,p}, pairs then views in ascending order summed in fp32 and added once; rows no view routes to are not
+ *       touched.  P = 0 does nothing. */
+int edg_views_bwd_drop_pairs(const float* pooled, const float* mmax, const int32_t* arg, const float* gates,
+                             const float* g_xy, int32_t V, const int32_t* sent_ptr, const int32_t* row_sent, int32_t N,
+                             const int32_t* pair_ptr, const int32_t* pair_row_ptr, int32_t P, int32_t D,
+                             const int64_t* seed, float p, void* dh, int dtype, int64_t lddh, float* dgates, int acc_view,
+                             edg_stream stream);
 /* edg_trigger_scatter_add per pair: dx[pair_start[p] + anchor[p]] += da[p] + sum_k extra[k][p], the pairs of a
  * sentence in ascending order (pairs may share a row). */
 int edg_trigger_scatter_add_pairs(const float* da, const float* extra, int32_t n_extra, int32_t S, const int32_t* pair_ptr,

@@ -12,7 +12,13 @@ forward, with CUDA events over ``--steps`` calls after ``--warmup``.  Reported: 
 bytes per batch (the x rows in bf16 plus the integer arrays each arm needs), and the card name and power limit read in
 the same run.  Writes one JSON line to stdout and, with ``--out``, to that file.
 
+``--dropout P`` runs both arms in train() mode with gate dropout P (the reference trainer's default is 0.25): the
+grouped arm with ``pair_dropout=True`` (per-pair masked passes over the sentence rows), the expanded arm on the existing
+path (masked copies of the expanded rows).  Both arms draw their masks from the same seed, so they compute the same
+result.
+
     python tools/bench_pairs.py --sentences 149 --steps 100 --warmup 10 --rounds 3 --out profiles/r04_a_bench_pairs.json
+    python tools/bench_pairs.py --dropout 0.25 --out profiles/r05_a_bench_pairs_dropout.json
 """
 from __future__ import annotations
 
@@ -45,6 +51,7 @@ def main():
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--rounds", type=int, default=3)
     ap.add_argument("--seed", type=int, default=14181)
+    ap.add_argument("--dropout", type=float, default=0.0)
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
 
@@ -65,7 +72,8 @@ def main():
     e_sp[1:] = np.cumsum(batch.lengths[owner])
 
     torch.manual_seed(args.seed)
-    stack = E.GatedGCNStack(D, n_layers=Lyr, n_classes=C, compute_dtype=cd).to(dev)
+    stack = E.GatedGCNStack(D, n_layers=Lyr, n_classes=C, compute_dtype=cd, dropout=args.dropout,
+                            pair_dropout=args.dropout > 0).to(dev)
     head = E.DenseHead(2 * D, C).to(dev)
     x_host = torch.randn(batch.n_rows, D, generator=torch.Generator().manual_seed(args.seed + 1)).to(cd)
     tgt = (torch.arange(P) % C).to(dev)
@@ -106,7 +114,9 @@ def main():
         return fn
 
     # same results: the grouped arm must reproduce the expanded one
+    torch.manual_seed(args.seed + 2)                   # the same dropout seed for both arms
     lg = fwd_step(arms["grouped"])().float()
+    torch.manual_seed(args.seed + 2)
     le = fwd_step(arms["expanded"])().float()
     max_rel_logits = float((lg - le).abs().max() / le.abs().max())
 
@@ -132,6 +142,7 @@ def main():
     name, pl = card()
     res = {"tool": "bench_pairs", "gpu": name, "power_limit": pl, "sentences": batch.n_graphs, "pairs": P,
            "sentence_rows": batch.n_rows, "expanded_rows": int(len(rows)), "D": D, "L": Lyr, "dtype": "bf16",
+           "dropout": args.dropout,
            "steps": args.steps, "warmup": args.warmup, "rounds": args.rounds, "max_rel_logits_grouped_vs_expanded":
            max_rel_logits, "arms": {}}
     for n in arms:
