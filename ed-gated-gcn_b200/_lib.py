@@ -36,15 +36,13 @@ SIGNATURES = {
     "edg_tree_dist": (c_int, [_P, _P, _P, _P, _I, _I, _P, _P]),
     "edg_dist_pad": (c_int, [_P, _P, _I, _I, c_int, _P, _P]),
     "edg_aggregate": (c_int, [_P, c_int, _L, _P, c_int, _L, _I, _I, _P, _P, c_int, _P, _P, _I, _I, _P]),
-    "edg_aggregate_patched": (c_int, [_P, c_int, _L, _P, c_int, _L, _I, _I, _P, _P, c_int, _P, _P, _I, _I, _P, _P, _I, _P]),
     "edg_fused_tile_rows": (c_int, [_I, _I]),
     "edg_views_bwd_hmax": (c_int, [_P, _P, _P, _I, _I, _I, _P, _L, _P, c_int, _P]),
     "edg_head_du_workspace": (_Z, [_I]),
     "edg_head_du": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P, _L, _P, _P, _P, _Z, _P]),
     "edg_tile_plan": (c_int, [_P, _P, _I, _I, _P, _P, _P]),
     "edg_gcn_layer": (c_int, [_P, _L, _I, _I, _P, _L, _I, _P, c_int, _P, _P, _P, _P, _P, _I, _P, _L, _P, _P, _L, _P, _P,
-                              _L, _P, c_int, _P, _Z, _P, _P]),
-    "edg_row_meta": (c_int, [_P, _P, _P, _P, _I, _P, _P]),
+                              _L, _P, c_int, _P, _Z, _P]),
     "edg_adam_multi": (c_int, [_I, _P, _P, _P, _P, _P, _P, c_float, c_float, c_float, c_float, c_float, c_float, _P]),
     "edg_dense_head_fwd": (c_int, [_P, _L, _P, _L, _P, _L, _P, _I, _I, _I, _P, _L, _P]),
     "edg_dense_head_bwd_workspace": (_Z, [_I, _I, _I]),
@@ -76,7 +74,6 @@ SIGNATURES = {
     "edg_diversity_fwd": (c_int, [_P, _I, _I, _I, _P, _P, _P]),
     "edg_views_bwd": (c_int, [_P, _P, _P, _P, c_int, _L, _I, _I, _I, _P, _P, _P, _L, _P, c_int, _P]),
     "edg_views_bwd_parts": (c_int, [_P, _P, _P, _P, c_int, _L, _I, _I, _I, _P, _P, _P, _L, _P, c_int, c_int, _P]),
-    "edg_views_patch": (c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _P, c_int, _P]),
     "edg_scores_kl_fwd": (c_int, [_P, c_int, _L, _P, _I, _I, _P, _P, _P, _P, c_int, _P, _P, _P, _P, _P, _P, _P, _I, _I, _P]),
     "edg_fc_head_fwd": (c_int, [_P, _L, _P, _L, _P, _P, _L, _I, _I, _I, _P, _P, _P]),
     "edg_fc_head_bwd_workspace": (_Z, [_I, _I, _I]),

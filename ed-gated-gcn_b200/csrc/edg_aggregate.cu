@@ -6,8 +6,6 @@
 // request is a fully used 32-byte sector stream.  A row's neighbours live in the same
 // sentence (a few KB away), so the 2-3 extra row reads per output row hit L1/L2; compulsory
 // DRAM traffic is one read + one write of the [N,D] matrix plus 16 B/row of CSR.
-#include <stdlib.h>
-
 #include "edg_staged.cuh"
 
 namespace edg {
@@ -29,39 +27,10 @@ template <> __device__ __forceinline__ void store_chunk<__nv_bfloat16, 4>(__nv_b
   *reinterpret_cast<uint2*>(p) = make_uint2(*reinterpret_cast<uint32_t*>(&a), *reinterpret_cast<uint32_t*>(&b));
 }
 
-// Optional epilogue of the adjoint pass: y[patch_arg[b,d], d] += patch_val[b,d] -- the gradient that the gated
-// max-pool views of layer 1 (bert_amir5.py:627-636) route to their arg-max rows, folded into the kernel that
-// produces d h_1 instead of a separate scattered read-modify-write pass (edg_views_patch builds the two arrays).
-struct AggPatch { const int16_t* loc; const float* val; const int32_t* row_sent; const int32_t* sent_ptr; int D, ldp; };
-
-// loc = sentence-local row index per (sentence, column) or -1, pitch ldp (multiple of 8): one 8- or 16-byte load
-// covers the thread's E columns
-template <int E>
-__device__ __forceinline__ void apply_patch_at(const AggPatch& p, int64_t o, int lr, float (&acc)[E]) {
-  uint32_t w[E / 2];
-  if (E == 8) {
-    const uint4 q = __ldg(reinterpret_cast<const uint4*>(p.loc + o));
-    w[0] = q.x; w[1] = q.y; w[E / 2 - 2] = q.z; w[E / 2 - 1] = q.w;
-  } else {
-    const uint2 q = __ldg(reinterpret_cast<const uint2*>(p.loc + o));
-    w[0] = q.x; w[1] = q.y;
-  }
-#pragma unroll
-  for (int k = 0; k < E; ++k) {
-    const int l = (int)(int16_t)((k & 1) ? (w[k >> 1] >> 16) : (w[k >> 1] & 0xffffu));
-    if (l == lr) acc[k] += __ldg(p.val + o + k);
-  }
-}
-template <int E>
-__device__ __forceinline__ void apply_patch(const AggPatch& p, int row, int c, float (&acc)[E]) {
-  const int b = __ldg(p.row_sent + row);
-  apply_patch_at<E>(p, (int64_t)b * p.ldp + c, row - __ldg(p.sent_ptr + b), acc);
-}
-
 template <typename TI, typename TO, int MODE>
 __global__ void __launch_bounds__(256)
 aggregate_flat_kernel(const TI* __restrict__ x, int64_t ldx, TO* __restrict__ y, int64_t ldy, int N, int chunks,
-                 const int32_t* __restrict__ row_ptr, const int32_t* __restrict__ col, AggPatch patch) {
+                 const int32_t* __restrict__ row_ptr, const int32_t* __restrict__ col) {
   constexpr int E = Vec16<TI>::kElems;
   const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int row = (int)(idx / chunks);
@@ -104,7 +73,6 @@ aggregate_flat_kernel(const TI* __restrict__ x, int64_t ldx, TO* __restrict__ y,
 #pragma unroll
     for (int k = 0; k < E; ++k) acc[k] = acc[k] / den;
   }
-  if (patch.loc) apply_patch<E>(patch, row, c, acc);
   store_chunk<TO, E>(y + (int64_t)row * ldy + c, acc);
 }
 
@@ -121,7 +89,7 @@ __device__ __forceinline__ uint32_t agg_smem_u32(const void* p) { return (uint32
 template <typename TI, typename TO, int MODE>
 __device__ __noinline__ void aggregate_rows_global(const TI* __restrict__ x, int64_t ldx, TO* __restrict__ y, int64_t ldy,
                                                    int r0, int r1, const int32_t* __restrict__ row_ptr,
-                                                   const int32_t* __restrict__ col, const AggPatch& patch) {
+                                                   const int32_t* __restrict__ col) {
   constexpr int E = Vec16<TI>::kElems;
   const int c = threadIdx.x * E;
   for (int row = r0 + threadIdx.y; row < r1; row += blockDim.y) {
@@ -142,19 +110,18 @@ __device__ __noinline__ void aggregate_rows_global(const TI* __restrict__ x, int
 #pragma unroll
       for (int k = 0; k < E; ++k) acc[k] *= inv;
     }
-    if (patch.loc) apply_patch<E>(patch, row, c, acc);
     store_chunk<TO, E>(y + (int64_t)row * ldy + c, acc);
   }
 }
 
-// PATCH / MAXT are compile-time so that the default instantiation (no patch arrays, 384-thread blocks) carries
-// neither the patch code nor the 64-register cap of 1024-thread blocks (they cost ~2-4 us per launch at C2)
-template <typename TI, typename TO, int MODE, bool PATCH, int MAXT>
+// MAXT is compile-time so that the default instantiation (384-thread blocks) does not carry the 64-register cap of
+// 1024-thread blocks (it costs ~2-4 us per launch at C2)
+template <typename TI, typename TO, int MODE, int MAXT>
 __global__ void __launch_bounds__(MAXT)
 aggregate_staged_kernel(const TI* __restrict__ x, int64_t ldx, TO* __restrict__ y, int64_t ldy, int N, int B,
                         int tile_rows, int cap_rows, const int32_t* __restrict__ sent_ptr,
                         const int32_t* __restrict__ row_sent, const int32_t* __restrict__ row_ptr,
-                        const int32_t* __restrict__ col, AggPatch patch) {
+                        const int32_t* __restrict__ col) {
   constexpr int E = Vec16<TI>::kElems;
   extern __shared__ __align__(128) uint8_t agg_smem[];
   __shared__ __align__(8) uint64_t bar;
@@ -165,8 +132,6 @@ aggregate_staged_kernel(const TI* __restrict__ x, int64_t ldx, TO* __restrict__ 
   int32_t* rp_s = reinterpret_cast<int32_t*>(agg_smem + (size_t)cap_rows * pitch);   // [cap_rows + 1] (+3 pad)
   int32_t* col_s = rp_s + cap_rows + 4;                                             // [4 * cap_rows] tile-local ids
   float* inv_s = reinterpret_cast<float*>(col_s + 4 * cap_rows);                    // [cap_rows] 1/(deg+1)
-  int32_t* poff_s = reinterpret_cast<int32_t*>(inv_s + cap_rows);                   // [cap_rows] sentence * ldp   (patch)
-  int32_t* plr_s = poff_s + cap_rows;                                               // [cap_rows] row - sentence start
   const int cap_nnz = 4 * cap_rows;
   const uint32_t b32 = agg_smem_u32(&bar);
   if (tid == 0) {
@@ -192,7 +157,7 @@ aggregate_staged_kernel(const TI* __restrict__ x, int64_t ldx, TO* __restrict__ 
   const int r0 = range[0], r1 = range[1], n = r1 - r0;
   if (n <= 0) return;
   if (n > cap_rows) {                               // nothing was staged
-    aggregate_rows_global<TI, TO, MODE>(x, ldx, y, ldy, r0, r1, row_ptr, col, patch);
+    aggregate_rows_global<TI, TO, MODE>(x, ldx, y, ldy, r0, r1, row_ptr, col);
     return;
   }
   // the tile's slice of the CSR (as tile-local ids) and 1/(deg+1) go to shared memory while the bulk copy flies
@@ -203,12 +168,6 @@ aggregate_staged_kernel(const TI* __restrict__ x, int64_t ldx, TO* __restrict__ 
   if (fits)
     for (int i = tid; i < nnz; i += nthreads) col_s[i] = __ldg(col + e0 + i) - r0;
   for (int i = tid; i < n; i += nthreads) inv_s[i] = __frcp_rn((float)(rp_s[i + 1] - rp_s[i] + 1));
-  if (PATCH && patch.loc)                           // per staged row: where its sentence's patch entries start, and
-    for (int i = tid; i < n; i += nthreads) {       // its sentence-local index (two dependent loads, once per row)
-      const int b = __ldg(patch.row_sent + r0 + i);
-      poff_s[i] = b * patch.ldp;
-      plr_s[i] = r0 + i - __ldg(patch.sent_ptr + b);
-    }
   __syncthreads();
   {
     uint32_t ok = 0;
@@ -218,7 +177,7 @@ aggregate_staged_kernel(const TI* __restrict__ x, int64_t ldx, TO* __restrict__ 
     }
   }
   if (!fits) {                                      // dense-ish graph: keep the staged copy unused, gather from global
-    aggregate_rows_global<TI, TO, MODE>(x, ldx, y, ldy, r0, r1, row_ptr, col, patch);
+    aggregate_rows_global<TI, TO, MODE>(x, ldx, y, ldy, r0, r1, row_ptr, col);
     return;
   }
   // ---- hot loop: shared memory only -------------------------------------------------------------------
@@ -263,22 +222,14 @@ aggregate_staged_kernel(const TI* __restrict__ x, int64_t ldx, TO* __restrict__ 
 #pragma unroll
       for (int k = 0; k < E; ++k) acc[k] *= inv;
     }
-    if (PATCH && patch.loc) apply_patch_at<E>(patch, (int64_t)poff_s[lr] + threadIdx.x * E, plr_s[lr], acc);
     store_chunk<TO, E>(yrow, acc);
   }
-}
-
-// experiment switch (bring-up only): EDG_AGG_VARIANT = 0 flat gather from global, 3 = shared-memory staged (default)
-static int agg_variant() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("EDG_AGG_VARIANT"); v = e ? atoi(e) : 3; }
-  return v;
 }
 
 template <typename TI, typename TO>
 static int launch_aggregate(const void* x, int64_t ldx, void* y, int64_t ldy, int N, int D,
                             const int32_t* row_ptr, const int32_t* col, int mode, const int32_t* sent_ptr,
-                            const int32_t* row_sent, int B, int max_len, const AggPatch& patch, cudaStream_t s) {
+                            const int32_t* row_sent, int B, int max_len, cudaStream_t s) {
   constexpr int E = Vec16<TI>::kElems;
   const int chunks = (D + E - 1) / E;
   if (ldx < (int64_t)chunks * E || ldy < (int64_t)chunks * E) return EDG_ERR_ALIGN;
@@ -296,35 +247,28 @@ static int launch_aggregate(const void* x, int64_t ldx, void* y, int64_t ldy, in
     tile_rows = cap_rows - max_len + 1;
     max_threads = 1024;
   }
-  const bool staged = agg_variant() >= 3 && sent_ptr && row_sent && B > 0 && max_len > 0 && tile_rows >= 8;
+  const bool staged = sent_ptr && row_sent && B > 0 && max_len > 0 && tile_rows >= 8;
   if (!staged) {
     const int64_t total = (int64_t)N * chunks;
     const unsigned blocks = (unsigned)((total + 255) / 256);
-    if (mode == 0) aggregate_flat_kernel<TI, TO, 0><<<blocks, 256, 0, s>>>((const TI*)x, ldx, (TO*)y, ldy, N, chunks, row_ptr, col, patch);
-    else aggregate_flat_kernel<TI, TO, 1><<<blocks, 256, 0, s>>>((const TI*)x, ldx, (TO*)y, ldy, N, chunks, row_ptr, col, patch);
+    if (mode == 0) aggregate_flat_kernel<TI, TO, 0><<<blocks, 256, 0, s>>>((const TI*)x, ldx, (TO*)y, ldy, N, chunks, row_ptr, col);
+    else aggregate_flat_kernel<TI, TO, 1><<<blocks, 256, 0, s>>>((const TI*)x, ldx, (TO*)y, ldy, N, chunks, row_ptr, col);
     return check_launch();
-  }
-  {
-    static int forced = -1;                 // experiment switch (bring-up only): EDG_AGG_THREADS = threads per block
-    if (forced < 0) { const char* e = getenv("EDG_AGG_THREADS"); forced = e ? atoi(e) : 0; }
-    if (forced >= 64 && forced <= 1024) max_threads = forced;
   }
   int rpb = max_threads / chunks;
   if (rpb > 32) rpb = 32;
   if (rpb < 1) rpb = 1;
   dim3 block(chunks, rpb);
-  const size_t smem = (size_t)cap_rows * pitch + (size_t)(8 * cap_rows + 8) * sizeof(int32_t);
+  const size_t smem = (size_t)cap_rows * pitch + (size_t)(6 * cap_rows + 8) * sizeof(int32_t);
   const unsigned blocks = (unsigned)((N + tile_rows - 1) / tile_rows);
-  // four instantiations per (mode): {patch, no patch} x {<= 384-thread, <= 1024-thread blocks}
-  const bool pt = patch.loc != nullptr, big = max_threads > 384;
+  // two instantiations per mode: <= 384-thread and <= 1024-thread blocks
+  const bool big = max_threads > 384;
   void (*kern)(const TI*, int64_t, TO*, int64_t, int, int, int, int, const int32_t*, const int32_t*, const int32_t*,
-               const int32_t*, AggPatch);
-  if (mode == 0) kern = pt ? (big ? aggregate_staged_kernel<TI, TO, 0, true, 1024> : aggregate_staged_kernel<TI, TO, 0, true, 384>)
-                           : (big ? aggregate_staged_kernel<TI, TO, 0, false, 1024> : aggregate_staged_kernel<TI, TO, 0, false, 384>);
-  else kern = pt ? (big ? aggregate_staged_kernel<TI, TO, 1, true, 1024> : aggregate_staged_kernel<TI, TO, 1, true, 384>)
-                 : (big ? aggregate_staged_kernel<TI, TO, 1, false, 1024> : aggregate_staged_kernel<TI, TO, 1, false, 384>);
+               const int32_t*);
+  if (mode == 0) kern = big ? aggregate_staged_kernel<TI, TO, 0, 1024> : aggregate_staged_kernel<TI, TO, 0, 384>;
+  else kern = big ? aggregate_staged_kernel<TI, TO, 1, 1024> : aggregate_staged_kernel<TI, TO, 1, 384>;
   if (int rc_ = ensure_dyn_smem((const void*)kern, smem)) return rc_;
-  kern<<<blocks, block, smem, s>>>((const TI*)x, ldx, (TO*)y, ldy, N, B, tile_rows, cap_rows, sent_ptr, row_sent, row_ptr, col, patch);
+  kern<<<blocks, block, smem, s>>>((const TI*)x, ldx, (TO*)y, ldy, N, B, tile_rows, cap_rows, sent_ptr, row_sent, row_ptr, col);
   return check_launch();
 }
 
@@ -332,39 +276,18 @@ static int launch_aggregate(const void* x, int64_t ldx, void* y, int64_t ldy, in
 
 using namespace edg;
 
-static int aggregate_entry(const void* x, int x_dtype, int64_t ldx, void* y, int y_dtype, int64_t ldy,
-                           int32_t N, int32_t D, const int32_t* row_ptr, const int32_t* col, int mode,
-                           const int32_t* sent_ptr, const int32_t* row_sent, int32_t B, int32_t max_len,
-                           const int16_t* patch_loc, const float* patch_val, int32_t ldp, edg_stream stream) {
-  if (N < 0 || D <= 0 || (mode != 0 && mode != 1)) return EDG_ERR_ARG;
-  if (N == 0) return EDG_OK;
-  if (!x || !y || !row_ptr || !col) return EDG_ERR_ARG;
-  if ((patch_loc != nullptr) != (patch_val != nullptr)) return EDG_ERR_ARG;
-  if (patch_loc && (!row_sent || !sent_ptr || ldp < D || (ldp & 7) || !aligned16(patch_loc) || !aligned16(patch_val)))
-    return EDG_ERR_ARG;
-  if (!aligned16(x) || !aligned16(y) || !row_pitch_ok(x_dtype, ldx) || !row_pitch_ok(y_dtype, ldy)) return EDG_ERR_ALIGN;
-  cudaStream_t s = (cudaStream_t)stream;
-  AggPatch patch{patch_loc, patch_val, row_sent, sent_ptr, D, ldp};
-  if (x_dtype == EDG_BF16 && y_dtype == EDG_BF16) return launch_aggregate<__nv_bfloat16, __nv_bfloat16>(x, ldx, y, ldy, N, D, row_ptr, col, mode, sent_ptr, row_sent, B, max_len, patch, s);
-  if (x_dtype == EDG_F32 && y_dtype == EDG_F32) return launch_aggregate<float, float>(x, ldx, y, ldy, N, D, row_ptr, col, mode, sent_ptr, row_sent, B, max_len, patch, s);
-  if (x_dtype == EDG_F32 && y_dtype == EDG_BF16) return launch_aggregate<float, __nv_bfloat16>(x, ldx, y, ldy, N, D, row_ptr, col, mode, sent_ptr, row_sent, B, max_len, patch, s);
-  if (x_dtype == EDG_BF16 && y_dtype == EDG_F32) return launch_aggregate<__nv_bfloat16, float>(x, ldx, y, ldy, N, D, row_ptr, col, mode, sent_ptr, row_sent, B, max_len, patch, s);
-  return EDG_ERR_DTYPE;
-}
-
 extern "C" int edg_aggregate(const void* x, int x_dtype, int64_t ldx, void* y, int y_dtype, int64_t ldy,
                              int32_t N, int32_t D, const int32_t* row_ptr, const int32_t* col, int mode,
                              const int32_t* sent_ptr, const int32_t* row_sent, int32_t B, int32_t max_len,
                              edg_stream stream) {
-  return aggregate_entry(x, x_dtype, ldx, y, y_dtype, ldy, N, D, row_ptr, col, mode, sent_ptr, row_sent, B, max_len, nullptr,
-                         nullptr, 0, stream);
-}
-
-extern "C" int edg_aggregate_patched(const void* x, int x_dtype, int64_t ldx, void* y, int y_dtype, int64_t ldy,
-                                     int32_t N, int32_t D, const int32_t* row_ptr, const int32_t* col, int mode,
-                                     const int32_t* sent_ptr, const int32_t* row_sent, int32_t B, int32_t max_len,
-                                     const int16_t* patch_loc, const float* patch_val, int32_t ldp,
-                                     edg_stream stream) {
-  return aggregate_entry(x, x_dtype, ldx, y, y_dtype, ldy, N, D, row_ptr, col, mode, sent_ptr, row_sent, B, max_len, patch_loc,
-                         patch_val, ldp, stream);
+  if (N < 0 || D <= 0 || (mode != 0 && mode != 1)) return EDG_ERR_ARG;
+  if (N == 0) return EDG_OK;
+  if (!x || !y || !row_ptr || !col) return EDG_ERR_ARG;
+  if (!aligned16(x) || !aligned16(y) || !row_pitch_ok(x_dtype, ldx) || !row_pitch_ok(y_dtype, ldy)) return EDG_ERR_ALIGN;
+  cudaStream_t s = (cudaStream_t)stream;
+  if (x_dtype == EDG_BF16 && y_dtype == EDG_BF16) return launch_aggregate<__nv_bfloat16, __nv_bfloat16>(x, ldx, y, ldy, N, D, row_ptr, col, mode, sent_ptr, row_sent, B, max_len, s);
+  if (x_dtype == EDG_F32 && y_dtype == EDG_F32) return launch_aggregate<float, float>(x, ldx, y, ldy, N, D, row_ptr, col, mode, sent_ptr, row_sent, B, max_len, s);
+  if (x_dtype == EDG_F32 && y_dtype == EDG_BF16) return launch_aggregate<float, __nv_bfloat16>(x, ldx, y, ldy, N, D, row_ptr, col, mode, sent_ptr, row_sent, B, max_len, s);
+  if (x_dtype == EDG_BF16 && y_dtype == EDG_F32) return launch_aggregate<__nv_bfloat16, float>(x, ldx, y, ldy, N, D, row_ptr, col, mode, sent_ptr, row_sent, B, max_len, s);
+  return EDG_ERR_DTYPE;
 }

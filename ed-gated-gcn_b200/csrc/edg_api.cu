@@ -1,6 +1,5 @@
 // C-ABI entry points that dispatch between the fp32 (FFMA) and bf16 (tcgen05) GEMM kernels,
 // plus version / error reporting.
-#include <stdlib.h>
 #include <string.h>
 
 #include <mutex>
@@ -50,17 +49,6 @@ int launch_wgrad_tc_batch(int n, const void* const* A, int64_t lda, int K1, cons
                           float* const* dW, int64_t lddw, float* const* dbias, int bias_of, float* ws, cudaStream_t s);
 size_t wgrad_tc_batch_workspace(int n, int R, int K1, int K2);
 
-// Bring-up switch for the GPU tests only: EDG_FORCE_SIMT=1 routes bf16 GEMMs through the FFMA
-// kernels so a tcgen05 result can be cross-checked on the same inputs.  Not a product path.
-static bool force_simt() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("EDG_FORCE_SIMT");
-    v = (e && e[0] == '1') ? 1 : 0;
-  }
-  return v == 1;
-}
-
 }  // namespace edg
 
 using namespace edg;
@@ -96,19 +84,14 @@ extern "C" int edg_linear(const void* A, int ab_dtype, int64_t lda, int32_t M, i
   if (!row_pitch_ok(ab_dtype, lda) || !row_pitch_ok(ab_dtype, ldw) || !row_pitch_ok(c_dtype, ldc)) return EDG_ERR_ALIGN;
   cudaStream_t s = (cudaStream_t)stream;
   if (ab_dtype == EDG_F32) return launch_linear_simt<float>(A, lda, M, K, W, ldw, Nout, bias, act, C, c_dtype, ldc, s);
-  if (ab_dtype == EDG_BF16) {
-    if (force_simt()) return launch_linear_simt<__nv_bfloat16>(A, lda, M, K, W, ldw, Nout, bias, act, C, c_dtype, ldc, s);
-    return launch_linear_tc(A, lda, M, K, W, ldw, Nout, bias, act, C, c_dtype, ldc, s);
-  }
+  if (ab_dtype == EDG_BF16) return launch_linear_tc(A, lda, M, K, W, ldw, Nout, bias, act, C, c_dtype, ldc, s);
   return EDG_ERR_DTYPE;
 }
 
 extern "C" size_t edg_wgrad_workspace(int32_t R, int32_t K1, int32_t K2, int dtype) {
   if (R <= 0 || K1 <= 0 || K2 <= 0) return 16;
-  size_t a = wgrad_simt_workspace(R, K1, K2);
-  size_t b = (dtype == EDG_BF16) ? wgrad_tc_workspace(R, K1, K2) : 0;
+  size_t m = (dtype == EDG_BF16) ? wgrad_tc_workspace(R, K1, K2) : wgrad_simt_workspace(R, K1, K2);
   size_t c = edg_colsum_workspace(R, K1 > K2 ? K1 : K2);
-  size_t m = a > b ? a : b;
   return m + c + 256;
 }
 
@@ -130,15 +113,11 @@ extern "C" int edg_wgrad(const void* A, int64_t lda, int32_t K1, const void* B, 
   if (lda < K1 || ldb < K2) return EDG_ERR_ARG;
   if (!aligned16(A) || !aligned16(B) || !aligned16(ws) || !row_pitch_ok(dtype, lda) || !row_pitch_ok(dtype, ldb)) return EDG_ERR_ALIGN;
   if (ws_bytes < edg_wgrad_workspace(R, K1, K2, dtype)) return EDG_ERR_WORKSPACE;
-  int rc;
-  const bool tc = (dtype == EDG_BF16) && !force_simt();
-  size_t gemm_ws = tc ? wgrad_tc_workspace(R, K1, K2) : wgrad_simt_workspace(R, K1, K2);
-  if (dtype == EDG_F32) rc = launch_wgrad_simt<float>(A, lda, K1, B, ldb, K2, R, dW, lddw, accumulate, (float*)ws, s);
-  else if (tc) return launch_wgrad_tc(A, lda, K1, B, ldb, K2, R, dW, lddw, dbias, bias_of, accumulate, (float*)ws, s);
-  else rc = launch_wgrad_simt<__nv_bfloat16>(A, lda, K1, B, ldb, K2, R, dW, lddw, accumulate, (float*)ws, s);
+  if (dtype == EDG_BF16) return launch_wgrad_tc(A, lda, K1, B, ldb, K2, R, dW, lddw, dbias, bias_of, accumulate, (float*)ws, s);
+  int rc = launch_wgrad_simt<float>(A, lda, K1, B, ldb, K2, R, dW, lddw, accumulate, (float*)ws, s);
   if (rc) return rc;
   if (bias_of) {
-    char* cws = (char*)ws + ((gemm_ws + 255) & ~(size_t)255);
+    char* cws = (char*)ws + ((wgrad_simt_workspace(R, K1, K2) + 255) & ~(size_t)255);
     const void* X = bias_of == 1 ? A : B;
     const int64_t ldx = bias_of == 1 ? lda : ldb;
     const int Cc = bias_of == 1 ? K1 : K2;

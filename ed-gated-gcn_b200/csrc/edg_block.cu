@@ -168,48 +168,6 @@ views_bwd_kernel(const float* __restrict__ pooled, const int32_t* __restrict__ a
   }
 }
 
-// The same gradients WITHOUT touching dh: what the views send to their arg-max rows is written as one
-// (sentence-local row, value) pair per (sentence, column) for the aggregation kernel that produces dh to add on
-// the fly (edg_aggregate_patched).  Pure [B,D] streaming: h at the arg-max row is the column maximum `hmax`
-// that edg_pool_fwd returns.  Positive gates (sigmoid outputs) as in edg_pool_fwd: the views then share their
-// arg-max row; a view whose gate is exactly 0 contributes nothing to dh.
-__global__ void __launch_bounds__(256)
-views_patch_kernel(const float* __restrict__ pooled, const int32_t* __restrict__ arg, const float* __restrict__ gates,
-                   const float* __restrict__ hmax, const int32_t* __restrict__ sent_ptr, int V, int B, int D, int ldp,
-                   const float* __restrict__ g_xy, const float* __restrict__ g_pooled, int16_t* __restrict__ patch_loc,
-                   float* __restrict__ patch_val, float* __restrict__ dgates, int acc_view) {
-  const int64_t BD = (int64_t)B * D;
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= (int64_t)B * ldp) return;
-  const int b = (int)(i / ldp), d = (int)(i - (int64_t)b * ldp);
-  if (d >= D) { patch_loc[i] = -1; patch_val[i] = 0.f; return; }
-  const int64_t o = (int64_t)b * D + d;
-  const float gxy = g_xy ? (__ldg(g_xy) / (float)B) : 0.f;
-  float tot = 0.f;
-  for (int v = 0; v < V; ++v) tot += pooled[v * BD + o];
-  const float hm = hmax[o];
-  int prow = -1;
-  float pval = 0.f;
-  for (int v = 0; v < V; ++v) {
-    float dp = gxy * (tot - pooled[v * BD + o]);
-    if (g_pooled) dp += g_pooled[v * BD + o];
-    const int r = arg[v * BD + o];
-    float dgv = 0.f;
-    if (r >= 0) {
-      dgv = dp * hm;
-      const float contrib = dp * gates[v * BD + o];
-      if (contrib != 0.f) {
-        if (prow < 0) prow = r;
-        if (r == prow) pval += contrib;
-      }
-    }
-    dgates[v * BD + o] = (v == acc_view) ? dgates[v * BD + o] + dgv : dgv;
-  }
-  const int loc = prow >= 0 ? prow - sent_ptr[b] : -1;
-  patch_loc[i] = (int16_t)((loc >= 0 && loc < 32767) ? loc : -1);
-  patch_val[i] = (loc >= 0 && loc < 32767) ? pval : 0.f;
-}
-
 // ---- importance scores + softmax product ("kl") ---------------------------------
 template <int I64> __device__ __forceinline__ float dist_at(const void* dist, int64_t i) {
   return I64 ? (float)reinterpret_cast<const long long*>(dist)[i] : (float)reinterpret_cast<const int32_t*>(dist)[i];
@@ -517,12 +475,6 @@ int head_bwd_staged(const void* h, int64_t ldh, const int32_t* sent_ptr, const i
                     const float* kl_b, const float* g_kl, const float* g_scores, const float* g_pooled, const int32_t* arg,
                     const void* g_xout, int64_t ldgx, void* dh, int64_t lddh, float* dgate, float* dv, float* dc,
                     cudaStream_t s);
-// bring-up switch: EDG_STAGED=0 keeps the per-sentence kernels
-static bool staged_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("EDG_STAGED"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v == 1;
-}
 }  // namespace edg
 
 using namespace edg;
@@ -589,10 +541,8 @@ extern "C" int edg_pool_fwd(const void* h, int dtype, int64_t ldh, const int32_t
   if (!aligned16(h) || !row_pitch_ok(dtype, ldh)) return EDG_ERR_ALIGN;
   cudaStream_t s = (cudaStream_t)stream;
   EDG_DISPATCH_T(dtype, {
-    if (staged_enabled()) {
-      const int rc = pool_fwd_staged<T>(h, ldh, sent_ptr, row_sent, N, B, D, max_len, gates, V, pooled, arg, hmax, s);
-      if (rc <= 0) return rc;
-    }
+    const int rc = pool_fwd_staged<T>(h, ldh, sent_ptr, row_sent, N, B, D, max_len, gates, V, pooled, arg, hmax, s);
+    if (rc <= 0) return rc;
     return pool_fwd_dispatch<T>(h, ldh, sent_ptr, B, D, gates, V, pooled, arg, hmax, s);
   })
 }
@@ -645,19 +595,6 @@ extern "C" int edg_views_bwd_parts(const float* pooled, const int32_t* arg, cons
                          stream);
 }
 
-extern "C" int edg_views_patch(const float* pooled, const int32_t* arg, const float* gates, const float* hmax,
-                               const int32_t* sent_ptr, int32_t V, int32_t B, int32_t D, int32_t ldp, const float* g_xy,
-                               const float* g_pooled, int16_t* patch_loc, float* patch_val, float* dgates, int acc_view,
-                               edg_stream stream) {
-  if (V <= 0 || B < 0 || D <= 0 || ldp < D || (ldp & 7)) return EDG_ERR_ARG;
-  if (B == 0) return EDG_OK;
-  if (!pooled || !arg || !gates || !hmax || !sent_ptr || !patch_loc || !patch_val || !dgates) return EDG_ERR_ARG;
-  cudaStream_t s = (cudaStream_t)stream;
-  views_patch_kernel<<<blocks_for((int64_t)B * ldp, 256), 256, 0, s>>>(pooled, arg, gates, hmax, sent_ptr, V, B, D, ldp, g_xy,
-                                                                      g_pooled, patch_loc, patch_val, dgates, acc_view);
-  return check_launch();
-}
-
 extern "C" int edg_scores_kl_fwd(const void* h, int dtype, int64_t ldh, const int32_t* sent_ptr, int32_t B,
                                  int32_t D, const float* gate, const float* v, const float* c,
                                  const void* dist, int dist_i64, float* scores, float* kl_b,
@@ -674,11 +611,9 @@ extern "C" int edg_scores_kl_fwd(const void* h, int dtype, int64_t ldh, const in
     constexpr int E = Vec16<T>::kElems;
     const int chunks = (D + E - 1) / E;
     if (chunks > 32 * ScoresQ<T>::value) return EDG_ERR_UNSUPPORTED;
-    if (staged_enabled()) {
-      const int rc = scores_kl_staged<T>(h, ldh, sent_ptr, row_sent, N, B, D, max_len, gate, v, c, dist, dist_i64, scores, kl_b,
-                                         dv_unit, dc_unit, u_unit, sf_unit, s);
-      if (rc <= 0) return rc;
-    }
+    const int rc = scores_kl_staged<T>(h, ldh, sent_ptr, row_sent, N, B, D, max_len, gate, v, c, dist, dist_i64, scores, kl_b,
+                                       dv_unit, dc_unit, u_unit, sf_unit, s);
+    if (rc <= 0) return rc;
     if (dist_i64) scores_kl_fwd_kernel<T, 1><<<blocks, 128, 0, s>>>((const T*)h, ldh, sent_ptr, B, D, chunks, gate, v, c, dist, scores, kl_b, dv_unit, dc_unit, u_unit, sf_unit);
     else scores_kl_fwd_kernel<T, 0><<<blocks, 128, 0, s>>>((const T*)h, ldh, sent_ptr, B, D, chunks, gate, v, c, dist, scores, kl_b, dv_unit, dc_unit, u_unit, sf_unit);
   })
@@ -708,11 +643,9 @@ extern "C" int edg_head_bwd(const void* h, int dtype, int64_t ldh, const int32_t
     constexpr int E = Vec16<T>::kElems;
     const int chunks = (D + E - 1) / E;
     if (chunks > 256) return EDG_ERR_UNSUPPORTED;
-    if (staged_enabled()) {
-      const int rc = head_bwd_staged<T>(h, ldh, sent_ptr, row_sent, N, B, D, max_len, gate, v, dist, dist_i64, scores, kl_b, g_kl,
-                                        g_scores, g_pooled, arg, g_xout, ldgx, dh, lddh, dgate, dv, dc, s);
-      if (rc <= 0) return rc;
-    }
+    const int rc = head_bwd_staged<T>(h, ldh, sent_ptr, row_sent, N, B, D, max_len, gate, v, dist, dist_i64, scores, kl_b, g_kl,
+                                      g_scores, g_pooled, arg, g_xout, ldgx, dh, lddh, dgate, dv, dc, s);
+    if (rc <= 0) return rc;
     int threads = ((chunks + 31) / 32) * 32;
     if (threads < 32) threads = 32;
     if (dist_i64) head_bwd_kernel<T, 1><<<B, threads, smem, s>>>((const T*)h, ldh, sent_ptr, B, D, chunks, gate, v, dist, scores, kl_b, g_kl, g_scores, g_pooled, arg, (const T*)g_xout, ldgx, (T*)dh, lddh, dgate, dv, dc);

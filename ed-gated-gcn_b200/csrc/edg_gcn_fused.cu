@@ -29,6 +29,8 @@
 // side, so the second read of the tile's rows is an L2 hit.
 //
 // Unity build: included after edg_gemm_tc.cu (PTX wrappers, descriptors, TMA map helper).
+#include <stdlib.h>
+
 #include "edg_common.cuh"
 
 namespace edg {
@@ -738,22 +740,12 @@ static FusedPlan plan_fused(int K, int Nout) {
   return p;
 }
 
-// edg_gcn_fused2.cu (the version with the aggregation on the tensor cores; EDG_FUSED_V=1 selects the kernel above)
-static bool fused_v2() { return fused_env("EDG_FUSED_V", 1) == 2; }
-static int fused2_tile_rows(int K, int Nout);
-static int launch_gcn_layer2(const void* x, int64_t ldx, int32_t N, int32_t K, const void* w, int64_t ldw, int32_t Nout,
-                             const float* bias, int mode, const int32_t* row_ptr, const int32_t* col, const int32_t* sent_ptr,
-                             const int32_t* tile_info, const int32_t* n_tiles, int32_t tile_rows, void* y, int64_t ldy, float* hmax,
-                             int32_t* harg, int64_t ldpool, const float* patch_val, const int32_t* patch_arg, int64_t ldpatch,
-                             float* colsum, int colsum_accumulate, void* ws, size_t ws_bytes, const void* row_meta, cudaStream_t s);
-
 }  // namespace edg
 
 using namespace edg;
 
 /* see include/edgcn.h */
 extern "C" int edg_fused_tile_rows(int32_t K, int32_t Nout) {
-  if (fused_v2()) return fused2_tile_rows(K, Nout);
   const FusedPlan p = plan_fused(K, Nout);
   return p.ok ? p.rows_cap : 0;
 }
@@ -786,7 +778,7 @@ extern "C" int edg_gcn_layer(const void* x, int64_t ldx, int32_t N, int32_t K, c
                              const int32_t* sent_ptr, const int32_t* tile_info, const int32_t* n_tiles, int32_t tile_rows,
                              void* y, int64_t ldy, float* hmax, int32_t* harg, int64_t ldpool, const float* patch_val,
                              const int32_t* patch_arg, int64_t ldpatch, float* colsum, int colsum_accumulate, void* ws,
-                             size_t ws_bytes, const void* row_meta, edg_stream stream) {
+                             size_t ws_bytes, edg_stream stream) {
   if (N < 0 || K <= 0 || Nout <= 0 || (mode != 0 && mode != 1)) return EDG_ERR_ARG;
   if (N == 0) return EDG_OK;
   if (!x || !w || !y || !row_ptr || !col || !sent_ptr || !tile_info || !n_tiles) return EDG_ERR_ARG;
@@ -796,9 +788,6 @@ extern "C" int edg_gcn_layer(const void* x, int64_t ldx, int32_t N, int32_t K, c
   if (ldx < K || ldw < K || ldy < Nout) return EDG_ERR_ARG;
   if (!aligned16(x) || !aligned16(w) || !aligned16(y) || (ldx & 7) || (ldw & 7) || (ldy & 7)) return EDG_ERR_ALIGN;
   cudaStream_t s = (cudaStream_t)stream;
-  if (fused_v2())
-    return launch_gcn_layer2(x, ldx, N, K, w, ldw, Nout, bias, mode, row_ptr, col, sent_ptr, tile_info, n_tiles, tile_rows, y, ldy,
-                             hmax, harg, ldpool, patch_val, patch_arg, ldpatch, colsum, colsum_accumulate, ws, ws_bytes, row_meta, s);
   const FusedPlan p = plan_fused(K, Nout);
   if (!p.ok || tile_rows > p.rows_cap) return EDG_ERR_UNSUPPORTED;
   const int groups = kNumSMs / p.n_split;

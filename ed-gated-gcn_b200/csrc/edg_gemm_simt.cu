@@ -1,6 +1,5 @@
 // FFMA GEMMs of the fp32-parity mode (SURVEY hard part 1: single-pass TF32 misses the
-// 1e-5 bar, so the fp32 mode stays on the fp32 pipe).  Also instantiated for bf16 inputs as
-// the known-good cross-check of the tcgen05 kernels in the GPU tests.
+// 1e-5 bar, so the fp32 mode stays on the fp32 pipe).
 //   linear: C[M,Nout] = act(A[M,K] * W[Nout,K]^T + bias)
 //   wgrad : P[s][K1,K2] = sum_{r in split s} A[r,K1]^T B[r,K2]  (+ deterministic split reduce)
 #include <type_traits>
@@ -440,7 +439,6 @@ int launch_linear_simt(const void* A, int64_t lda, int M, int K, const void* W, 
   return check_launch();
 }
 template int launch_linear_simt<float>(const void*, int64_t, int, int, const void*, int64_t, int, const float*, int, void*, int, int64_t, cudaStream_t);
-template int launch_linear_simt<__nv_bfloat16>(const void*, int64_t, int, int, const void*, int64_t, int, const float*, int, void*, int, int64_t, cudaStream_t);
 
 template <typename T>
 int launch_wgrad_simt(const void* A, int64_t lda, int K1, const void* B, int64_t ldb, int K2, int R,
@@ -469,7 +467,6 @@ size_t wgrad_simt_workspace(int R, int K1, int K2) {
   return (size_t)sp * K1 * K2 * sizeof(float);
 }
 template int launch_wgrad_simt<float>(const void*, int64_t, int, const void*, int64_t, int, int, float*, int64_t, int, float*, cudaStream_t);
-template int launch_wgrad_simt<__nv_bfloat16>(const void*, int64_t, int, const void*, int64_t, int, int, float*, int64_t, int, float*, cudaStream_t);
 
 }  // namespace edg
 

@@ -10,7 +10,6 @@
 // linear_tc is persistent over (m,n) tiles with two TMEM accumulator stages, so the epilogue
 // of tile i overlaps the MMAs of tile i+1.
 #include <cuda.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "edg_common.cuh"
@@ -982,13 +981,6 @@ int launch_linear_split(const void* A2, int64_t lda, const float* amax_a, int M,
   return check_launch();
 }
 
-// bring-up switch: EDG_LINEAR_WS=0 forces the streaming kernel
-static bool ws_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("EDG_LINEAR_WS"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v == 1;
-}
-
 int launch_linear_tc(const void* A, int64_t lda, int M, int K, const void* W, int64_t ldw, int Nout,
                      const float* bias, int act, void* C, int c_dtype, int64_t ldc, cudaStream_t s) {
   if (Nout > kMaxBias) return EDG_ERR_UNSUPPORTED;
@@ -1005,7 +997,7 @@ int launch_linear_tc(const void* A, int64_t lda, int M, int K, const void* W, in
     const size_t w_bytes = (size_t)num_kb * block_n * kBlockK * 2;
     const size_t fixed = 1024 + kMaxBias * sizeof(float) + 512;
     const size_t budget = 227 * 1024;
-    if (ws_enabled() && w_bytes + fixed + 4 * kABytes <= budget && n_tiles <= kNumSMs && M >= 4 * kBlockM) {
+    if (w_bytes + fixed + 4 * kABytes <= budget && n_tiles <= kNumSMs && M >= 4 * kBlockM) {
       int stages = (int)((budget - fixed - w_bytes) / kABytes);
       if (stages > kWsMaxStages) stages = kWsMaxStages;
       const size_t smem = fixed + w_bytes + (size_t)stages * kABytes;
@@ -1063,11 +1055,6 @@ static TallPlan plan_wgrad_tall(int R, int K1e, int K2e, int max_rows = 0) {
   p.splits = (R + p.rows_per - 1) / p.rows_per;
   return p;
 }
-static bool tall_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("EDG_WGRAD_TALL"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v == 1;
-}
 
 size_t wgrad_tc_workspace(int R, int K1, int K2, int max_rows) {
   size_t best = 0;
@@ -1096,7 +1083,7 @@ static int run_wgrad_tc(const void* A, int64_t lda, int K1, const void* B, int64
   const int K1e = K1 + (bias_of == 2 ? 1 : 0), K2e = K2 + (bias_of == 1 ? 1 : 0);
   const int ones_a = (plant && bias_of == 2) ? K1 : -1, ones_b = (plant && bias_of == 1) ? K2 : -1;
   const TallPlan t = plan_wgrad_tall(R, K1e, K2e, max_rows);
-  if (t.ok && tall_enabled()) {
+  if (t.ok) {
     if (int rc_ = ensure_dyn_smem((const void*)wgrad_tall_kernel, kTallSmem)) return rc_;
     CUtensorMap ma, mb;
     int rc = make_map_bf16(&ma, A, R, K1, lda, 64, kBlockK);

@@ -43,16 +43,9 @@ GATE_ARCHS = {
 
 def _chain_ok(cd: torch.dtype, D: int, n_gates: int, gate_linears: int) -> bool:
     """The fused gate-MLP kernel (``edg_mlp_chain``) covers bf16, D <= 320, <= 4 gates, <= 3 Linears per gate;
-    everything else runs one ``edg_linear`` per layer.  EDG_MLP_CHAIN=0 forces the per-layer kernels (bring-up)."""
+    everything else runs one ``edg_linear`` per layer."""
     return (cd == torch.bfloat16 and 16 <= D <= ops.MLP_CHAIN_MAX_D and n_gates <= ops.MLP_CHAIN_MAX_GROUPS
-            and gate_linears <= ops.MLP_CHAIN_MAX_STAGES and os.environ.get("EDG_MLP_CHAIN", "1") != "0")
-
-
-# Opt-in (EDG_VIEWS_PATCH=1): the views' backward folded into the adjoint aggregation (edg_views_patch +
-# edg_aggregate_patched).  Correct (GPU suite passes with it) but measured SLOWER at C2: the patched aggregation
-# costs +26 us (two dependent index loads and eight compares per thread-row in an instruction-bound loop) and the
-# [B,D] patch kernel 40 us (twelve 4.9 MB fp32 arrays), against 54 us for the scattered edg_views_bwd pass.
-_PATCH_VIEWS = os.environ.get("EDG_VIEWS_PATCH", "0") == "1"
+            and gate_linears <= ops.MLP_CHAIN_MAX_STAGES)
 
 # Two-stream overlap inside the autograd node (EDG_OVERLAP=0 disables it).  The gate MLPs (64 CTAs, latency-bound)
 # and the view pooling are independent of the aggregate -> projection chain until their results meet, so they are
@@ -61,11 +54,6 @@ _PATCH_VIEWS = os.environ.get("EDG_VIEWS_PATCH", "0") == "1"
 # record_stream: the side stream always waits for the caller's current position before it starts, and the caller's
 # stream always joins the side stream before the node returns.
 _OVERLAP = os.environ.get("EDG_OVERLAP", "1") != "0"
-# opt-in: also the weight gradient of a layer next to its input gradient.  Measured slower at C2 (0.994 vs 0.971 ms):
-# wgrad_tall and linear_ws each want a whole SM (~200 KB of shared memory), so they queue for residency instead
-# of overlapping, and the two HBM streams thrash each other's L2 lines (only the upper layers' weight gradients on
-# the idle side stream: 0.983 vs 0.965 ms -- same cause)
-_OVERLAP_WGRAD = _OVERLAP and os.environ.get("EDG_OVERLAP_WGRAD", "0") == "1"
 _SIDE_STREAMS = {}
 # SMs the input-gradient projection uses while the bucket all-reduce (grad_bucket_hook) runs next to it: the rest is
 # what the collective's CTAs get
@@ -116,13 +104,12 @@ def _masked_view_pool(h, graph: DepGraph, gates: torch.Tensor, view_len: torch.T
     return torch.where(empty, torch.full_like(pooled, -1e12), pooled), torch.where(empty, torch.full_like(arg, -1), arg)
 
 
-def _side_stream(device: torch.device, which: int = 0) -> "torch.cuda.Stream":
+def _side_stream(device: torch.device) -> "torch.cuda.Stream":
     idx = torch.device(device).index if torch.device(device).index is not None else torch.cuda.current_device()
-    key = (idx, which)
-    st = _SIDE_STREAMS.get(key)
+    st = _SIDE_STREAMS.get(idx)
     if st is None:
         st = torch.cuda.Stream(device=idx)
-        _SIDE_STREAMS[key] = st
+        _SIDE_STREAMS[idx] = st
     return st
 
 
@@ -130,11 +117,11 @@ class _Side:
     """``with side.region():`` runs the body on the side stream after everything enqueued so far on the caller's
     stream; ``side.join()`` makes the caller's stream wait for all side work.  Disabled = plain in-order code."""
 
-    def __init__(self, enabled: bool, device, which: int = 0):
+    def __init__(self, enabled: bool, device):
         self.enabled = enabled
         if enabled:
             self.main = torch.cuda.current_stream(device)
-            self.side = _side_stream(device, which)
+            self.side = _side_stream(device)
         self.dirty = False
 
     def region(self):
@@ -429,18 +416,17 @@ def _layer_fwd(h, wt, b, graph: DepGraph, cd: torch.dtype, relu: bool, fused, wa
     return h, m, split, None, None
 
 
-def _unfused_layer_bwd(ctx, l: int, dh, hs, ms, params, grads_out, grad_hook, side_w: _Side):
-    """Layer l of the unfused chain backward from d h_l: the ReLU mask, the weight gradient (in ``side_w``'s region,
-    handed to ``grad_hook``) and d h_l W_l^T, which the caller aggregates with A^T."""
+def _unfused_layer_bwd(ctx, l: int, dh, hs, ms, params, grads_out, grad_hook):
+    """Layer l of the unfused chain backward from d h_l: the ReLU mask, the weight gradient (handed to ``grad_hook``)
+    and d h_l W_l^T, which the caller aggregates with A^T."""
     w, b = params[2 * l], params[2 * l + 1]
     if ctx.cfg["relu"]:
         dh = ops.as_rows(dh * (hs[l] > 0), ctx.cfg["cdtype"])
     split = ctx.ms_split[l]
     dh2 = gcn.layer_dy_split(dh, split)                                 # shared by dW and the input gradient
-    with side_w.region():
-        dW, db = gcn.layer_wgrad(ms[l], split, dh, dh2, bias_of=2)
-        grads_out[2 * l], grads_out[2 * l + 1] = dW.to(w.dtype), db.to(b.dtype)
-        grad_hook(grads_out[2 * l:2 * l + 2])
+    dW, db = gcn.layer_wgrad(ms[l], split, dh, dh2, bias_of=2)
+    grads_out[2 * l], grads_out[2 * l + 1] = dW.to(w.dtype), db.to(b.dtype)
+    grad_hook(grads_out[2 * l:2 * l + 2])
     return gcn.layer_dgrad(dh, dh2, ctx.w_n[l])                          # w_n[l] [in,out] = B operand of dh W^T
 
 
@@ -532,8 +518,6 @@ class _GatedStackFn(torch.autograd.Function):
                             v_pooled[v], v_arg[v] = pv[0], av[0]
                     elif cfg.get("view_len") is not None:
                         v_pooled, v_arg = _masked_view_pool(hs[0], graph, gates, cfg["view_len"])
-                    elif _PATCH_VIEWS:
-                        v_pooled, v_arg, v_hmax = ops.pool_fwd(hs[0], graph, gates, want_hmax=True)
                     else:
                         v_pooled, v_arg = ops.pool_fwd(hs[0], graph, gates)
                     if Lyr > 1:
@@ -618,20 +602,9 @@ class _GatedStackFn(torch.autograd.Function):
         views_active = g_xy is not None and Lyr > 1 and gated
         dgates = torch.empty((Lyr, B, D), dtype=torch.float32, device=dev)
         side = _Side(_OVERLAP and gated, dev)
-        patch = patch_ev = None
-        # (the unpatched default keeps ONE edg_views_bwd launch at layer 1: issuing its dgates half early on the side
+        # (the unfused path keeps ONE edg_views_bwd launch at layer 1: issuing its dgates half early on the side
         # stream was measured slower, 0.989 vs 0.965 ms/step -- the two halves re-read the same [B,D] arrays)
         fused = ctx.fused
-        early_views = views_active and not drop and _PATCH_VIEWS and fused is None
-        if early_views:
-            # the dgates half of the views' backward needs only forward tensors and d xy: it runs on the side stream
-            # from the very start, so the gate MLPs' backward can follow right after edg_head_bwd; what goes to d h_1
-            # comes back as patch arrays for the adjoint aggregation of layer 2
-            with side.region():
-                patch = ops.views_patch(v_pooled, v_arg, gates, ctx.v_hmax, graph, g_xy, None, dgates, acc_view=-1)
-                if side.enabled:
-                    patch_ev = torch.cuda.Event()
-                    patch_ev.record(side.side)
         # ---- d v, d c: the per-unit gradients of the forward sweep times d kl, or (when scores itself carries
         # gradient) pass A over h_L; then the fc and classifier heads
         dvc = None
@@ -649,8 +622,7 @@ class _GatedStackFn(torch.autograd.Function):
         # ---- pass B over h_L: dh_L, dgate_L
         if not views_active and Lyr > 1:
             dgates[:Lyr - 1].zero_()                                  # no diversity gradient: the other gates get none
-        # (early views: dgates[L-1] already holds the views' share, head_bwd writes elsewhere)
-        dgL = torch.empty((B, D), dtype=torch.float32, device=dev) if early_views else dgates[Lyr - 1]
+        dgL = dgates[Lyr - 1]
         du_top = db_top = None
         if fused is not None and g_xout is None:
             # top of the chain straight in aggregated form: du_L = A^T dh_L, db_L, d gate_L from [N]- and [B,D]-sized
@@ -691,13 +663,7 @@ class _GatedStackFn(torch.autograd.Function):
             grads_out[o:o + len(gg)] = gg
             return da_g, da_x
 
-        # (opt-in) the weight gradient of a layer next to its input gradient: both start from dh
-        side_w = _Side(_OVERLAP_WGRAD, dev, which=1)
         da_gate = da_extra = None
-        if early_views:
-            with side.region():                   # after head_bwd: dgates are complete
-                dgates[Lyr - 1].add_(dgL)
-                da_gate, da_extra = gate_backward()
         if fused is not None:
             if du_top is not None:
                 du, db_next = du_top, db_top
@@ -723,7 +689,6 @@ class _GatedStackFn(torch.autograd.Function):
                 # every parameter gradient of the block exists now (the gate MLPs' come from the side stream): hand
                 # them to the all-reduce and let it run NEXT to the input-gradient projection, which leaves it SMs
                 side.join()
-                side_w.join()
                 grads_out[-2], grads_out[-1] = d_fcw, d_fcb
                 n_out = len(grads_out)
                 reduced = bucket_hook(list(grads_out) + list(head_grads))
@@ -744,19 +709,16 @@ class _GatedStackFn(torch.autograd.Function):
                         ops.views_bwd(v_pooled[vi:vi + 1], v_arg[vi:vi + 1], gates[vi:vi + 1], drop[2][vi], None,
                                       dp[vi:vi + 1].contiguous(), tmp, dgates[vi:vi + 1], acc_view=0 if vi == Lyr - 1 else -1)
                         ops.dropout_rows(tmp, drop[1], vi, drop[0], out=dh, accumulate=True)
-                elif l == 0 and views_active and not _PATCH_VIEWS:
+                elif l == 0 and views_active:
                     # gated views of h_1 feed xy (:627-638): add their gradient to d h_1 before leaving layer 1
                     ops.views_bwd(v_pooled, v_arg, gates, hs[0], g_xy, None, dh, dgates, acc_view=Lyr - 1)
-                if l == 0 and gated and not early_views:
+                if l == 0 and gated:
                     with side.region():               # dgates are complete from here on
                         da_gate, da_extra = gate_backward()
-                dm = _unfused_layer_bwd(ctx, l, dh, hs, ms, params, grads_out, grad_hook, side_w)
-                if l == 1 and patch is not None and patch_ev is not None:
-                    torch.cuda.current_stream(dev).wait_event(patch_ev)       # the patch arrays come from the side stream
-                dh = ops.aggregate(dm, graph, mode=1, patch=patch if l == 1 else None)
+                dm = _unfused_layer_bwd(ctx, l, dh, hs, ms, params, grads_out, grad_hook)
+                dh = ops.aggregate(dm, graph, mode=1)
         dx = dh
         side.join()
-        side_w.join()
         da = ga_head.float() if ga_head is not None else None
         if da_extra is not None and ctx.ext_aspect:   # the caller gets d aspect as a tensor: sum the gates' slabs here
             da_gate, da_extra = (da_extra.sum(0) if da_extra.shape[0] > 1 else da_extra[0]), None
@@ -937,7 +899,6 @@ class _GatedPairsFn(torch.autograd.Function):
                                   patch)
             dh = ops.linear(du, ctx.w_n[0], None)
         else:
-            no_side = _Side(False, dev)
             for l in range(Lyr - 1, -1, -1):
                 if l == 0 and views_active and drop:
                     # the views' share of d h_1: every pair's view arg-max rows under that view's mask
@@ -948,8 +909,7 @@ class _GatedPairsFn(torch.autograd.Function):
                     zero = torch.zeros((1, graph.n_graphs, D), dtype=torch.float32, device=dev)
                     ops.views_bwd(zero, harg1.unsqueeze(0), zero + 1.0, hs[0], None, patch_val.unsqueeze(0), dh, None,
                                   parts=1)
-                dh = ops.aggregate(_unfused_layer_bwd(ctx, l, dh, hs, ms, params, grads_out, grad_hook, no_side),
-                                   graph, mode=1)
+                dh = ops.aggregate(_unfused_layer_bwd(ctx, l, dh, hs, ms, params, grads_out, grad_hook), graph, mode=1)
         dx = dh
         # ---- d x at the trigger rows: the head's and the gate MLPs' d a of every pair, in pair order
         da = ga_head.float() if ga_head is not None else None

@@ -34,19 +34,6 @@ class DepGraph:
     def device(self):
         return self.row_ptr.device
 
-    def row_meta(self) -> torch.Tensor:
-        """Two 16-byte words per packed row (``edg_row_meta``: neighbour ids | degree, sentence) for the fused layer
-        kernel; built on first use."""
-        rm = self.__dict__.get("_row_meta")
-        if rm is None:
-            dev = self.device
-            rm = torch.empty((max(self.n_rows, 1), 8), dtype=torch.int32, device=dev)
-            with torch.cuda.device(dev):
-                L.call("edg_row_meta", L.ptr(self.row_ptr), L.ptr(self.col), L.ptr(self.row_sent), L.ptr(self.sent_ptr),
-                       self.n_rows, L.ptr(rm), L.stream())
-            self.__dict__["_row_meta"] = rm
-        return rm
-
     def tile_plan(self, max_rows: int):
         """Sentence-aligned row tiles for the fused layer kernel (``edg_gcn_layer``): ``(tile_info int32
         [B+1, 8], n_tiles int32 [1])``, built by one small kernel on first use and cached per ``max_rows``.

@@ -53,17 +53,10 @@ def _f32c(t: torch.Tensor) -> torch.Tensor:
 
 
 # ---------------------------------------------------------------------------
-def aggregate(x: torch.Tensor, graph, mode: int, out_dtype: Optional[torch.dtype] = None, patch=None) -> torch.Tensor:
-    """``patch`` = (patch_arg int32 [B,D], patch_val fp32 [B,D]) from :func:`views_patch`: added to the rows it
-    names while the output is produced."""
+def aggregate(x: torch.Tensor, graph, mode: int, out_dtype: Optional[torch.dtype] = None) -> torch.Tensor:
     N, D = x.shape
     # the kernel walks 16-byte chunks of the INPUT dtype, so the output pitch must cover the same columns
     out = alloc_rows(N, D, out_dtype or x.dtype, x.device, min_ld=row_pitch(D, x.dtype))
-    if patch is not None:
-        L.call("edg_aggregate_patched", L.ptr(x), L.dt(x), ld(x), L.ptr(out), L.dt(out), ld(out), N, D,
-               L.ptr(graph.row_ptr), L.ptr(graph.col), mode, L.ptr(graph.sent_ptr), L.ptr(graph.row_sent),
-               graph.n_graphs, graph.max_len, L.ptr(patch[0]), L.ptr(patch[1]), patch[0].shape[1], L.stream())
-        return out
     L.call("edg_aggregate", L.ptr(x), L.dt(x), ld(x), L.ptr(out), L.dt(out), ld(out), N, D,
            L.ptr(graph.row_ptr), L.ptr(graph.col), mode, L.ptr(graph.sent_ptr), L.ptr(graph.row_sent),
            graph.n_graphs, graph.max_len, L.stream())
@@ -199,7 +192,7 @@ def gcn_layer(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], gr
     L.call("edg_gcn_layer", L.ptr(x), ld(x), N, K, L.ptr(w), ld(w), Nout, L.ptr(bias), int(mode), L.ptr(graph.row_ptr),
            L.ptr(graph.col), L.ptr(graph.sent_ptr), L.ptr(info), L.ptr(n_tiles), int(tile_rows), L.ptr(y), ld(y),
            L.ptr(hmax), L.ptr(harg), Nout, L.ptr(pv), L.ptr(pa), pv.stride(0) if pv is not None else 0, L.ptr(colsum), 0,
-           L.ptr(ws), ws.numel() * 4 if ws is not None else 0, L.ptr(graph.row_meta()), L.stream())
+           L.ptr(ws), ws.numel() * 4 if ws is not None else 0, L.stream())
     return y, hmax, harg, colsum
 
 
@@ -395,18 +388,6 @@ def views_bwd(pooled, arg, gates, h, g_xy, g_pooled, dh, dgates, acc_view: int =
     V, B, D = pooled.shape
     L.call("edg_views_bwd_parts", L.ptr(pooled), L.ptr(arg), L.ptr(gates), L.ptr(h), L.dt(h), ld(h), V, B, D, L.ptr(g_xy),
            L.ptr(g_pooled), L.ptr(dh), ld(dh) if dh is not None else 0, L.ptr(dgates), int(acc_view), int(parts), L.stream())
-
-
-def views_patch(pooled, arg, gates, hmax, graph, g_xy, g_pooled, dgates, acc_view: int = -1):
-    """Backward of the gated views + diversity term without touching dh: writes dgates and returns
-    (patch_loc int16 [B,ldp], patch_val fp32 [B,ldp]) for :func:`aggregate` (``patch=``)."""
-    V, B, D = pooled.shape
-    ldp = _round_up(D, 8)
-    patch_loc = torch.empty((B, ldp), dtype=torch.int16, device=pooled.device)
-    patch_val = torch.empty((B, ldp), dtype=torch.float32, device=pooled.device)
-    L.call("edg_views_patch", L.ptr(pooled), L.ptr(arg), L.ptr(gates), L.ptr(hmax), L.ptr(graph.sent_ptr), V, B, D, ldp,
-           L.ptr(g_xy), L.ptr(g_pooled), L.ptr(patch_loc), L.ptr(patch_val), L.ptr(dgates), int(acc_view), L.stream())
-    return patch_loc, patch_val
 
 
 def _dist_flag(dist: torch.Tensor) -> int:

@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define EDG_ABI_VERSION 3
+#define EDG_ABI_VERSION 4
 
 typedef enum {
   EDG_OK = 0,
@@ -135,16 +135,6 @@ int edg_aggregate(const void* x, int x_dtype, int64_t ldx, void* y, int y_dtype,
                   const int32_t* sent_ptr, const int32_t* row_sent, int32_t B, int32_t max_len,
                   edg_stream stream);
 
-/* edg_aggregate followed by y[sent_ptr[b] + patch_loc[b,d], d] += patch_val[b,d] for every sentence b and column d
- * (patch_loc int16 [B,ldp] sentence-local row, -1 = none; patch_val fp32 [B,ldp]; ldp = D rounded up to a multiple
- * of 8; sent_ptr and row_sent required): the gradient the gated max-pool views send to their arg-max rows
- * (edg_views_patch) is added while d h_1 is being produced by the adjoint aggregation, before its single
- * rounding -- no separate scattered pass over d h_1. */
-int edg_aggregate_patched(const void* x, int x_dtype, int64_t ldx, void* y, int y_dtype, int64_t ldy,
-                          int32_t N, int32_t D, const int32_t* row_ptr, const int32_t* col, int mode,
-                          const int32_t* sent_ptr, const int32_t* row_sent, int32_t B, int32_t max_len,
-                          const int16_t* patch_loc, const float* patch_val, int32_t ldp, edg_stream stream);
-
 /* One graph-convolution layer as ONE kernel (projection on tcgen05, the degree-normalised aggregation of the
  * sentence tree and the gated max-pool in its epilogue), replacing the matmul + bmm + divide + bias of
  * models/gcn.py:33-45 and the torch.max pools of bert_amir5.py:627-640 without materialising `adj @ hidden`:
@@ -179,12 +169,7 @@ int edg_gcn_layer(const void* x, int64_t ldx, int32_t N, int32_t K, const void* 
                   const int32_t* sent_ptr, const int32_t* tile_info, const int32_t* n_tiles, int32_t tile_rows,
                   void* y, int64_t ldy, float* hmax, int32_t* harg, int64_t ldpool, const float* patch_val,
                   const int32_t* patch_arg, int64_t ldpatch, float* colsum, int colsum_accumulate, void* ws,
-                  size_t ws_bytes, const void* row_meta, edg_stream stream);
-/* row_meta [N][2] 16-byte words for edg_gcn_layer, 32 bytes per packed row: the sentence-local ids (u8) of the row itself and
- * of its first fifteen other neighbours in CSR order (0xff = unused) | the number of CSR entries of the row, its sentence, 0, 0.
- * Depends on the graph only: build it once per batch next to the CSR (graph.py:62-75 builds the dense matrix instead). */
-int edg_row_meta(const int32_t* row_ptr, const int32_t* col, const int32_t* row_sent, const int32_t* sent_ptr,
-                 int32_t N, void* row_meta, edg_stream stream);
+                  size_t ws_bytes, edg_stream stream);
 
 /* C[M,Nout] = act(A[M,K] * W^T + bias), W given as [Nout,K] with K contiguous
  * (nn.Linear layout).  Replaces torch.matmul(text, weight) of gcn.py:34 (with a
@@ -271,7 +256,7 @@ int edg_trigger_scatter_add(const float* da, const float* extra, int32_t n_extra
  * starting in a window are brought in by one bulk async copy instead of one dependent load per row;
  * the same holds for edg_scores_kl_fwd and edg_head_bwd.
  * hmax (optional, fp32 [B,D]): the plain column maximum max_t h[t,:] of every sentence -- h at the arg-max row,
- * which the backward of the views needs (edg_views_patch). */
+ * from which the views' forward and backward follow for positive gates (edg_views_bwd_hmax, edg_views_bwd_hmax_pairs). */
 int edg_pool_fwd(const void* h, int dtype, int64_t ldh, const int32_t* sent_ptr, int32_t B,
                  int32_t D, const float* gates, int32_t V, float* pooled, int32_t* arg,
                  const int32_t* row_sent, int32_t N, int32_t max_len, float* hmax, edg_stream stream);
@@ -314,16 +299,6 @@ int edg_views_bwd_parts(const float* pooled, const int32_t* arg, const float* ga
                         int dtype, int64_t ldh, int32_t V, int32_t B, int32_t D, const float* g_xy,
                         const float* g_pooled, void* dh, int64_t lddh, float* dgates, int acc_view, int parts,
                         edg_stream stream);
-
-/* edg_views_bwd without the read-modify-write of dh and without the gather of h at the arg-max rows (hmax fp32
- * [B,D] = the column maximum edg_pool_fwd returns): dgates as there; what would be added to dh comes back as
- * patch_loc int16 [B,ldp] (sentence-local row, -1 = nothing) / patch_val fp32 [B,ldp] for edg_aggregate_patched.
- * Assumes what edg_pool_fwd guarantees for positive gates (sigmoid outputs): the views of a (sentence, column)
- * share their arg-max row; a view whose gate is exactly 0 contributes nothing to dh. */
-int edg_views_patch(const float* pooled, const int32_t* arg, const float* gates, const float* hmax,
-                    const int32_t* sent_ptr, int32_t V, int32_t B, int32_t D, int32_t ldp, const float* g_xy,
-                    const float* g_pooled, int16_t* patch_loc, float* patch_val, float* dgates, int acc_view,
-                    edg_stream stream);
 
 /* bert_amir5.py:645-646 collapsed (SURVEY A9): the per-sentence operands of the importance scores,
  *   [v_b | va_b] = logits_b @ fc.weight   (fc.weight [C, 2D], nn.Linear layout; C <= 64),

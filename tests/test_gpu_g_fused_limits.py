@@ -1,13 +1,10 @@
-"""The fused layer kernels at the limits of their tiles, on both variants (EDG_FUSED_V=1: edg_gcn_fused.cu, 2:
-edg_gcn_fused2.cu) and for edg_head_du, against fp64 references over EVERY sentence of the batch.
+"""The fused layer kernel (edg_gcn_fused.cu) at the limits of its tiles, and edg_head_du, against fp64 references over
+EVERY sentence of the batch.
 
 The limits under test:
-  - a tile holds at most rows_cap rows (128; 127 in v2, whose adjacency row 127 carries the column-sum weights),
-    6 sentences and 512 CSR entries;
-  - v1 stages slot 0 = the row itself + 7 other neighbours per row, reads the second half of that word only above
-    4 entries and the global CSR above 8; v2 keeps 15 neighbours per row word (edg_row_meta) and builds rows with
-    more than 16 entries from the global CSR, after which the next tile of the same CTA re-zeroes its adjacency tile
-    (otherwise it clears only the entries of the tile before).
+  - a tile holds at most rows_cap (128) rows, 6 sentences and 512 CSR entries;
+  - the kernel stages slot 0 = the row itself + 7 other neighbours per row, reads the second half of that word only
+    above 4 entries and the global CSR above 8.
 The batches are built from explicit head arrays: hubs with exactly k CSR entries (k = 4, 5, 8, 9, 16, 17, 64,
 rows_cap) whose own entry sits in the first, a middle and the last slot of their CSR row; sentences that fill a tile
 exactly (rows, sentences, both); runs of 1-token sentences; empty sentences inside tiles; a path of rows_cap tokens;
@@ -25,15 +22,8 @@ from test_gpu_f_fused import check_tile_plan
 pytestmark = pytest.mark.gpu
 
 N_SM = 148
-ROWS_CAP = {1: 128, 2: 127}
+ROWS_CAP = 128
 HUB_K = (4, 5, 8, 9, 16, 17, 64)          # + rows_cap
-
-
-@pytest.fixture(params=[1, 2], ids=["v1", "v2"])
-def variant(request, monkeypatch):
-    # read by the library on every call (edg_fused_tile_rows, edg_gcn_layer); DepGraph caches plans per max_rows
-    monkeypatch.setenv("EDG_FUSED_V", str(request.param))
-    return request.param
 
 
 # ------------------------------------------------------------------------------------------------ graph builders
@@ -117,13 +107,13 @@ def limits_batch(R, seed=0):
 _BATCHES = {}
 
 
-def limits_setup(variant, K, Nout):
-    """(batch, graph, rows, plan) for the variant's tile height, checked to be rows_cap."""
+def limits_setup(K, Nout):
+    """(batch, graph, rows, plan) for the kernel's tile height, checked to be rows_cap."""
     import ed_gated_gcn_b200 as E
     from ed_gated_gcn_b200 import ops
-    R = ROWS_CAP[variant]
+    R = ROWS_CAP
     rows = ops.fused_tile_rows(K, Nout)
-    assert rows == R, (variant, K, Nout, rows)
+    assert rows == R, (K, Nout, rows)
     if R not in _BATCHES:
         _BATCHES[R] = limits_batch(R)
     batch = _BATCHES[R]
@@ -183,9 +173,9 @@ def inputs(batch, K, Nout, seed):
     return xr, wr, bias, u
 
 
-# ------------------------------------------------------------------------------------------------ plan and row words
-def test_tile_plan_at_the_limits(variant):
-    batch, g, rows, plan = limits_setup(variant, 300, 300)
+# ------------------------------------------------------------------------------------------------ tile plan
+def test_tile_plan_at_the_limits():
+    batch, g, rows, plan = limits_setup(300, 300)
     sp = batch.sent_ptr
     info = check_tile_plan(sp, g, rows, plan)
     nt = len(info)
@@ -203,31 +193,12 @@ def test_tile_plan_at_the_limits(variant):
     assert set(int(e) for e in ent) >= {4, 5, 8, 9, 16, 17, 64, rows}
 
 
-def test_row_meta_matches_its_definition(variant):
-    """edg_row_meta, bit for bit: word 0 = own sentence-local id, then up to 15 other neighbours in CSR order, 0xff
-    for unused slots; word 1 = CSR entries of the row, sentence, 0, 0."""
-    batch, g, _, _ = limits_setup(variant, 300, 300)
-    rm = g.row_meta().cpu().numpy()[:batch.n_rows]
-    want = np.zeros((batch.n_rows, 8), dtype=np.int64)
-    w0 = np.full((batch.n_rows, 16), 0xff, dtype=np.uint8)
-    for b, h in enumerate(batch.heads_list()):
-        a = O.dense_adjacency_from_heads(h, len(h))
-        for i in range(len(h)):
-            r = batch.sent_ptr[b] + i
-            nb = [j for j in np.nonzero(a[i])[0] if j != i][:15]
-            w0[r, 0] = i
-            w0[r, 1:1 + len(nb)] = nb
-            want[r, 4:6] = (a[i].sum(), b)
-    want[:, :4] = w0.view("<u4").astype(np.int64)
-    assert np.array_equal(rm.astype(np.int64) & 0xffffffff, want & 0xffffffff)
-
-
 # ------------------------------------------------------------------------------------------------ edg_gcn_layer
 @pytest.mark.parametrize("shape", [(300, 300), (320, 320), (64, 64), (300, 161), (20, 300)])
-def test_layer_forward_and_pool_at_the_limits(variant, shape):
+def test_layer_forward_and_pool_at_the_limits(shape):
     from ed_gated_gcn_b200 import ops
     K, Nout = shape
-    batch, g, rows, plan = limits_setup(variant, K, Nout)
+    batch, g, rows, plan = limits_setup(K, Nout)
     xr, wr, bias, u = inputs(batch, K, Nout, seed=K + Nout)
     y, hmax, harg, _ = ops.gcn_layer(xr, wr, bias.to(DEV), g, 0, plan, rows, want_pool=True)
     ah = adj_hat(batch)
@@ -250,10 +221,10 @@ def test_layer_forward_and_pool_at_the_limits(variant, shape):
 
 
 @pytest.mark.parametrize("shape", [(300, 300), (64, 64), (300, 161)])
-def test_layer_adjoint_patch_and_colsum_at_the_limits(variant, shape):
+def test_layer_adjoint_patch_and_colsum_at_the_limits(shape):
     from ed_gated_gcn_b200 import ops
     K, Nout = shape
-    batch, g, rows, plan = limits_setup(variant, K, Nout)
+    batch, g, rows, plan = limits_setup(K, Nout)
     xr, wr, _, u = inputs(batch, K, Nout, seed=3 * K + Nout)
     B = batch.n_graphs
     rng = np.random.default_rng(K + Nout)
@@ -286,12 +257,12 @@ def test_layer_adjoint_patch_and_colsum_at_the_limits(variant, shape):
 
 # ------------------------------------------------------------------------------------------------ edg_head_du
 @pytest.mark.parametrize("D", [300, 64])
-def test_head_du_at_the_limits(variant, D):
+def test_head_du_at_the_limits(D):
     """edg_head_du on the same tiles, with the arg-max rows of hub sentences on the hub (phase 4 then scatters into a
     row list longer than 8): against head_bwd -> aggregate (mode 1) and against the fp64 definition on every sentence."""
     import ed_gated_gcn_b200 as E
     from ed_gated_gcn_b200 import ops
-    batch, g, rows, plan = limits_setup(variant, D, D)
+    batch, g, rows, plan = limits_setup(D, D)
     B, N = batch.n_graphs, batch.n_rows
     gen = torch.Generator().manual_seed(D)
     h = ops.as_rows(torch.randn(N, D, generator=gen).to(DEV), torch.bfloat16)
@@ -371,13 +342,13 @@ def _spy_fused_plan(monkeypatch):
     return seen
 
 
-def test_stack_at_the_tile_limits_vs_oracle_and_unfused(variant, monkeypatch):
+def test_stack_at_the_tile_limits_vs_oracle_and_unfused(monkeypatch):
     """bf16 GatedGCNStack (D = 300, L = 2) on sentences of 90..rows_cap tokens with hubs and 1-token sentences: the fused
     path against the oracle (gradients under its own max-pool routing), then the unfused kernels on the same inputs."""
     import ed_gated_gcn_b200 as E
     from ed_gated_gcn_b200 import gated
     from test_gpu_c_models import _check_routing, _compare, _oracle_run
-    R = ROWS_CAP[variant]
+    R = ROWS_CAP
     batch = _stack_batch(R)
     assert batch.lengths.max() == R
     D, C, B, Lyr = 300, 34, batch.n_graphs, 2

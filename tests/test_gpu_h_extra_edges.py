@@ -1,6 +1,6 @@
 """Dependency graphs that are not forests on the packed path: heads plus extra undirected edges -> CSR on the GPU
 (edg_csr_from_heads_edges through graph.build_graph), bit for bit against an oracle CSR of the dense matrix, and the
-gated-GCN stack on such graphs against the per-sentence oracle, on both fused-layer variants and on the unfused
+gated-GCN stack on such graphs against the per-sentence oracle, on the fused layer kernel and on the unfused
 kernels."""
 import numpy as np
 import pytest
@@ -13,12 +13,6 @@ from test_gpu_g_fused_limits import _run_stack, _spy_fused_plan
 from test_host_extra_edges import enhanced_items, rebuild
 
 pytestmark = pytest.mark.gpu
-
-
-@pytest.fixture(params=[1, 2], ids=["v1", "v2"])
-def variant(request, monkeypatch):
-    monkeypatch.setenv("EDG_FUSED_V", str(request.param))
-    return request.param
 
 
 # ------------------------------------------------------------------------------------------------ helpers
@@ -246,7 +240,7 @@ def _stack_case(batch, dtype, seed):
     return stack, dense, graph, anchor, dist, xp, targets, sents, Lyr
 
 
-def test_bf16_stack_with_extra_edges_vs_oracle_and_unfused(variant, monkeypatch):
+def test_bf16_stack_with_extra_edges_vs_oracle_and_unfused(monkeypatch):
     from ed_gated_gcn_b200 import gated, synth
     from test_gpu_c_models import _check_routing, _compare, _oracle_run
     batch = synth.with_extra_edges(synth.config_batch("C2", n_graphs=160), rate=0.3, seed=8)

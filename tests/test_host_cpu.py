@@ -35,7 +35,7 @@ def test_library_exports_every_declared_symbol():
 def test_version_and_error_strings_without_gpu():
     from ed_gated_gcn_b200 import _lib
     lib = _lib.load()
-    assert lib.edg_version() == 3
+    assert lib.edg_version() == 4
     assert b"aligned" in lib.edg_strerror(-2)
     assert lib.edg_strerror(0) == b"ok"
 

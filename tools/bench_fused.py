@@ -55,8 +55,8 @@ bench("linear (unfused)", lambda i: ops.linear(xs[i], w, bias))
 bench("pool_fwd V=1 (unfused)", lambda i: ops.pool_fwd(xs[i], graph, gates), N * D * 2)
 bench("torch copy (ref)", lambda i: xs[(i + 1) % RING].copy_(xs[i]), 2 * N * D * 2)
 
-KEYS = ("V", "EPI_WARPS", "STAGES", "ROWS", "PF", "DEBUG", "SLEEP", "BOXROWS")
-sweeps = [dict(), dict(EPI_WARPS=12), dict(STAGES=3), dict(V=2)]
+KEYS = ("EPI_WARPS", "STAGES", "ROWS", "PF", "DEBUG", "SLEEP", "BOXROWS")
+sweeps = [dict(), dict(EPI_WARPS=12), dict(STAGES=3)]
 only_plain = False
 if len(sys.argv) > 1 and sys.argv[1] == "pipe":       # load-pipeline study: epilogue work switched off
     only_plain = True

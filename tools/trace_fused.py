@@ -26,7 +26,7 @@ for rep in range(3):
     L.call("edg_gcn_layer", L.ptr(x), ops.ld(x), N, D, L.ptr(w), ops.ld(w), D, L.ptr(bias), 0, L.ptr(graph.row_ptr),
            L.ptr(graph.col), L.ptr(graph.sent_ptr), L.ptr(info), L.ptr(n_tiles), rows, L.ptr(y), ops.ld(y),
            L.ptr(hmax) if pool else None, L.ptr(harg) if pool else None, D, None, None, 0, None, 0, L.ptr(ws), ws.numel() * 8,
-           L.ptr(graph.row_meta()), L.stream())
+           L.stream())
     torch.cuda.synchronize()
 t = ws.cpu().view(3, 160).tolist()
 t0 = min(v for r in t for v in r if v)
