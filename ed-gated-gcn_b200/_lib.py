@@ -48,6 +48,11 @@ SIGNATURES = {
     "edg_dense_head_bwd_workspace": (_Z, [_I, _I, _I]),
     "edg_dense_head_bwd": (c_int, [_P, _L, _P, _L, _P, _L, _P, _L, _I, _I, _I, c_int, _P, _L, _P, _P, _P, _P, _P, _L, _P, _P, _Z,
                                    _P]),
+    "edg_block_head_fwd": (c_int, [_P, _L, _P, _L, _P, _L, _P, _L, _P, _L, _P, _P, _L, _P, _I, _I, _I, _P, _P, _P, _P, _P]),
+    "edg_block_head_bwd": (c_int, [_P, _P, _L, _P, _L, c_int, _P, _L, _P, _L, _P, _P, _P, _P, _P, _P, _I, _I, _I, _P, _P,
+                                   _P, _P]),
+    "edg_block_head_wgrad_workspace": (_Z, [_I, _I, _I]),
+    "edg_block_head_wgrad": (c_int, [_P, _P, _P, _L, _P, _L, _P, _L, _P, _P, _P, _I, _I, _I, _P, _P, _P, _P, _P, _Z, _P]),
     "edg_cross_entropy_workspace": (_Z, [_I]),
     "edg_cross_entropy_fwd": (c_int, [_P, _L, _P, _I, _I, _L, _P, _P, _P, _Z, _P]),
     "edg_cross_entropy_bwd": (c_int, [_P, _L, _P, _I, _I, _L, _P, _P, _P, _L, _P]),
@@ -158,6 +163,8 @@ def _kernels_of(name: str, args) -> int:
         return 0 if args[4] == 0 else (3 if (args[5] == 0 or args[6] == 0) else 7)
     if name == "edg_wgrad_split":
         return 4
+    if name == "edg_block_head_wgrad":
+        return 2
     if name == "edg_dense_head_bwd":
         return 2 if (args[11] & 2) else 1
     if name == "edg_split_f16":

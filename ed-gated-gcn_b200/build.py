@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(CSRC, "libedgcn.so")
 SOURCES = ["libedgcn.cu", "edg_api.cu", "edg_graph.cu", "edg_aggregate.cu", "edg_gemm_simt.cu", "edg_gemm_tc.cu", "edg_split.cu",
-           "edg_block.cu", "edg_block_staged.cu", "edg_pairs.cu", "edg_staged.cuh", "edg_head.cu", "edg_dense_head.cu", "edg_segment.cu", "edg_optim.cu", "edg_mlp_chain.cu", "edg_gcn_fused.cu", "edg_head_fused.cu", "edg_common.cuh", os.path.join("..", "..", "include", "edgcn.h")]
+           "edg_block.cu", "edg_block_staged.cu", "edg_pairs.cu", "edg_staged.cuh", "edg_head.cu", "edg_dense_head.cu", "edg_block_head.cu", "edg_segment.cu", "edg_optim.cu", "edg_mlp_chain.cu", "edg_gcn_fused.cu", "edg_head_fused.cu", "edg_common.cuh", os.path.join("..", "..", "include", "edgcn.h")]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]

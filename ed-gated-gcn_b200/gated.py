@@ -308,51 +308,82 @@ def _gates_bwd(gates, dgates, saved, gate_p, w_t, lead: bool, cd: torch.dtype, u
     return da_gate, da_extra, grads
 
 
-def _head_fwd(ctx, a_raw, pooled, a_fc, fc_w, fc_b):
+def _head_fwd(ctx, a_raw, pooled, a_fc, fc_w, fc_b, hmax=None, gate=None):
     """Classifier head: ``logits_fn`` is the model's own dense head (host torch, :643); a head.DenseHead (= the
     reference's nn.Linear on cat[a, pooled]) is run by the block's own kernels: no inner autograd graph, its weight and
     bias are head_params[0:2].  Then the per-row operands of the collapsed scores, [v_b | va_b] = logits_b @ fc.weight
-    and c_b = a_b . va_b + logits_b . fc.bias  (= logits_b . (Wfc[:, D:] a_b + bfc), SURVEY A9), in one kernel.
-    Returns (logits, v, c); what :func:`_head_bwd` reads stays on ``ctx``."""
+    and c_b = a_b . va_b + logits_b . fc.bias  (= logits_b . (Wfc[:, D:] a_b + bfc), SURVEY A9).  A DenseHead runs
+    both in ONE launch (``edg_block_head_fwd``), a torch head is followed by ``edg_fc_head_fwd``.  ``pooled`` None:
+    pooled = gate * hmax (written by that launch).  Returns (logits, v, c, pooled); what :func:`_head_bwd` reads stays
+    on ``ctx``."""
     cfg = ctx.cfg
     dense_head = cfg.get("dense_head")
     a_leaf = p_leaf = None
     if dense_head is not None:
         hp = cfg["head_params"]
-        logits = ops.dense_head_fwd(a_raw, pooled, hp[0], hp[1] if len(hp) > 1 else None)
+        p, g = (hmax, gate) if pooled is None else (pooled, None)
+        pooled, logits, v, c = ops.block_head_fwd(a_raw, a_fc, p, g, hp[0], hp[1] if len(hp) > 1 else None,
+                                                  _f32(fc_w), _f32(fc_b))
+        lg = logits
     else:
+        if pooled is None:
+            pooled = gate * hmax
         with torch.enable_grad():
             a_leaf = a_raw.detach().requires_grad_(True)
             p_leaf = pooled.detach().requires_grad_(True)
             logits = cfg["logits_fn"](a_leaf, p_leaf)
         if logits.requires_grad and cfg["grad_enabled"]:
             _check_head_leaves(logits, (a_leaf, p_leaf), cfg["head_params"])
-    lg = logits.detach().float().contiguous()
-    v, c = ops.fc_head_fwd(lg, _f32(fc_w), _f32(fc_b), a_fc)
+        lg = logits.detach().float().contiguous()
+        v, c = ops.fc_head_fwd(lg, _f32(fc_w), _f32(fc_b), a_fc)
     ctx.head = (a_leaf, p_leaf, logits, lg, a_raw, v)
     # (detached alias: `pooled` itself is an output of this node, and an output stored on its own node is a reference
     # cycle that keeps the whole graph -- and its AccumulateGrad nodes with their stream -- alive until the cyclic GC)
     ctx.pooled_head = pooled.detach() if dense_head is not None else None
-    return logits, v, c
+    return logits, v, c, pooled
 
 
 def _head_bwd(ctx, g_logits, g_pooled, dvc, fc_w, fc_b, side: Optional[_Side], grad_hook):
-    """Backward of :func:`_head_fwd`.  ``dvc = (d v, d c, scale)`` when the scores carry gradient (else None): the fc
-    head's backward adds its d logits to ``g_logits``, then the classifier head's backward gives d a, d pooled and the
-    head parameters' gradients.  With ``side``, each launch runs as parts=1 here and parts=2 (the parameter gradients,
-    which nothing downstream waits for) in ``side``'s region, where ``grad_hook`` receives them; with ``side=None`` each
-    runs once as parts=3 and the caller hands the gradients on.
-    Returns (d a or None, d pooled or None, d fc.weight, d fc.bias, head parameter gradients)."""
+    """Backward of :func:`_head_fwd`.  ``dvc = (d v, d c, scale)`` when the scores carry gradient (else None).  A
+    DenseHead: d a, d pooled and d logits in ONE launch (``edg_block_head_bwd``), then every parameter gradient of the
+    two heads in one partial launch plus one reduction (``edg_block_head_wgrad``).  A torch head: the fc head's
+    backward adds its d logits to ``g_logits``, then the head's own autograd graph gives d a, d pooled and the head
+    parameters' gradients.  With ``side``, the parameter gradients (which nothing downstream waits for) run in
+    ``side``'s region, where ``grad_hook`` receives them; with ``side=None`` they run inline and the caller hands them
+    on.  Returns (d a or None, d pooled or None, d fc.weight, d fc.bias, head parameter gradients)."""
     cfg = ctx.cfg
     a_leaf, p_leaf, logits, lg, a_raw, v = ctx.head
     dense = cfg.get("dense_head") is not None
     region = side.region if side is not None else contextlib.nullcontext
-    d_fcw = d_fcb = da_fc = g_lg2 = None
+    d_fcw = d_fcb = da_fc = None
     g_lg = g_logits.float() if g_logits is not None else None
+    head_grads: List[Optional[torch.Tensor]] = [None] * ctx.n_head
+    a_fc = ctx.fc_sig[2] if ctx.fc_sig else a_raw
+    fcw32, fcb32 = _f32(fc_w), _f32(fc_b)
+    if dense:
+        if g_lg is None and dvc is None:
+            return None, g_pooled, None, None, head_grads
+        hp = cfg["head_params"]
+        dv, dc, scale = dvc if dvc is not None else (None, None, None)
+        # d a and d pooled leave with everything else that flows into a / pooled already added (g_pooled)
+        dlg, ga_head, gp_total = ops.block_head_bwd(lg, a_raw, a_fc, bool(ctx.fc_sig), hp[0], fcw32, fcb32, dv, dc,
+                                                    scale, g_lg, g_pooled)
+        with region():
+            d_hw, d_hb, d_fcw, d_fcb = ops.block_head_wgrad(lg, dlg, a_raw, a_fc, ctx.pooled_head, dv, dc, scale,
+                                                            want_bias=len(hp) > 1)
+            if d_fcw is not None:
+                d_fcw, d_fcb = d_fcw.to(fc_w.dtype), d_fcb.to(fc_b.dtype)
+                if side is not None:
+                    grad_hook([d_fcw, d_fcb])
+            if hp[0].requires_grad:
+                head_grads[0] = d_hw.to(hp[0].dtype)
+            if len(hp) > 1 and hp[1].requires_grad:
+                head_grads[1] = d_hb.to(hp[1].dtype)
+            if side is not None:
+                grad_hook([g for g in head_grads if g is not None and g.dtype == torch.float32])
+        return ga_head, gp_total, d_fcw, d_fcb, head_grads
     if dvc is not None:
         # backward of [v | va] = logits @ fc.weight, c = a . va + logits . fc.bias  (one kernel + a reduction)
-        a_fc = ctx.fc_sig[2] if ctx.fc_sig else a_raw
-        fcw32, fcb32 = _f32(fc_w), _f32(fc_b)
         d_lg, da_fc, d_fcw, d_fcb = ops.fc_head_bwd(lg, fcw32, fcb32, a_fc, *dvc, parts=3 if side is None else 1)
         with region():
             if side is not None:
@@ -362,30 +393,10 @@ def _head_bwd(ctx, g_logits, g_pooled, dvc, fc_w, fc_b, side: Optional[_Side], g
                 grad_hook([d_fcw, d_fcb])
         if ctx.fc_sig:
             da_fc = da_fc * a_fc * (1.0 - a_fc)                   # through sigmoid(a)
-        if dense and g_lg is not None:
-            g_lg2 = d_lg                      # the fused head adds the two d logits terms while it loads them
-        else:
-            g_lg = d_lg if g_lg is None else g_lg + d_lg
+        g_lg = d_lg if g_lg is None else g_lg + d_lg
     # ---- classifier head backward: d a, d pooled, and .grad of the parameters it closes over
     ga_head = gp_head = None
-    head_grads: List[Optional[torch.Tensor]] = [None] * ctx.n_head
-    if g_lg is not None and dense:
-        hp = cfg["head_params"]
-        # d a and d pooled leave with everything else that flows into a / pooled already added (da_fc, g_pooled)
-        ga_head, gp_head, d_hw, d_hb = ops.dense_head_bwd(g_lg, a_raw, ctx.pooled_head, hp[0],
-                                                          parts=3 if side is None else 1, g2=g_lg2,
-                                                          da_add=da_fc, dp_add=g_pooled)
-        da_fc = g_pooled = None
-        with region():
-            if side is not None:
-                _, _, d_hw, d_hb = ops.dense_head_bwd(g_lg, a_raw, ctx.pooled_head, hp[0], parts=2, g2=g_lg2)
-            if hp[0].requires_grad:
-                head_grads[0] = d_hw.to(hp[0].dtype)
-            if len(hp) > 1 and hp[1].requires_grad:
-                head_grads[1] = d_hb.to(hp[1].dtype)
-            if side is not None:
-                grad_hook([g for g in head_grads if g is not None and g.dtype == torch.float32])
-    elif g_lg is not None and logits.requires_grad:
+    if g_lg is not None and logits.requires_grad:
         cap = [(i, p) for i, p in enumerate(cfg["head_params"]) if p.requires_grad]
         res = torch.autograd.grad([logits], [a_leaf, p_leaf] + [p for _, p in cap], [g_lg.to(logits.dtype)],
                                   allow_unused=True, retain_graph=True)
@@ -527,7 +538,7 @@ class _GatedStackFn(torch.autograd.Function):
         gL = gates[Lyr - 1]
         if fused is not None:
             hL, hmaxL, p_arg = hs[-1], hm, ha
-            pooled = gL * hmaxL                        # the arg-max rows came with the maxima
+            pooled = None                              # gL * hmaxL, from the head launch; the arg-max rows came with the maxima
         else:
             hL = ops.dropout_rows(hs[-1], seed, Lyr - 1, drop_p) if drop_p > 0 else hs[-1]
             hmaxL = None
@@ -540,7 +551,7 @@ class _GatedStackFn(torch.autograd.Function):
         # BertAmir54: fc = Sequential(Sigmoid, Linear) (:464-465): the scores read z = sigmoid(x_out) (materialised
         # rows, unit gate) and sigmoid(a); everything downstream is the same kernels
         a_fc = torch.sigmoid(a_raw) if fc_sig else a_raw
-        logits, v, c = _head_fwd(ctx, a_raw, pooled, a_fc, fc_w, fc_b)
+        logits, v, c, pooled = _head_fwd(ctx, a_raw, pooled, a_fc, fc_w, fc_b, hmaxL, gL)
         # ---- importance scores and the softmax product (:645-648)
         # (also d kl/d v, d kl/d c per unit gradient: saves the backward pass one sweep over h_L)
         if fc_sig:
@@ -805,7 +816,7 @@ class _GatedPairsFn(torch.autograd.Function):
         ctx.set_materialize_grads(False)
         ctx.cfg = cfg
         ctx.fc_sig = None
-        logits, v, c = _head_fwd(ctx, a_raw, pooled, a_raw, fc_w, fc_b)
+        logits, v, c, pooled = _head_fwd(ctx, a_raw, pooled, a_raw, fc_w, fc_b)
         if drop_p > 0:
             scores, kl_b, kl, dvu, dcu = ops.scores_kl_drop_pairs_fwd(hL, graph, pairs, gL, v, c, cfg["dist"], seed,
                                                                       Lyr - 1, drop_p)

@@ -491,6 +491,65 @@ def dense_head_bwd(g: torch.Tensor, a: torch.Tensor, p: torch.Tensor, w: torch.T
     return da, dp, dW, db
 
 
+def block_head_fwd(a, a_fc, p, g, w, bias, fc_w, fc_b):
+    """``edg_block_head_fwd``: ``pooled = g * p`` (``p`` itself when ``g`` is None), ``logits = cat([a, pooled]) @ w.T
+    + bias``, and the scores' operands ``v = logits @ fc_w[:, :D]``, ``c = logits . (fc_w[:, D:] a_fc + fc_b)`` in one
+    launch.  All fp32 ``[B, D]`` rows.  Returns ``(pooled, logits [B,C], v [B,D], c [B])``."""
+    a, a_fc, p, w, fc_w, fc_b = (_f32c(t) for t in (a, a_fc, p, w, fc_w, fc_b))
+    g = _f32c(g) if g is not None else None
+    bias = _f32c(bias) if bias is not None else None
+    B, D = a.shape
+    C = w.shape[0]
+    assert p.shape == (B, D) and a_fc.shape == (B, D) and w.shape[1] == 2 * D and fc_w.shape == (C, 2 * D)
+    dev = a.device
+    pooled = torch.empty((B, D), dtype=torch.float32, device=dev) if g is not None else p
+    logits = torch.empty((B, C), dtype=torch.float32, device=dev)
+    v = torch.empty((B, D), dtype=torch.float32, device=dev)
+    c = torch.empty((B,), dtype=torch.float32, device=dev)
+    L.call("edg_block_head_fwd", L.ptr(a), ld(a), L.ptr(a_fc), ld(a_fc), L.ptr(p), ld(p), L.ptr(g),
+           ld(g) if g is not None else 0, L.ptr(w), ld(w), L.ptr(bias), L.ptr(fc_w), ld(fc_w), L.ptr(fc_b), B, D, C,
+           L.ptr(pooled) if g is not None else None, L.ptr(logits), L.ptr(v), L.ptr(c), L.stream())
+    return pooled, logits, v, c
+
+
+def block_head_bwd(logits, a, a_fc, fc_sigmoid: bool, w, fc_w, fc_b, dv=None, dc=None, scale=None, g_logits=None,
+                   g_pooled=None):
+    """``edg_block_head_bwd`` -> ``(d logits [B,C], d a [B,D], d pooled [B,D])`` of :func:`block_head_fwd`, with the
+    scores' ``dv`` / ``dc`` (times the device scalar ``scale``; both None when the scores carry no gradient) and the
+    direct gradients ``g_logits`` / ``g_pooled`` (each optional) flowing in."""
+    logits, a, a_fc, w, fc_w, fc_b = (_f32c(t) for t in (logits, a, a_fc, w, fc_w, fc_b))
+    dv, dc, scale, g_logits, g_pooled = (_f32c(t) if t is not None else None for t in (dv, dc, scale, g_logits, g_pooled))
+    B, D = a.shape
+    C = w.shape[0]
+    dev = a.device
+    dlg = torch.empty((B, C), dtype=torch.float32, device=dev)
+    da = torch.empty((B, D), dtype=torch.float32, device=dev)
+    dp = torch.empty((B, D), dtype=torch.float32, device=dev)
+    L.call("edg_block_head_bwd", L.ptr(logits), L.ptr(a), ld(a), L.ptr(a_fc), ld(a_fc), int(bool(fc_sigmoid)), L.ptr(w),
+           ld(w), L.ptr(fc_w), ld(fc_w), L.ptr(fc_b), L.ptr(dv), L.ptr(dc), L.ptr(scale), L.ptr(g_logits),
+           L.ptr(g_pooled), B, D, C, L.ptr(dlg), L.ptr(da), L.ptr(dp), L.stream())
+    return dlg, da, dp
+
+
+def block_head_wgrad(logits, dlg, a, a_fc, pooled, dv=None, dc=None, scale=None, want_bias: bool = True):
+    """``edg_block_head_wgrad`` -> ``(dW [C,2D], dbias [C], d fc_w [C,2D], d fc_b [C])``: the head's parameter gradients
+    when ``dlg`` is given (``dbias`` None unless ``want_bias``), the fc's when ``dv`` / ``dc`` are (else None)."""
+    logits, a, a_fc, pooled = (_f32c(t) for t in (logits, a, a_fc, pooled))
+    dlg, dv, dc, scale = (_f32c(t) if t is not None else None for t in (dlg, dv, dc, scale))
+    B, D = a.shape
+    C = logits.shape[1]
+    dev = a.device
+    new = lambda *s: torch.empty(s, dtype=torch.float32, device=dev)
+    dW, dbias = (new(C, 2 * D), new(C) if want_bias else None) if dlg is not None else (None, None)
+    d_fw, d_fb = (new(C, 2 * D), new(C)) if dv is not None else (None, None)
+    nbytes = L.load().edg_block_head_wgrad_workspace(B, D, C)
+    ws = torch.empty((nbytes + 3) // 4, dtype=torch.float32, device=dev)
+    L.call("edg_block_head_wgrad", L.ptr(logits), L.ptr(dlg), L.ptr(a), ld(a), L.ptr(a_fc), ld(a_fc), L.ptr(pooled),
+           ld(pooled), L.ptr(dv), L.ptr(dc), L.ptr(scale), B, D, C, L.ptr(dW), L.ptr(dbias), L.ptr(d_fw), L.ptr(d_fb),
+           L.ptr(ws), ws.numel() * 4, L.stream())
+    return dW, dbias, d_fw, d_fb
+
+
 def cross_entropy_fwd(logits: torch.Tensor, target: torch.Tensor, ignore_index: int = -100):
     """``edg_cross_entropy_fwd`` -> ``(out fp32 [2] = {mean loss, counted rows}, bad int32 [1])``."""
     B, C = logits.shape

@@ -494,6 +494,39 @@ int edg_dense_head_bwd(const float* g, int64_t ldg, const float* a, int64_t lda,
                        int64_t ldg2, const float* da_add, const float* dp_add, float* da, float* dp, float* dW,
                        int64_t lddw, float* dbias, void* ws, size_t ws_bytes, edg_stream stream);
 
+/* The block's classifier head and the collapsed-scores operands as ONE launch (what edg_dense_head_fwd followed by
+ * edg_fc_head_fwd compute, without the memset, the atomics and the round trip of the logits through HBM).  Per row b:
+ *   pooled_b = g_b * p_b              (written to pooled [B, D] contiguous; when g == NULL pooled_b = p_b, nothing written)
+ *   logits_b = W [a_b | pooled_b] + bias                  (W fp32 [C, 2D], bias [C] or NULL; logits [B, C] contiguous)
+ *   va_b = logits_b^T fc_w[:, D:],  c_b = a_fc_b . va_b + logits_b . fc_b,  v_b = logits_b^T fc_w[:, :D]  (v [B, D] contiguous)
+ * a_fc is a, or sigmoid(a) for fc = Sequential(Sigmoid, Linear).  All fp32, C <= 64; the same bits as edg_dense_head_fwd
+ * followed by edg_fc_head_fwd (their summation order). */
+int edg_block_head_fwd(const float* a, int64_t lda, const float* a_fc, int64_t ldf, const float* p, int64_t ldp,
+                       const float* g, int64_t ldg, const float* W, int64_t ldw, const float* bias, const float* fc_w,
+                       int64_t ldfw, const float* fc_b, int32_t B, int32_t D, int32_t C, float* pooled, float* logits,
+                       float* v, float* c, edg_stream stream);
+
+/* Its input gradients as ONE launch.  With s = *scale (1 when NULL) and u_b = [s dv_b | s dc_b a_fc_b]:
+ *   dlg_b = g_logits_b + fc_w u_b + s dc_b fc_b                                               (dlg [B, C] contiguous)
+ *   da_b  = s dc_b (logits_b^T fc_w[:, D:]) (times a_fc (1 - a_fc) when fc_sigmoid) + dlg_b^T W[:, :D]
+ *   dp_b  = dlg_b^T W[:, D:] + g_pooled_b                                          (da, dp [B, D] contiguous)
+ * dv [B, D] / dc [B] (contiguous) are both NULL when the scores carry no gradient; g_logits [B, C] and g_pooled [B, D]
+ * (contiguous) may be NULL.  logits [B, C] contiguous.  The same bits as edg_fc_head_bwd + edg_dense_head_bwd. */
+int edg_block_head_bwd(const float* logits, const float* a, int64_t lda, const float* a_fc, int64_t ldf, int fc_sigmoid,
+                       const float* W, int64_t ldw, const float* fc_w, int64_t ldfw, const float* fc_b, const float* dv,
+                       const float* dc, const float* scale, const float* g_logits, const float* g_pooled, int32_t B,
+                       int32_t D, int32_t C, float* dlg, float* da, float* dp, edg_stream stream);
+
+/* The parameter gradients of the two: per-block partials in one launch, summed in block order by a second one.
+ *   dv / dc given:  d_fc_w [C, 2D] = logits^T u,  d_fc_b [C] = logits^T (s dc)
+ *   dlg given:      dW [C, 2D] = dlg^T [a | pooled],  dbias [C] = colsum(dlg)  (dbias may be NULL)
+ * (all outputs contiguous, overwritten).  ws: edg_block_head_wgrad_workspace bytes. */
+size_t edg_block_head_wgrad_workspace(int32_t B, int32_t D, int32_t C);
+int edg_block_head_wgrad(const float* logits, const float* dlg, const float* a, int64_t lda, const float* a_fc,
+                         int64_t ldf, const float* pooled, int64_t ldp, const float* dv, const float* dc,
+                         const float* scale, int32_t B, int32_t D, int32_t C, float* dW, float* dbias, float* d_fc_w,
+                         float* d_fc_b, void* ws, size_t ws_bytes, edg_stream stream);
+
 /* nn.CrossEntropyLoss (mean reduction, ignore_index): out = device float[2] {mean loss over the rows whose target is not
  * ignore_index, number of such rows}; bad = device int[1], OR-ed with 1 when a target lies outside [0, C) (checked by the
  * caller when it chooses to: nothing here synchronises).  The backward writes
