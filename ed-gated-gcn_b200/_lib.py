@@ -103,6 +103,8 @@ SIGNATURES = {
                                    _P, _L, _P, _P, _P, _P, _P]),
     "edg_views_bwd_hmax_pairs": (c_int, [_P, _P, _P, _I, _I, _P, _I, _I, _P, _L, _P, c_int, _P]),
     "edg_trigger_scatter_add_pairs": (c_int, [_P, _P, _I, _I, _P, _I, _I, _P, _P, _P, c_int, _L, _P]),
+    "edg_lr_pool_pairs_fwd": (c_int, [_P, c_int, _L, _P, _P, _P, _I, _I, _I, _I, _P, _P, _P]),
+    "edg_lr_pool_pairs_bwd": (c_int, [_P, _P, _P, _P, _I, _I, _I, _P, c_int, _L, _P]),
     "edg_pool_drop_pairs": (c_int, [_P, c_int, _L, _P, _P, _P, _I, _I, _P, _I, _P, _I, _F, _P, _P, _P, _P]),
     "edg_scores_kl_drop_pairs_fwd": (c_int, [_P, c_int, _L, _P, _P, _P, _I, _I, _P, _P, _P, _P, c_int, _P, _P, _P, _P, _P,
                                              _P, _P, _I, _F, _P]),

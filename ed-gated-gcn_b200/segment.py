@@ -115,16 +115,61 @@ class _LRPoolFn(torch.autograd.Function):
         return (dh if dh.dtype == hdt else dh.to(hdt)), None, None, None, None
 
 
+class _LRPoolPairsFn(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, h, sent_ptr, pair_ptr, anchor, T_pad, cdtype):
+        hr = ops.as_rows(h, cdtype)
+        N, D = hr.shape
+        S, P = sent_ptr.numel() - 1, anchor.numel()
+        pooled = torch.empty((P, 2 * D), dtype=torch.float32, device=h.device)
+        arg = torch.empty((P, 2 * D), dtype=torch.int32, device=h.device)
+        L.call("edg_lr_pool_pairs_fwd", L.ptr(hr), L.dt(hr), ops.ld(hr), L.ptr(sent_ptr), L.ptr(pair_ptr), L.ptr(anchor), S,
+               P, D, int(T_pad), L.ptr(pooled), L.ptr(arg), L.stream())
+        ctx.save_for_backward(arg, sent_ptr, pair_ptr)
+        ctx.meta = (N, D, cdtype, h.dtype)
+        ctx.mark_non_differentiable(arg)
+        return pooled, arg
+
+    @staticmethod
+    def backward(ctx, g, _garg=None):
+        arg, sent_ptr, pair_ptr = ctx.saved_tensors
+        N, D, cd, hdt = ctx.meta
+        dh = ops.alloc_rows(N, D, cd, g.device)            # every sentence row is written by the kernel
+        L.call("edg_lr_pool_pairs_bwd", L.ptr(g.float().contiguous()), L.ptr(arg), L.ptr(sent_ptr), L.ptr(pair_ptr),
+               sent_ptr.numel() - 1, arg.shape[0], D, L.ptr(dh), L.dt(dh), ops.ld(dh), L.stream())
+        return (dh if dh.dtype == hdt else dh.to(hdt)), None, None, None, None, None
+
+
 def lr_pool(h: torch.Tensor, graph, anchor_index: torch.Tensor, T_pad: Optional[int] = None, compute_dtype=None,
-            return_arg: bool = False):
+            return_arg: bool = False, pairs=None):
     """BertDM dynamic pooling (bertdm.py:174-185) on packed rows: ``[B, 2D]`` = ``cat(pooledL, pooledR) - 1``.
     ``T_pad`` = the padded length the reference would use (``sentence_length.max()``, bertdm.py:148; default
-    ``graph.max_len``): it decides whether the left pool sees a masked zero."""
+    ``graph.max_len``): it decides whether the left pool sees a masked zero.
+
+    With ``pairs`` (a :class:`TriggerPairs` over ``graph``), ``h`` holds every sentence once (``graph.n_rows`` rows),
+    ``anchor_index`` is the sentence-local anchor of every pair (``[P]``, usually ``pairs.anchor``) and the result is
+    ``[P, 2D]`` in pair order: bit for bit what the call gives on the expanded batch (each sentence's rows copied once
+    per pair), with ``arg`` naming sentence rows.  Each sentence's rows are read twice, not once per pair, and the
+    gradient sums over a sentence's pairs in ascending pair order.  The default ``T_pad`` = ``graph.max_len`` is the
+    expanded batch's padded length whenever every sentence has a pair, as in every
+    ``collate_packed(group_sentences=True)`` batch; a caller with pair-less sentences passes the expanded batch's
+    ``T_pad`` (its longest sentence that has a pair).  The trigger row of each pair stays a row gather:
+    ``words[pairs.pair_start + pairs.anchor]``."""
     if not h.is_cuda:
         raise L.EdgError("lr_pool runs on CUDA tensors only (there is no CPU path)")
     cd = _compute_dtype(compute_dtype) if compute_dtype is not None else (h.dtype if h.dtype in L.DTYPES else torch.float32)
     anchor = anchor_index.to(device=h.device, dtype=torch.int32).contiguous()
-    pooled, arg = _LRPoolFn.apply(h, graph.sent_ptr, anchor, T_pad if T_pad is not None else graph.max_len, cd)
+    T_pad = T_pad if T_pad is not None else graph.max_len
+    if pairs is None:
+        pooled, arg = _LRPoolFn.apply(h, graph.sent_ptr, anchor, T_pad, cd)
+    else:
+        if pairs.n_sentences != graph.n_graphs:
+            raise L.EdgError(f"pairs cover {pairs.n_sentences} sentences, the graph has {graph.n_graphs}")
+        if h.dim() != 2 or h.shape[0] != graph.n_rows:
+            raise L.EdgError(f"with pairs, h must hold every sentence once: [{graph.n_rows}, D], got {tuple(h.shape)}")
+        if anchor.dim() != 1 or anchor.numel() != pairs.n_pairs:
+            raise L.EdgError(f"anchor_index must give one anchor per pair: [{pairs.n_pairs}], got {tuple(anchor.shape)}")
+        pooled, arg = _LRPoolPairsFn.apply(h, graph.sent_ptr, pairs.pair_ptr, anchor, T_pad, cd)
     return (pooled, arg) if return_arg else pooled
 
 

@@ -637,6 +637,24 @@ int edg_views_bwd_drop_pairs(const float* pooled, const float* mmax, const int32
 int edg_trigger_scatter_add_pairs(const float* da, const float* extra, int32_t n_extra, int32_t S, const int32_t* pair_ptr,
                                   int32_t P, int32_t D, const int32_t* pair_start, const int32_t* anchor, void* dx,
                                   int dtype, int64_t lddx, edg_stream stream);
+/* N4 (edg_lr_pool_fwd) per pair over the sentence rows h [N, ldh]: pair p of sentence s with anchor a = anchor[p]
+ * (sentence-local, inside the sentence) gets pooled[p] = [max over rows t <= a | max over rows a < t < n] of the
+ * sentence, as edg_lr_pool_fwd gives p's copy of the sentence: the same T_pad rule for the left pool's masked zero, the
+ * same (m + 1) - 1 rounding and the same first-index ties (a real 0 beats the left's masked 0; a right row must be
+ * strictly positive), so values and arg are bit for bit the expanded batch's with arg = the global SENTENCE row.
+ * pooled fp32 [P, 2D], arg int32 [P, 2D] (-1 where a masked zero won).  Pairs may come in any order within their
+ * sentence and may share an anchor.  Each sentence's rows are read twice (an ascending and a descending pass), whatever
+ * its pair count; a sentence of more than 512 rows or 2048 pairs is scanned once per pair instead. */
+int edg_lr_pool_pairs_fwd(const void* h, int dtype, int64_t ldh, const int32_t* sent_ptr, const int32_t* pair_ptr,
+                          const int32_t* anchor, int32_t S, int32_t P, int32_t D, int32_t T_pad, float* pooled,
+                          int32_t* arg, edg_stream stream);
+/* its adjoint: dh[t, j] = sum_{p of s} ([arg[p, j] = t] g[p, j] + [arg[p, D + j] = t] g[p, D + j]) for the rows t of
+ * sentence s, pairs in ascending order, summed in one thread (fp64 for fp32 dh, fp32 for bf16 dh) and rounded once.
+ * g fp32 [P, 2D].
+ * Every row of every sentence is written (0 where nothing routes, sentences without pairs included), so dh needs no
+ * clearing; P = 0 writes zeros (g and arg may then be NULL). */
+int edg_lr_pool_pairs_bwd(const float* g, const int32_t* arg, const int32_t* sent_ptr, const int32_t* pair_ptr, int32_t S,
+                          int32_t P, int32_t D, void* dh, int dtype, int64_t lddh, edg_stream stream);
 
 #ifdef __cplusplus
 }
