@@ -112,6 +112,10 @@ SIGNATURES = {
                                         _P, _P, _P, _P, _L, _P, _P, _P, _P, _P, _I, _F, _P]),
     "edg_views_bwd_drop_pairs": (c_int, [_P, _P, _P, _P, _P, _I, _P, _P, _I, _P, _P, _I, _I, _P, _F, _P, c_int, _L, _P,
                                          c_int, _P]),
+    "edg_scores_kl_sig_pairs_fwd": (c_int, [_P, c_int, _L, _P, _P, _P, _I, _I, _P, _P, _P, _P, c_int, _P, _P, _P, _P, _P,
+                                            _I, _F, _P]),
+    "edg_head_bwd_sig_pairs": (c_int, [_P, c_int, _L, _P, _I, _P, _I, _P, _P, _P, _I, _I, _P, _P, _P, c_int, _P, _P, _P, _P,
+                                       _P, _P, _P, _P, _L, _P, _P, _P, _P, _P, _I, _F, _P]),
 }
 
 
@@ -179,7 +183,7 @@ def _kernels_of(name: str, args) -> int:
         return 2 if args[0] else 0
     if name == "edg_head_bwd_pairs":
         return 2 if args[22] else 1
-    if name == "edg_head_bwd_drop_pairs":
+    if name in ("edg_head_bwd_drop_pairs", "edg_head_bwd_sig_pairs"):
         return 2 if args[23] else 1
     if name == "edg_views_bwd_drop_pairs":
         return (1 if args[15] else 0) + (1 if args[18] else 0)

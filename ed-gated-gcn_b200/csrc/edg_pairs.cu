@@ -11,19 +11,25 @@
 // applies to that row's copy, keep(seed, stream, pair_row_ptr[p] + t, column) -- every pair draws its own mask.  The
 // masks are regenerated from the seed wherever they are needed; nothing is stored per (pair, row).
 //
+// BertAmir54 (GatedGCNStack(fc_sigmoid=True, pair_fc_sigmoid=True)): fc = Sequential(Sigmoid, Linear), so the scores
+// read z_{p,t} = T(sigmoid(g_p * h_t)) against v_p (unit gate).  g_p does not factor out of the sigmoid, so z is never
+// materialised: the kernels' Sig = true instantiations form it from each row as they read it.
+//
 // Included after edg_block.cu (softmax_stats, dist_at, ScoresQ).
 
 namespace edg {
 
 // ---- row mask policies of the per-pair kernels --------------------------------------------------------------------
 // NoMask: the rows as stored.  GateDrop: the gate-dropout mask of one stream; a kept element reads as
-// T(h * scale) (the value edg_dropout_rows stores), a dropped one as 0.
+// T(h * scale) (the value edg_dropout_rows stores), a dropped one as 0.  kept(): the value a kept element reads as.
 struct NoMask {
   static constexpr bool kDrop = false;
   struct Key {};
   __device__ __forceinline__ Key key() const { return Key{}; }
   template <typename T, int E>
   __device__ __forceinline__ void apply(Key, float (&)[E], int, int) const {}
+  template <typename T>
+  __device__ __forceinline__ float kept(float f) const { return f; }
 };
 struct GateDrop {
   static constexpr bool kDrop = true;
@@ -41,12 +47,24 @@ struct GateDrop {
 #pragma unroll
     for (int i = 0; i < E; ++i) f[i] = keep(k, row, c + i) ? to_f32(from_f32<T>(f[i] * scale)) : 0.f;
   }
+  template <typename T>
+  __device__ __forceinline__ float kept(float f) const { return to_f32(from_f32<T>(f * scale)); }
 };
+
+// z = T(sigmoid(g h)), the value edg_gate_rows_act stores, and its slope z (1 - z) as the backward uses it
+template <typename T>
+__device__ __forceinline__ float sig_row(float gh) { return to_f32(from_f32<T>(sigmoidf_(gh))); }
+template <typename T>
+__device__ __forceinline__ float sig_slope(float gh) {
+  const float z = sig_row<T>(gh);
+  return z * (1.f - z);
+}
 
 // ---- scores, softmax product and d kl / d (v, c) units per pair -----------------------------------------
 // One warp per pair (the per-pair twin of scores_kl_fwd_kernel): the sentence's rows are read through L1 / L2, where
 // the consecutive pairs of a sentence -- consecutive warps of a block -- find them.
-template <typename T, int I64, class Mask>
+// Sig: scores_t = z_t . v + c with z_t = sig_row(g * h_t), dv_unit = sum_t u_t z_t (no gate factor); sf_unit unused.
+template <typename T, int I64, class Mask, bool Sig = false>
 __global__ void __launch_bounds__(128)
 scores_kl_pairs_kernel(const T* __restrict__ h, int64_t ldh, const int32_t* __restrict__ sent_ptr,
                        const int32_t* __restrict__ pair_sent, const int32_t* __restrict__ pair_row_ptr, int P, int D,
@@ -63,14 +81,22 @@ scores_kl_pairs_kernel(const T* __restrict__ h, int64_t ldh, const int32_t* __re
   const int beg = __ldg(sent_ptr + s), end = __ldg(sent_ptr + s + 1), n = end - beg;
   const int o0 = __ldg(pair_row_ptr + p);                 // this pair's rows in the per-pair layout
   const typename Mask::Key key = mask.key();
-  float w[kMaxQ][E];
+  float w[kMaxQ][E];                          // g * v, or v alone under Sig (g then lives in gq)
+  float gq[Sig ? kMaxQ : 1][E];
 #pragma unroll
   for (int q = 0; q < kMaxQ; ++q) {
     const int c = (lane + 32 * q) * E;
 #pragma unroll
-    for (int k = 0; k < E; ++k)
-      w[q][k] = (lane + 32 * q < chunks && c + k < D)
-                    ? __ldg(gate + (int64_t)p * D + c + k) * __ldg(vvec + (int64_t)p * D + c + k) : 0.f;
+    for (int k = 0; k < E; ++k) {
+      if constexpr (Sig) {
+        const bool in = lane + 32 * q < chunks && c + k < D;
+        gq[q][k] = in ? __ldg(gate + (int64_t)p * D + c + k) : 0.f;
+        w[q][k] = in ? __ldg(vvec + (int64_t)p * D + c + k) : 0.f;
+      } else {
+        w[q][k] = (lane + 32 * q < chunks && c + k < D)
+                      ? __ldg(gate + (int64_t)p * D + c + k) * __ldg(vvec + (int64_t)p * D + c + k) : 0.f;
+      }
+    }
   }
   const float cb = cvec ? __ldg(cvec + p) : 0.f;
   constexpr int U = 4;                        // rows in flight per warp
@@ -90,7 +116,10 @@ scores_kl_pairs_kernel(const T* __restrict__ h, int64_t ldh, const int32_t* __re
           if (t + u < n) {
             mask.template apply<T>(key, f[u], o0 + t + u, (lane + 32 * q) * E);
 #pragma unroll
-            for (int k = 0; k < E; ++k) sacc[u] = fmaf(f[u][k], w[q][k], sacc[u]);
+            for (int k = 0; k < E; ++k) {
+              if constexpr (Sig) sacc[u] = fmaf(sig_row<T>(gq[q][k] * f[u][k]), w[q][k], sacc[u]);
+              else sacc[u] = fmaf(f[u][k], w[q][k], sacc[u]);
+            }
           }
       }
     }
@@ -131,7 +160,10 @@ scores_kl_pairs_kernel(const T* __restrict__ h, int64_t ldh, const int32_t* __re
         Vec16<T>::load(h + (int64_t)(beg + t) * ldh + (lane + 32 * q) * E, f);
         mask.template apply<T>(key, f, o0 + t, (lane + 32 * q) * E);
 #pragma unroll
-        for (int k = 0; k < E; ++k) dvu[q][k] = fmaf(u, f[k], dvu[q][k]);
+        for (int k = 0; k < E; ++k) {
+          if constexpr (Sig) dvu[q][k] = fmaf(u, sig_row<T>(gq[q][k] * f[k]), dvu[q][k]);
+          else dvu[q][k] = fmaf(u, f[k], dvu[q][k]);
+        }
       }
     }
   }
@@ -141,7 +173,7 @@ scores_kl_pairs_kernel(const T* __restrict__ h, int64_t ldh, const int32_t* __re
 #pragma unroll
     for (int k = 0; k < E; ++k)
       if (lane + 32 * q < chunks && c + k < D) {
-        dv_unit[(int64_t)p * D + c + k] = dvu[q][k] * __ldg(gate + (int64_t)p * D + c + k);
+        dv_unit[(int64_t)p * D + c + k] = Sig ? dvu[q][k] : dvu[q][k] * __ldg(gate + (int64_t)p * D + c + k);
         if (sf_unit) sf_unit[(int64_t)p * D + c + k] = dvu[q][k];
       }
   }
@@ -152,7 +184,8 @@ scores_kl_pairs_kernel(const T* __restrict__ h, int64_t ldh, const int32_t* __re
 // One warp per pair.  ds_t = g_kl / P * P_t (Q_t - kl_b) + g_scores_t goes to the workspace (the row pass below reads
 // it); with sf = sum_t ds_t h_t:  dv = g * sf,  dc = sum_t ds_t,  dgate = v * sf + g_pooled * h[arg].
 // Under GateDrop h_t is the pair's masked row and h[arg] its masked column maximum (mask.mmax).
-template <typename T, int I64, class Mask>
+// Sig (z_t = sig_row(g h_t)):  dv = sum_t ds_t z_t,  dgate = v * sum_t ds_t z_t (1 - z_t) h_t + g_pooled * h[arg].
+template <typename T, int I64, class Mask, bool Sig = false>
 __global__ void __launch_bounds__(128)
 head_pairs_kernel(const T* __restrict__ h, int64_t ldh, const int32_t* __restrict__ sent_ptr,
                   const int32_t* __restrict__ pair_sent, const int32_t* __restrict__ pair_row_ptr, int P, int D, int chunks,
@@ -195,10 +228,18 @@ head_pairs_kernel(const T* __restrict__ h, int64_t ldh, const int32_t* __restric
   if (!dv && !dgate) return;
   __syncwarp();                               // ds_ws of every lane is visible to the whole warp
   float sf[kMaxQ][E];
+  float gq[Sig ? kMaxQ : 1][E], sg[Sig ? kMaxQ : 1][E];     // Sig: the gate, sum_t ds_t z_t (1 - z_t) h_t
 #pragma unroll
   for (int q = 0; q < kMaxQ; ++q)
 #pragma unroll
-    for (int k = 0; k < E; ++k) sf[q][k] = 0.f;
+    for (int k = 0; k < E; ++k) {
+      sf[q][k] = 0.f;
+      if constexpr (Sig) {
+        const int c = (lane + 32 * q) * E + k;
+        gq[q][k] = (lane + 32 * q < chunks && c < D) ? __ldg(gate + (int64_t)p * D + c) : 0.f;
+        sg[q][k] = 0.f;
+      }
+    }
   if (have_s) {
     for (int t = 0; t < n; ++t) {
       const float dst = ds_ws[o0 + t];
@@ -209,7 +250,15 @@ head_pairs_kernel(const T* __restrict__ h, int64_t ldh, const int32_t* __restric
           Vec16<T>::load(h + (int64_t)(beg + t) * ldh + (lane + 32 * q) * E, f);
           mask.template apply<T>(key, f, o0 + t, (lane + 32 * q) * E);
 #pragma unroll
-          for (int k = 0; k < E; ++k) sf[q][k] = fmaf(dst, f[k], sf[q][k]);
+          for (int k = 0; k < E; ++k) {
+            if constexpr (Sig) {
+              const float z = sig_row<T>(gq[q][k] * f[k]);
+              sf[q][k] = fmaf(dst, z, sf[q][k]);
+              sg[q][k] = fmaf(dst * (z * (1.f - z)), f[k], sg[q][k]);
+            } else {
+              sf[q][k] = fmaf(dst, f[k], sf[q][k]);
+            }
+          }
         }
       }
     }
@@ -221,9 +270,11 @@ head_pairs_kernel(const T* __restrict__ h, int64_t ldh, const int32_t* __restric
     for (int k = 0; k < E; ++k)
       if (lane + 32 * q < chunks && c + k < D) {
         const int64_t o = (int64_t)p * D + c + k;
-        if (dv) dv[o] = __ldg(gate + o) * sf[q][k];
+        if (dv) dv[o] = Sig ? sf[q][k] : __ldg(gate + o) * sf[q][k];
         if (dgate) {
-          float dg = vvec ? __ldg(vvec + o) * sf[q][k] : 0.f;
+          float dg;
+          if constexpr (Sig) dg = vvec ? __ldg(vvec + o) * sg[q][k] : 0.f;
+          else dg = vvec ? __ldg(vvec + o) * sf[q][k] : 0.f;
           if (g_pooled) {
             if constexpr (Mask::kDrop) {
               dg = fmaf(__ldg(g_pooled + o), __ldg(mask.mmax + o), dg);
@@ -243,13 +294,15 @@ head_pairs_kernel(const T* __restrict__ h, int64_t ldh, const int32_t* __restric
 // the pairs of the row's sentence in ascending order.  Every row is written (0 where the sentence has no pairs).
 // Under GateDrop each pair's term is multiplied by its mask (keep / (1 - p), regenerated per element) and the arg-max
 // rows are the pair's own ([P,D]):  dh_t = sum_p keep_{p,t} s (ds_{p,t} g_p v_p + [t = arg_p] g_p g_pooled_p).
-template <typename T, class Mask>
+// Sig reads the row h_L[t] once (h, ldh) and multiplies each pair's ds term by z (1 - z) of the pair's own
+// z = sig_row(g_p h~_{p,t}), h~ = the value the pair reads (kept: mask.kept; a dropped element's term is masked out).
+template <typename T, class Mask, bool Sig = false>
 __global__ void __launch_bounds__(128)
 dh_pairs_kernel(const int32_t* __restrict__ sent_ptr, const int32_t* __restrict__ row_sent,
                 const int32_t* __restrict__ pair_ptr, const int32_t* __restrict__ pair_row_ptr, int N, int D, int chunks,
                 const float* __restrict__ gate, const float* __restrict__ vvec, const float* __restrict__ g_pooled,
                 const int32_t* __restrict__ arg, const float* __restrict__ ds_ws, int have_s, T* __restrict__ dh,
-                int64_t lddh, Mask mask) {
+                int64_t lddh, Mask mask, const T* __restrict__ h, int64_t ldh) {
   constexpr int E = Vec16<T>::kElems;
   const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int t = (int)(idx / chunks);
@@ -258,6 +311,10 @@ dh_pairs_kernel(const int32_t* __restrict__ sent_ptr, const int32_t* __restrict_
   const int s = __ldg(row_sent + t);
   const int loc = t - __ldg(sent_ptr + s);
   const int p0 = __ldg(pair_ptr + s), p1 = __ldg(pair_ptr + s + 1);
+  float hr[Sig ? E : 1];
+  if constexpr (Sig) {
+    if (have_s) Vec16<T>::load(h + (int64_t)t * ldh + c, hr);
+  }
   if constexpr (Mask::kDrop) {
     const typename Mask::Key key = mask.key();
     float o[E];
@@ -272,6 +329,9 @@ dh_pairs_kernel(const int32_t* __restrict__ sent_ptr, const int32_t* __restrict_
         if (c + k < D) {
           const float g = __ldg(gate + po + k);
           float term = have_s ? dst * (g * __ldg(vvec + po + k)) : 0.f;
+          if constexpr (Sig) {
+            if (have_s) term *= sig_slope<T>(g * mask.template kept<T>(hr[k]));
+          }
           if (g_pooled && __ldg(arg + po + k) == t) term = fmaf(g, __ldg(g_pooled + po + k), term);
           if (mask.keep(key, rk, c + k)) o[k] = fmaf(mask.scale, term, o[k]);
         }
@@ -295,7 +355,14 @@ dh_pairs_kernel(const int32_t* __restrict__ sent_ptr, const int32_t* __restrict_
       const float dst = __ldg(ds_ws + __ldg(pair_row_ptr + p) + loc);
 #pragma unroll
       for (int k = 0; k < E; ++k)
-        if (c + k < D) o[k] = fmaf(dst, __ldg(gate + po + k) * __ldg(vvec + po + k), o[k]);
+        if (c + k < D) {
+          if constexpr (Sig) {
+            const float g = __ldg(gate + po + k);
+            o[k] = fmaf(dst * sig_slope<T>(g * hr[k]), g * __ldg(vvec + po + k), o[k]);
+          } else {
+            o[k] = fmaf(dst, __ldg(gate + po + k) * __ldg(vvec + po + k), o[k]);
+          }
+        }
     }
     if (hit) {
 #pragma unroll
@@ -494,7 +561,7 @@ using namespace edg;
 
 namespace edg {
 
-template <class Mask>
+template <class Mask, bool Sig = false>
 static int scores_kl_pairs_launch(const void* h, int dtype, int64_t ldh, const int32_t* sent_ptr, const int32_t* pair_sent,
                                   const int32_t* pair_row_ptr, int32_t P, int32_t D, const float* gate, const float* v,
                                   const float* c, const void* dist, int dist_i64, float* scores, float* kl_b,
@@ -512,18 +579,18 @@ static int scores_kl_pairs_launch(const void* h, int dtype, int64_t ldh, const i
     const int chunks = (D + E - 1) / E;
     if (chunks > 32 * ScoresQ<T>::value) return EDG_ERR_UNSUPPORTED;
     if (dist_i64)
-      scores_kl_pairs_kernel<T, 1><<<blocks, 128, 0, s>>>((const T*)h, ldh, sent_ptr, pair_sent, pair_row_ptr, P, D, chunks,
+      scores_kl_pairs_kernel<T, 1, Mask, Sig><<<blocks, 128, 0, s>>>((const T*)h, ldh, sent_ptr, pair_sent, pair_row_ptr, P, D, chunks,
                                                           gate, v, c, dist, scores, kl_b, dv_unit, dc_unit, u_unit, sf_unit,
                                                           mask);
     else
-      scores_kl_pairs_kernel<T, 0><<<blocks, 128, 0, s>>>((const T*)h, ldh, sent_ptr, pair_sent, pair_row_ptr, P, D, chunks,
+      scores_kl_pairs_kernel<T, 0, Mask, Sig><<<blocks, 128, 0, s>>>((const T*)h, ldh, sent_ptr, pair_sent, pair_row_ptr, P, D, chunks,
                                                           gate, v, c, dist, scores, kl_b, dv_unit, dc_unit, u_unit, sf_unit,
                                                           mask);
   })
   return check_launch();
 }
 
-template <class Mask>
+template <class Mask, bool Sig = false>
 static int head_bwd_pairs_launch(const void* h, int dtype, int64_t ldh, const int32_t* sent_ptr, int32_t S,
                                  const int32_t* row_sent, int32_t N, const int32_t* pair_ptr, const int32_t* pair_sent,
                                  const int32_t* pair_row_ptr, int32_t P, int32_t D, const float* gate, const float* v,
@@ -551,18 +618,19 @@ static int head_bwd_pairs_launch(const void* h, int dtype, int64_t ldh, const in
     if (P > 0) {
       const unsigned blocks = (unsigned)((P + 3) / 4);
       if (dist_i64)
-        head_pairs_kernel<T, 1><<<blocks, 128, 0, s>>>((const T*)h, ldh, sent_ptr, pair_sent, pair_row_ptr, P, D, chunks, gate,
+        head_pairs_kernel<T, 1, Mask, Sig><<<blocks, 128, 0, s>>>((const T*)h, ldh, sent_ptr, pair_sent, pair_row_ptr, P, D, chunks, gate,
                                                        v, dist, scores, kl_b, g_kl, g_scores, g_pooled, arg, ds_ws, dgate, dv, dc,
                                                        mask);
       else
-        head_pairs_kernel<T, 0><<<blocks, 128, 0, s>>>((const T*)h, ldh, sent_ptr, pair_sent, pair_row_ptr, P, D, chunks, gate,
+        head_pairs_kernel<T, 0, Mask, Sig><<<blocks, 128, 0, s>>>((const T*)h, ldh, sent_ptr, pair_sent, pair_row_ptr, P, D, chunks, gate,
                                                        v, dist, scores, kl_b, g_kl, g_scores, g_pooled, arg, ds_ws, dgate, dv, dc,
                                                        mask);
     }
     if (dh && N > 0) {
       const unsigned blocks = (unsigned)(((int64_t)N * chunks + 127) / 128);
-      dh_pairs_kernel<T><<<blocks, 128, 0, s>>>(sent_ptr, row_sent, pair_ptr, pair_row_ptr, N, D, chunks, gate, v, g_pooled,
-                                                arg, ds_ws, have_s, (T*)dh, lddh, mask);
+      dh_pairs_kernel<T, Mask, Sig><<<blocks, 128, 0, s>>>(sent_ptr, row_sent, pair_ptr, pair_row_ptr, N, D, chunks, gate,
+                                                           v, g_pooled, arg, ds_ws, have_s, (T*)dh, lddh, mask,
+                                                           (const T*)h, ldh);
     }
   })
   return check_launch();
@@ -625,6 +693,43 @@ extern "C" int edg_head_bwd_drop_pairs(const void* h, int dtype, int64_t ldh, co
   return head_bwd_pairs_launch(h, dtype, ldh, sent_ptr, S, row_sent, N, pair_ptr, pair_sent, pair_row_ptr, P, D, gate, v,
                                dist, dist_i64, scores, kl_b, g_kl, g_scores, g_pooled, arg, dh, lddh, dgate, dv, dc, ds_ws,
                                m, stream);
+}
+
+extern "C" int edg_scores_kl_sig_pairs_fwd(const void* h, int dtype, int64_t ldh, const int32_t* sent_ptr,
+                                           const int32_t* pair_sent, const int32_t* pair_row_ptr, int32_t P, int32_t D,
+                                           const float* gate, const float* v, const float* c, const void* dist,
+                                           int dist_i64, float* scores, float* kl_b, float* dv_unit, float* dc_unit,
+                                           const int64_t* seed, int32_t stream_id, float p, edg_stream stream) {
+  if (P < 0 || D <= 0) return EDG_ERR_ARG;
+  if (P == 0) return EDG_OK;
+  if (!seed)
+    return scores_kl_pairs_launch<NoMask, true>(h, dtype, ldh, sent_ptr, pair_sent, pair_row_ptr, P, D, gate, v, c, dist,
+                                                dist_i64, scores, kl_b, dv_unit, dc_unit, nullptr, nullptr, NoMask{},
+                                                stream);
+  GateDrop m;
+  if (const int rc = gate_drop(seed, stream_id, p, nullptr, m)) return rc;
+  return scores_kl_pairs_launch<GateDrop, true>(h, dtype, ldh, sent_ptr, pair_sent, pair_row_ptr, P, D, gate, v, c, dist,
+                                                dist_i64, scores, kl_b, dv_unit, dc_unit, nullptr, nullptr, m, stream);
+}
+
+extern "C" int edg_head_bwd_sig_pairs(const void* h, int dtype, int64_t ldh, const int32_t* sent_ptr, int32_t S,
+                                      const int32_t* row_sent, int32_t N, const int32_t* pair_ptr,
+                                      const int32_t* pair_sent, const int32_t* pair_row_ptr, int32_t P, int32_t D,
+                                      const float* gate, const float* v, const void* dist, int dist_i64,
+                                      const float* scores, const float* kl_b, const float* g_kl, const float* g_scores,
+                                      const float* g_pooled, const int32_t* arg, const float* mmax, void* dh,
+                                      int64_t lddh, float* dgate, float* dv, float* dc, float* ds_ws,
+                                      const int64_t* seed, int32_t stream_id, float p, edg_stream stream) {
+  if (!seed)
+    return head_bwd_pairs_launch<NoMask, true>(h, dtype, ldh, sent_ptr, S, row_sent, N, pair_ptr, pair_sent,
+                                               pair_row_ptr, P, D, gate, v, dist, dist_i64, scores, kl_b, g_kl, g_scores,
+                                               g_pooled, arg, dh, lddh, dgate, dv, dc, ds_ws, NoMask{}, stream);
+  GateDrop m;
+  if (P > 0 && g_pooled && !mmax) return EDG_ERR_ARG;
+  if (const int rc = gate_drop(seed, stream_id, p, mmax, m)) return rc;
+  return head_bwd_pairs_launch<GateDrop, true>(h, dtype, ldh, sent_ptr, S, row_sent, N, pair_ptr, pair_sent,
+                                               pair_row_ptr, P, D, gate, v, dist, dist_i64, scores, kl_b, g_kl, g_scores,
+                                               g_pooled, arg, dh, lddh, dgate, dv, dc, ds_ws, m, stream);
 }
 
 extern "C" int edg_pool_drop_pairs(const void* h, int dtype, int64_t ldh, const int32_t* sent_ptr, const int32_t* pair_sent,

@@ -72,8 +72,11 @@ def _dropout_seed(device) -> torch.Tensor:
 
 def _fused_plan(cfg, cd, D, graph, drop_p):
     """(tile_rows, plan) when the whole GCN chain can run on ``edg_gcn_layer``: bf16, no ReLU, no gate dropout, no
-    BertAmir54 head, every sentence fits a tile.  Otherwise None (the unfused kernels cover everything)."""
-    if not _FUSED or cd != torch.bfloat16 or cfg["relu"] or drop_p > 0 or cfg["fc_sigmoid"] or cfg.get("view_len") is not None:
+    BertAmir54 head on unpaired batches (their fused backward enters the chain through ``edg_head_du``, which has no
+    sigmoid form; the pairs backward materialises d h_L whatever the head), every sentence fits a tile.  Otherwise None
+    (the unfused kernels cover everything)."""
+    fc_sig_unpaired = cfg["fc_sigmoid"] and cfg.get("pairs") is None
+    if not _FUSED or cd != torch.bfloat16 or cfg["relu"] or drop_p > 0 or fc_sig_unpaired or cfg.get("view_len") is not None:
         return None
     rows = ops.fused_tile_rows(D, D)
     if rows <= 0:
@@ -815,9 +818,16 @@ class _GatedPairsFn(torch.autograd.Function):
         # ---- classifier head on [P,D], then the per-pair scores / kl over the sentence rows
         ctx.set_materialize_grads(False)
         ctx.cfg = cfg
-        ctx.fc_sig = None
-        logits, v, c, pooled = _head_fwd(ctx, a_raw, pooled, a_raw, fc_w, fc_b)
-        if drop_p > 0:
+        fc_sig = cfg["fc_sigmoid"]
+        # BertAmir54 (pair_fc_sigmoid): the fc head reads sigmoid(a); the scores read z = sigmoid(g_p * h_t), which the
+        # per-pair kernels form from each row as they read it (no z rows: ctx.fc_sig carries only sigmoid(a))
+        a_fc = torch.sigmoid(a_raw) if fc_sig else a_raw
+        ctx.fc_sig = (None, None, a_fc) if fc_sig else None
+        logits, v, c, pooled = _head_fwd(ctx, a_raw, pooled, a_fc, fc_w, fc_b)
+        if fc_sig:
+            scores, kl_b, kl, dvu, dcu = ops.scores_kl_sig_pairs_fwd(hL, graph, pairs, gL, v, c, cfg["dist"],
+                                                                     seed if drop_p > 0 else None, Lyr - 1, drop_p)
+        elif drop_p > 0:
             scores, kl_b, kl, dvu, dcu = ops.scores_kl_drop_pairs_fwd(hL, graph, pairs, gL, v, c, cfg["dist"], seed,
                                                                       Lyr - 1, drop_p)
         else:
@@ -860,9 +870,15 @@ class _GatedPairsFn(torch.autograd.Function):
         dgates = torch.empty((Lyr, P, D), dtype=torch.float32, device=dev)
         drop = ctx.drop
         if drop:
-            # the head backward on every pair's masked rows of h_L (stream L-1), with the pair's own final-pool rows
             drop_p, seed, v_pooled, v_mmax, v_arg, p_arg, mmaxL = drop
+        if ctx.fc_sig:
+            # BertAmir54: through z = sigmoid(g_p * h_t) per (pair, row), masked as in the forward pass
+            pool_seed = (p_arg, mmaxL, seed, Lyr - 1, drop_p) if drop else (hargL, None, None, 0, 0.0)
 
+            def head_bwd(*a, **kw):
+                return ops.head_bwd_sig_pairs(*a, *pool_seed, **kw)
+        elif drop:
+            # the head backward on every pair's masked rows of h_L (stream L-1), with the pair's own final-pool rows
             def head_bwd(*a, **kw):
                 return ops.head_bwd_drop_pairs(*a, p_arg, mmaxL, seed, Lyr - 1, drop_p, **kw)
         else:
@@ -940,7 +956,7 @@ class GatedGCNStack(nn.Module):
 
     def __init__(self, hidden: int, n_layers: int = 2, n_classes: int = 2, gate_arch: str = "sig-2",
                  relu: bool = False, dropout: float = 0.0, compute_dtype="f32", gated: bool = True,
-                 fc_sigmoid: bool = False, pair_dropout: bool = False):
+                 fc_sigmoid: bool = False, pair_dropout: bool = False, pair_fc_sigmoid: bool = False):
         super().__init__()
         if hidden % 4:
             raise ValueError("hidden size must be a multiple of 4 (16-byte fp32 rows)")
@@ -952,6 +968,9 @@ class GatedGCNStack(nn.Module):
         # train-mode gate dropout on the pairs= path (per-pair passes over the sentence rows instead of [P,D] products:
         # the caller asks for that cost explicitly); no effect without pairs, in eval mode, at p = 0 or ungated
         self.pair_dropout = pair_dropout
+        # BertAmir54's sigmoid fc head on the pairs= path (every pair's z = sigmoid(g_p * h_t) formed in per-pair passes
+        # over the sentence rows); no effect without fc_sigmoid or without pairs
+        self.pair_fc_sigmoid = pair_fc_sigmoid
         self.compute_dtype = _compute_dtype(compute_dtype)
         for l in range(1, n_layers + 1):
             setattr(self, f"gc{l}", GraphConvolution(hidden, hidden, None, compute_dtype=self.compute_dtype))
@@ -1009,9 +1028,11 @@ class GatedGCNStack(nn.Module):
         ``pair_dropout=True``: each pair then applies the masks the expanded batch would apply to its copy of the
         sentence (keyed on the per-pair packed row ``pairs.pair_row_ptr[p] + t``), so for the same
         ``last_dropout_seed`` the result equals the expanded run's, every pair with its own masks; the views and the
-        final pool become per-pair passes over the sentence rows.  Not covered (``EdgError``): train-mode gate dropout
-        without ``pair_dropout``, ``fc_sigmoid``, ``view_len``, ``aspect``, ``return_x_out`` and 3-D dense-compat
-        ``x``."""
+        final pool become per-pair passes over the sentence rows.  BertAmir54's head (``fc_sigmoid``) needs
+        ``pair_fc_sigmoid=True``: each pair's scores then read ``sigmoid(g_p * h_t)``, formed per (pair, row) as the
+        sentence rows are read (with or without ``pair_dropout``).  Not covered (``EdgError``): train-mode gate dropout
+        without ``pair_dropout``, ``fc_sigmoid`` without ``pair_fc_sigmoid``, ``view_len``, ``aspect``,
+        ``return_x_out`` and 3-D dense-compat ``x``."""
         if not x.is_cuda:
             raise L.EdgError("GatedGCNStack runs on CUDA tensors only (there is no CPU path)")
         if pairs is not None:
@@ -1063,8 +1084,8 @@ class GatedGCNStack(nn.Module):
         drop = self.training and self.dropout_p > 0 and self.gated
         if drop and not self.pair_dropout:
             declined.append("train-mode gate dropout (p > 0) unless GatedGCNStack(pair_dropout=True)")
-        if self.fc_sigmoid:
-            declined.append("fc_sigmoid")
+        if self.fc_sigmoid and not self.pair_fc_sigmoid:
+            declined.append("fc_sigmoid unless GatedGCNStack(pair_fc_sigmoid=True)")
         if view_len is not None:
             declined.append("view_len")
         if aspect is not None:

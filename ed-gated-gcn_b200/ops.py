@@ -741,6 +741,52 @@ def head_bwd_drop_pairs(h, graph, pairs, gate, v, dist, scores, kl_b, g_kl, g_sc
     return dh, dgate, dv, dc
 
 
+def scores_kl_sig_pairs_fwd(h, graph, pairs, gate, v, c, dist, seed: Optional[torch.Tensor] = None, stream_id: int = 0,
+                            p: float = 0.0):
+    """BertAmir54's scores / kl per pair (``edg_scores_kl_sig_pairs_fwd``): :func:`scores_kl_pairs_fwd` on
+    ``z = sigmoid(gate_p * h_t)`` with a unit gate (``dv_unit`` has no gate factor); with ``seed`` on the pairs' masked
+    rows of dropout stream ``stream_id``."""
+    P, D = gate.shape
+    dev = h.device
+    R = pairs.n_pair_rows
+    scores = torch.empty((max(R, 1),), dtype=torch.float32, device=dev)[:R]
+    kl_b = torch.empty((P,), dtype=torch.float32, device=dev)
+    dvu = torch.empty((P, D), dtype=torch.float32, device=dev)
+    dcu = torch.empty((P,), dtype=torch.float32, device=dev)
+    L.call("edg_scores_kl_sig_pairs_fwd", L.ptr(h), L.dt(h), ld(h), L.ptr(graph.sent_ptr), L.ptr(pairs.pair_sent),
+           L.ptr(pairs.pair_row_ptr), P, D, L.ptr(gate), L.ptr(v), L.ptr(c), L.ptr(dist), _dist_flag(dist), L.ptr(scores),
+           L.ptr(kl_b), L.ptr(dvu), L.ptr(dcu), L.ptr(seed), int(stream_id), float(p), L.stream())
+    kl = torch.empty((), dtype=torch.float32, device=dev)
+    L.call("edg_sum_scaled", L.ptr(kl_b), P, 1.0 / max(P, 1), L.ptr(kl), L.stream())
+    return scores, kl_b, kl, dvu, dcu
+
+
+def head_bwd_sig_pairs(h, graph, pairs, gate, v, dist, scores, kl_b, g_kl, g_scores, g_pooled, arg, mmax,
+                       seed: Optional[torch.Tensor], stream_id: int, p: float, want_dh: bool,
+                       dgate_out: Optional[torch.Tensor] = None):
+    """Backward of :func:`scores_kl_sig_pairs_fwd` and the final pool (``edg_head_bwd_sig_pairs``), the two passes of
+    :func:`head_bwd_pairs`.  ``seed`` None: ``arg`` int32 ``[S,D]`` per sentence (``mmax`` unused); otherwise ``arg`` /
+    ``mmax`` ``[P,D]`` of :func:`pool_drop_pairs` on the same dropout stream."""
+    P, D = gate.shape
+    N = h.shape[0]
+    dev = h.device
+    dh = alloc_rows(N, D, h.dtype, dev) if want_dh else None
+    dgate = (dgate_out if dgate_out is not None else torch.empty((P, D), dtype=torch.float32, device=dev)) \
+        if want_dh else None
+    dv = None if want_dh else torch.empty((P, D), dtype=torch.float32, device=dev)
+    dc = None if want_dh else torch.empty((P,), dtype=torch.float32, device=dev)
+    ds_ws = torch.empty((max(pairs.n_pair_rows, 1),), dtype=torch.float32, device=dev)
+    if want_dh and graph.row_sent is None:
+        raise L.EdgError("the pairs head backward needs graph.row_sent (build_graph / graph_from_dense set it)")
+    L.call("edg_head_bwd_sig_pairs", L.ptr(h), L.dt(h), ld(h), L.ptr(graph.sent_ptr), graph.n_graphs,
+           L.ptr(graph.row_sent) if N > 0 else None, N, L.ptr(pairs.pair_ptr),
+           L.ptr(pairs.pair_sent), L.ptr(pairs.pair_row_ptr), P, D, L.ptr(gate), L.ptr(v), L.ptr(dist),
+           _dist_flag(dist) if dist is not None else 0, L.ptr(scores), L.ptr(kl_b), L.ptr(g_kl), L.ptr(g_scores),
+           L.ptr(g_pooled), L.ptr(arg), L.ptr(mmax), L.ptr(dh), ld(dh) if dh is not None else 0, L.ptr(dgate), L.ptr(dv),
+           L.ptr(dc), L.ptr(ds_ws), L.ptr(seed), int(stream_id), float(p), L.stream())
+    return dh, dgate, dv, dc
+
+
 def views_bwd_drop_pairs(pooled, mmax, arg, gates, g_xy, graph, pairs, seed: torch.Tensor, p: float,
                          dh: Optional[torch.Tensor] = None, dgates: Optional[torch.Tensor] = None,
                          acc_view: int = -1) -> None:

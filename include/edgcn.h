@@ -621,6 +621,36 @@ int edg_head_bwd_drop_pairs(const void* h, int dtype, int64_t ldh, const int32_t
                             const float* g_scores, const float* g_pooled, const int32_t* arg, const float* mmax, void* dh,
                             int64_t lddh, float* dgate, float* dv, float* dc, float* ds_ws, const int64_t* seed,
                             int32_t stream_id, float p, edg_stream stream);
+/* BertAmir54 on the pairs (bert_amir5.py:464-465 fc = Sequential(Sigmoid, Linear), applied at :538 before the scores
+ * of :645-648): pair p scores the sigmoid of its gated rows, z_{p,t} = T(sigmoid(gate_p * h~_{p,t})) -- the value
+ * edg_gate_rows_act stores, T the row dtype -- against v_p with a unit gate.  h~_{p,t} is row t of the pair's sentence
+ * as stored (seed = NULL) or under the pair's mask of dropout stream stream_id (seed given; as edg_scores_kl_drop_pairs_fwd).
+ * gate_p does not factor out of the sigmoid, so z is formed from each row as it is read; nothing is stored per
+ * (pair, row).  Replaces the materialised z rows of the unpaired BertAmir54 path (edg_gate_rows_act + edg_scores_kl_fwd
+ * with a unit gate) for a batch holding each sentence once.
+ *
+ * Forward: scores_{p,t} = sum_d z_{p,t,d} v_{p,d} + c_p, kl_b as edg_scores_kl_pairs_fwd, optional dv_unit [P,D] =
+ * sum_t u_t z_{p,t} (no gate factor), dc_unit [P] = sum_t u_t.  Same empty-sentence, P = 0 and D rules. */
+int edg_scores_kl_sig_pairs_fwd(const void* h, int dtype, int64_t ldh, const int32_t* sent_ptr, const int32_t* pair_sent,
+                                const int32_t* pair_row_ptr, int32_t P, int32_t D, const float* gate, const float* v,
+                                const float* c, const void* dist, int dist_i64, float* scores, float* kl_b,
+                                float* dv_unit, float* dc_unit, const int64_t* seed, int32_t stream_id, float p,
+                                edg_stream stream);
+/* Its backward with the final pool, the two-pass contract of edg_head_bwd_pairs, ds_{p,t} as there:
+ *   dc_p = sum_t ds_{p,t},  dv_p = sum_t ds_{p,t} z_{p,t},
+ *   dgate_p = v_p * sum_t ds_{p,t} z (1 - z) h~_{p,t} + g_pooled_p * h[arg],
+ *   dh_t = sum_{p of s} [keep_{p,t} / (1-p)] gate_p * (ds_{p,t} v_p z (1 - z)) + (arg-max term),
+ * one thread per (row, 16-byte chunk) reading h_t once and the sentence's pairs in ascending order.  seed = NULL:
+ * arg int32 [S,D] per sentence and the arg-max term of edg_head_bwd_pairs (mmax unused); seed given: arg / mmax [P,D]
+ * per pair and the arg-max term of edg_head_bwd_drop_pairs.  Every row of dh is written (0 where the sentence has no
+ * pairs; P = 0 gives dh = 0 and the per-pair arrays may be NULL). */
+int edg_head_bwd_sig_pairs(const void* h, int dtype, int64_t ldh, const int32_t* sent_ptr, int32_t S,
+                           const int32_t* row_sent, int32_t N, const int32_t* pair_ptr, const int32_t* pair_sent,
+                           const int32_t* pair_row_ptr, int32_t P, int32_t D, const float* gate, const float* v,
+                           const void* dist, int dist_i64, const float* scores, const float* kl_b, const float* g_kl,
+                           const float* g_scores, const float* g_pooled, const int32_t* arg, const float* mmax, void* dh,
+                           int64_t lddh, float* dgate, float* dv, float* dc, float* ds_ws, const int64_t* seed,
+                           int32_t stream_id, float p, edg_stream stream);
 /* Backward of the masked views (streams 0..V-1) and the diversity term from edg_pool_drop_pairs' pooled / mmax / arg
  * [V,P,D], with dP_{v,p} = g_xy / P * (sum_{v'} pooled_{v',p} - pooled_{v,p}):
  *   dgates (optional) [V,P,D]:  dgates[v,p] (+)= dP_{v,p} * mmax_{v,p}   (+= for v = acc_view)

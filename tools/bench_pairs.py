@@ -17,8 +17,14 @@ grouped arm with ``pair_dropout=True`` (per-pair masked passes over the sentence
 path (masked copies of the expanded rows).  Both arms draw their masks from the same seed, so they compute the same
 result.
 
+``--fc-sigmoid`` runs BertAmir54's block in both arms (``fc_sigmoid=True``; the grouped arm with
+``pair_fc_sigmoid=True``, which forms every pair's sigmoid rows inside the per-pair kernels).  ``--hidden`` sets D
+(BertAmir54's LSTM output is 256 wide).
+
     python tools/bench_pairs.py --sentences 149 --steps 100 --warmup 10 --rounds 3 --out profiles/r04_a_bench_pairs.json
     python tools/bench_pairs.py --dropout 0.25 --out profiles/r05_a_bench_pairs_dropout.json
+    python tools/bench_pairs.py --fc-sigmoid --hidden 256 --out profiles/r08_a_bench_pairs_fc_sigmoid.json
+    python tools/bench_pairs.py --fc-sigmoid --hidden 256 --dropout 0.25 --out profiles/r08_b_bench_pairs_fc_sigmoid_dropout.json
 """
 from __future__ import annotations
 
@@ -52,6 +58,8 @@ def main():
     ap.add_argument("--rounds", type=int, default=3)
     ap.add_argument("--seed", type=int, default=14181)
     ap.add_argument("--dropout", type=float, default=0.0)
+    ap.add_argument("--fc-sigmoid", action="store_true")
+    ap.add_argument("--hidden", type=int, default=300)
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
 
@@ -59,7 +67,7 @@ def main():
     from ed_gated_gcn_b200 import synth
     from ed_gated_gcn_b200.runtime import GraphedStep
     dev = torch.device("cuda", torch.cuda.current_device())
-    D, Lyr, C = 300, 2, 34
+    D, Lyr, C = args.hidden, 2, 34
     cd = torch.bfloat16
     batch = synth.make_batch(args.sentences, 5, 50, seed=args.seed)
     pp, an = synth.candidate_pairs(batch)
@@ -73,7 +81,8 @@ def main():
 
     torch.manual_seed(args.seed)
     stack = E.GatedGCNStack(D, n_layers=Lyr, n_classes=C, compute_dtype=cd, dropout=args.dropout,
-                            pair_dropout=args.dropout > 0).to(dev)
+                            pair_dropout=args.dropout > 0, fc_sigmoid=args.fc_sigmoid,
+                            pair_fc_sigmoid=args.fc_sigmoid).to(dev)
     head = E.DenseHead(2 * D, C).to(dev)
     x_host = torch.randn(batch.n_rows, D, generator=torch.Generator().manual_seed(args.seed + 1)).to(cd)
     tgt = (torch.arange(P) % C).to(dev)
@@ -142,7 +151,7 @@ def main():
     name, pl = card()
     res = {"tool": "bench_pairs", "gpu": name, "power_limit": pl, "sentences": batch.n_graphs, "pairs": P,
            "sentence_rows": batch.n_rows, "expanded_rows": int(len(rows)), "D": D, "L": Lyr, "dtype": "bf16",
-           "dropout": args.dropout,
+           "dropout": args.dropout, "fc_sigmoid": args.fc_sigmoid,
            "steps": args.steps, "warmup": args.warmup, "rounds": args.rounds, "max_rel_logits_grouped_vs_expanded":
            max_rel_logits, "arms": {}}
     for n in arms:
