@@ -44,10 +44,6 @@ SIGNATURES = {
     "edg_gcn_layer": (c_int, [_P, _L, _I, _I, _P, _L, _I, _P, c_int, _P, _P, _P, _P, _P, _I, _P, _L, _P, _P, _L, _P, _P,
                               _L, _P, c_int, _P, _Z, _P]),
     "edg_adam_multi": (c_int, [_I, _P, _P, _P, _P, _P, _P, c_float, c_float, c_float, c_float, c_float, c_float, _P]),
-    "edg_dense_head_fwd": (c_int, [_P, _L, _P, _L, _P, _L, _P, _I, _I, _I, _P, _L, _P]),
-    "edg_dense_head_bwd_workspace": (_Z, [_I, _I, _I]),
-    "edg_dense_head_bwd": (c_int, [_P, _L, _P, _L, _P, _L, _P, _L, _I, _I, _I, c_int, _P, _L, _P, _P, _P, _P, _P, _L, _P, _P, _Z,
-                                   _P]),
     "edg_block_head_fwd": (c_int, [_P, _L, _P, _L, _P, _L, _P, _L, _P, _L, _P, _P, _L, _P, _I, _I, _I, _P, _P, _P, _P, _P]),
     "edg_block_head_bwd": (c_int, [_P, _P, _L, _P, _L, c_int, _P, _L, _P, _L, _P, _P, _P, _P, _P, _P, _I, _I, _I, _P, _P,
                                    _P, _P]),
@@ -80,9 +76,6 @@ SIGNATURES = {
     "edg_views_bwd": (c_int, [_P, _P, _P, _P, c_int, _L, _I, _I, _I, _P, _P, _P, _L, _P, c_int, _P]),
     "edg_views_bwd_parts": (c_int, [_P, _P, _P, _P, c_int, _L, _I, _I, _I, _P, _P, _P, _L, _P, c_int, c_int, _P]),
     "edg_scores_kl_fwd": (c_int, [_P, c_int, _L, _P, _I, _I, _P, _P, _P, _P, c_int, _P, _P, _P, _P, _P, _P, _P, _I, _I, _P]),
-    "edg_fc_head_fwd": (c_int, [_P, _L, _P, _L, _P, _P, _L, _I, _I, _I, _P, _P, _P]),
-    "edg_fc_head_bwd_workspace": (_Z, [_I, _I, _I]),
-    "edg_fc_head_bwd": (c_int, [_P, _L, _P, _L, _P, _P, _L, _P, _P, _P, _I, _I, _I, c_int, _P, _L, _P, _P, _L, _P, _P, _Z, _P]),
     "edg_head_bwd": (c_int, [_P, c_int, _L, _P, _I, _I, _P, _P, _P, c_int, _P, _P, _P, _P, _P, _P, _P, _L,
                              _P, _L, _P, _P, _P, _I, _P, _I, _P]),
     "edg_segment_mean": (c_int, [_P, c_int, _L, _P, _P, _I, _I, _P, c_int, _L, _P]),
@@ -171,11 +164,9 @@ def _kernels_of(name: str, args) -> int:
         return 4
     if name == "edg_block_head_wgrad":
         return 2
-    if name == "edg_dense_head_bwd":
-        return 2 if (args[11] & 2) else 1
     if name == "edg_split_f16":
         return 2
-    if name in ("edg_csr_from_dense_count", "edg_diversity_fwd", "edg_colsum", "edg_fc_head_bwd", "edg_wgrad_batch", "edg_head_du"):
+    if name in ("edg_csr_from_dense_count", "edg_diversity_fwd", "edg_colsum", "edg_wgrad_batch", "edg_head_du"):
         return 2
     if name == "edg_gcn_layer":
         return 2 if args[23] else 1

@@ -7,33 +7,38 @@
 //     dlg_b = g_logits_b + Wfc u_b + s dc_b bfc
 //     da_b  = s dc_b (logits_b^T Wfc[:, D:]) (* af (1 - af) under fc_sigmoid) + dlg_b^T W[:, :D]
 //     dp_b  = dlg_b^T W[:, D:] + g_pooled_b
-// edg_dense_head_* and edg_fc_head_* compute the same maps as a chain of launches, each split into two column-half
-// blocks that meet through atomics or a reduction launch; here a block owns 8 sentences and both column halves, so v,
-// c and the input gradients follow the logits without leaving the SM.  [B,*] work is bound by latency and by how many
-// blocks carry it, not by bytes (DESIGN section 5): 512 blocks of 128 threads at C2, all resident at once.
+// Either head may be left out (template flags HEAD / FC): without the dense head (a torch logits_fn) the logits are an
+// input and only the fc terms are formed; without fc (a DenseHead called on its own) only the logits and their input
+// gradients are.  A block owns 8 sentences and both column halves, so v, c and the input gradients follow the logits
+// without leaving the SM.  [B,*] work is bound by latency and by how many blocks carry it, not by bytes (DESIGN
+// section 5): 512 blocks of 128 threads at C2, all resident at once.
 //
-// Every result has the bits the launch chain gives: each sum keeps that chain's fp32 order (lane-strided fmaf chains
-// closed by an xor butterfly for the K = D reductions, classes in ascending order for the K = C products, sentences in
-// blocks of 32 then blocks in order for the parameter gradients).  A training run therefore does not drift from the
-// one the chain gave -- which matters here: d kl / d c is zero analytically (the softmax over a sentence's scores does
-// not see a shift), so d fc.bias is pure rounding, and Adam turns any reordering of it into different parameters.
+// Every sum has a fixed fp32 order (lane-strided fmaf chains closed by an xor butterfly for the K = D reductions,
+// classes in ascending order for the K = C products, sentences in blocks of 32 then blocks in order for the parameter
+// gradients), and the order of each sum is the same whichever heads a launch runs: the combined launch gives the bits
+// of the dense-only and fc-only launches composed.  A torch-head and a DenseHead training run therefore follow the same
+// arithmetic -- which matters here: d kl / d c is zero analytically (the softmax over a sentence's scores does not see
+// a shift), so d fc.bias is pure rounding, and Adam turns any reordering of it into different parameters.
 // Phase 1 (the K = D reductions) stages the pass's rows in shared memory and reads the weights through L1; a warp
 // takes 4 sentences x 8 classes and reduces the 32 lane-partial sums in one scattering butterfly.  Phase 2 (the K = C
 // products) reads the weights through L1 with 128-bit loads, a thread owning 4 sentences x 4 columns.  The parameter
-// gradients (edg_block_head_wgrad) are one partial launch plus one reduction in block order.  (Included after
-// edg_dense_head.cu: shares its staging helpers and constants.)
+// gradients (edg_block_head_wgrad) are one partial launch plus one reduction in block order.
 #include "edg_common.cuh"
 
 namespace edg {
 
+constexpr int kHeadMaxC = 64;
+constexpr int kHeadGraphs = 32;           // sentences per block (parameter-gradient kernel)
+constexpr int kHeadThreads = 256;
+constexpr int kHeadPitch = 320;           // columns staged per pass (compile-time: shared-memory offsets become immediates)
 constexpr int kBhS = 8;                   // sentences per block (forward / input-gradient kernels)
 constexpr int kBhWarps = 4;
 constexpr int kBhThreads = 32 * kBhWarps;
 constexpr int kBhP = kHeadPitch;          // columns per phase-1 pass (a multiple of 32: lane residues stay aligned)
 
 // rows [b0, b0 + nb) of x[:, col0 : col0 + lim) into Xs[kBhS][kBhP] (zero beyond nb / lim), each element times m[., .]
-// when m is given (the product is also written to `out` [B, ldo] when given) or times rs[row] when rs is given -- the
-// same single roundings as the staging of edg_fc_head_bwd and the torch product gate * hmax
+// when m is given (the product is also written to `out` [B, ldo] when given) or times rs[row] when rs is given -- one
+// rounding per product, as in the torch product gate * hmax
 template <bool VEC>
 __device__ __forceinline__ void bh_stage_rows(float* __restrict__ Xs, const float* __restrict__ x, int64_t ldx,
                                               const float* __restrict__ m, int64_t ldm, float* __restrict__ out,
@@ -77,10 +82,9 @@ __device__ __forceinline__ void bh_stage_rows(float* __restrict__ Xs, const floa
 
 // Phase 1 of one pass: for both halves h (rows Xs[h] against W[:, wcol[h] + d0 + .]), every sentence and class,
 //     out[h][s][c] += warp_sum over lanes r of ( sum over the pass columns jj = r, r + 32, ... of x[s][jj] W[c][jj] )
-// -- the order of edg_dense_head_fwd / edg_fc_head_bwd (lane-strided fmaf chains, xor-butterfly across the lanes), so
-// the results are the same bits.  A warp takes 4 sentences x 8 classes at a time (every staged x and every W element
-// loaded feeds 8 or 4 fmas) and reduces those 32 sums in one xor-butterfly that scatters them over the lanes: 31
-// shuffles instead of 32 x 5, with each sum built from the same pairs as warp_sum's.
+// (lane-strided fmaf chains, xor-butterfly across the lanes).  A warp takes 4 sentences x 8 classes at a time (every
+// staged x and every W element loaded feeds 8 or 4 fmas) and reduces those 32 sums in one xor-butterfly that scatters
+// them over the lanes: 31 shuffles instead of 32 x 5, with each sum built from the same pairs as warp_sum's.
 template <int NCG8>
 __device__ __forceinline__ void bh_pass(const float* __restrict__ Xs, const float* __restrict__ W, int64_t ldw,
                                         int wcol0, int wcol1, int d0, int lim, int C, float* __restrict__ out) {
@@ -163,7 +167,8 @@ __device__ __forceinline__ void bh_mix(const float (*coef)[kBhS], const float* _
 }
 
 // ---- forward ----------------------------------------------------------------------------------------------------
-template <int NCG8, bool VEC>
+// HEAD: the logits from [a | pooled] (else read from `logits`); FC: v and c from the logits.
+template <int NCG8, bool VEC, bool HEAD, bool FC>
 __global__ void __launch_bounds__(kBhThreads, 4)
 block_head_fwd_kernel(const float* __restrict__ a, int64_t lda, const float* __restrict__ af, int64_t ldf,
                       const float* __restrict__ p, int64_t ldp, const float* __restrict__ g, int64_t ldg,
@@ -178,26 +183,33 @@ block_head_fwd_kernel(const float* __restrict__ a, int64_t lda, const float* __r
   const int b0 = blockIdx.x * kBhS;
   const int nb = min(kBhS, B - b0);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  for (int i = threadIdx.x; i < 2 * kBhS * CP; i += kBhThreads) part[i] = 0.f;
-  for (int d0 = 0; d0 < D; d0 += kBhP) {
-    const int lim = min(kBhP, D - d0);
-    __syncthreads();                                                     // previous pass consumed (part zeroed)
-    bh_stage_rows<VEC>(Xs, a, lda, nullptr, 0, nullptr, 0, nullptr, b0, nb, d0, lim);
-    bh_stage_rows<VEC>(Xs + kBhS * kBhP, p, ldp, g, ldg, pooled, D, nullptr, b0, nb, d0, lim);
+  if constexpr (HEAD) {
+    for (int i = threadIdx.x; i < 2 * kBhS * CP; i += kBhThreads) part[i] = 0.f;
+    for (int d0 = 0; d0 < D; d0 += kBhP) {
+      const int lim = min(kBhP, D - d0);
+      __syncthreads();                                                   // previous pass consumed (part zeroed)
+      bh_stage_rows<VEC>(Xs, a, lda, nullptr, 0, nullptr, 0, nullptr, b0, nb, d0, lim);
+      bh_stage_rows<VEC>(Xs + kBhS * kBhP, p, ldp, g, ldg, pooled, D, nullptr, b0, nb, d0, lim);
+      __syncthreads();
+      bh_pass<NCG8>(Xs, W, ldw, 0, D, d0, lim, C, part);
+    }
     __syncthreads();
-    bh_pass<NCG8>(Xs, W, ldw, 0, D, d0, lim, C, part);
   }
-  __syncthreads();
-  // logits = (W[:, :D] a + bias) + W[:, D:] pooled: edg_dense_head_fwd's two commuting additions onto zero
+  // logits = (W[:, :D] a + bias) + W[:, D:] pooled
   for (int i = threadIdx.x; i < kBhS * CP; i += kBhThreads) {
     const int s = i / CP, c = i - s * CP;
     float l = 0.f;
     if (s < nb && c < C) {
-      l = (part[s * CP + c] + (bias ? __ldg(bias + c) : 0.f)) + part[(kBhS + s) * CP + c];
-      logits[(int64_t)(b0 + s) * C + c] = l;
+      if constexpr (HEAD) {
+        l = (part[s * CP + c] + (bias ? __ldg(bias + c) : 0.f)) + part[(kBhS + s) * CP + c];
+        logits[(int64_t)(b0 + s) * C + c] = l;
+      } else {
+        l = __ldg(logits + (int64_t)(b0 + s) * C + c);
+      }
     }
     lg_t[c][s] = l;
   }
+  if constexpr (!FC) return;
   __syncthreads();
   // v = logits^T Wfc[:, :D]
   bh_mix<CP, VEC>(lg_t, Wf, ldfw, C, D, nb, [&](int s0, int j, const float (&o)[4][4]) {
@@ -210,7 +222,7 @@ block_head_fwd_kernel(const float* __restrict__ a, int64_t lda, const float* __r
     }
   });
   // c = warp_sum over lanes of (sum over d = lane, lane + 32, ... of af[d] va[d]) + logits . bfc, va = logits^T
-  // Wfc[:, D:] -- edg_fc_head_fwd's order; va goes through shared memory a pass at a time, a warp owns 2 sentences
+  // Wfc[:, D:]; va goes through shared memory a pass at a time, a warp owns 2 sentences
   float* va = Xs;                                                        // [kBhS][kBhP]
   float cacc[2] = {0.f, 0.f};
   for (int d0 = 0; d0 < D; d0 += kBhP) {
@@ -245,9 +257,9 @@ block_head_fwd_kernel(const float* __restrict__ a, int64_t lda, const float* __r
 }
 
 // ---- input gradients -----------------------------------------------------------------------------------------------
-// The order of edg_fc_head_bwd (parts = 1) followed by edg_dense_head_bwd (parts = 1): dlg = g + ((Wfc[:, :D] (s dv) +
-// s dc bfc) + Wfc[:, D:] (s dc af)), da = dlg^T W[:, :D] + (s dc) (logits^T Wfc[:, D:]), dp = dlg^T W[:, D:] + g_pooled.
-template <int NCG8, bool VEC>
+// dlg = g + ((Wfc[:, :D] (s dv) + s dc bfc) + Wfc[:, D:] (s dc af)), da = dlg^T W[:, :D] + (s dc) (logits^T Wfc[:, D:]),
+// dp = dlg^T W[:, D:] + g_pooled.  FC: the fc terms (when dv is given); HEAD: the dense head's terms and dp.
+template <int NCG8, bool VEC, bool HEAD, bool FC>
 __global__ void __launch_bounds__(kBhThreads, 4)
 block_head_bwd_kernel(const float* __restrict__ lg, const float* __restrict__ a, int64_t lda,
                       const float* __restrict__ af, int64_t ldf, int fc_sigmoid, const float* __restrict__ W, int64_t ldw,
@@ -263,7 +275,7 @@ block_head_bwd_kernel(const float* __restrict__ lg, const float* __restrict__ a,
   __shared__ float rs_v[kBhS], dc_s[kBhS];
   const int b0 = blockIdx.x * kBhS;
   const int nb = min(kBhS, B - b0);
-  const bool scores = dv != nullptr;
+  const bool scores = FC && dv != nullptr;
   const float sc = (scores && scale) ? __ldg(scale) : 1.f;
   if (threadIdx.x < kBhS) {
     const int s = threadIdx.x;
@@ -285,7 +297,7 @@ block_head_bwd_kernel(const float* __restrict__ lg, const float* __restrict__ a,
     float d = 0.f, l = 0.f;
     if (s < nb && c < C) {
       const int64_t o = (int64_t)(b0 + s) * C + c;
-      l = __ldg(lg + o);
+      if (FC) l = __ldg(lg + o);
       if (scores) {
         d = fmaf(dc_s[s], __ldg(bf + c), part[s * CP + c]) + part[(kBhS + s) * CP + c];
         if (g_lg) d = __ldg(g_lg + o) + d;
@@ -309,15 +321,19 @@ block_head_bwd_kernel(const float* __restrict__ lg, const float* __restrict__ a,
     float t1[4][4] = {}, t2[4][4] = {};
 #pragma unroll 4
     for (int c = 0; c < C; ++c) {
-      float w1[4], w2[4];
+      float w1[4] = {}, w2[4] = {};
       if (VEC) {
-        const float4 x = __ldg(reinterpret_cast<const float4*>(Wf + (int64_t)c * ldfw + D + j));
-        const float4 y = __ldg(reinterpret_cast<const float4*>(W + (int64_t)c * ldw + j));
-        w1[0] = x.x; w1[1] = x.y; w1[2] = x.z; w1[3] = x.w;
-        w2[0] = y.x; w2[1] = y.y; w2[2] = y.z; w2[3] = y.w;
+        if (FC) {
+          const float4 x = __ldg(reinterpret_cast<const float4*>(Wf + (int64_t)c * ldfw + D + j));
+          w1[0] = x.x; w1[1] = x.y; w1[2] = x.z; w1[3] = x.w;
+        }
+        if (HEAD) {
+          const float4 y = __ldg(reinterpret_cast<const float4*>(W + (int64_t)c * ldw + j));
+          w2[0] = y.x; w2[1] = y.y; w2[2] = y.z; w2[3] = y.w;
+        }
       } else {
-        w1[0] = __ldg(Wf + (int64_t)c * ldfw + D + j); w2[0] = __ldg(W + (int64_t)c * ldw + j);
-        w1[1] = w1[2] = w1[3] = w2[1] = w2[2] = w2[3] = 0.f;
+        if (FC) w1[0] = __ldg(Wf + (int64_t)c * ldfw + D + j);
+        if (HEAD) w2[0] = __ldg(W + (int64_t)c * ldw + j);
       }
       const float4 k = *reinterpret_cast<const float4*>(&lg_t[c][s0]);
       const float4 d = *reinterpret_cast<const float4*>(&dlg_t[c][s0]);
@@ -335,14 +351,14 @@ block_head_bwd_kernel(const float* __restrict__ lg, const float* __restrict__ a,
       float o[4];
 #pragma unroll
       for (int q = 0; q < 4; ++q) {
-        o[q] = t2[i][q];
+        o[q] = HEAD ? t2[i][q] : 0.f;
         if (scores && q < nj) {
           float f = dc_s[s0 + i] * t1[i][q];
           if (fc_sigmoid) {
             const float z = __ldg(af + b * ldf + j + q);
             f = (f * z) * (1.f - z);
           }
-          o[q] = o[q] + f;
+          o[q] = HEAD ? o[q] + f : f;
         }
       }
       float* dst = da + b * D + j;
@@ -351,7 +367,7 @@ block_head_bwd_kernel(const float* __restrict__ lg, const float* __restrict__ a,
     }
   }
   // d p = dlg^T W[:, D:] + g_pooled
-  bh_mix<CP, VEC>(dlg_t, W + D, ldw, C, D, nb, [&](int s0, int j, const float (&o)[4][4]) {
+  if constexpr (HEAD) bh_mix<CP, VEC>(dlg_t, W + D, ldw, C, D, nb, [&](int s0, int j, const float (&o)[4][4]) {
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
       if (s0 + i >= nb) break;
@@ -368,6 +384,27 @@ block_head_bwd_kernel(const float* __restrict__ lg, const float* __restrict__ a,
       }
     }
   });
+}
+
+// rows [b0, b0+nb) of x[:, d0 : d0+kHeadPitch) into Xs [32][kHeadPitch], zero beyond nb / lim
+__device__ __forceinline__ void stage_rows_chunk(float* __restrict__ Xs, const float* __restrict__ x, int64_t ldx, int b0,
+                                                 int nb, int d0, int lim, bool vec4) {
+  if (vec4) {
+    constexpr int P4 = kHeadPitch / 4;
+#pragma unroll 4
+    for (int i = threadIdx.x; i < kHeadGraphs * P4; i += kHeadThreads) {
+      const int g = i / P4, jj = (i - g * P4) << 2;
+      float4 u = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (g < nb && jj < lim) u = __ldg(reinterpret_cast<const float4*>(x + (int64_t)(b0 + g) * ldx + d0 + jj));
+      *reinterpret_cast<float4*>(Xs + g * kHeadPitch + jj) = u;
+    }
+  } else {
+#pragma unroll 4
+    for (int i = threadIdx.x; i < kHeadGraphs * kHeadPitch; i += kHeadThreads) {
+      const int g = i / kHeadPitch, jj = i - g * kHeadPitch;
+      Xs[i] = (g < nb && jj < lim) ? __ldg(x + (int64_t)(b0 + g) * ldx + d0 + jj) : 0.f;
+    }
+  }
 }
 
 // ---- parameter gradients: per-block partials [nblocks][C][4D + 2] -----------------------------------------------
@@ -460,6 +497,21 @@ block_head_wgrad_reduce_kernel(const float* __restrict__ partial, int nblocks, i
   *dst = s;
 }
 
+// the instantiation for C, the row alignment and the heads present (at least one)
+template <bool HEAD, bool FC, class Launch>
+int bh_fwd_launch(int C, bool vec4, Launch launch) {
+  if (C <= 8) return vec4 ? launch(block_head_fwd_kernel<1, true, HEAD, FC>) : launch(block_head_fwd_kernel<1, false, HEAD, FC>);
+  if (C <= 40) return vec4 ? launch(block_head_fwd_kernel<5, true, HEAD, FC>) : launch(block_head_fwd_kernel<5, false, HEAD, FC>);
+  return vec4 ? launch(block_head_fwd_kernel<8, true, HEAD, FC>) : launch(block_head_fwd_kernel<8, false, HEAD, FC>);
+}
+
+template <bool HEAD, bool FC, class Launch>
+int bh_bwd_launch(int C, bool vec4, Launch launch) {
+  if (C <= 8) return vec4 ? launch(block_head_bwd_kernel<1, true, HEAD, FC>) : launch(block_head_bwd_kernel<1, false, HEAD, FC>);
+  if (C <= 40) return vec4 ? launch(block_head_bwd_kernel<5, true, HEAD, FC>) : launch(block_head_bwd_kernel<5, false, HEAD, FC>);
+  return vec4 ? launch(block_head_bwd_kernel<8, true, HEAD, FC>) : launch(block_head_bwd_kernel<8, false, HEAD, FC>);
+}
+
 }  // namespace edg
 
 using namespace edg;
@@ -469,11 +521,13 @@ extern "C" int edg_block_head_fwd(const float* a, int64_t lda, const float* a_fc
                                   const float* bias, const float* fc_w, int64_t ldfw, const float* fc_b, int32_t B,
                                   int32_t D, int32_t C, float* pooled, float* logits, float* v, float* c,
                                   edg_stream stream) {
-  if (B < 0 || D <= 0 || C <= 0) return EDG_ERR_ARG;
+  const bool head = W != nullptr, fc = fc_w != nullptr;
+  if (B < 0 || D <= 0 || C <= 0 || (!head && !fc)) return EDG_ERR_ARG;
   if (C > kHeadMaxC) return EDG_ERR_UNSUPPORTED;
   if (B == 0) return EDG_OK;
-  if (!a || !a_fc || !p || !W || !fc_w || !fc_b || !logits || !v || !c || (g && !pooled)) return EDG_ERR_ARG;
-  if (lda < D || ldf < D || ldp < D || (g && ldg < D) || ldw < 2 * D || ldfw < 2 * D) return EDG_ERR_ARG;
+  if (!logits || (head && (!a || !p || (g && !pooled))) || (fc && (!a_fc || !fc_b || !v || !c))) return EDG_ERR_ARG;
+  if ((head && (lda < D || ldp < D || (g && ldg < D) || ldw < 2 * D)) || (fc && (ldf < D || ldfw < 2 * D)))
+    return EDG_ERR_ARG;
   const bool vec4 = (D & 3) == 0 && (lda & 3) == 0 && (ldf & 3) == 0 && (ldp & 3) == 0 && (ldg & 3) == 0 &&
                     (ldw & 3) == 0 && (ldfw & 3) == 0 && aligned16(a) && aligned16(a_fc) && aligned16(p) &&
                     aligned16(g) && aligned16(W) && aligned16(fc_w) && aligned16(pooled) && aligned16(v);
@@ -484,9 +538,9 @@ extern "C" int edg_block_head_fwd(const float* a, int64_t lda, const float* a_fc
                                        logits, v, c);
     return check_launch();
   };
-  if (C <= 8) return vec4 ? launch(block_head_fwd_kernel<1, true>) : launch(block_head_fwd_kernel<1, false>);
-  if (C <= 40) return vec4 ? launch(block_head_fwd_kernel<5, true>) : launch(block_head_fwd_kernel<5, false>);
-  return vec4 ? launch(block_head_fwd_kernel<8, true>) : launch(block_head_fwd_kernel<8, false>);
+  if (!head) return bh_fwd_launch<false, true>(C, vec4, launch);
+  if (!fc) return bh_fwd_launch<true, false>(C, vec4, launch);
+  return bh_fwd_launch<true, true>(C, vec4, launch);
 }
 
 extern "C" int edg_block_head_bwd(const float* logits, const float* a, int64_t lda, const float* a_fc, int64_t ldf,
@@ -494,11 +548,13 @@ extern "C" int edg_block_head_bwd(const float* logits, const float* a, int64_t l
                                   const float* fc_b, const float* dv, const float* dc, const float* scale,
                                   const float* g_logits, const float* g_pooled, int32_t B, int32_t D, int32_t C,
                                   float* dlg, float* da, float* dp, edg_stream stream) {
-  if (B < 0 || D <= 0 || C <= 0) return EDG_ERR_ARG;
+  const bool head = W != nullptr, fc = fc_w != nullptr;
+  if (B < 0 || D <= 0 || C <= 0 || (!head && !fc)) return EDG_ERR_ARG;
   if (C > kHeadMaxC) return EDG_ERR_UNSUPPORTED;
   if (B == 0) return EDG_OK;
-  if (!logits || !a || !a_fc || !W || !fc_w || !fc_b || !dlg || !da || !dp || (!dv) != (!dc)) return EDG_ERR_ARG;
-  if (lda < D || ldf < D || ldw < 2 * D || ldfw < 2 * D) return EDG_ERR_ARG;
+  if (!a || !dlg || !da || (head && !dp) || (!dv) != (!dc) || (!fc && dv)) return EDG_ERR_ARG;
+  if (fc && (!logits || !a_fc || !fc_b)) return EDG_ERR_ARG;
+  if (lda < D || (head && ldw < 2 * D) || (fc && (ldf < D || ldfw < 2 * D))) return EDG_ERR_ARG;
   const bool vec4 = (D & 3) == 0 && (lda & 3) == 0 && (ldf & 3) == 0 && (ldw & 3) == 0 && (ldfw & 3) == 0 &&
                     aligned16(a) && aligned16(a_fc) && aligned16(W) && aligned16(fc_w) && aligned16(dv) &&
                     aligned16(g_pooled) && aligned16(da) && aligned16(dp);
@@ -509,9 +565,9 @@ extern "C" int edg_block_head_bwd(const float* logits, const float* a, int64_t l
                                        g_logits, g_pooled, B, D, C, dlg, da, dp);
     return check_launch();
   };
-  if (C <= 8) return vec4 ? launch(block_head_bwd_kernel<1, true>) : launch(block_head_bwd_kernel<1, false>);
-  if (C <= 40) return vec4 ? launch(block_head_bwd_kernel<5, true>) : launch(block_head_bwd_kernel<5, false>);
-  return vec4 ? launch(block_head_bwd_kernel<8, true>) : launch(block_head_bwd_kernel<8, false>);
+  if (!head) return bh_bwd_launch<false, true>(C, vec4, launch);
+  if (!fc) return bh_bwd_launch<true, false>(C, vec4, launch);
+  return bh_bwd_launch<true, true>(C, vec4, launch);
 }
 
 extern "C" size_t edg_block_head_wgrad_workspace(int32_t B, int32_t D, int32_t C) {
@@ -542,7 +598,7 @@ extern "C" int edg_block_head_wgrad(const float* logits, const float* dlg, const
     return check_launch();
   }
   if (!fc && !head) return EDG_OK;
-  if (!logits || !ws || (fc && !a_fc) || (head && (!a || !pooled))) return EDG_ERR_ARG;
+  if (!ws || (fc && (!logits || !a_fc)) || (head && (!a || !pooled))) return EDG_ERR_ARG;
   if ((head && (lda < D || ldp < D)) || (fc && ldf < D)) return EDG_ERR_ARG;
   if (ws_bytes < edg_block_head_wgrad_workspace(B, D, C)) return EDG_ERR_WORKSPACE;
   const int vec4 = ((D & 3) == 0 && (lda & 3) == 0 && (ldf & 3) == 0 && (ldp & 3) == 0 && aligned16(a) &&

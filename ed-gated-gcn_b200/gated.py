@@ -312,22 +312,20 @@ def _gates_bwd(gates, dgates, saved, gate_p, w_t, lead: bool, cd: torch.dtype, u
 
 
 def _head_fwd(ctx, a_raw, pooled, a_fc, fc_w, fc_b, hmax=None, gate=None):
-    """Classifier head: ``logits_fn`` is the model's own dense head (host torch, :643); a head.DenseHead (= the
-    reference's nn.Linear on cat[a, pooled]) is run by the block's own kernels: no inner autograd graph, its weight and
-    bias are head_params[0:2].  Then the per-row operands of the collapsed scores, [v_b | va_b] = logits_b @ fc.weight
-    and c_b = a_b . va_b + logits_b . fc.bias  (= logits_b . (Wfc[:, D:] a_b + bfc), SURVEY A9).  A DenseHead runs
-    both in ONE launch (``edg_block_head_fwd``), a torch head is followed by ``edg_fc_head_fwd``.  ``pooled`` None:
-    pooled = gate * hmax (written by that launch).  Returns (logits, v, c, pooled); what :func:`_head_bwd` reads stays
-    on ``ctx``."""
+    """Classifier head and the per-row operands of the collapsed scores, [v_b | va_b] = logits_b @ fc.weight and
+    c_b = a_b . va_b + logits_b . fc.bias  (= logits_b . (Wfc[:, D:] a_b + bfc), SURVEY A9), in ONE launch
+    (``edg_block_head_fwd``).  ``logits_fn`` is the model's own dense head (host torch, :643): it runs first under
+    autograd and the launch takes its logits.  A head.DenseHead (= the reference's nn.Linear on cat[a, pooled]) runs
+    inside the launch: no inner autograd graph, its weight and bias are head_params[0:2].  ``pooled`` None: pooled =
+    gate * hmax (written by the launch for a DenseHead).  Returns (logits, v, c, pooled); what :func:`_head_bwd` reads
+    stays on ``ctx``."""
     cfg = ctx.cfg
-    dense_head = cfg.get("dense_head")
-    a_leaf = p_leaf = None
-    if dense_head is not None:
+    dense = cfg.get("dense_head") is not None
+    a_leaf = p_leaf = lg = w = bias = p = g = None
+    if dense:
         hp = cfg["head_params"]
+        w, bias = hp[0], hp[1] if len(hp) > 1 else None
         p, g = (hmax, gate) if pooled is None else (pooled, None)
-        pooled, logits, v, c = ops.block_head_fwd(a_raw, a_fc, p, g, hp[0], hp[1] if len(hp) > 1 else None,
-                                                  _f32(fc_w), _f32(fc_b))
-        lg = logits
     else:
         if pooled is None:
             pooled = gate * hmax
@@ -338,69 +336,69 @@ def _head_fwd(ctx, a_raw, pooled, a_fc, fc_w, fc_b, hmax=None, gate=None):
         if logits.requires_grad and cfg["grad_enabled"]:
             _check_head_leaves(logits, (a_leaf, p_leaf), cfg["head_params"])
         lg = logits.detach().float().contiguous()
-        v, c = ops.fc_head_fwd(lg, _f32(fc_w), _f32(fc_b), a_fc)
+    n_head = w.shape[0] if dense else lg.shape[1]
+    if n_head != fc_w.shape[0]:
+        # the scores are <logits, fc(...)>: both heads have to give the same classes
+        raise L.EdgError(f"logits_fn gives {n_head} classes, the stack's fc head {fc_w.shape[0]} (n_classes)")
+    p_out, lg, v, c = ops.block_head_fwd(a_raw, a_fc, p, g, w, bias, _f32(fc_w), _f32(fc_b), logits=lg)
+    if dense:
+        pooled, logits = p_out, lg
     ctx.head = (a_leaf, p_leaf, logits, lg, a_raw, v)
     # (detached alias: `pooled` itself is an output of this node, and an output stored on its own node is a reference
     # cycle that keeps the whole graph -- and its AccumulateGrad nodes with their stream -- alive until the cyclic GC)
-    ctx.pooled_head = pooled.detach() if dense_head is not None else None
+    ctx.pooled_head = pooled.detach() if dense else None
     return logits, v, c, pooled
 
 
 def _head_bwd(ctx, g_logits, g_pooled, dvc, fc_w, fc_b, side: Optional[_Side], grad_hook):
-    """Backward of :func:`_head_fwd`.  ``dvc = (d v, d c, scale)`` when the scores carry gradient (else None).  A
-    DenseHead: d a, d pooled and d logits in ONE launch (``edg_block_head_bwd``), then every parameter gradient of the
-    two heads in one partial launch plus one reduction (``edg_block_head_wgrad``).  A torch head: the fc head's
-    backward adds its d logits to ``g_logits``, then the head's own autograd graph gives d a, d pooled and the head
-    parameters' gradients.  With ``side``, the parameter gradients (which nothing downstream waits for) run in
-    ``side``'s region, where ``grad_hook`` receives them; with ``side=None`` they run inline and the caller hands them
-    on.  Returns (d a or None, d pooled or None, d fc.weight, d fc.bias, head parameter gradients)."""
+    """Backward of :func:`_head_fwd`.  ``dvc = (d v, d c, scale)`` when the scores carry gradient (else None).  ONE
+    launch (``edg_block_head_bwd``) gives d logits (``g_logits`` plus the fc's terms) and d a -- and for a DenseHead d
+    pooled -- then every parameter gradient of the fc and of a DenseHead comes from one partial launch plus one
+    reduction (``edg_block_head_wgrad``).  A torch head runs its own autograd graph on that d logits for its share of
+    d a, d pooled and its parameters' gradients.  With ``side``, the parameter gradients (which nothing downstream
+    waits for) run in ``side``'s region, where ``grad_hook`` receives them; with ``side=None`` they run inline and the
+    caller hands them on.  Returns (d a or None, d pooled or None, d fc.weight, d fc.bias, head parameter
+    gradients)."""
     cfg = ctx.cfg
     a_leaf, p_leaf, logits, lg, a_raw, v = ctx.head
     dense = cfg.get("dense_head") is not None
+    hp = cfg["head_params"]
     region = side.region if side is not None else contextlib.nullcontext
-    d_fcw = d_fcb = da_fc = None
+    d_fcw = d_fcb = None
     g_lg = g_logits.float() if g_logits is not None else None
     head_grads: List[Optional[torch.Tensor]] = [None] * ctx.n_head
-    a_fc = ctx.fc_sig[2] if ctx.fc_sig else a_raw
-    fcw32, fcb32 = _f32(fc_w), _f32(fc_b)
-    if dense:
-        if g_lg is None and dvc is None:
-            return None, g_pooled, None, None, head_grads
-        hp = cfg["head_params"]
+    da_k, gp_total = None, g_pooled
+    # (a torch head without scores gradient: d logits is g_logits itself, nothing for the kernels to add)
+    if dvc is not None or (dense and g_lg is not None):
+        a_fc = ctx.fc_sig[2] if ctx.fc_sig else a_raw
         dv, dc, scale = dvc if dvc is not None else (None, None, None)
-        # d a and d pooled leave with everything else that flows into a / pooled already added (g_pooled)
-        dlg, ga_head, gp_total = ops.block_head_bwd(lg, a_raw, a_fc, bool(ctx.fc_sig), hp[0], fcw32, fcb32, dv, dc,
-                                                    scale, g_lg, g_pooled)
+        w = hp[0] if dense else None
+        # for a DenseHead d a and d pooled leave with everything else that flows into a / pooled already added
+        g_lg, da_k, dp_k = ops.block_head_bwd(lg, a_raw, a_fc, bool(ctx.fc_sig), w, _f32(fc_w), _f32(fc_b), dv, dc,
+                                              scale, g_lg, g_pooled if dense else None)
+        if dense:
+            gp_total = dp_k
         with region():
-            d_hw, d_hb, d_fcw, d_fcb = ops.block_head_wgrad(lg, dlg, a_raw, a_fc, ctx.pooled_head, dv, dc, scale,
-                                                            want_bias=len(hp) > 1)
+            d_hw, d_hb, d_fcw, d_fcb = ops.block_head_wgrad(lg, g_lg if dense else None, a_raw, a_fc,
+                                                            ctx.pooled_head, dv, dc, scale,
+                                                            want_bias=dense and len(hp) > 1)
             if d_fcw is not None:
                 d_fcw, d_fcb = d_fcw.to(fc_w.dtype), d_fcb.to(fc_b.dtype)
                 if side is not None:
                     grad_hook([d_fcw, d_fcb])
-            if hp[0].requires_grad:
-                head_grads[0] = d_hw.to(hp[0].dtype)
-            if len(hp) > 1 and hp[1].requires_grad:
-                head_grads[1] = d_hb.to(hp[1].dtype)
-            if side is not None:
-                grad_hook([g for g in head_grads if g is not None and g.dtype == torch.float32])
-        return ga_head, gp_total, d_fcw, d_fcb, head_grads
-    if dvc is not None:
-        # backward of [v | va] = logits @ fc.weight, c = a . va + logits . fc.bias  (one kernel + a reduction)
-        d_lg, da_fc, d_fcw, d_fcb = ops.fc_head_bwd(lg, fcw32, fcb32, a_fc, *dvc, parts=3 if side is None else 1)
-        with region():
-            if side is not None:
-                _, _, d_fcw, d_fcb = ops.fc_head_bwd(lg, fcw32, fcb32, a_fc, *dvc, parts=2)
-            d_fcw, d_fcb = d_fcw.to(fc_w.dtype), d_fcb.to(fc_b.dtype)
-            if side is not None:
-                grad_hook([d_fcw, d_fcb])
-        if ctx.fc_sig:
-            da_fc = da_fc * a_fc * (1.0 - a_fc)                   # through sigmoid(a)
-        g_lg = d_lg if g_lg is None else g_lg + d_lg
-    # ---- classifier head backward: d a, d pooled, and .grad of the parameters it closes over
+            if dense:
+                if hp[0].requires_grad:
+                    head_grads[0] = d_hw.to(hp[0].dtype)
+                if len(hp) > 1 and hp[1].requires_grad:
+                    head_grads[1] = d_hb.to(hp[1].dtype)
+                if side is not None:
+                    grad_hook([g for g in head_grads if g is not None and g.dtype == torch.float32])
+    if dense:
+        return da_k, gp_total, d_fcw, d_fcb, head_grads
+    # ---- a torch head's own backward: d a, d pooled, and .grad of the parameters it closes over
     ga_head = gp_head = None
     if g_lg is not None and logits.requires_grad:
-        cap = [(i, p) for i, p in enumerate(cfg["head_params"]) if p.requires_grad]
+        cap = [(i, p) for i, p in enumerate(hp) if p.requires_grad]
         res = torch.autograd.grad([logits], [a_leaf, p_leaf] + [p for _, p in cap], [g_lg.to(logits.dtype)],
                                   allow_unused=True, retain_graph=True)
         ga_head, gp_head = res[0], res[1]
@@ -408,9 +406,8 @@ def _head_bwd(ctx, g_logits, g_pooled, dvc, fc_w, fc_b, side: Optional[_Side], g
             head_grads[i] = g
         if side is not None:
             grad_hook([g for g in head_grads if g is not None and g.dtype == torch.float32])
-    if da_fc is not None:
-        ga_head = da_fc if ga_head is None else ga_head.float() + da_fc
-    gp_total = g_pooled
+    if da_k is not None:
+        ga_head = da_k if ga_head is None else ga_head.float() + da_k
     if gp_head is not None:
         gp_total = gp_head.float() if gp_total is None else gp_total + gp_head.float()
     return ga_head, gp_total, d_fcw, d_fcb, head_grads

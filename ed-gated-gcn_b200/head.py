@@ -3,7 +3,8 @@
 Reference: ``self.dense = nn.Linear(2 * hidden, polarities)`` applied to ``torch.cat([aspect, pooled], 1)``
 (models/bert_amir5.py:573, :643) and ``criterion = nn.CrossEntropyLoss()`` (train.py:96, :121).  Both are
 ``[B, *]``-sized work that torch runs as a dozen small library launches between the forward and the backward pass of
-the block; here the head is two kernels (``edg_dense_head_fwd/bwd``) and the loss two (``edg_cross_entropy_fwd/bwd``).
+the block; here the head runs on the block head's kernels with the fc part left out (``edg_block_head_fwd``, and
+``edg_block_head_bwd`` + ``edg_block_head_wgrad`` backward) and the loss is two (``edg_cross_entropy_fwd/bwd``).
 """
 from __future__ import annotations
 
@@ -19,14 +20,17 @@ class _DenseHeadFn(torch.autograd.Function):
     def forward(ctx, a, p, weight, bias):
         ctx.save_for_backward(a, p, weight)
         ctx.has_bias = bias is not None
-        return ops.dense_head_fwd(a, p, weight, bias)
+        return ops.block_head_fwd(a, None, p, None, weight, bias, None, None)[1]
 
     @staticmethod
     def backward(ctx, g):
         a, p, weight = ctx.saved_tensors
-        da, dp, dW, db = ops.dense_head_bwd(g, a, p, weight, parts=3 if (ctx.needs_input_grad[0] or ctx.needs_input_grad[1]) else 2)
+        da = dp = None
+        if ctx.needs_input_grad[0] or ctx.needs_input_grad[1]:
+            _, da, dp = ops.block_head_bwd(None, a, None, False, weight, None, None, g_logits=g)
+        dW, db, _, _ = ops.block_head_wgrad(None, g, a, None, p, want_bias=ctx.has_bias)
         return (da.to(a.dtype) if da is not None else None, dp.to(p.dtype) if dp is not None else None,
-                dW.to(weight.dtype), db if ctx.has_bias else None)
+                dW.to(weight.dtype), db)
 
 
 class DenseHead(nn.Linear):

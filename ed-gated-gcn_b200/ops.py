@@ -422,92 +422,38 @@ def scores_kl_fwd(h, graph, gate, v, c, dist, want_units: bool = False, want_row
     return scores, kl_b, kl
 
 
-def fc_head_fwd(logits: torch.Tensor, fc_w: torch.Tensor, fc_b: torch.Tensor, a: torch.Tensor):
-    """``[v | va] = logits @ fc_w``, ``c = a . va + logits . fc_b`` (fp32): v [B,D], c [B]."""
-    B, C = logits.shape
-    D = a.shape[1]
-    v = torch.empty((B, D), dtype=torch.float32, device=a.device)
-    c = torch.empty((B,), dtype=torch.float32, device=a.device)
-    L.call("edg_fc_head_fwd", L.ptr(logits), ld(logits), L.ptr(fc_w), ld(fc_w), L.ptr(fc_b), L.ptr(a), ld(a), B, D, C,
-           L.ptr(v), L.ptr(c), L.stream())
-    return v, c
-
-
-def fc_head_bwd(logits, fc_w, fc_b, a, dv, dc, scale: Optional[torch.Tensor] = None, parts: int = 3):
-    """Backward of :func:`fc_head_fwd` -> d_logits [B,C], d_a [B,D] (``parts & 1``), d_fc_w [C,2D], d_fc_b [C]
-    (``parts & 2``); ``dv``/``dc`` are multiplied by the device scalar ``scale`` when given."""
-    B, C = logits.shape
-    D = a.shape[1]
-    dev = a.device
-    d_lg = torch.empty((B, C), dtype=torch.float32, device=dev) if parts & 1 else None
-    d_a = torch.empty((B, D), dtype=torch.float32, device=dev) if parts & 1 else None
-    d_w = torch.empty((C, 2 * D), dtype=torch.float32, device=dev) if parts & 2 else None
-    d_b = torch.empty((C,), dtype=torch.float32, device=dev) if parts & 2 else None
-    nbytes = L.load().edg_fc_head_bwd_workspace(B, D, C)
-    ws = torch.empty((nbytes + 3) // 4, dtype=torch.float32, device=dev)
-    L.call("edg_fc_head_bwd", L.ptr(logits), ld(logits), L.ptr(fc_w), ld(fc_w), L.ptr(fc_b), L.ptr(a), ld(a),
-           L.ptr(dv), L.ptr(dc), L.ptr(scale), B, D, C, int(parts), L.ptr(d_lg), C, L.ptr(d_a), L.ptr(d_w), 2 * D,
-           L.ptr(d_b), L.ptr(ws), ws.numel() * 4, L.stream())
-    return d_lg, d_a, d_w, d_b
-
-
 DENSE_HEAD_MAX_CLASSES = 64
 
 
-def dense_head_fwd(a: torch.Tensor, p: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor]) -> torch.Tensor:
-    """``edg_dense_head_fwd``: ``cat([a, p], 1) @ w.T + bias`` with ``a, p`` fp32 ``[B, D]``, ``w`` fp32 ``[C, 2D]``."""
-    a, p, w = _f32c(a), _f32c(p), _f32c(w)
-    B, D = a.shape
-    C = w.shape[0]
-    assert p.shape == (B, D) and w.shape[1] == 2 * D
-    bias = _f32c(bias) if bias is not None else None
-    logits = torch.empty((B, C), dtype=torch.float32, device=a.device)
-    L.call("edg_dense_head_fwd", L.ptr(a), ld(a), L.ptr(p), ld(p), L.ptr(w), ld(w), L.ptr(bias), B, D, C,
-           L.ptr(logits), C, L.stream())
-    return logits
+def _f32c_opt(*ts):
+    return tuple(_f32c(t) if t is not None else None for t in ts)
 
 
-def dense_head_bwd(g: torch.Tensor, a: torch.Tensor, p: torch.Tensor, w: torch.Tensor, parts: int = 3,
-                   g2: Optional[torch.Tensor] = None, da_add: Optional[torch.Tensor] = None,
-                   dp_add: Optional[torch.Tensor] = None):
-    """``edg_dense_head_bwd`` -> ``(da [B,D], dp [B,D])`` (``parts & 1``), ``(dW [C,2D], dbias [C])`` (``parts & 2``)
-    from ``d logits = g (+ g2) [B,C]``; ``da_add`` / ``dp_add`` (fp32 ``[B,D]``) are added to ``da`` / ``dp``."""
-    g, a, p, w = _f32c(g), _f32c(a), _f32c(p), _f32c(w)
-    g2 = _f32c(g2) if g2 is not None else None
-    da_add = _f32c(da_add) if da_add is not None else None
-    dp_add = _f32c(dp_add) if dp_add is not None else None
-    B, D = a.shape
-    C = w.shape[0]
-    dev = a.device
-    da = torch.empty((B, D), dtype=torch.float32, device=dev) if parts & 1 else None
-    dp = torch.empty((B, D), dtype=torch.float32, device=dev) if parts & 1 else None
-    dW = torch.empty((C, 2 * D), dtype=torch.float32, device=dev) if parts & 2 else None
-    db = torch.empty((C,), dtype=torch.float32, device=dev) if parts & 2 else None
-    nbytes = L.load().edg_dense_head_bwd_workspace(B, D, C)
-    ws = torch.empty((nbytes + 3) // 4, dtype=torch.float32, device=dev)
-    L.call("edg_dense_head_bwd", L.ptr(g), ld(g), L.ptr(a), ld(a), L.ptr(p), ld(p), L.ptr(w), ld(w), B, D, C, int(parts),
-           L.ptr(g2), ld(g2) if g2 is not None else 0, L.ptr(da_add), L.ptr(dp_add),
-           L.ptr(da), L.ptr(dp), L.ptr(dW), 2 * D, L.ptr(db), L.ptr(ws), ws.numel() * 4, L.stream())
-    return da, dp, dW, db
+def _ld_opt(t) -> int:
+    return ld(t) if t is not None else 0
 
 
-def block_head_fwd(a, a_fc, p, g, w, bias, fc_w, fc_b):
+def block_head_fwd(a, a_fc, p, g, w, bias, fc_w, fc_b, logits=None):
     """``edg_block_head_fwd``: ``pooled = g * p`` (``p`` itself when ``g`` is None), ``logits = cat([a, pooled]) @ w.T
     + bias``, and the scores' operands ``v = logits @ fc_w[:, :D]``, ``c = logits . (fc_w[:, D:] a_fc + fc_b)`` in one
-    launch.  All fp32 ``[B, D]`` rows.  Returns ``(pooled, logits [B,C], v [B,D], c [B])``."""
-    a, a_fc, p, w, fc_w, fc_b = (_f32c(t) for t in (a, a_fc, p, w, fc_w, fc_b))
-    g = _f32c(g) if g is not None else None
-    bias = _f32c(bias) if bias is not None else None
+    launch.  All fp32 ``[B, D]`` rows.  With ``w`` None the given ``logits`` are used and only ``v``, ``c`` are formed;
+    with ``fc_w`` None only ``pooled`` and ``logits`` are.  Returns ``(pooled, logits [B,C], v [B,D], c [B])``, None
+    for what is not formed."""
+    a, a_fc, p, g, w, bias, fc_w, fc_b, logits = _f32c_opt(a, a_fc, p, g, w, bias, fc_w, fc_b, logits)
     B, D = a.shape
-    C = w.shape[0]
-    assert p.shape == (B, D) and a_fc.shape == (B, D) and w.shape[1] == 2 * D and fc_w.shape == (C, 2 * D)
+    C = (w if w is not None else fc_w).shape[0]
+    assert w is None or (p.shape == (B, D) and w.shape[1] == 2 * D)
+    assert fc_w is None or (a_fc.shape == (B, D) and fc_w.shape == (C, 2 * D))
+    assert w is not None or logits.shape == (B, C)
     dev = a.device
-    pooled = torch.empty((B, D), dtype=torch.float32, device=dev) if g is not None else p
-    logits = torch.empty((B, C), dtype=torch.float32, device=dev)
-    v = torch.empty((B, D), dtype=torch.float32, device=dev)
-    c = torch.empty((B,), dtype=torch.float32, device=dev)
-    L.call("edg_block_head_fwd", L.ptr(a), ld(a), L.ptr(a_fc), ld(a_fc), L.ptr(p), ld(p), L.ptr(g),
-           ld(g) if g is not None else 0, L.ptr(w), ld(w), L.ptr(bias), L.ptr(fc_w), ld(fc_w), L.ptr(fc_b), B, D, C,
+    new = lambda *s: torch.empty(s, dtype=torch.float32, device=dev)
+    pooled = None
+    if w is not None:
+        pooled = new(B, D) if g is not None else p
+        logits = new(B, C)
+    v, c = (new(B, D), new(B)) if fc_w is not None else (None, None)
+    L.call("edg_block_head_fwd", L.ptr(a), ld(a), L.ptr(a_fc), _ld_opt(a_fc), L.ptr(p), _ld_opt(p), L.ptr(g),
+           _ld_opt(g), L.ptr(w), _ld_opt(w), L.ptr(bias), L.ptr(fc_w), _ld_opt(fc_w), L.ptr(fc_b), B, D, C,
            L.ptr(pooled) if g is not None else None, L.ptr(logits), L.ptr(v), L.ptr(c), L.stream())
     return pooled, logits, v, c
 
@@ -516,37 +462,38 @@ def block_head_bwd(logits, a, a_fc, fc_sigmoid: bool, w, fc_w, fc_b, dv=None, dc
                    g_pooled=None):
     """``edg_block_head_bwd`` -> ``(d logits [B,C], d a [B,D], d pooled [B,D])`` of :func:`block_head_fwd`, with the
     scores' ``dv`` / ``dc`` (times the device scalar ``scale``; both None when the scores carry no gradient) and the
-    direct gradients ``g_logits`` / ``g_pooled`` (each optional) flowing in."""
-    logits, a, a_fc, w, fc_w, fc_b = (_f32c(t) for t in (logits, a, a_fc, w, fc_w, fc_b))
-    dv, dc, scale, g_logits, g_pooled = (_f32c(t) if t is not None else None for t in (dv, dc, scale, g_logits, g_pooled))
+    direct gradients ``g_logits`` / ``g_pooled`` (each optional) flowing in.  With ``w`` None only the fc terms are
+    formed (d pooled is None); with ``fc_w`` None only the dense head's (``dv`` / ``dc`` None)."""
+    logits, a, a_fc, w, fc_w, fc_b = _f32c_opt(logits, a, a_fc, w, fc_w, fc_b)
+    dv, dc, scale, g_logits, g_pooled = _f32c_opt(dv, dc, scale, g_logits, g_pooled)
     B, D = a.shape
-    C = w.shape[0]
+    C = (w if w is not None else fc_w).shape[0]
     dev = a.device
     dlg = torch.empty((B, C), dtype=torch.float32, device=dev)
     da = torch.empty((B, D), dtype=torch.float32, device=dev)
-    dp = torch.empty((B, D), dtype=torch.float32, device=dev)
-    L.call("edg_block_head_bwd", L.ptr(logits), L.ptr(a), ld(a), L.ptr(a_fc), ld(a_fc), int(bool(fc_sigmoid)), L.ptr(w),
-           ld(w), L.ptr(fc_w), ld(fc_w), L.ptr(fc_b), L.ptr(dv), L.ptr(dc), L.ptr(scale), L.ptr(g_logits),
-           L.ptr(g_pooled), B, D, C, L.ptr(dlg), L.ptr(da), L.ptr(dp), L.stream())
+    dp = torch.empty((B, D), dtype=torch.float32, device=dev) if w is not None else None
+    L.call("edg_block_head_bwd", L.ptr(logits), L.ptr(a), ld(a), L.ptr(a_fc), _ld_opt(a_fc), int(bool(fc_sigmoid)),
+           L.ptr(w), _ld_opt(w), L.ptr(fc_w), _ld_opt(fc_w), L.ptr(fc_b), L.ptr(dv), L.ptr(dc), L.ptr(scale),
+           L.ptr(g_logits), L.ptr(g_pooled), B, D, C, L.ptr(dlg), L.ptr(da), L.ptr(dp), L.stream())
     return dlg, da, dp
 
 
 def block_head_wgrad(logits, dlg, a, a_fc, pooled, dv=None, dc=None, scale=None, want_bias: bool = True):
     """``edg_block_head_wgrad`` -> ``(dW [C,2D], dbias [C], d fc_w [C,2D], d fc_b [C])``: the head's parameter gradients
-    when ``dlg`` is given (``dbias`` None unless ``want_bias``), the fc's when ``dv`` / ``dc`` are (else None)."""
-    logits, a, a_fc, pooled = (_f32c(t) for t in (logits, a, a_fc, pooled))
-    dlg, dv, dc, scale = (_f32c(t) if t is not None else None for t in (dlg, dv, dc, scale))
+    when ``dlg`` is given (``dbias`` None unless ``want_bias``), the fc's when ``dv`` / ``dc`` are (else None).
+    ``logits`` / ``a_fc`` are only read for the fc's, ``pooled`` only for the head's."""
+    logits, dlg, a, a_fc, pooled, dv, dc, scale = _f32c_opt(logits, dlg, a, a_fc, pooled, dv, dc, scale)
     B, D = a.shape
-    C = logits.shape[1]
+    C = (logits if logits is not None else dlg).shape[1]
     dev = a.device
     new = lambda *s: torch.empty(s, dtype=torch.float32, device=dev)
     dW, dbias = (new(C, 2 * D), new(C) if want_bias else None) if dlg is not None else (None, None)
     d_fw, d_fb = (new(C, 2 * D), new(C)) if dv is not None else (None, None)
     nbytes = L.load().edg_block_head_wgrad_workspace(B, D, C)
     ws = torch.empty((nbytes + 3) // 4, dtype=torch.float32, device=dev)
-    L.call("edg_block_head_wgrad", L.ptr(logits), L.ptr(dlg), L.ptr(a), ld(a), L.ptr(a_fc), ld(a_fc), L.ptr(pooled),
-           ld(pooled), L.ptr(dv), L.ptr(dc), L.ptr(scale), B, D, C, L.ptr(dW), L.ptr(dbias), L.ptr(d_fw), L.ptr(d_fb),
-           L.ptr(ws), ws.numel() * 4, L.stream())
+    L.call("edg_block_head_wgrad", L.ptr(logits), L.ptr(dlg), L.ptr(a), ld(a), L.ptr(a_fc), _ld_opt(a_fc), L.ptr(pooled),
+           _ld_opt(pooled), L.ptr(dv), L.ptr(dc), L.ptr(scale), B, D, C, L.ptr(dW), L.ptr(dbias), L.ptr(d_fw),
+           L.ptr(d_fb), L.ptr(ws), ws.numel() * 4, L.stream())
     return dW, dbias, d_fw, d_fb
 
 

@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define EDG_ABI_VERSION 4
+#define EDG_ABI_VERSION 5
 
 typedef enum {
   EDG_OK = 0,
@@ -300,27 +300,6 @@ int edg_views_bwd_parts(const float* pooled, const int32_t* arg, const float* ga
                         const float* g_pooled, void* dh, int64_t lddh, float* dgates, int acc_view, int parts,
                         edg_stream stream);
 
-/* bert_amir5.py:645-646 collapsed (SURVEY A9): the per-sentence operands of the importance scores,
- *   [v_b | va_b] = logits_b @ fc.weight   (fc.weight [C, 2D], nn.Linear layout; C <= 64),
- *   c_b          = a_b . va_b + logits_b . fc.bias,
- * so that scores[b,t] = x_out[b,t,:] . v_b + c_b  (edg_scores_kl_fwd).  All fp32.  v [B,D], c [B]. */
-int edg_fc_head_fwd(const float* logits, int64_t ldl, const float* fc_w, int64_t ldw, const float* fc_b,
-                    const float* a, int64_t lda, int32_t B, int32_t D, int32_t C, float* v, float* c,
-                    edg_stream stream);
-
-/* backward of edg_fc_head_fwd.  dv [B,D], dc [B] (both multiplied by the device scalar *scale when scale != NULL:
- * the per-unit gradients of edg_scores_kl_fwd times the upstream d kl):
- *   parts & 1:  d_logits[b,:] = [dv_b | dc_b a_b] @ fc.weight^T + dc_b fc.bias        (overwritten, [B, lddl])
- *               d_a[b,:]      = dc_b va_b                                             (overwritten, [B, D])
- *   parts & 2:  d_fc_w        = logits^T @ [dv | dc a],  d_fc_b = logits^T dc         (overwritten; fixed summation order)
- * The two parts may be issued as two calls on two streams (nothing downstream waits for the parameter gradients);
- * outputs of a part that is not requested may be NULL.  ws: edg_fc_head_bwd_workspace() bytes. */
-size_t edg_fc_head_bwd_workspace(int32_t B, int32_t D, int32_t C);
-int edg_fc_head_bwd(const float* logits, int64_t ldl, const float* fc_w, int64_t ldw, const float* fc_b,
-                    const float* a, int64_t lda, const float* dv, const float* dc, const float* scale,
-                    int32_t B, int32_t D, int32_t C, int parts, float* d_logits, int64_t lddl, float* d_a,
-                    float* d_fc_w, int64_t lddw, float* d_fc_b, void* ws, size_t ws_bytes, edg_stream stream);
-
 /* backward of x_out = gate*h_L through scores/kl, the final max-pool and an
  * optional direct gradient on x_out:
  *   ds[i]   = g_kl/B * P_i*(Q_i - kl_b) + g_scores[i]
@@ -478,29 +457,17 @@ int edg_wgrad_split(const void* A2, int64_t lda, const float* amax_a, int32_t K1
 /* Classifier head and loss (bert_amir5.py:643 self.dense, train.py:121)      */
 /* ------------------------------------------------------------------------- */
 
-/* logits fp32 [B, C] = [a | p] W^T + bias with a, p fp32 [B, D], W fp32 [C, 2D] (nn.Linear(2D, C).weight), bias [C] or
- * NULL: `self.dense(torch.cat([aspect, pooled], 1))` without the cat.  C <= 64. */
-int edg_dense_head_fwd(const float* a, int64_t lda, const float* p, int64_t ldp, const float* W, int64_t ldw,
-                       const float* bias, int32_t B, int32_t D, int32_t C, float* logits, int64_t ldl, edg_stream stream);
-
-/* Its backward from g = d logits [B, C]:  da = g W[:, :D], dp = g W[:, D:] (fp32 [B, D] contiguous; either may be NULL),
- * dW [C, 2D] = g^T [a | p], dbias [C] = colsum(g); fixed summation order.  parts: bit 0 = da / dp, bit 1 = dW / dbias (two
- * calls on two streams keep the parameter gradients off the critical path).  Optional: g2 [B, C] is added to g on load,
- * da_add / dp_add [B, D] (contiguous) are added to da / dp on store -- the sums torch would run as separate elementwise
- * launches.  ws: edg_dense_head_bwd_workspace bytes. */
-size_t edg_dense_head_bwd_workspace(int32_t B, int32_t D, int32_t C);
-int edg_dense_head_bwd(const float* g, int64_t ldg, const float* a, int64_t lda, const float* p, int64_t ldp,
-                       const float* W, int64_t ldw, int32_t B, int32_t D, int32_t C, int parts, const float* g2,
-                       int64_t ldg2, const float* da_add, const float* dp_add, float* da, float* dp, float* dW,
-                       int64_t lddw, float* dbias, void* ws, size_t ws_bytes, edg_stream stream);
-
-/* The block's classifier head and the collapsed-scores operands as ONE launch (what edg_dense_head_fwd followed by
- * edg_fc_head_fwd compute, without the memset, the atomics and the round trip of the logits through HBM).  Per row b:
+/* The classifier head and the collapsed-scores operands (bert_amir5.py:643-646, SURVEY A9) as ONE launch.  Per row b:
  *   pooled_b = g_b * p_b              (written to pooled [B, D] contiguous; when g == NULL pooled_b = p_b, nothing written)
  *   logits_b = W [a_b | pooled_b] + bias                  (W fp32 [C, 2D], bias [C] or NULL; logits [B, C] contiguous)
  *   va_b = logits_b^T fc_w[:, D:],  c_b = a_fc_b . va_b + logits_b . fc_b,  v_b = logits_b^T fc_w[:, :D]  (v [B, D] contiguous)
- * a_fc is a, or sigmoid(a) for fc = Sequential(Sigmoid, Linear).  All fp32, C <= 64; the same bits as edg_dense_head_fwd
- * followed by edg_fc_head_fwd (their summation order). */
+ * so that scores[b,t] = x_out[b,t,:] . v_b + c_b (edg_scores_kl_fwd).  a_fc is a, or sigmoid(a) for fc =
+ * Sequential(Sigmoid, Linear).  All fp32, C <= 64.  Either head may be left out (not both):
+ *   W == NULL (the logits come from a torch head): logits is an input; only v and c are written (a, p, g, pooled, bias
+ *     unused);
+ *   fc_w == NULL (a DenseHead on its own): only logits (and pooled when g is given) are written (a_fc, fc_b, v, c
+ *     unused).
+ * Each sum has the same order in every mode, so the combined launch gives the bits of the two composed. */
 int edg_block_head_fwd(const float* a, int64_t lda, const float* a_fc, int64_t ldf, const float* p, int64_t ldp,
                        const float* g, int64_t ldg, const float* W, int64_t ldw, const float* bias, const float* fc_w,
                        int64_t ldfw, const float* fc_b, int32_t B, int32_t D, int32_t C, float* pooled, float* logits,
@@ -511,7 +478,12 @@ int edg_block_head_fwd(const float* a, int64_t lda, const float* a_fc, int64_t l
  *   da_b  = s dc_b (logits_b^T fc_w[:, D:]) (times a_fc (1 - a_fc) when fc_sigmoid) + dlg_b^T W[:, :D]
  *   dp_b  = dlg_b^T W[:, D:] + g_pooled_b                                          (da, dp [B, D] contiguous)
  * dv [B, D] / dc [B] (contiguous) are both NULL when the scores carry no gradient; g_logits [B, C] and g_pooled [B, D]
- * (contiguous) may be NULL.  logits [B, C] contiguous.  The same bits as edg_fc_head_bwd + edg_dense_head_bwd. */
+ * (contiguous) may be NULL.  logits [B, C] contiguous.  As in the forward, either head may be left out:
+ *   W == NULL: dlg and da get the fc terms only; dp is not written (may be NULL);
+ *   fc_w == NULL: dv and dc must be NULL; dlg = g_logits, da = dlg W[:, :D], dp = dlg W[:, D:] + g_pooled (logits,
+ *     a_fc, fc_b unused).
+ * The combined launch gives the bits of the fc-only launch followed by the dense-only one with g_logits = its dlg, the
+ * two d a summed as da_dense + da_fc. */
 int edg_block_head_bwd(const float* logits, const float* a, int64_t lda, const float* a_fc, int64_t ldf, int fc_sigmoid,
                        const float* W, int64_t ldw, const float* fc_w, int64_t ldfw, const float* fc_b, const float* dv,
                        const float* dc, const float* scale, const float* g_logits, const float* g_pooled, int32_t B,
@@ -519,7 +491,8 @@ int edg_block_head_bwd(const float* logits, const float* a, int64_t lda, const f
 
 /* The parameter gradients of the two: per-block partials in one launch, summed in block order by a second one.
  *   dv / dc given:  d_fc_w [C, 2D] = logits^T u,  d_fc_b [C] = logits^T (s dc)
- *   dlg given:      dW [C, 2D] = dlg^T [a | pooled],  dbias [C] = colsum(dlg)  (dbias may be NULL)
+ *   dlg given:      dW [C, 2D] = dlg^T [a | pooled],  dbias [C] = colsum(dlg)  (dbias may be NULL; logits may be NULL
+ *                   when dv / dc are not given)
  * (all outputs contiguous, overwritten).  ws: edg_block_head_wgrad_workspace bytes. */
 size_t edg_block_head_wgrad_workspace(int32_t B, int32_t D, int32_t C);
 int edg_block_head_wgrad(const float* logits, const float* dlg, const float* a, int64_t lda, const float* a_fc,

@@ -159,15 +159,18 @@ def test_scores_kl(dtype, i64):
 
 
 @pytest.mark.parametrize("shape", [(4096, 300, 34), (37, 256, 2), (1, 16, 1), (130, 768, 34), (64, 300, 64)])
-def test_fc_head_forward_backward(shape):
+def test_block_head_fc_only_forward_backward(shape):
     """[v | va] = logits @ fc.weight, c = a.va + logits.fc.bias (bert_amir5.py:645-646 collapsed) and its
-    backward, against the torch formulation in fp64."""
+    backward, against the torch formulation in fp64: the block head's launches without the dense head (the logits of
+    a torch logits_fn as input), the parameter gradients from edg_block_head_wgrad without d logits."""
     from ed_gated_gcn_b200 import ops
     B, D, C = shape
     g = torch.Generator().manual_seed(B + D + C)
     lg, W, bfc = torch.randn(B, C, generator=g), torch.randn(C, 2 * D, generator=g) / C ** 0.5, torch.randn(C, generator=g)
     a, dv, dc = torch.randn(B, D, generator=g), torch.randn(B, D, generator=g), torch.randn(B, generator=g)
-    v, c = ops.fc_head_fwd(lg.to(DEV), W.to(DEV), bfc.to(DEV), a.to(DEV))
+    lg_, W_, bfc_, a_, dv_, dc_ = (t.to(DEV) for t in (lg, W, bfc, a, dv, dc))
+    _, lg_out, v, c = ops.block_head_fwd(a_, a_, None, None, None, None, W_, bfc_, logits=lg_)
+    assert torch.equal(lg_out, lg_)
     lgd, Wd, bd, ad = (t.double().requires_grad_(True) for t in (lg, W, bfc, a))
     vva = lgd @ Wd
     v_ref = vva[:, :D]
@@ -177,15 +180,18 @@ def test_fc_head_forward_backward(shape):
         s = 1.0 if scale is None else scale
         want = torch.autograd.grad([v_ref, c_ref], [lgd, ad, Wd, bd], [s * dv.double(), s * dc.double()], retain_graph=True)
         sc = None if scale is None else torch.tensor(scale, device=DEV)
-        got = ops.fc_head_bwd(lg.to(DEV), W.to(DEV), bfc.to(DEV), a.to(DEV), dv.to(DEV), dc.to(DEV), sc)
-        for name, x, y in zip(["d_logits", "d_a", "d_fc_w", "d_fc_b"], got, want):
+        d_lg, d_a, dp = ops.block_head_bwd(lg_, a_, a_, False, None, W_, bfc_, dv_, dc_, sc)
+        _, _, d_fw, d_fb = ops.block_head_wgrad(lg_, None, a_, a_, None, dv_, dc_, sc)
+        assert dp is None
+        for name, x, y in zip(["d_logits", "d_a", "d_fc_w", "d_fc_b"], (d_lg, d_a, d_fw, d_fb), want):
             assert rel(x, y) < 2e-6, (name, shape, scale)
-        # the two halves of the work as separate calls (input gradients / parameter gradients) give the same bits
-        g1 = ops.fc_head_bwd(lg.to(DEV), W.to(DEV), bfc.to(DEV), a.to(DEV), dv.to(DEV), dc.to(DEV), sc, parts=1)
-        g2 = ops.fc_head_bwd(lg.to(DEV), W.to(DEV), bfc.to(DEV), a.to(DEV), dv.to(DEV), dc.to(DEV), sc, parts=2)
-        assert g1[2] is None and g2[0] is None
-        assert torch.equal(g1[0], got[0]) and torch.equal(g1[1], got[1])
-        assert torch.equal(g2[2], got[2]) and torch.equal(g2[3], got[3])
+        # where the modes overlap (a dense head of zeros adds exact zeros to d a), the combined launches give the
+        # same bits
+        zw, p = torch.zeros_like(W_), torch.randn(B, D, generator=g).to(DEV)
+        dlg2, da2, _ = ops.block_head_bwd(lg_, a_, a_, False, zw, W_, bfc_, dv_, dc_, sc)
+        _, _, d_fw2, d_fb2 = ops.block_head_wgrad(lg_, dlg2, a_, a_, p, dv_, dc_, sc)
+        assert torch.equal(dlg2, d_lg) and torch.equal(da2, d_a)
+        assert torch.equal(d_fw2, d_fw) and torch.equal(d_fb2, d_fb)
 
 
 @pytest.mark.parametrize("D", [300, 256, 200, 64, 320])

@@ -635,8 +635,9 @@ def test_tensors_on_a_second_gpu_with_device_0_current():
 
 @pytest.mark.parametrize("dtype", DTYPES, ids=["f32", "bf16"])
 def test_dense_head_and_fused_loss_equal_the_torch_head(dtype):
-    """`E.DenseHead` passed as logits_fn (run inside the block by edg_dense_head_fwd/bwd) + `E.cross_entropy` against the
-    same stack with torch's nn.Linear-on-cat head and F.cross_entropy: same loss, same gradients everywhere."""
+    """`E.DenseHead` passed as logits_fn (run inside the block's head launches, edg_block_head_*) + `E.cross_entropy`
+    against the same stack with torch's nn.Linear-on-cat head (the fc-only launches) and F.cross_entropy: same loss,
+    same gradients everywhere."""
     import ed_gated_gcn_b200 as E
     from ed_gated_gcn_b200 import synth
     torch.manual_seed(5)

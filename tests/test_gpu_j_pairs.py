@@ -335,7 +335,7 @@ def test_declined_combinations_raise():
     anchor = torch.from_numpy(an).to(DEV)
     dist = E.tree_distance(graph, anchor, pairs=pairs)
     x = torch.randn(batch.n_rows, D, device=DEV)
-    dense = torch.nn.Linear(2 * D, 34).to(DEV)
+    dense = torch.nn.Linear(2 * D, 2).to(DEV)                  # as many classes as the stacks' fc (n_classes=2)
     fn = lambda a, p: dense(torch.cat([a, p], 1))
 
     def call(stack, **kw):
@@ -346,6 +346,10 @@ def test_declined_combinations_raise():
     call(s, match="gate dropout")
     s.eval()
     s(x, graph, anchor, dist, fn, head_params=list(dense.parameters()), pairs=pairs)     # eval mode: dropout is off
+    wide = torch.nn.Linear(2 * D, 34).to(DEV)                  # more classes than the fc head scores
+    with pytest.raises(E.EdgError, match="classes"):
+        s(x, graph, anchor, dist, lambda a, p: wide(torch.cat([a, p], 1)), head_params=list(wide.parameters()),
+          pairs=pairs)
     call(E.GatedGCNStack(D, fc_sigmoid=True).to(DEV), match="fc_sigmoid")
     base = E.GatedGCNStack(D).to(DEV)
     call(base, match="view_len", view_len=torch.ones(batch.n_graphs, dtype=torch.int64, device=DEV))

@@ -1,5 +1,5 @@
 """edg_block_head_fwd / _bwd / _wgrad (the block's classifier head and collapsed-scores algebra, one launch each way)
-against fp64 torch and against the launch chains they replace (edg_dense_head_* + edg_fc_head_*)."""
+against fp64 torch, and the combined launches against their dense-only and fc-only modes composed."""
 import pytest
 import torch
 
@@ -93,21 +93,27 @@ def test_block_head_without_gate_reads_pooled():
 
 
 @pytest.mark.parametrize("B,D,C", [(4096, 300, 34), (33, 768, 34), (33, 302, 64)])
-def test_block_head_equals_the_launch_chain_bitwise(B, D, C):
-    """The same bits as edg_dense_head_* followed by edg_fc_head_*: the fused kernels keep their summation order, so a
-    training run does not drift from the one the launch chain gave."""
+@pytest.mark.parametrize("fc_sigmoid", [False, True])
+def test_block_head_equals_its_two_modes_composed(B, D, C, fc_sigmoid):
+    """The same bits as the dense-only and the fc-only launches composed (dense forward -> fc forward on its logits,
+    fc backward -> dense backward on its d logits, d a summed, one parameter-gradient launch per head): every sum
+    keeps its order in every mode, so a torch head (fc-only) and a DenseHead (combined) give the same training run."""
     from ed_gated_gcn_b200 import ops
-    t = _inputs(B, D, C, seed=11)
-    got = _run(t, False)
-    pooled = t["gate"] * t["hmax"]
-    lg = ops.dense_head_fwd(t["a"], pooled, t["W"], t["bias"])
-    v, c = ops.fc_head_fwd(lg, t["Wf"], t["bf"], t["a"])
-    d_lg, da_fc, dWf, dbf = ops.fc_head_bwd(lg, t["Wf"], t["bf"], t["a"], t["dv"], t["dc"], t["scale"], parts=3)
-    da, dp, dW, db = ops.dense_head_bwd(t["g_lg"], t["a"], pooled, t["W"], parts=3, g2=d_lg, da_add=da_fc,
-                                        dp_add=t["g_p"])
-    old = dict(pooled=pooled, logits=lg, v=v, c=c, dlg=t["g_lg"] + d_lg, da=da, dp=dp, dW=dW, dbias=db, dWf=dWf,
-               dbf=dbf)
-    for k, w in old.items():
+    t = _inputs(B, D, C, seed=11, fc_sigmoid=fc_sigmoid)
+    got = _run(t, fc_sigmoid)
+    sv = (t["dv"], t["dc"], t["scale"])
+    pooled, lg, v0, c0 = ops.block_head_fwd(t["a"], None, t["hmax"], t["gate"], t["W"], t["bias"], None, None)
+    _, _, v, c = ops.block_head_fwd(t["a"], t["af"], None, None, None, None, t["Wf"], t["bf"], logits=lg)
+    dlg, da_fc, dp_fc = ops.block_head_bwd(lg, t["a"], t["af"], fc_sigmoid, None, t["Wf"], t["bf"], *sv,
+                                           g_logits=t["g_lg"])
+    dlg_d, da_dense, dp = ops.block_head_bwd(None, t["a"], None, False, t["W"], None, None, g_logits=dlg,
+                                             g_pooled=t["g_p"])
+    dW, dbias, _, _ = ops.block_head_wgrad(None, dlg, t["a"], None, pooled)
+    _, _, dWf, dbf = ops.block_head_wgrad(lg, None, t["a"], t["af"], None, *sv)
+    assert v0 is None and c0 is None and dp_fc is None and torch.equal(dlg_d, dlg)
+    composed = dict(pooled=pooled, logits=lg, v=v, c=c, dlg=dlg, da=da_dense + da_fc, dp=dp, dW=dW, dbias=dbias,
+                    dWf=dWf, dbf=dbf)
+    for k, w in composed.items():
         assert torch.equal(got[k], w), (k, rel(got[k], w))
 
 

@@ -35,7 +35,7 @@ def test_library_exports_every_declared_symbol():
 def test_version_and_error_strings_without_gpu():
     from ed_gated_gcn_b200 import _lib
     lib = _lib.load()
-    assert lib.edg_version() == 4
+    assert lib.edg_version() == 5
     assert b"aligned" in lib.edg_strerror(-2)
     assert lib.edg_strerror(0) == b"ok"
 
@@ -335,7 +335,7 @@ def test_host_side_planning_entry_points_of_the_round_2_additions():
     # three products: the hi x hi launch in short chains (more slabs) + two cross-term launches
     assert lib.edg_wgrad_split_workspace(204800, 300, 300) > 3 * 301 * 300 * 4
     assert lib.edg_wgrad_split_workspace(0, 300, 300) == 16
-    assert lib.edg_dense_head_bwd_workspace(4096, 300, 34) == 128 * 34 * 601 * 4
+    assert lib.edg_block_head_wgrad_workspace(4096, 300, 34) == 128 * 34 * 1202 * 4
     assert lib.edg_cross_entropy_workspace(4096) == (2 * 512 + 1) * 4
     prev = lib.edg_set_sm_budget(116)
     assert prev == 148 and lib.edg_set_sm_budget(1000) == 116 and lib.edg_set_sm_budget(148) == 148

@@ -1,7 +1,6 @@
-"""Micro-benchmark of the block's head at config-C2 size (B = 4096, D = 300, C = 34, fp32 operands): the launch chain of
-edg_dense_head_* + edg_fc_head_* (forward: memset + dense head, torch gate * hmax, fc head; backward: fc head parts=1 +
-its reduction, dense head parts=1; parameter gradients: both parts=2 kernels + their two reductions) against
-edg_block_head_fwd / _bwd / _wgrad (1 + 1 + 2 launches).
+"""Micro-benchmark of the block's head at config-C2 size (B = 4096, D = 300, C = 34, fp32 operands):
+edg_block_head_fwd / _bwd / _wgrad in their three modes -- both heads (a DenseHead in the block), fc only (the logits
+of a torch logits_fn as input) and dense only (a DenseHead called on its own).
 
 Each direction is captured as a CUDA graph over a ring of input sets larger than L2 (so every replay reads HBM, as in
 the training step), replayed many times between two CUDA events.  Prints microseconds per call of each direction.
@@ -33,29 +32,33 @@ def main():
     ring = [dict(a=r(B, D), hmax=r(B, D), gate=torch.rand(B, D, device=dev, generator=g), dv=r(B, D), dc=r(B),
                  g_lg=r(B, C)) for _ in range(args.ring)]
 
-    def old_fwd(t):
-        t["pooled"] = t["gate"] * t["hmax"]
-        t["lg"] = ops.dense_head_fwd(t["a"], t["pooled"], W, bias)
-        t["v"], t["c"] = ops.fc_head_fwd(t["lg"], Wf, bf, t["a"])
-
-    def old_bwd(t):
-        d_lg, da_fc, _, _ = ops.fc_head_bwd(t["lg"], Wf, bf, t["a"], t["dv"], t["dc"], scale, parts=1)
-        ops.dense_head_bwd(t["g_lg"], t["a"], t["pooled"], W, parts=1, g2=d_lg, da_add=da_fc)
-        t["d_lg"] = d_lg
-
-    def old_wgrad(t):
-        ops.fc_head_bwd(t["lg"], Wf, bf, t["a"], t["dv"], t["dc"], scale, parts=2)
-        ops.dense_head_bwd(t["g_lg"], t["a"], t["pooled"], W, parts=2, g2=t["d_lg"])
-
-    def new_fwd(t):
+    def both_fwd(t):
         t["pooled"], t["lg"], t["v"], t["c"] = ops.block_head_fwd(t["a"], t["a"], t["hmax"], t["gate"], W, bias, Wf, bf)
 
-    def new_bwd(t):
+    def both_bwd(t):
         t["dlg"], _, _ = ops.block_head_bwd(t["lg"], t["a"], t["a"], False, W, Wf, bf, t["dv"], t["dc"], scale,
                                             t["g_lg"], None)
 
-    def new_wgrad(t):
+    def both_wgrad(t):
         ops.block_head_wgrad(t["lg"], t["dlg"], t["a"], t["a"], t["pooled"], t["dv"], t["dc"], scale)
+
+    def fc_fwd(t):
+        ops.block_head_fwd(t["a"], t["a"], None, None, None, None, Wf, bf, logits=t["lg"])
+
+    def fc_bwd(t):
+        ops.block_head_bwd(t["lg"], t["a"], t["a"], False, None, Wf, bf, t["dv"], t["dc"], scale, t["g_lg"], None)
+
+    def fc_wgrad(t):
+        ops.block_head_wgrad(t["lg"], None, t["a"], t["a"], None, t["dv"], t["dc"], scale)
+
+    def dense_fwd(t):
+        ops.block_head_fwd(t["a"], None, t["pooled"], None, W, bias, None, None)
+
+    def dense_bwd(t):
+        ops.block_head_bwd(None, t["a"], None, False, W, None, None, g_logits=t["g_lg"])
+
+    def dense_wgrad(t):
+        ops.block_head_wgrad(None, t["g_lg"], t["a"], None, t["pooled"])
 
     def time_graph(fn):
         s = torch.cuda.Stream()
@@ -78,11 +81,13 @@ def main():
         torch.cuda.synchronize()
         return 1e3 * e0.elapsed_time(e1) / (args.reps * len(ring))
 
+    for t in ring:                          # forward outputs the other modes and the backward read
+        both_fwd(t)
+        both_bwd(t)
     res = {}
-    for name, (fwd, bwd, wg) in dict(chain=(old_fwd, old_bwd, old_wgrad), block=(new_fwd, new_bwd, new_wgrad)).items():
-        for t in ring:                      # forward outputs the backward reads
-            fwd(t)
-            bwd(t)
+    modes = dict(both=(both_fwd, both_bwd, both_wgrad), fc_only=(fc_fwd, fc_bwd, fc_wgrad),
+                 dense_only=(dense_fwd, dense_bwd, dense_wgrad))
+    for name, (fwd, bwd, wg) in modes.items():
         res[name] = dict(fwd_us=time_graph(fwd), bwd_us=time_graph(bwd), wgrad_us=time_graph(wg))
     res["device"] = torch.cuda.get_device_name()
     print(json.dumps(res))
