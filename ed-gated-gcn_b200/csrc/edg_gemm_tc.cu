@@ -212,12 +212,20 @@ __device__ __forceinline__ float apply_act(float x, int act) {
   return x;
 }
 
-// one 32-column chunk of one accumulator row -> bias, activation, convert, 128-bit stores
+// first column a CTA's N tile does not own: the next tile's first column, or the row pitch on the last tile (which
+// also writes the row padding).  A tile that is not a multiple of 32 columns wide ends inside its last chunk.
+__device__ __forceinline__ int tile_col_end(int n_tile, int n_tiles, int n0, int block_n, int64_t ldc) {
+  const int64_t e = (n_tile == n_tiles - 1) ? ldc : (int64_t)n0 + block_n;
+  return (int)(e < ldc ? e : ldc);
+}
+
+// one 32-column chunk of one accumulator row -> bias, activation, convert, 128-bit stores; only columns below
+// `col_end` are written (what this CTA's N tile owns: n0 + block_n, or ldc on the last N tile so its padding is zeroed)
 template <typename TC>
-__device__ __forceinline__ void epilogue_chunk(const uint32_t (&r)[32], int col0, int Nout, int64_t ldc, int act,
+__device__ __forceinline__ void epilogue_chunk(const uint32_t (&r)[32], int col0, int Nout, int col_end, int act,
                                                const float* __restrict__ bias_s, TC* __restrict__ crow) {
   constexpr int G = OutVec<TC>::G;
-  if (col0 + 32 <= Nout) {                      // interior chunk: no per-element guards
+  if (col0 + 32 <= Nout && col0 + 32 <= col_end) {   // interior chunk: no per-element guards
 #pragma unroll
     for (int g = 0; g < 32; g += G) {
       float v[G];
@@ -225,11 +233,11 @@ __device__ __forceinline__ void epilogue_chunk(const uint32_t (&r)[32], int col0
       for (int j = 0; j < G; ++j) v[j] = apply_act(__uint_as_float(r[g + j]) + bias_s[col0 + g + j], act);
       OutVec<TC>::store(crow + col0 + g, v);
     }
-  } else {                                      // last chunk of the row: zero the padding, skip what is past ldc
+  } else {                                      // last chunk of the tile: zero the padding, skip what is past col_end
 #pragma unroll
     for (int g = 0; g < 32; g += G) {
       const int col = col0 + g;
-      if (col + G <= ldc) {
+      if (col + G <= col_end) {
         float v[G];
 #pragma unroll
         for (int j = 0; j < G; ++j) {
@@ -320,6 +328,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
       const int as = it & 1;
       const uint32_t aphase = (it >> 1) & 1;
       const int m0 = (tile / n_tiles) * kBlockM, n0 = (tile % n_tiles) * block_n;
+      const int col_end = tile_col_end(tile % n_tiles, n_tiles, n0, block_n, ldc);
       mbar_wait(L.tfull(as), aphase);
       tc_fence_after();
       const int row = m0 + q * 32 + lane;
@@ -333,13 +342,13 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
         tmem_wait_ld();
         const int nxt = ci + 2;
         if (nxt < n_chunks) tmem_ld_32x32_nowait(tbase + nxt * 32, rb);
-        if (row_ok && n0 + ci * 32 < ldc) epilogue_chunk<TC>(ra, n0 + ci * 32, Nout, ldc, act, bias_s, crow);
+        if (row_ok && n0 + ci * 32 < ldc) epilogue_chunk<TC>(ra, n0 + ci * 32, Nout, col_end, act, bias_s, crow);
         ci = nxt;
         if (ci >= n_chunks) break;
         tmem_wait_ld();
         const int nx2 = ci + 2;
         if (nx2 < n_chunks) tmem_ld_32x32_nowait(tbase + nx2 * 32, ra);
-        if (row_ok && n0 + ci * 32 < ldc) epilogue_chunk<TC>(rb, n0 + ci * 32, Nout, ldc, act, bias_s, crow);
+        if (row_ok && n0 + ci * 32 < ldc) epilogue_chunk<TC>(rb, n0 + ci * 32, Nout, col_end, act, bias_s, crow);
         ci = nx2;
       }
       tc_fence_before();
@@ -512,12 +521,10 @@ linear_ws_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
     const int half = (warp - 2) >> 2;
     const int n_chunks = (block_n + 31) / 32;
     float inv_a = 1.f, inv_w = 1.f;
-    int col_end = 0;
+    const int col_end = tile_col_end(n_tile, n_tiles, n0, block_n, ldc);
     if (SPLIT) {
       inv_a = split_inv_scale(__ldg(amax_a));
       inv_w = split_inv_scale(__ldg(amax_w));
-      col_end = (n_tile == n_tiles - 1) ? (int)ldc : n0 + block_n;
-      if (col_end > (int)ldc) col_end = (int)ldc;
     }
     int it = 0;
     for (int mt = m_first; mt < m_tiles; mt += m_step, ++it) {
@@ -535,7 +542,7 @@ linear_ws_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
         if constexpr (SPLIT) {
           epilogue_chunk_scaled(r, n0 + ci * 32, Nout, col_end, act, inv_a, inv_w, bias_s, reinterpret_cast<float*>(crow));
         } else {
-          if (n0 + ci * 32 < ldc) epilogue_chunk<TC>(r, n0 + ci * 32, Nout, ldc, act, bias_s, crow);
+          if (n0 + ci * 32 < ldc) epilogue_chunk<TC>(r, n0 + ci * 32, Nout, col_end, act, bias_s, crow);
         }
       };
       int ci = half;
